@@ -2,6 +2,7 @@
 """Benchmark of the hot path: AVSeparationTransformer.forward on SyntheticAVDataset-shaped input.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--config c1|c2|c3|c4] [--batch B] [--impl ours|reference]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -246,6 +247,27 @@ def total_flops(B):
     return kernel_work(B)[2]
 
 
+DUMP_BYTES = 64 * 10**6       # --dump-outputs writes at most this many bytes in all
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: writes each (name, tensor) of one step's outputs as out_dir/<name>.npy in float32, so that two
+    builds run with the same arguments (hence the same seeded inputs and weights) can be compared output for output.
+    Whole utterances (dim 0) are kept; when all of them would exceed DUMP_BYTES, every array keeps the same seeded
+    sample of utterances, in index order.  Returns the number of utterances written."""
+    import numpy as np
+    import torch
+    n = arrays[0][1].shape[0]
+    per_utt = sum(t[0].numel() * 4 for _, t in arrays)
+    keep = min(n, (DUMP_BYTES - 1024 * len(arrays)) // per_utt)       # 1 KB per file for the .npy header
+    idx = None if keep == n else torch.from_numpy(np.sort(np.random.default_rng(0).choice(n, keep, replace=False)))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays:
+        t = t.detach() if idx is None else t.detach()[idx.to(t.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), t.float().cpu().numpy())
+    return keep
+
+
 # ----------------------------------------------------------------------------------------------
 # the reference's own CPU implementation -- the ONLY place bench.py touches oracle/
 # ----------------------------------------------------------------------------------------------
@@ -321,8 +343,10 @@ def run_reference(args, rank, world):
         fwd(mixed, frames)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        fwd(mixed, frames)
+        out = fwd(mixed, frames)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, [("separated", out[0]), ("masks", out[1])])
     value = args.steps * CPU_SAMPLE_B * CLIP_SECONDS / dt
     sample = (f"B={CPU_SAMPLE_B} utterances of the same workload per step (CPU throughput is flat beyond B~32); "
               + ("the unmodified reference modules (oracle/_ref, model.py:227-276), eval mode, no_grad" if kind == "reference"
@@ -438,6 +462,10 @@ def run_ours(args, rank, local_rank, world):
     phase("warm-up done")
     launches_per_step = eng.launch_count()
     ms_sharded = timed(step, args.steps, 0, sampler)
+    if world == 1 and args.dump_outputs:      # the later passes below overwrite sep / masks
+        n_dumped = dump_outputs(args.dump_outputs, [("separated", sep), ("masks", masks)])
+        print(f"bench.py: wrote separated, masks of the last timed step ({n_dumped} of {B} utterances) to "
+              f"{args.dump_outputs}", file=sys.stderr)
 
     # ---- N > 1 headline: scatter from the root, forward, gather to the root (copy engines over NVLink peer memory) ----
     sharded_entry, sg = None, None
@@ -508,6 +536,11 @@ def run_ours(args, rank, local_rank, world):
             return ok
 
         verified = sg_verify(sg)
+        if rank == 0 and args.dump_outputs:      # the global batch gathered into the root's buffers by the last step
+            gsep, gmasks = sg.root_out[(args.steps - 1) & 1]
+            n_dumped = dump_outputs(args.dump_outputs, [("separated", gsep), ("masks", gmasks)])
+            print(f"bench.py: wrote separated, masks of the last timed step ({n_dumped} of {world * B} utterances) "
+                  f"to {args.dump_outputs}", file=sys.stderr)
         barrier()
         # side entry: the same step with the other wire format
         wire_what = {
@@ -875,7 +908,12 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-sweep", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last timed step's outputs as DIR/separated.npy and "
+                         "DIR/masks.npy (float32, whole utterances; a fixed seeded sample of them above 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
     cfg = select_config(args.config)
     if args.batch is None:
@@ -889,7 +927,8 @@ def main():
                "--master-addr", "127.0.0.1", "--master-port", str(29500 + os.getpid() % 1000), os.path.abspath(__file__),
                "--gpus", str(args.gpus), "--steps", str(args.steps), "--warmup", str(args.warmup),
                "--config", args.config, "--batch", str(args.batch)] + \
-              (["--no-cpu-baseline"] if args.no_cpu_baseline else []) + (["--no-sweep"] if args.no_sweep else [])
+              (["--no-cpu-baseline"] if args.no_cpu_baseline else []) + (["--no-sweep"] if args.no_sweep else []) + \
+              (["--dump-outputs", os.path.abspath(args.dump_outputs)] if args.dump_outputs else [])
         raise SystemExit(subprocess.call(cmd))
     if args.impl == "reference":
         run_reference(args, rank, world)

@@ -67,3 +67,41 @@ def test_gather_wire_format_follows_the_traffic_through_the_root():
     assert bench.choose_wire(8, i_b, o_b, fwd, "auto") == "masks"
     with pytest.raises(SystemExit):
         bench.choose_wire(2, i_b, o_b, fwd, "bf16")
+
+
+def test_dump_outputs_of_the_reference_arm_repeat_run_to_run(tmp_path):
+    import subprocess
+    import sys
+    import numpy as np
+    runs = []
+    for k in range(2):
+        out = tmp_path / f"run{k}"
+        res = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--config", "c1",
+                              "--steps", "1", "--warmup", "1", "--dump-outputs", str(out)],
+                             capture_output=True, text=True, timeout=600)
+        assert res.returncode == 0, res.stderr[-3000:]
+        assert json.loads(res.stdout.strip().splitlines()[-1])["steps"] == 1
+        runs.append({n: np.load(out / f"{n}.npy") for n in ("separated", "masks")})
+    for n in ("separated", "masks"):
+        assert runs[0][n].dtype == np.float32 and runs[0][n].shape == (8, 2, 257, 63), n
+        assert np.array_equal(runs[0][n], runs[1][n]), n          # seeded inputs and weights: identical outputs
+    assert runs[0]["masks"].min() >= 0.0 and runs[0]["masks"].max() <= 1.0
+    res = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "0"], capture_output=True, text=True)
+    assert res.returncode != 0 and "--steps" in res.stderr
+
+
+def test_dump_outputs_samples_whole_utterances_under_the_cap(tmp_path, monkeypatch):
+    import numpy as np
+    import torch
+    import bench
+    a = torch.arange(10 * 2 * 3 * 4, dtype=torch.float64).view(10, 2, 3, 4)
+    b = -a
+    monkeypatch.setattr(bench, "DUMP_BYTES", 2 * 1024 + 4 * 2 * a[0].numel() * 4)      # room for 4 of 10 utterances
+    assert bench.dump_outputs(str(tmp_path), [("x", a), ("y", b)]) == 4
+    x, y = np.load(tmp_path / "x.npy"), np.load(tmp_path / "y.npy")
+    assert x.dtype == np.float32 and x.shape == (4, 2, 3, 4) and np.array_equal(y, -x)
+    rows = [int(r[0, 0, 0]) // a[0].numel() for r in x]
+    assert rows == sorted(set(rows)) and all(np.array_equal(x[i], a[r].numpy()) for i, r in enumerate(rows))
+    monkeypatch.setattr(bench, "DUMP_BYTES", 10**6)
+    assert bench.dump_outputs(str(tmp_path), [("x", a), ("y", b)]) == 10
+    assert np.array_equal(np.load(tmp_path / "x.npy"), a.float().numpy())
