@@ -411,7 +411,9 @@ class Engine:
         return waves
 
     def set_option(self, name: str, value: int):
-        """Execution options: 'fuse_ln' (0/1), 'host_chunk' (utterances per pipeline chunk of forward_host)."""
+        """Execution options of avsep_set_option (include/avsep.h): 'use_graph', 'two_stream', 'pdl' (0/1), 'attn_tc'
+        (0 never, 1 long sequences, 2 whenever usable), 'host_chunk', 'host_lanes' (0 = auto), 'profile_spin_us'.
+        An unknown name raises RuntimeError."""
         self._check(self.lib.avsep_set_option(self.h, name.encode(), int(value)), "avsep_set_option")
 
     # ---- profiling -------------------------------------------------------------------------------

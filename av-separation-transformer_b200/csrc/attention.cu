@@ -473,22 +473,12 @@ const char* launch_t(cudaStream_t s, const AttnDev& d, int B, int H, int Lq) {
 
 }  // namespace
 
-namespace {
-int g_tc_mode = 1;
-int g_tc_min_len = 96;
-bool g_small = true;      // single-tile kernel for Lq, Lk <= 64
-}  // namespace
-
-void attention_set_small(bool on) { g_small = on; }
-
-void attention_set_tc(int mode, int min_len) {
-  g_tc_mode = mode;
-  if (min_len > 0) g_tc_min_len = min_len;
-}
+// tc_mode 1: the tcgen05 kernel takes sequences this long or longer on both sides; shorter ones stay on mma.sync.
+constexpr int ATTN_TC_MIN_LEN = 96;
 
 bool attention_tc_wanted(int prec, const AttnProblem& p) {
-  if (g_tc_mode == 0 || !attention_tc_usable(prec, p)) return false;
-  return g_tc_mode == 2 || (p.Lq < p.Lk ? p.Lq : p.Lk) >= g_tc_min_len;
+  if (p.tc_mode == 0 || !attention_tc_usable(prec, p)) return false;
+  return p.tc_mode == 2 || (p.Lq < p.Lk ? p.Lq : p.Lk) >= ATTN_TC_MIN_LEN;
 }
 
 const char* launch_attention(cudaStream_t s, int prec, const AttnProblem& p) {
@@ -507,7 +497,7 @@ const char* launch_attention(cudaStream_t s, int prec, const AttnProblem& p) {
   if (split) {
     if ((p.ldq & 3) || (p.ldo & 1) || (p.ldkv & 3)) return "attention: misaligned leading dimension";
   } else {
-    if (g_small && p.hd == 64 && p.Lq <= QT && p.Lk <= KT && !(p.ldq & 7) && !(p.ldo & 1) && !(lerp ? (p.ldkv & 3) : (p.ldkv & 7)))
+    if (p.hd == 64 && p.Lq <= QT && p.Lk <= KT && !(p.ldq & 7) && !(p.ldo & 1) && !(lerp ? (p.ldkv & 3) : (p.ldkv & 7)))
       return lerp ? launch_small<true>(s, d, p.B, p.H) : launch_small<false>(s, d, p.B, p.H);
   }
   if (!split) {

@@ -107,10 +107,8 @@ struct avsep_handle {
   std::string err;
   std::map<std::string, HostTensor> host_w;
   bool finalized = false;
-  bool fuse_ln = true;   // residual+LayerNorm in the GEMM epilogue when the row fits one tile
   bool use_graph = true; // replay the forward as a CUDA graph (captured per shape + buffer set on its 2nd use)
-  bool fuse_ffn = true;   // linear1 -> act -> linear2 -> +residual -> LayerNorm in one kernel (d_model = 256, bf16)
-  int ffn_fused_min_rows = 2048;   // below this the unfused pair spreads over more CTAs and wins
+  int attn_tc = 1;       // AttnProblem::tc_mode of every attention launch
   bool two_stream = true; // audio and visual branches on two streams (fork/join), so partial waves overlap
   cudaStream_t aux_stream = nullptr;
   cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
@@ -126,21 +124,13 @@ struct avsep_handle {
   const float *pe_a = nullptr, *pe_v = nullptr, *fng = nullptr, *fnb = nullptr;
   CnnWeights cnn{};
   const uint8_t *cnn_w2_slabs = nullptr, *cnn_w3_rows = nullptr;   // tcgen05 CNN operands
-  const uint8_t* cnn_w3_img = nullptr;                             // conv3 weights as shared-memory images (cnn_ig)
-  bool cnn_tc = true;     // tensor-core (tcgen05) CNN for 32x32 frames on the bf16 path
-  bool cnn_ig = false;    // ... as shifted-view implicit GEMMs (visual_cnn_ig_sm100.cu; parity-tested, 157 us L2-warm but
-                          // 192 us inside the step against 185 us for the TMEM-im2col kernel: off by default)
   std::vector<EncLayerW> enc_a, enc_v;
   std::vector<FusLayerW> fus;
   // prepacked weight streams / vector blocks of the fused transformer-stack kernel (null when the config cannot use it)
   const uint8_t *xs_a = nullptr, *xs_v = nullptr, *xs_f = nullptr;
   bool xs_f_decoder = false;   // the fusion stream continues with the SeparationDecoder block
   const uint8_t *xs_a_np = nullptr, *xs_v_np = nullptr;   // encoder streams past their input-projection items
-  bool fuse_proj = true;       // Conv1d #2 / frame_proj inside the encoder stack kernels (option "fuse_proj")
   bool xs_v_kvp = false;       // the visual stream ends with the fusion layers' K | V projection block
-  bool fuse_kvp = true;        // interpolation + K | V projection inside the visual stack kernel (option "fuse_kvp")
-  bool fuse_decoder = true;    // run the decoder inside the fusion stack kernel (option "fuse_decoder")
-  bool fuse_stack = true;   // whole encoder / fusion stacks in one persistent kernel (d_model = 256, 4 heads, bf16, len <= 128)
   // cached library-owned workspace
   void* own_ws = nullptr;
   size_t own_ws_bytes = 0;
@@ -311,12 +301,8 @@ int snapshot(avsep_handle* h, cudaStream_t s, const char* name, const void* ptr,
 // ---- stage helpers -----------------------------------------------------------------------------
 const char* run_visual_cnn(avsep_handle* h, cudaStream_t s, const float* frames, int M, int Hh, int Ww, void* pooled,
                            unsigned long long* trace = nullptr) {
-  if (h->cnn_tc && Hh == 32 && Ww == 32 && h->cfg.precision == AVSEP_PREC_BF16) {
-    if (h->cnn_ig)       // (its trace is clock64 stamps: [grid][64] long long, see tools/cnn_trace.py --ig)
-      return launch_visual_cnn_ig(s, frames, M, h->cnn, h->cnn_w2_slabs, h->cnn_w3_img, pooled, h->num_sms,
-                                  reinterpret_cast<long long*>(trace));
+  if (Hh == 32 && Ww == 32 && h->cfg.precision == AVSEP_PREC_BF16)
     return launch_visual_cnn_tc(s, frames, M, h->cnn, h->cnn_w2_slabs, h->cnn_w3_rows, pooled, h->num_sms, trace);
-  }
   return launch_visual_cnn(s, h->cfg.precision, frames, M, Hh, Ww, h->cnn, pooled, h->num_sms);
 }
 
@@ -343,7 +329,7 @@ int gemm_resid_ln(avsep_handle* h, cudaStream_t s, const char* label, const Gemm
                   const float* resid, float* x_out, const float* g, const float* b, void* out_op, int rows_out,
                   float* y) {
   const int prec = h->cfg.precision;
-  if (h->fuse_ln && gemm_ln_fusable(p.N)) {
+  if (gemm_ln_fusable(p.N)) {
     e.kind = EPI_LN;
     e.resid = resid;
     e.out_f32 = x_out; e.ld_f32 = p.N;
@@ -376,7 +362,7 @@ int linear_resid_ln(avsep_handle* h, cudaStream_t s, const char* label, const vo
 }
 
 bool stack_fusable(const avsep_handle* h, int len) {
-  return h->fuse_stack && h->xs_a != nullptr && xformer_stack_usable(h->cfg.precision, h->cfg.d_model, h->cfg.nhead, len);
+  return h->xs_a != nullptr && xformer_stack_usable(h->cfg.precision, h->cfg.d_model, h->cfg.nhead, len);
 }
 
 // A whole stack in one kernel (xformer_stack_sm100.cu).  which: 0 audio encoder, 1 visual encoder, 2 fusion.
@@ -408,6 +394,10 @@ int run_stack(avsep_handle* h, cudaStream_t s, int which, const float* x_in, flo
   return 0;
 }
 
+// One fused kernel per feed-forward sub-layer (ffn_fused_sm100.cu) from this many rows on; below it the unfused GEMM
+// pair spreads over more CTAs and wins.
+constexpr int FFN_FUSED_MIN_ROWS = 2048;
+
 // nn.TransformerEncoderLayer x L (pre-norm, ReLU FFN; model.py:48-52,59; torch transformer.py:946-950).
 // In: x (fp32 residual stream), a_op = LN_{layer0.norm1}(x).  Out: x, a_op = LN_{final}(x) (or cast when final_g == null).
 int encoder_stack(avsep_handle* h, cudaStream_t s, const std::vector<EncLayerW>& layers, int B, int L, float* x,
@@ -423,13 +413,13 @@ int encoder_stack(avsep_handle* h, cudaStream_t s, const std::vector<EncLayerW>&
     ap.v = static_cast<const uint8_t*>(qkv) + static_cast<size_t>(2 * d) * os;
     ap.ldkv = 3 * d;
     ap.out = attn; ap.ldo = d;
-    ap.B = B; ap.H = H; ap.hd = d / H; ap.Lq = L; ap.Lk = L; ap.lerp_src = 0;
+    ap.B = B; ap.H = H; ap.hd = d / H; ap.Lq = L; ap.Lk = L; ap.lerp_src = 0; ap.tc_mode = h->attn_tc;
     CKL("attn.self", launch_attention(s, prec, ap));
     if (linear_resid_ln(h, s, "gemm.out_proj", attn, M, d, w.wo, w.bo, d, x, w.n2g, w.n2b, a_op, y)) return 1;
     const bool last = (l + 1 == layers.size());
     const float* g = last ? final_g : layers[l + 1].n1g;
     const float* b = last ? final_b : layers[l + 1].n1b;
-    if (h->fuse_ffn && ffn_fusable(prec, d) && M >= h->ffn_fused_min_rows) {
+    if (ffn_fusable(prec, d) && M >= FFN_FUSED_MIN_ROWS) {
       CKL("ffn.fused", launch_ffn_fused(s, a_op, w.w1, w.b1, w.w2, w.b2, ACT_RELU, x, x,
                                                                              g, b, a_op, M, h->num_sms, nullptr));
     } else {
@@ -516,7 +506,7 @@ int fusion_stack_fused(avsep_handle* h, cudaStream_t s, Workspace& w, int L_src,
     CKL("lerp_kv", launch_lerp_rows(s, w.x_v, d, B, L_src, T, d, w.attn_a, d));
     if (linear(h, s, "gemm.cross_kv", w.attn_a, Ma, d, h->wkv_all, h->bkv_all, Lf * 2 * d, ACT_NONE, nullptr, w.kvb)) return 1;
   }
-  *decoded = h->fuse_decoder && h->xs_f_decoder && !h->debug && masks != nullptr;
+  *decoded = h->xs_f_decoder && !h->debug && masks != nullptr;
   if (*decoded)
     return run_stack(h, s, 2, w.x_a, nullptr, nullptr, h->fng, h->fnb, w.kvb, Lf * 2 * d, B, T, nullptr, mixed, separated, masks);
   if (run_stack(h, s, 2, w.x_a, h->debug ? w.x_a : nullptr, w.a_op, h->fng, h->fnb, w.kvb, Lf * 2 * d, B, T)) return 1;
@@ -538,7 +528,7 @@ int fusion_stack(avsep_handle* h, cudaStream_t s, Workspace& w, int L_src) {
     ap.v = w.kvn + static_cast<size_t>(l) * 2 * d + d;
     ap.ldkv = Lf * 2 * d;
     ap.out = w.attn_a; ap.ldo = d;
-    ap.B = B; ap.H = H; ap.hd = d / H; ap.Lq = T; ap.Lk = T; ap.lerp_src = L_src;
+    ap.B = B; ap.H = H; ap.hd = d / H; ap.Lq = T; ap.Lk = T; ap.lerp_src = L_src; ap.tc_mode = h->attn_tc;
     {
       // Long sequences: materialise the interpolated K/V rows once (bf16, in the unused 2d columns' worth of the
       // Q buffer) so the tcgen05 kernel can stage them by TMA; short ones interpolate on load inside the kernel.
@@ -557,7 +547,7 @@ int fusion_stack(avsep_handle* h, cudaStream_t s, Workspace& w, int L_src) {
     const bool last = (l + 1 == Lf);
     const float* g = last ? h->fng : h->fus[l + 1].n1g;
     const float* b = last ? h->fnb : h->fus[l + 1].n1b;
-    if (h->fuse_ffn && ffn_fusable(prec, d) && Ma >= h->ffn_fused_min_rows) {
+    if (ffn_fusable(prec, d) && Ma >= FFN_FUSED_MIN_ROWS) {
       CKL("ffn.fused", launch_ffn_fused(s, w.a_op, fw.w1, fw.b1, fw.w2, fw.b2, ACT_GELU,
                                                                              w.x_a, w.x_a, g, b, w.a_op, Ma, h->num_sms,
                                                                              nullptr));
@@ -609,13 +599,13 @@ int forward_device(avsep_handle* h, cudaStream_t s, Workspace& w, const float* m
   const bool fa = stack_fusable(h, w.T), fv = stack_fusable(h, w.N);
   const bool ff = fa && fv;            // the fused fusion stack reads the fp32 residual rows of both encoders
   // --- visual branch (enqueued first: its CNN is the longest kernel) ---
-  const bool fp = h->fuse_proj && !h->debug;     // input projections inside the stack kernels (no stage snapshots then)
+  const bool fp = !h->debug;     // input projections inside the stack kernels (no stage snapshots then)
   bool kvp = false;
   if (visual_frontend(h, sv, w, frames, h->enc_v[0].n1g, h->enc_v[0].n1b, fv, fv && fp)) return 1;
   if (fv) {
     // out: x_v (fp32) for the interpolation in front of the K/V projection; v_op (bf16 cast) only for the unfused fusion
     // fused K | V projection: needs the fused fusion stack behind it and the audio frames inside a visual tile slot
-    kvp = ff && h->fuse_kvp && h->xs_v_kvp && !h->debug &&
+    kvp = ff && h->xs_v_kvp && !h->debug &&
           xformer_kvp_usable(h->cfg.num_fusion_layers * 2 * d, w.N, w.T);
     if (run_stack(h, sv, 1, w.x_v, kvp ? nullptr : w.x_v, (ff || kvp) ? nullptr : w.v_op, nullptr, nullptr, nullptr, 0, w.B,
                   w.N, nullptr, nullptr, nullptr, nullptr, fp ? w.pooled : nullptr, kvp ? w.kvb : nullptr, w.T))
@@ -944,9 +934,6 @@ int avsep_finalize_weights(avsep_handle* h, void* cuda_stream) {
     visual_cnn_tc_pack(folded[1].data(), folded[2].data(), tc2.data(), tc3.data());
     off["tcw2"] = ar.add(tc2.data(), tc2.size());
     off["tcw3"] = ar.add(tc3.data(), tc3.size());
-    std::vector<uint8_t> ig3(visual_cnn_ig_w3_bytes());
-    visual_cnn_ig_pack(folded[2].data(), ig3.data());
-    off["igw3"] = ar.add(ig3.data(), ig3.size());
     off["cw1"] = ar.add(p1.data(), p1.size() * 4);
     off["cw2"] = ar.add(p2.data(), p2.size() * 4);
     off["cw3"] = ar.add(p3.data(), p3.size() * 4);
@@ -1131,7 +1118,6 @@ int avsep_finalize_weights(avsep_handle* h, void* cuda_stream) {
   h->cnn.w3l = reinterpret_cast<const uint32_t*>(P("cw3l"));
   h->cnn_w2_slabs = static_cast<const uint8_t*>(P("tcw2"));
   h->cnn_w3_rows = static_cast<const uint8_t*>(P("tcw3"));
-  h->cnn_w3_img = static_cast<const uint8_t*>(P("igw3"));
   h->xs_a = h->xs_v = h->xs_f = nullptr;
   if (pack_stacks) {
     h->xs_a = static_cast<const uint8_t*>(P("xs_a")); h->xs_v = static_cast<const uint8_t*>(P("xs_v"));
@@ -1744,24 +1730,12 @@ int avsep_test_fusion_decoder(avsep_handle* h, const float* x_in, const void* kv
 
 int avsep_set_option(avsep_handle* h, const char* name, int32_t value) {
   if (!h || !name) return 1;
-  if (strcmp(name, "fuse_ln") == 0) { h->fuse_ln = value != 0; drop_graphs(h); return 0; }
   if (strcmp(name, "host_chunk") == 0) { h->host_chunk = value; return 0; }
   if (strcmp(name, "host_lanes") == 0) { h->host_lanes = value; return 0; }
   if (strcmp(name, "pdl") == 0) { h->pdl = value != 0; pdl_set(h->pdl && !h->profile); drop_graphs(h); return 0; }
-  if (strcmp(name, "cnn_tc") == 0) { h->cnn_tc = value != 0; drop_graphs(h); return 0; }
-  if (strcmp(name, "cnn_ig") == 0) { h->cnn_ig = value != 0; drop_graphs(h); return 0; }
   if (strcmp(name, "use_graph") == 0) { h->use_graph = value != 0; return 0; }
-  if (strcmp(name, "fuse_ffn") == 0) { h->fuse_ffn = value != 0; drop_graphs(h); return 0; }
-  if (strcmp(name, "fuse_stack") == 0) { h->fuse_stack = value != 0; drop_graphs(h); return 0; }
-  if (strcmp(name, "fuse_decoder") == 0) { h->fuse_decoder = value != 0; drop_graphs(h); return 0; }
-  if (strcmp(name, "fuse_proj") == 0) { h->fuse_proj = value != 0; drop_graphs(h); return 0; }
-  if (strcmp(name, "fuse_kvp") == 0) { h->fuse_kvp = value != 0; drop_graphs(h); return 0; }
-  if (strcmp(name, "ffn_fused_min_rows") == 0) { h->ffn_fused_min_rows = value; drop_graphs(h); return 0; }
   if (strcmp(name, "two_stream") == 0) { h->two_stream = value != 0; drop_graphs(h); return 0; }
-  if (strcmp(name, "attn_small") == 0) { attention_set_small(value != 0); drop_graphs(h); return 0; }
-  if (strcmp(name, "attn_tc") == 0) { attention_set_tc(value, 0); drop_graphs(h); return 0; }
-  if (strcmp(name, "attn_tc_min_len") == 0) { attention_set_tc(1, value); drop_graphs(h); return 0; }
-  if (strcmp(name, "epilogue_tma") == 0) { gemm_set_epilogue_tma(value != 0); drop_graphs(h); return 0; }
+  if (strcmp(name, "attn_tc") == 0) { h->attn_tc = value; drop_graphs(h); return 0; }
   if (strcmp(name, "profile_spin_us") == 0) { h->profile_spin_us = value; return 0; }
   return fail(h, std::string("unknown option ") + name);
 }
@@ -1784,7 +1758,7 @@ int avsep_test_attention(avsep_handle* h, const void* q, const void* k, const vo
   if (!h) return 1;
   AttnProblem ap{};
   ap.q = q; ap.ldq = H * hd; ap.k = k; ap.v = v; ap.ldkv = H * hd; ap.out = out; ap.ldo = H * hd;
-  ap.B = B; ap.H = H; ap.hd = hd; ap.Lq = Lq; ap.Lk = Lk; ap.lerp_src = lerp_src;
+  ap.B = B; ap.H = H; ap.hd = hd; ap.Lq = Lq; ap.Lk = Lk; ap.lerp_src = lerp_src; ap.tc_mode = h->attn_tc;
   cudaStream_t s = static_cast<cudaStream_t>(cuda_stream);
   void* scratch = nullptr;
   if (lerp_src > 0) {   // same routing as fusion_stack: K then V columns side by side in one interpolated buffer

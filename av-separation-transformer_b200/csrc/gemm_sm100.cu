@@ -910,7 +910,6 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
 // ------------------------------------------------------------------------------------------
 PFN_cuTensorMapEncodeTiled_v12000 g_encode = nullptr;
 int g_num_sms = 0;
-bool g_epi_tma = true;   // A/B switch (gemm_set_epilogue_tma)
 
 const char* encode_2d(CUtensorMap* map, bool tf32, const void* ptr, uint64_t inner, uint64_t outer, uint64_t ld_elems,
                       uint32_t box_inner, uint32_t box_outer) {
@@ -966,8 +965,6 @@ const char* gemm_init() {
   return nullptr;
 }
 
-void gemm_set_epilogue_tma(bool on) { g_epi_tma = on; }
-
 bool gemm_ln_fusable(int N) { return N <= BN_MAX && N >= 32 && (N % 32) == 0; }
 
 const char* launch_gemm(cudaStream_t s, int prec, const GemmProblem& p, const GemmEpilogue& e, int force_bn,
@@ -1010,7 +1007,7 @@ const char* launch_gemm(cudaStream_t s, int prec, const GemmProblem& p, const Ge
   if (const char* err = encode_2d(&tw, tf32, p.W, static_cast<uint64_t>(p.ldw), p.N, p.ldw, box_k, n_tile)) return err;
   // Epilogue I/O through TMA slabs: rows map one-to-one (no Conv1d halo remap), columns in 64-wide units.
   CUtensorMap top = ta, tf32m = ta;   // placeholders when unused
-  bool use_tma = g_epi_tma && e.kind != EPI_TAIL && e.rowmap == ROW_IDENT && (p.N % 64 == 0) && (n_tile % 64 == 0);
+  bool use_tma = e.kind != EPI_TAIL && e.rowmap == ROW_IDENT && (p.N % 64 == 0) && (n_tile % 64 == 0);
   if (e.kind == EPI_STD && e.out_f32 != nullptr && e.out_op != nullptr && !tf32) use_tma = false;   // one slab, one output
   if (e.kind == EPI_LN) {
     use_tma = use_tma && n_tile == 256 && (e.resid == nullptr || e.resid == e.out_f32 || e.out_f32 == nullptr);

@@ -80,7 +80,6 @@ const char* gemm_init();   // resolves cuTensorMapEncodeTiled, sets smem attribu
 const char* launch_gemm(cudaStream_t s, int prec, const GemmProblem& p, const GemmEpilogue& e, int force_bn = 0,
                         unsigned long long* trace = nullptr);   // trace: [grid][8] globaltimer stamps (debug)
 bool gemm_ln_fusable(int N);   // EPI_LN usable for this row width
-void gemm_set_epilogue_tma(bool on);   // A/B switch: epilogue I/O through TMA slabs (default on)
 
 // Fused FFN sub-layer (d_model = 256, bf16): x += W2 act(W1 a + b1) + b2 ; out_op = LayerNorm(x)  (ffn_fused_sm100.cu)
 bool ffn_fusable(int prec, int d_model);
@@ -167,15 +166,14 @@ struct AttnProblem {
   void* out; int ldo;              // operand precision [B*Lq, ldo]
   int B, H, hd, Lq, Lk;
   int lerp_src;                    // 0 = plain; >0 = K/V hold lerp_src source rows per utterance, interpolated to Lk rows
+  int tc_mode;                     // tcgen05 kernel: 0 = never, 1 = when min(Lq, Lk) >= 96, 2 = whenever usable
 };
 const char* launch_attention(cudaStream_t s, int prec, const AttnProblem& p);
 // tcgen05 flash attention (attention_tc.cu): bf16, head dim 64, materialised K/V rows.  launch_attention dispatches
-// to it by itself; mode 0 = never, 1 = when min(Lq, Lk) >= min_len, 2 = whenever usable.
+// to it by itself when attention_tc_wanted.
 bool attention_tc_usable(int prec, const AttnProblem& p);
-bool attention_tc_wanted(int prec, const AttnProblem& p);      // usable and selected by the current mode
+bool attention_tc_wanted(int prec, const AttnProblem& p);      // usable and selected by p.tc_mode
 const char* launch_attention_tc(cudaStream_t s, const AttnProblem& p);
-void attention_set_tc(int mode, int min_len);
-void attention_set_small(bool on);                             // single-tile kernel for Lq, Lk <= 64 (bf16, head dim 64)                  // min_len <= 0 keeps the current value
 // dst[b*L + t, 0:cols] (bf16) = linear interpolation (align_corners=False) of src rows [b*nsrc + i, 0:cols] (fp32)
 const char* launch_lerp_rows(cudaStream_t s, const float* src, int ld_src, int B, int nsrc, int L, int cols,
                              void* dst_bf16, int ld_dst);
@@ -196,11 +194,6 @@ void visual_cnn_tc_pack(const float* w2, const float* w3, uint8_t* w2_slabs, uin
 const char* launch_visual_cnn_tc(cudaStream_t s, const float* frames, int M, const CnnWeights& w, const uint8_t* w2_slabs,
                                  const uint8_t* w3_rows, void* pooled, int num_sms,
                                  unsigned long long* trace = nullptr);
-// shifted-view implicit GEMM variant (visual_cnn_ig_sm100.cu): no im2col gather; conv3 weights as pre-swizzled images
-size_t visual_cnn_ig_w3_bytes();
-void visual_cnn_ig_pack(const float* w3, uint8_t* w3_img);
-const char* launch_visual_cnn_ig(cudaStream_t s, const float* frames, int M, const CnnWeights& w, const uint8_t* w2_slabs,
-                                 const uint8_t* w3_img, void* pooled, int num_sms, long long* trace = nullptr);
 size_t visual_cnn_pack_sizes(int which);   // elements of packed w1/w2/w3 (uint32)
 void visual_cnn_pack(const float* w1, const float* w2, const float* w3, uint32_t* p1, uint32_t* p2, uint32_t* p3,
                      bool lo_part = false);

@@ -114,30 +114,18 @@ AVSEP_API int avsep_set_debug(avsep_handle* h, int32_t enable);
 /* Copies a snapshot to a HOST buffer of `capacity` floats; returns the element count in *count. Synchronises. */
 AVSEP_API int avsep_debug_get_stage(avsep_handle* h, const char* name, float* host_out, size_t capacity, size_t* count);
 
-/* Execution options (A/B switches; every position is parity-tested).  name -> meaning (default):
- *   "fuse_ln" (1)            residual + LayerNorm inside the GEMM epilogue (0: separate add+LayerNorm kernel)
- *   "epilogue_tma" (1)       TMA-slab GEMM epilogues (0: cooperative stores)
- *   "fuse_stack" (1)         every layer of an encoder / fusion stack in one persistent kernel when d_model = 256, 4 heads,
- *                            bf16 and the clip has at most 128 frames (xformer_stack_sm100.cu); the switches below refine it
- *   "fuse_proj" (1)          ... with Conv1d #2 + ReLU + PE / frame_proj + PE fused in front of the encoder stacks
- *   "fuse_kvp" (1)           ... with the interpolation + K|V projection of the fusion layers fused behind the visual stack
- *   "fuse_decoder" (1)       ... with the final LayerNorm + SeparationDecoder fused behind the fusion stack
- *   "cnn_ig" (0)             shifted-view implicit-GEMM CNN (visual_cnn_ig_sm100.cu) instead of the TMEM-im2col one
- *   "fuse_ffn" (1)           one kernel per feed-forward sub-layer when d_model = 256, bf16, rows >= ffn_fused_min_rows
- *   "ffn_fused_min_rows" (2048)
- *   "cnn_tc" (1)             tcgen05 CNN for 32x32 frames (0: generic mma.sync kernel)
- *   "attn_tc" (1)            1: tcgen05 attention when min(Lq, Lk) >= attn_tc_min_len; 0: never; 2: whenever usable
- *   "attn_tc_min_len" (96)
- *   "attn_small" (1)         single-tile attention kernel (72 registers, 7 CTAs/SM) when Lq, Lk <= 64, bf16, head dim 64
+/* Execution options.  Apart from them, kernel choice follows from the configuration, the shapes and debug mode alone.
+ * name -> meaning (default):
  *   "use_graph" (1)          CUDA-graph replay keyed by (shape, buffers)
  *   "two_stream" (1)         audio and visual branches on two streams
  *   "pdl" (1)                programmatic dependent launch between consecutive kernels
+ *   "attn_tc" (1)            1: tcgen05 attention when usable and min(Lq, Lk) >= 96; 0: never; 2: whenever usable
  *   "host_chunk" (0), "host_lanes" (0)    host-buffer pipeline: utterances per chunk, concurrent compute lanes; 0 = auto
  *                            (56 x 2 lanes for avsep_forward_host, 128 x 1 lane for avsep_forward_host_async)
  *   "profile_spin_us"        length of the GPU spin kernel that precedes a profiled forward
- * The environment variable AVSEP_OPTS="name=value,name=value" applies options at avsep_create (measurement runs).
- * Kernel-selection switches ("epilogue_tma", "attn_tc", "attn_tc_min_len", "attn_small", "pdl") are process-wide:
- * they apply to every handle of the process, not only to `h`. */
+ * Any other name is an error.  The environment variable AVSEP_OPTS="name=value,name=value" applies options at
+ * avsep_create (measurement runs).  "pdl" is process-wide: it applies to every handle of the process, not only to `h`;
+ * every other option applies to `h` alone. */
 AVSEP_API int avsep_set_option(avsep_handle* h, const char* name, int32_t value);
 
 /* Per-kernel timing: when enabled every launch of the forward is bracketed by a cudaEvent pair on the launching

@@ -250,12 +250,12 @@ def test_add_layernorm(eng, M, d):
     assert torch.equal(out2, x.bfloat16())
 
 
-@pytest.mark.parametrize("Hh,Ww,M,tc", [(32, 32, 50, 2), (32, 32, 8, 2), (32, 32, 1, 2), (32, 32, 7, 2), (32, 32, 1203, 2),
-                                         (32, 32, 2501, 2), (32, 32, 50, 1), (32, 32, 8, 1), (32, 32, 1203, 1),
-                                         (32, 32, 50, 0), (16, 16, 21, 0), (15, 18, 7, 0), (32, 32, 601, 0)])
-def test_visual_cnn(Hh, Ww, M, tc):
-    """tc = 2: shifted-view implicit-GEMM tcgen05 kernel (visual_cnn_ig_sm100.cu, 32x32 only); 1: the TMEM-im2col tcgen05
-    kernel (visual_cnn_tc.cu); 0: generic mma.sync kernel (any frame size)."""
+@pytest.mark.parametrize("Hh,Ww,M", [(32, 32, 1), (32, 32, 7), (32, 32, 8), (32, 32, 50), (32, 32, 601), (32, 32, 1203),
+                                      (32, 32, 2501), (16, 16, 21), (15, 18, 7), (16, 16, 601), (31, 32, 50), (32, 31, 50),
+                                      (64, 64, 50)])
+def test_visual_cnn(Hh, Ww, M):
+    """The frame size picks the kernel: 32x32 frames run the tcgen05 kernel (visual_cnn_tc.cu), every other size the
+    generic mma.sync kernel (visual_cnn.cu)."""
     from oracle.weights import CONFIGS, make_state_dict
     from avsep_b200.engine import Engine, EngineConfig
     cfg = CONFIGS["tiny"]
@@ -263,8 +263,6 @@ def test_visual_cnn(Hh, Ww, M, tc):
     e = Engine(EngineConfig(**cfg.as_dict()), 0)
     try:
         e.load_state({k: v for k, v in P.items() if v.ndim > 0})
-        e.set_option("cnn_tc", 1 if tc else 0)
-        e.set_option("cnn_ig", 1 if tc == 2 else 0)
         g = torch.Generator(device="cuda").manual_seed(M)
         frames = torch.rand(M, Hh, Ww, device="cuda", generator=g)
         pooled = torch.zeros(M, 128, device="cuda", dtype=torch.bfloat16)

@@ -10,15 +10,13 @@ sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "av-separation-t
 from avsep_b200 import AVSeparationTransformer
 from avsep_b200.synth import synthetic_batch
 
-ap = argparse.ArgumentParser(); ap.add_argument("--precision", default="bf16"); ap.add_argument("--profile", action="store_true"); ap.add_argument("--ffn-min-rows", type=int, default=-1); ap.add_argument("--small", action="store_true"); args = ap.parse_args()
+ap = argparse.ArgumentParser(); ap.add_argument("--precision", default="bf16"); ap.add_argument("--profile", action="store_true"); ap.add_argument("--small", action="store_true"); args = ap.parse_args()
 
 def run(model_kw, B, T, N, seconds, label, iters=30):
     torch.manual_seed(0)
     m = AVSeparationTransformer(**model_kw, precision=args.precision).cuda()
     mixed, frames = synthetic_batch(B, model_kw.get("freq_bins", 257), T, N, 32, 32, seed=1, device="cuda")
     m.prepack("cuda")
-    if args.ffn_min_rows >= 0:
-        m.engine.set_option("ffn_fused_min_rows", args.ffn_min_rows)
     for _ in range(4):
         m(mixed, frames)
     torch.cuda.synchronize()
@@ -46,7 +44,7 @@ scaled = dict(freq_bins=257, d_model=512, nhead=8, num_encoder_layers=6, num_fus
 res = []
 if args.small:
     for B in (8, 16, 32, 64, 96, 128):
-        run(default, B, 63, 50, 1.0, f"B={B} ffn_min_rows={args.ffn_min_rows}")
+        run(default, B, 63, 50, 1.0, f"B={B}")
     sys.exit(0)
 if args.profile:
     run(default, 32, 1251, 500, 10.0, "C3 long-form B=32", iters=5)

@@ -6,7 +6,6 @@ sys.path.insert(0, os.path.join(ROOT, "av-separation-transformer_b200"))
 from avsep_b200.engine import Engine, EngineConfig
 
 eng = Engine(EngineConfig(65, 64, 4, 1, 1, 2, "bf16"), 0)
-eng.set_option("epilogue_tma", int(os.environ.get("EPI_TMA", "1")))
 for (M, N, K, ln, act, tag) in [(16128, 256, 768, 1, 0, "K=768 LN (conv1d_2-sized, plain rows)"), (16128, 256, 768, 0, 0, "K=768 std"), (16128, 768, 256, 0, 0, "qkv"), (12800, 768, 256, 0, 0, "qkv visual"), (16128, 256, 256, 0, 0, "cross_q"), (16128, 1024, 256, 0, 1, "ffn1 relu"), (16128, 1024, 256, 0, 2, "ffn1 gelu"), (16128, 256, 1024, 1, 0, "ffn2 LN"), (16128, 256, 256, 1, 0, "LN full"), (16128, 256, 256, 2, 0, "LN no-resid-load"),
                                 (16128, 256, 256, 3, 0, "LN no-x'-store"), (16128, 256, 256, 4, 0, "LN no-bf16-store"),
                                 (16128, 256, 256, 5, 0, "LN no resid, no x' store"), (16128, 256, 256, 6, 0, "LN cast only (no stats)")]:
