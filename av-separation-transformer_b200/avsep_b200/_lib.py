@@ -42,6 +42,7 @@ SIGNATURES = {
     "avsep_finalize_weights": (C.c_int, [_P, _P]),
     "avsep_workspace_bytes": (C.c_size_t, [_P, _I, _I, _I, _I, _I]),
     "avsep_forward": (C.c_int, [_P, _P, _P, _I, _I, _I, _I, _I, _P, _P, _P, C.c_size_t, _P]),
+    "avsep_forward_varlen": (C.c_int, [_P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _P, _P, _P, C.c_size_t, _P]),
     "avsep_forward_host": (C.c_int, [_P, _P, _P, _I, _I, _I, _I, _I, _P, _P, _P]),
     "avsep_forward_host_async": (C.c_int, [_P, _P, _P, _I, _I, _I, _I, _I, _P, _P, _I, _P]),
     "avsep_host_wait": (C.c_int, [_P, _I]),

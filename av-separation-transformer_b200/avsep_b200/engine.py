@@ -91,6 +91,7 @@ class Engine:
             raise RuntimeError("avsep_create: " + self.lib.avsep_last_error(None).decode())
         self.h = h
         self._keep = []
+        self._len_bufs = {}   # (name, stream) -> engine-owned int32 device buffer (stable graph key per stream)
 
     def close(self):
         if getattr(self, "h", None):
@@ -181,13 +182,49 @@ class Engine:
                     raise ValueError(f"{what}: output buffers must be contiguous float32 {want}, got {tuple(t.shape)}")
         return B, T, N, Hh, Ww
 
+    def _lengths(self, v, name: str, B: int, limit: int):
+        """Per-utterance lengths -> int32 device tensor (or None).  A list, numpy array or CPU integer tensor is
+        validated here (B entries, 1 <= v <= limit) and copied into an engine-owned buffer of the current stream, so
+        the pointer - and with it the CUDA-graph key - stays the same from call to call, and the copy is ordered after
+        the previous forward on that stream that read the buffer (one buffer per stream: forwards on two streams never
+        share one).  The copy goes through pinned memory and does not block the host.  An int32 tensor on the engine's
+        device is passed through without reading it: the library clamps its values to [1, limit]."""
+        if v is None:
+            return None
+        if isinstance(v, torch.Tensor) and v.is_cuda:
+            if v.device.index != self.device or v.dtype != torch.int32 or tuple(v.shape) != (B,) or not v.is_contiguous():
+                raise ValueError(f"forward: a device {name} tensor must be contiguous int32 ({B},) on cuda:{self.device}")
+            return v
+        a = v.numpy() if isinstance(v, torch.Tensor) else np.asarray(v)
+        if a.shape != (B,):
+            raise ValueError(f"forward: {name} must have one entry per utterance ({B}), got shape {a.shape}")
+        if a.dtype == np.bool_ or not np.issubdtype(a.dtype, np.integer):
+            raise ValueError(f"forward: {name} must hold integers, got {a.dtype}")
+        if a.min() < 1 or a.max() > limit:
+            raise ValueError(f"forward: {name} must lie in [1, {limit}], got [{a.min()}, {a.max()}]")
+        key = (name, torch.cuda.current_stream(self.device).cuda_stream)
+        buf = self._len_bufs.get(key)
+        if buf is None or buf.numel() < B:
+            buf = torch.empty(max(B, 256), dtype=torch.int32, device=torch.device("cuda", self.device))
+            self._len_bufs[key] = buf
+        # the pinned staging block is not reused before this copy has run (torch's host allocator records the stream)
+        buf[:B].copy_(torch.from_numpy(a.astype(np.int32)).pin_memory(), non_blocking=True)
+        return buf[:B]
+
     # ---- forward ---------------------------------------------------------------------------------
-    def forward(self, mixed: torch.Tensor, frames: torch.Tensor, out=None):
+    def forward(self, mixed: torch.Tensor, frames: torch.Tensor, out=None, lengths=None, frame_lengths=None):
         """Device tensors in, device tensors out.  ``out=(separated, masks)`` reuses caller-owned (B,S,F,T) float32
-        buffers: with fixed input and output buffers every call after the second is one CUDA-graph replay."""
+        buffers: with fixed input and output buffers every call after the second is one CUDA-graph replay.
+
+        Variable-length batch: ``lengths`` (B,) audio frames and ``frame_lengths`` (B,) lip frames per utterance, each
+        left-aligned in the padded (T, N) inputs; None = all T / all N.  Utterance b's outputs [b, :, :, :lengths[b]]
+        equal a forward of that utterance alone, the rest are 0, and the padding of the inputs is never read."""
         mixed = self._dev_f32(mixed, "mixed_spec")
         frames = self._dev_f32(frames, "lip_frames")
         B, T, N, Hh, Ww = self._check_inputs("forward", mixed=mixed, frames=frames, out=out)
+        with torch.cuda.device(self.device):
+            lens = self._lengths(lengths, "lengths", B, T)
+            flens = self._lengths(frame_lengths, "frame_lengths", B, N)
         F, S = self.cfg.freq_bins, self.cfg.num_speakers
         if out is None:
             # one allocation for both outputs: the caching allocator then recycles a handful of blocks, so the
@@ -199,14 +236,21 @@ class Engine:
             for t in out:
                 if not t.is_cuda or t.device.index != self.device:
                     raise ValueError(f"forward: output buffers must live on cuda:{self.device}")
-        args = (self.h, mixed.data_ptr(), frames.data_ptr(), B, T, N, Hh, Ww, sep.data_ptr(), masks.data_ptr(), None, 0,
-                self._stream())
+        if lens is None and flens is None:
+            fn, what = self.lib.avsep_forward, "avsep_forward"
+            args = (self.h, mixed.data_ptr(), frames.data_ptr(), B, T, N, Hh, Ww, sep.data_ptr(), masks.data_ptr(),
+                    None, 0, self._stream())
+        else:
+            fn, what = self.lib.avsep_forward_varlen, "avsep_forward_varlen"
+            args = (self.h, mixed.data_ptr(), frames.data_ptr(), None if lens is None else lens.data_ptr(),
+                    None if flens is None else flens.data_ptr(), B, T, N, Hh, Ww, sep.data_ptr(), masks.data_ptr(),
+                    None, 0, self._stream())
         if torch.cuda.current_device() == self.device:      # the library selects its device itself; only restore the
-            rc = self.lib.avsep_forward(*args)               # caller's when it differs
+            rc = fn(*args)                                   # caller's when it differs
         else:
             with torch.cuda.device(self.device):
-                rc = self.lib.avsep_forward(*args)
-        self._check(rc, "avsep_forward")
+                rc = fn(*args)
+        self._check(rc, what)
         return sep, masks
 
     @staticmethod

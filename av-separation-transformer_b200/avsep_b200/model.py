@@ -308,11 +308,20 @@ class AVSeparationTransformer(_InferenceOnly):
     def _engine_config(self):
         return self.config
 
-    def forward(self, mixed_spec: torch.Tensor, lip_frames: torch.Tensor, out=None):
+    def forward(self, mixed_spec: torch.Tensor, lip_frames: torch.Tensor, out=None, *, lengths=None,
+                frame_lengths=None):
         """``out=(separated, masks)``: optional caller-owned output buffers (not a reference argument); with fixed
-        input and output buffers the call is a single CUDA-graph replay."""
+        input and output buffers the call is a single CUDA-graph replay.
+
+        ``lengths`` / ``frame_lengths`` (not reference arguments; CUDA inputs only): per-utterance audio frames and lip
+        frames of a variable-length batch, see ``Engine.forward``.  Utterance b then gives what the model gives on its
+        first ``lengths[b]`` / ``frame_lengths[b]`` frames alone, and its outputs past ``lengths[b]`` are 0."""
         if mixed_spec.is_cuda:
-            return self._get_engine(mixed_spec.device).forward(mixed_spec, lip_frames, out)
+            return self._get_engine(mixed_spec.device).forward(mixed_spec, lip_frames, out, lengths=lengths,
+                                                               frame_lengths=frame_lengths)
+        if lengths is not None or frame_lengths is not None:
+            raise ValueError("forward: lengths / frame_lengths need CUDA inputs (the host-buffer path takes full "
+                             "batches only)")
         eng = self._get_engine(torch.device(self.host_device))
         return eng.forward_host(mixed_spec, lip_frames, *(out or ()))
 

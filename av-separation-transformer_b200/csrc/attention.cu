@@ -24,7 +24,25 @@ struct AttnDev {
   int H, Lq, Lk, nsrc;
   float scale_log2;
   float lerp_scale;   // (float)nsrc / Lk, as ATen computes it
+  // variable-length batch (null: all Lk / all nsrc): keys of utterance b, and its interpolation source rows.  Lk and
+  // nsrc stay the row pitch of the K/V buffers.
+  const int *k_lens, *src_lens;
 };
+
+// Keys of utterance b, its interpolation source rows and scale (ATen: (float)nsrc / (float)Lk).
+struct UttKeys {
+  int lk, nsrc;
+  float scale;
+};
+template <bool LERP>
+__device__ __forceinline__ UttKeys utt_keys(const AttnDev& p, int b) {
+  UttKeys u;
+  u.lk = utt_len(p.k_lens, b, p.Lk);
+  u.nsrc = LERP ? utt_len(p.src_lens, b, p.nsrc) : 0;
+  u.scale = (p.k_lens == nullptr && p.src_lens == nullptr) ? p.lerp_scale
+                                                           : static_cast<float>(u.nsrc) / static_cast<float>(u.lk);
+  return u;
+}
 
 __device__ __forceinline__ void ldmatrix_x4(uint32_t (&r)[4], uint32_t addr) {
   asm volatile("ldmatrix.sync.aligned.m8n8.x4.shared.b16 {%0,%1,%2,%3}, [%4];"
@@ -133,8 +151,10 @@ __device__ __forceinline__ void load_tile_split(__nv_bfloat16* dst_hi, __nv_bflo
 
 // SPLIT = fp32-grade path: Q/K/V are fp32 in global memory and are staged as bf16 hi + lo tiles; every contraction is
 // three tensor-core products (hi*hi + hi*lo + lo*hi); P is split the same way; the output is fp32.
+// The minimum-blocks bound keeps the bf16 head-dim 64 / 128 variants at 128 / 168 registers, i.e. 4 / 3 resident
+// CTAs per SM, which ptxas gives them without spills.
 template <int HD, bool LERP, bool SPLIT>
-__global__ void __launch_bounds__(128) attention_kernel(const AttnDev p) {
+__global__ void __launch_bounds__(128, SPLIT ? 0 : HD == 64 ? 4 : HD == 128 ? 3 : 0) attention_kernel(const AttnDev p) {
   constexpr int LDS = HD + 8;           // padded row (elements): 16-byte rows shifted by 4 banks -> conflict-free ldmatrix
   constexpr int KS = HD / 16;           // k-steps over the head dimension
   constexpr int NT_O = HD / 8;          // output n-tiles
@@ -153,26 +173,28 @@ __global__ void __launch_bounds__(128) attention_kernel(const AttnDev p) {
   const int b = blockIdx.z;
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
+  const int lk = utt_len(p.k_lens, b, p.Lk);
 
   auto load_kv = [&](int kv0) {
+    const UttKeys uk = utt_keys<LERP>(p, b);       // re-derived per tile: fewer registers live across the sweep
     if constexpr (SPLIT) {
       const int src_rows = LERP ? p.nsrc : p.Lk;
       const float* ksrc = reinterpret_cast<const float*>(p.k) + static_cast<size_t>(b) * src_rows * p.ldkv + h * HD;
       const float* vsrc = reinterpret_cast<const float*>(p.v) + static_cast<size_t>(b) * src_rows * p.ldkv + h * HD;
-      load_tile_split<HD>(sK, sKl, ksrc, p.ldkv, kv0, p.Lk, LERP ? p.nsrc : 0, p.lerp_scale);
-      load_tile_split<HD>(sV, sVl, vsrc, p.ldkv, kv0, p.Lk, LERP ? p.nsrc : 0, p.lerp_scale);
+      load_tile_split<HD>(sK, sKl, ksrc, p.ldkv, kv0, uk.lk, uk.nsrc, uk.scale);
+      load_tile_split<HD>(sV, sVl, vsrc, p.ldkv, kv0, uk.lk, uk.nsrc, uk.scale);
     } else if constexpr (LERP) {
       const float* ksrc = reinterpret_cast<const float*>(p.k) + static_cast<size_t>(b) * p.nsrc * p.ldkv + h * HD;
       const float* vsrc = reinterpret_cast<const float*>(p.v) + static_cast<size_t>(b) * p.nsrc * p.ldkv + h * HD;
-      load_tile_lerp<HD>(sK, ksrc, p.ldkv, kv0, p.Lk, p.nsrc, p.lerp_scale);
-      load_tile_lerp<HD>(sV, vsrc, p.ldkv, kv0, p.Lk, p.nsrc, p.lerp_scale);
+      load_tile_lerp<HD>(sK, ksrc, p.ldkv, kv0, uk.lk, uk.nsrc, uk.scale);
+      load_tile_lerp<HD>(sV, vsrc, p.ldkv, kv0, uk.lk, uk.nsrc, uk.scale);
     } else {
       const __nv_bfloat16* ksrc =
           reinterpret_cast<const __nv_bfloat16*>(p.k) + static_cast<size_t>(b) * p.Lk * p.ldkv + h * HD;
       const __nv_bfloat16* vsrc =
           reinterpret_cast<const __nv_bfloat16*>(p.v) + static_cast<size_t>(b) * p.Lk * p.ldkv + h * HD;
-      load_tile_bf16<HD>(sK, ksrc, p.ldkv, kv0, p.Lk);
-      load_tile_bf16<HD>(sV, vsrc, p.ldkv, kv0, p.Lk);
+      load_tile_bf16<HD>(sK, ksrc, p.ldkv, kv0, uk.lk);
+      load_tile_bf16<HD>(sV, vsrc, p.ldkv, kv0, uk.lk);
     }
   };
   // Q and the first K/V tile are staged together: one exposed global-load latency instead of two (at T <= 64 the
@@ -206,7 +228,7 @@ __global__ void __launch_bounds__(128) attention_kernel(const AttnDev p) {
   float m_run[2] = {-INFINITY, -INFINITY};
   float l_run[2] = {0.f, 0.f};
 
-  const int num_kv_tiles = (p.Lk + KT - 1) / KT;
+  const int num_kv_tiles = (lk + KT - 1) / KT;       // key tiles wholly past the utterance's keys are skipped
   for (int jt = 0; jt < num_kv_tiles; ++jt) {
     const int kv0 = jt * KT;
     if (jt > 0) {
@@ -247,7 +269,7 @@ __global__ void __launch_bounds__(128) attention_kernel(const AttnDev p) {
       const int c = kv0 + nt * 8 + 2 * (lane & 3);
 #pragma unroll
       for (int e = 0; e < 4; ++e) {
-        const bool ok = (c + (e & 1)) < p.Lk;
+        const bool ok = (c + (e & 1)) < lk;
         const float val = ok ? s[nt][e] * p.scale_log2 : -INFINITY;
         s[nt][e] = val;
         mx[e >> 1] = fmaxf(mx[e >> 1], val);
@@ -358,19 +380,20 @@ __global__ void __launch_bounds__(128, 7) attention_small_kernel(const AttnDev p
   griddep_wait();
   const int h = blockIdx.y, b = blockIdx.z;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const UttKeys uk = utt_keys<LERP>(p, b);
   {
     const __nv_bfloat16* qsrc = reinterpret_cast<const __nv_bfloat16*>(p.q) + static_cast<size_t>(b) * p.Lq * p.ldq + h * HD;
     load_tile_bf16<HD>(sQ, qsrc, p.ldq, 0, p.Lq);
     if constexpr (LERP) {
       const float* ksrc = reinterpret_cast<const float*>(p.k) + static_cast<size_t>(b) * p.nsrc * p.ldkv + h * HD;
       const float* vsrc = reinterpret_cast<const float*>(p.v) + static_cast<size_t>(b) * p.nsrc * p.ldkv + h * HD;
-      load_tile_lerp<HD>(sK, ksrc, p.ldkv, 0, p.Lk, p.nsrc, p.lerp_scale);
-      load_tile_lerp<HD>(sV, vsrc, p.ldkv, 0, p.Lk, p.nsrc, p.lerp_scale);
+      load_tile_lerp<HD>(sK, ksrc, p.ldkv, 0, uk.lk, uk.nsrc, uk.scale);
+      load_tile_lerp<HD>(sV, vsrc, p.ldkv, 0, uk.lk, uk.nsrc, uk.scale);
     } else {
       const __nv_bfloat16* ksrc = reinterpret_cast<const __nv_bfloat16*>(p.k) + static_cast<size_t>(b) * p.Lk * p.ldkv + h * HD;
       const __nv_bfloat16* vsrc = reinterpret_cast<const __nv_bfloat16*>(p.v) + static_cast<size_t>(b) * p.Lk * p.ldkv + h * HD;
-      load_tile_bf16<HD>(sK, ksrc, p.ldkv, 0, p.Lk);
-      load_tile_bf16<HD>(sV, vsrc, p.ldkv, 0, p.Lk);
+      load_tile_bf16<HD>(sK, ksrc, p.ldkv, 0, uk.lk);
+      load_tile_bf16<HD>(sV, vsrc, p.ldkv, 0, uk.lk);
     }
   }
   __syncthreads();
@@ -397,7 +420,7 @@ __global__ void __launch_bounds__(128, 7) attention_small_kernel(const AttnDev p
     const int c = nt * 8 + 2 * (lane & 3);
 #pragma unroll
     for (int e = 0; e < 4; ++e) {
-      const float val = (c + (e & 1)) < p.Lk ? s[nt][e] * p.scale_log2 : -INFINITY;
+      const float val = (c + (e & 1)) < uk.lk ? s[nt][e] * p.scale_log2 : -INFINITY;
       s[nt][e] = val;
       if (e < 2) mx0 = fmaxf(mx0, val); else mx1 = fmaxf(mx1, val);
     }
@@ -493,6 +516,7 @@ const char* launch_attention(cudaStream_t s, int prec, const AttnProblem& p) {
   d.H = p.H; d.Lq = p.Lq; d.Lk = p.Lk; d.nsrc = p.lerp_src;
   d.scale_log2 = 1.4426950408889634f / sqrtf(static_cast<float>(p.hd));
   d.lerp_scale = p.lerp_src > 0 ? static_cast<float>(p.lerp_src) / static_cast<float>(p.Lk) : 0.f;
+  d.k_lens = p.k_lens; d.src_lens = p.lerp_src > 0 ? p.src_lens : nullptr;
   const bool lerp = p.lerp_src > 0;
   if (split) {
     if ((p.ldq & 3) || (p.ldo & 1) || (p.ldkv & 3)) return "attention: misaligned leading dimension";

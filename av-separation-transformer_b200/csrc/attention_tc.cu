@@ -38,6 +38,7 @@ constexpr uint32_t TMEM_COLS = 256;
 struct AttnTcDev {
   int Lq, Lk;
   float scale_log2;
+  const int* k_lens;    // variable-length batch: keys of utterance b (null: all Lk)
 };
 
 __device__ __forceinline__ float ex2_approx(float x) {
@@ -78,7 +79,8 @@ attention_tc_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_consta
   const int q0 = blockIdx.x * QT;
   const int h = blockIdx.y;
   const int b = blockIdx.z;
-  const int nkv = (p.Lk + KT - 1) / KT;
+  const int lk = utt_len(p.k_lens, b, p.Lk);
+  const int nkv = (lk + KT - 1) / KT;                 // key tiles wholly past the utterance's keys are skipped
 
   if (threadIdx.x == 0) {
     mbar_init(q_full, 1);
@@ -177,7 +179,7 @@ attention_tc_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_consta
     };
 
     for (int j = 0; j < nkv; ++j) {
-      const int valid = p.Lk - j * KT;                  // columns of this tile that exist
+      const int valid = lk - j * KT;                    // columns of this tile that exist
       mbar_wait_sleep(s_full, j & 1);
       tc_fence_after();
       // pass 1: row max (four independent chains; the chunk that straddles Lk takes the masked branch)
@@ -292,9 +294,12 @@ attention_tc_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_consta
   if (warp == 1) tmem_dealloc(tmem_base, TMEM_COLS);
 }
 
-// out[b*L + t, :] = lerp of two fp32 source rows (ATen upsample_linear1d, align_corners=False; model.py:114-116)
+// out[b*L + t, :] = lerp of two fp32 source rows (ATen upsample_linear1d, align_corners=False; model.py:114-116).
+// src_lens / dst_lens (variable-length batch, else null): utterance b interpolates its first src_lens[b] source rows
+// to dst_lens[b] rows; the rows past dst_lens[b] take the same formula (finite filler for masked keys).
 __global__ void lerp_rows_kernel(const float* __restrict__ src, int ld_src, int nsrc, int L, int chunks, float scale,
-                                 __nv_bfloat16* __restrict__ dst, int ld_dst, long long total) {
+                                 __nv_bfloat16* __restrict__ dst, int ld_dst, long long total,
+                                 const int* __restrict__ src_lens, const int* __restrict__ dst_lens) {
   griddep_launch_dependents();
   griddep_wait();
   const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
@@ -303,10 +308,15 @@ __global__ void lerp_rows_kernel(const float* __restrict__ src, int ld_src, int 
   const long long rt = i / chunks;
   const int t = static_cast<int>(rt % L);
   const long long bb = rt / L;
+  int ns = nsrc;
+  if (src_lens != nullptr || dst_lens != nullptr) {
+    ns = utt_len(src_lens, static_cast<int>(bb), nsrc);
+    scale = static_cast<float>(ns) / static_cast<float>(utt_len(dst_lens, static_cast<int>(bb), L));
+  }
   const float sp = fmaxf(scale * (static_cast<float>(t) + 0.5f) - 0.5f, 0.0f);
   int i0 = static_cast<int>(sp);
-  if (i0 > nsrc - 1) i0 = nsrc - 1;
-  const int i1 = min(i0 + 1, nsrc - 1);
+  if (i0 > ns - 1) i0 = ns - 1;
+  const int i1 = min(i0 + 1, ns - 1);
   const float w1 = sp - static_cast<float>(i0), w0 = 1.0f - w1;
   const float4* p0 = reinterpret_cast<const float4*>(src + (bb * nsrc + i0) * ld_src + c * 8);
   const float4* p1 = reinterpret_cast<const float4*>(src + (bb * nsrc + i1) * ld_src + c * 8);
@@ -365,6 +375,7 @@ const char* launch_attention_tc(cudaStream_t s, const AttnProblem& p) {
   AttnTcDev d;
   d.Lq = p.Lq; d.Lk = p.Lk;
   d.scale_log2 = 1.4426950408889634f / sqrtf(static_cast<float>(HD));
+  d.k_lens = p.k_lens;
   dim3 grid((p.Lq + QT - 1) / QT, p.H, p.B);
   if (launch_pdl(attention_tc_kernel, grid, dim3(NTHREADS), SMEM_BYTES, s, tq, tk, tv, to, d) != cudaSuccess) {
     cudaGetLastError();
@@ -374,14 +385,15 @@ const char* launch_attention_tc(cudaStream_t s, const AttnProblem& p) {
 }
 
 const char* launch_lerp_rows(cudaStream_t s, const float* src, int ld_src, int B, int nsrc, int L, int cols,
-                             void* dst_bf16, int ld_dst) {
+                             void* dst_bf16, int ld_dst, const int* src_lens, const int* dst_lens) {
   if ((cols & 7) || (ld_src & 3) || (ld_dst & 7)) return "lerp_rows: misaligned";
   const int chunks = cols / 8;
   const long long total = static_cast<long long>(B) * L * chunks;
   const int threads = 256;
   const long long blocks = (total + threads - 1) / threads;
   launch_pdl(lerp_rows_kernel, dim3(static_cast<unsigned>(blocks)), dim3(threads), 0, s, src, ld_src, nsrc, L, chunks,
-             static_cast<float>(nsrc) / static_cast<float>(L), reinterpret_cast<__nv_bfloat16*>(dst_bf16), ld_dst, total);
+             static_cast<float>(nsrc) / static_cast<float>(L), reinterpret_cast<__nv_bfloat16*>(dst_bf16), ld_dst, total,
+             src_lens, dst_lens);
   return cudaGetLastError() == cudaSuccess ? nullptr : "lerp_rows: launch failed";
 }
 

@@ -60,9 +60,10 @@ __global__ void spin_kernel(unsigned long long ns) {
 struct GraphKey {
   int B, T, N, Hh, Ww;
   const void *mixed, *frames, *sep, *masks, *ws;
+  const int *lens, *frame_lens;   // the kernels read the lengths at run time: their contents are not part of the key
   bool operator==(const GraphKey& o) const {
     return B == o.B && T == o.T && N == o.N && Hh == o.Hh && Ww == o.Ww && mixed == o.mixed && frames == o.frames &&
-           sep == o.sep && masks == o.masks && ws == o.ws;
+           sep == o.sep && masks == o.masks && ws == o.ws && lens == o.lens && frame_lens == o.frame_lens;
   }
 };
 struct GraphEntry {
@@ -88,6 +89,9 @@ struct FusLayerW {
 
 struct Workspace {   // carved from one base pointer; all offsets 1 KB aligned
   int B = 0, T = 0, N = 0, Hh = 0, Ww = 0;
+  // variable-length batch (avsep_forward_varlen): device int32 [B] audio frames / lip frames per utterance, or null
+  // (all T / all N).  Every kernel where rows of different lengths meet reads them.
+  const int *lens = nullptr, *frame_lens = nullptr;
   size_t bytes = 0;
   // audio side
   void *xp, *h1, *a_op, *qkv_a, *attn_a, *ffn_a;
@@ -300,10 +304,11 @@ int snapshot(avsep_handle* h, cudaStream_t s, const char* name, const void* ptr,
 
 // ---- stage helpers -----------------------------------------------------------------------------
 const char* run_visual_cnn(avsep_handle* h, cudaStream_t s, const float* frames, int M, int Hh, int Ww, void* pooled,
-                           unsigned long long* trace = nullptr) {
+                           unsigned long long* trace = nullptr, const int* frame_lens = nullptr, int N = 1) {
   if (Hh == 32 && Ww == 32 && h->cfg.precision == AVSEP_PREC_BF16)
-    return launch_visual_cnn_tc(s, frames, M, h->cnn, h->cnn_w2_slabs, h->cnn_w3_rows, pooled, h->num_sms, trace);
-  return launch_visual_cnn(s, h->cfg.precision, frames, M, Hh, Ww, h->cnn, pooled, h->num_sms);
+    return launch_visual_cnn_tc(s, frames, M, h->cnn, h->cnn_w2_slabs, h->cnn_w3_rows, pooled, h->num_sms, trace,
+                                frame_lens, N);
+  return launch_visual_cnn(s, h->cfg.precision, frames, M, Hh, Ww, h->cnn, pooled, h->num_sms, frame_lens, N);
 }
 
 int linear(avsep_handle* h, cudaStream_t s, const char* label, const void* A, int M, int K, const void* W,
@@ -369,9 +374,10 @@ bool stack_fusable(const avsep_handle* h, int len) {
 int run_stack(avsep_handle* h, cudaStream_t s, int which, const float* x_in, float* out_x, void* out_op,
               const float* fin_g, const float* fin_b, const void* kv, int kv_ld, int B, int L, long long* trace = nullptr,
               const float* mixed = nullptr, float* separated = nullptr, float* masks = nullptr, const void* pro_a = nullptr,
-              void* kvp_out = nullptr, int kvp_L = 0) {
+              void* kvp_out = nullptr, int kvp_L = 0, const int* lens = nullptr, const int* kvp_lens = nullptr) {
   StackProblem sp{};
   sp.trace = trace;
+  sp.lens = lens; sp.kvp_lens = kvp_lens;
   if (kvp_out != nullptr) {      // which 1: the fusion layers' K | V rows are produced inside the kernel
     sp.kvp_out = kvp_out; sp.kvp_L = kvp_L; sp.kvp_n = h->cfg.num_fusion_layers * 2 * h->cfg.d_model; sp.kvp_ld = sp.kvp_n;
   }
@@ -400,8 +406,10 @@ constexpr int FFN_FUSED_MIN_ROWS = 2048;
 
 // nn.TransformerEncoderLayer x L (pre-norm, ReLU FFN; model.py:48-52,59; torch transformer.py:946-950).
 // In: x (fp32 residual stream), a_op = LN_{layer0.norm1}(x).  Out: x, a_op = LN_{final}(x) (or cast when final_g == null).
+// lens: keys per utterance of a variable-length batch, or null.
 int encoder_stack(avsep_handle* h, cudaStream_t s, const std::vector<EncLayerW>& layers, int B, int L, float* x,
-                  float* y, void* a_op, void* qkv, void* attn, void* ffn, const float* final_g, const float* final_b) {
+                  float* y, void* a_op, void* qkv, void* attn, void* ffn, const float* final_g, const float* final_b,
+                  const int* lens = nullptr) {
   const int d = h->cfg.d_model, H = h->cfg.nhead, M = B * L, prec = h->cfg.precision;
   const size_t os = op_size(h);
   for (size_t l = 0; l < layers.size(); ++l) {
@@ -414,6 +422,7 @@ int encoder_stack(avsep_handle* h, cudaStream_t s, const std::vector<EncLayerW>&
     ap.ldkv = 3 * d;
     ap.out = attn; ap.ldo = d;
     ap.B = B; ap.H = H; ap.hd = d / H; ap.Lq = L; ap.Lk = L; ap.lerp_src = 0; ap.tc_mode = h->attn_tc;
+    ap.k_lens = lens;
     CKL("attn.self", launch_attention(s, prec, ap));
     if (linear_resid_ln(h, s, "gemm.out_proj", attn, M, d, w.wo, w.bo, d, x, w.n2g, w.n2b, a_op, y)) return 1;
     const bool last = (l + 1 == layers.size());
@@ -438,13 +447,14 @@ int audio_frontend(avsep_handle* h, cudaStream_t s, Workspace& w, const float* m
   h->prof_stream = s;
   const int d = h->cfg.d_model, F = h->cfg.freq_bins, B = w.B, T = w.T, prec = h->cfg.precision;
   const int Map = B * (T + 2);
-  CKL("prep_audio", launch_prep_audio(s, prec, mixed, w.xp, B, F, T, h->Fp));
+  CKL("prep_audio", launch_prep_audio(s, prec, mixed, w.xp, B, F, T, h->Fp, w.lens));
   {
     GemmProblem p{};
     p.A = w.xp; p.lda = h->Fp; p.rowsA = Map; p.M = Map; p.W = h->wc1; p.ldw = 3 * h->Fp; p.N = d; p.K = h->Fp;
     p.taps = 3; p.tap_stride = h->Fp; p.row_shift = -1;
     GemmEpilogue e;
     e.bias = h->bc1; e.act = ACT_RELU; e.rowmap = ROW_PAD2PAD; e.Lp = T + 2;
+    e.lens = w.lens;
     e.out_op = w.h1; e.ld_op = d;
     CKL("gemm.conv1d_0", launch_gemm(s, prec, p, e));
   }
@@ -473,7 +483,7 @@ int visual_frontend(avsep_handle* h, cudaStream_t s, Workspace& w, const float* 
   h->prof_stream = s;
   const int d = h->cfg.d_model, B = w.B, N = w.N;
   const int Mv = B * N;
-  CKL("visual_cnn", run_visual_cnn(h, s, frames, Mv, w.Hh, w.Ww, w.pooled));
+  CKL("visual_cnn", run_visual_cnn(h, s, frames, Mv, w.Hh, w.Ww, w.pooled, nullptr, w.frame_lens, N));
   if (snapshot(h, s, "visual_pool", w.pooled, static_cast<size_t>(Mv) * 128, true)) return 1;
   if (cnn_only) return 0;        // frame_proj + PE run inside the encoder stack kernel, on the pooled features
   GemmProblem p{};
@@ -503,13 +513,16 @@ int fusion_stack_fused(avsep_handle* h, cudaStream_t s, Workspace& w, int L_src,
   const int d = h->cfg.d_model, B = w.B, T = w.T;
   const int Ma = B * T, Lf = h->cfg.num_fusion_layers;
   if (!have_kv) {                // else the visual stack kernel has already written w.kvb
-    CKL("lerp_kv", launch_lerp_rows(s, w.x_v, d, B, L_src, T, d, w.attn_a, d));
+    CKL("lerp_kv", launch_lerp_rows(s, w.x_v, d, B, L_src, T, d, w.attn_a, d, w.frame_lens, w.lens));
     if (linear(h, s, "gemm.cross_kv", w.attn_a, Ma, d, h->wkv_all, h->bkv_all, Lf * 2 * d, ACT_NONE, nullptr, w.kvb)) return 1;
   }
   *decoded = h->xs_f_decoder && !h->debug && masks != nullptr;
   if (*decoded)
-    return run_stack(h, s, 2, w.x_a, nullptr, nullptr, h->fng, h->fnb, w.kvb, Lf * 2 * d, B, T, nullptr, mixed, separated, masks);
-  if (run_stack(h, s, 2, w.x_a, h->debug ? w.x_a : nullptr, w.a_op, h->fng, h->fnb, w.kvb, Lf * 2 * d, B, T)) return 1;
+    return run_stack(h, s, 2, w.x_a, nullptr, nullptr, h->fng, h->fnb, w.kvb, Lf * 2 * d, B, T, nullptr, mixed, separated, masks,
+                     nullptr, nullptr, 0, w.lens);
+  if (run_stack(h, s, 2, w.x_a, h->debug ? w.x_a : nullptr, w.a_op, h->fng, h->fnb, w.kvb, Lf * 2 * d, B, T, nullptr, nullptr,
+                nullptr, nullptr, nullptr, nullptr, 0, w.lens))
+    return 1;
   return snapshot(h, s, "fused", w.a_op, static_cast<size_t>(Ma) * d, true);
 }
 
@@ -529,6 +542,7 @@ int fusion_stack(avsep_handle* h, cudaStream_t s, Workspace& w, int L_src) {
     ap.ldkv = Lf * 2 * d;
     ap.out = w.attn_a; ap.ldo = d;
     ap.B = B; ap.H = H; ap.hd = d / H; ap.Lq = T; ap.Lk = T; ap.lerp_src = L_src; ap.tc_mode = h->attn_tc;
+    ap.k_lens = w.lens; ap.src_lens = w.frame_lens;
     {
       // Long sequences: materialise the interpolated K/V rows once (bf16, in the unused 2d columns' worth of the
       // Q buffer) so the tcgen05 kernel can stage them by TMA; short ones interpolate on load inside the kernel.
@@ -537,7 +551,8 @@ int fusion_stack(avsep_handle* h, cudaStream_t s, Workspace& w, int L_src) {
       __nv_bfloat16* kvi = static_cast<__nv_bfloat16*>(w.qkv_a) + static_cast<size_t>(Ma) * d;
       tp.k = kvi; tp.v = kvi + d; tp.ldkv = 2 * d;
       if (attention_tc_wanted(prec, tp)) {
-        CKL("lerp_kv", launch_lerp_rows(s, w.kvn + static_cast<size_t>(l) * 2 * d, Lf * 2 * d, B, L_src, T, 2 * d, kvi, 2 * d));
+        CKL("lerp_kv", launch_lerp_rows(s, w.kvn + static_cast<size_t>(l) * 2 * d, Lf * 2 * d, B, L_src, T, 2 * d, kvi, 2 * d,
+                                        w.frame_lens, w.lens));
         ap = tp;
       }
     }
@@ -572,6 +587,7 @@ int decoder_stage(avsep_handle* h, cudaStream_t s, Workspace& w, const float* mi
   e.kind = EPI_TAIL;
   e.bias = h->bdec3;
   e.mixed = mixed; e.masks = masks; e.separated = separated; e.F = F; e.S = S; e.T = T;
+  e.lens = w.lens;
   CKL("gemm.dec3_tail", launch_gemm(s, h->cfg.precision, p, e));
   return 0;
 }
@@ -608,9 +624,11 @@ int forward_device(avsep_handle* h, cudaStream_t s, Workspace& w, const float* m
     kvp = ff && h->xs_v_kvp && !h->debug &&
           xformer_kvp_usable(h->cfg.num_fusion_layers * 2 * d, w.N, w.T);
     if (run_stack(h, sv, 1, w.x_v, kvp ? nullptr : w.x_v, (ff || kvp) ? nullptr : w.v_op, nullptr, nullptr, nullptr, 0, w.B,
-                  w.N, nullptr, nullptr, nullptr, nullptr, fp ? w.pooled : nullptr, kvp ? w.kvb : nullptr, w.T))
+                  w.N, nullptr, nullptr, nullptr, nullptr, fp ? w.pooled : nullptr, kvp ? w.kvb : nullptr, w.T, w.frame_lens,
+                  w.lens))
       return 1;
-  } else if (encoder_stack(h, sv, h->enc_v, w.B, w.N, w.x_v, w.y_v, w.v_op, w.qkv_v, w.attn_v, w.ffn_v, nullptr, nullptr)) {
+  } else if (encoder_stack(h, sv, h->enc_v, w.B, w.N, w.x_v, w.y_v, w.v_op, w.qkv_v, w.attn_v, w.ffn_v, nullptr, nullptr,
+                           w.frame_lens)) {
     return 1;
   }
   if (snapshot(h, sv, "visual_enc", w.x_v, static_cast<size_t>(Mv) * d, false)) return 1;
@@ -618,10 +636,10 @@ int forward_device(avsep_handle* h, cudaStream_t s, Workspace& w, const float* m
   if (audio_frontend(h, s, w, mixed, h->enc_a[0].n1g, h->enc_a[0].n1b, fa, fa && fp)) return 1;
   if (fa) {
     if (run_stack(h, s, 0, w.x_a, w.x_a, ff ? nullptr : w.a_op, h->fus[0].n1g, h->fus[0].n1b, nullptr, 0, w.B, w.T, nullptr,
-                  nullptr, nullptr, nullptr, fp ? w.h1 : nullptr))
+                  nullptr, nullptr, nullptr, fp ? w.h1 : nullptr, nullptr, 0, w.lens))
       return 1;
   } else if (encoder_stack(h, s, h->enc_a, w.B, w.T, w.x_a, w.y_a, w.a_op, w.qkv_a, w.attn_a, w.ffn_a, h->fus[0].n1g,
-                           h->fus[0].n1b)) {
+                           h->fus[0].n1b, w.lens)) {
     return 1;
   }
   if (snapshot(h, s, "audio_enc", w.x_a, static_cast<size_t>(Ma) * d, false)) return 1;
@@ -645,7 +663,7 @@ int forward_device(avsep_handle* h, cudaStream_t s, Workspace& w, const float* m
 int forward_cached(avsep_handle* h, cudaStream_t s, Workspace& w, const void* ws_base, const float* mixed,
                    const float* frames, float* separated, float* masks) {
   if (!h->use_graph || h->profile || h->debug) return forward_device(h, s, w, mixed, frames, separated, masks);
-  const GraphKey key{w.B, w.T, w.N, w.Hh, w.Ww, mixed, frames, separated, masks, ws_base};
+  const GraphKey key{w.B, w.T, w.N, w.Hh, w.Ww, mixed, frames, separated, masks, ws_base, w.lens, w.frame_lens};
   GraphEntry* ent = nullptr;
   for (auto& g : h->graphs)
     if (g.key == key) { ent = &g; break; }
@@ -1155,12 +1173,20 @@ size_t avsep_workspace_bytes(avsep_handle* h, int32_t B, int32_t T, int32_t N, i
 int avsep_forward(avsep_handle* h, const float* mixed_spec, const float* lip_frames, int32_t B, int32_t T, int32_t N,
                   int32_t Hh, int32_t Ww, float* separated, float* masks, void* workspace, size_t workspace_bytes,
                   void* cuda_stream) {
+  return avsep_forward_varlen(h, mixed_spec, lip_frames, nullptr, nullptr, B, T, N, Hh, Ww, separated, masks, workspace,
+                              workspace_bytes, cuda_stream);
+}
+
+int avsep_forward_varlen(avsep_handle* h, const float* mixed_spec, const float* lip_frames, const int32_t* lengths,
+                         const int32_t* frame_lengths, int32_t B, int32_t T, int32_t N, int32_t Hh, int32_t Ww,
+                         float* separated, float* masks, void* workspace, size_t workspace_bytes, void* cuda_stream) {
   if (!h) return 1;
   if (!mixed_spec || !lip_frames || !separated || !masks) return fail(h, "avsep_forward: null buffer");
   if (check_shape(h, B, T, N, Hh, Ww)) return 1;
   CUDA_OK(cudaSetDevice(h->cfg.device));
   Workspace w;
   if (get_workspace(h, w, workspace, workspace_bytes, B, T, N, Hh, Ww)) return 1;
+  w.lens = lengths; w.frame_lens = frame_lengths;
   h->launches = 0;
   return forward_cached(h, static_cast<cudaStream_t>(cuda_stream), w, workspace ? workspace : h->own_ws, mixed_spec,
                         lip_frames, separated, masks);

@@ -100,9 +100,12 @@ add_layernorm_kernel(const float* __restrict__ x, const float* __restrict__ y, c
 
 // mixed (B,F,T) fp32, T fastest  ->  xp (B, T+2, Fp), F fastest, rows 0 and T+1 zero (Conv1d padding=1,
 // model.py:38), columns [F,Fp) zero.  32x32 smem-tile transpose: reads coalesced along T, writes along F.
+// lens (variable-length batch, else null): rows t >= lens[b] are zero (the short clip's right-hand padding) and the
+// mixture is not read there.
 template <bool TF32>
 __global__ void __launch_bounds__(256)
-prep_audio_kernel(const float* __restrict__ mixed, void* __restrict__ xp, int F, int T, int Fp) {
+prep_audio_kernel(const float* __restrict__ mixed, void* __restrict__ xp, int F, int T, int Fp,
+                  const int* __restrict__ lens) {
   __shared__ float tile[32][33];
   griddep_launch_dependents();
   griddep_wait();
@@ -112,11 +115,12 @@ prep_audio_kernel(const float* __restrict__ mixed, void* __restrict__ xp, int F,
   const int tx = threadIdx.x & 31;
   const int ty = threadIdx.x >> 5;   // 0..7
   const float* src = mixed + static_cast<size_t>(b) * F * T;
+  const int Tb = utt_len(lens, b, T);
 #pragma unroll
   for (int i = 0; i < 4; ++i) {
     const int f = f0 + ty + 8 * i;
     const int t = t0 + tx;
-    tile[ty + 8 * i][tx] = (f < F && t < T) ? src[static_cast<size_t>(f) * T + t] : 0.f;
+    tile[ty + 8 * i][tx] = (f < F && t < Tb) ? src[static_cast<size_t>(f) * T + t] : 0.f;
   }
   __syncthreads();
   const size_t base = static_cast<size_t>(b) * (T + 2) * Fp;
@@ -158,10 +162,11 @@ const char* launch_add_layernorm(cudaStream_t s, int prec, const float* x, const
   return cudaGetLastError() == cudaSuccess ? nullptr : "layernorm: launch failed";
 }
 
-const char* launch_prep_audio(cudaStream_t s, int prec, const float* mixed, void* xp, int B, int F, int T, int Fp) {
+const char* launch_prep_audio(cudaStream_t s, int prec, const float* mixed, void* xp, int B, int F, int T, int Fp,
+                              const int* lens) {
   dim3 grid((T + 31) / 32, (Fp + 31) / 32, B);
-  if (prec == PREC_TF32) launch_pdl(prep_audio_kernel<true>, grid, dim3(256), 0, s, mixed, xp, F, T, Fp);
-  else launch_pdl(prep_audio_kernel<false>, grid, dim3(256), 0, s, mixed, xp, F, T, Fp);
+  if (prec == PREC_TF32) launch_pdl(prep_audio_kernel<true>, grid, dim3(256), 0, s, mixed, xp, F, T, Fp, lens);
+  else launch_pdl(prep_audio_kernel<false>, grid, dim3(256), 0, s, mixed, xp, F, T, Fp, lens);
   return cudaGetLastError() == cudaSuccess ? nullptr : "prep_audio: launch failed";
 }
 

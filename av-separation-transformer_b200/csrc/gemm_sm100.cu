@@ -190,7 +190,9 @@ __device__ __forceinline__ RowInfo row_info(const GemmEpilogue& e, int m, int M)
     const bool halo = (tp == 0) || (tp == e.Lp - 1);
     r.pos = tp - 1;
     if (e.rowmap == ROW_PAD2PAD) {
-      r.zero_row = halo;
+      // rows past a short utterance's length are its right-hand Conv1d padding (rows m >= M of the last tile have
+      // no utterance: lens is not read for them)
+      r.zero_row = halo || (r.valid && e.lens != nullptr && tp - 1 >= utt_len(e.lens, b, e.Lp - 2));
     } else {
       r.valid = r.valid && !halo;
       r.orow = static_cast<long long>(b) * (e.Lp - 2) + (tp - 1);
@@ -254,10 +256,16 @@ __device__ __forceinline__ void value_chunk(const GemmEpilogue& e, const RowInfo
 // even complete): column c = s*F + f sits c*T floats further in masks / separated and f*T further in mixed_spec.
 // Whole chunks that do not cross a speaker boundary take branch-free bodies - the per-element guards and the frequency
 // wrap cost more instructions than the sigmoid.  All tests except `valid` are warp-uniform.
+// live == false: the row lies past its utterance's length; mixed_spec is not read there and both outputs are 0.
 __device__ __forceinline__ void tail_load16(const GemmEpilogue& e, int N, int col0, const float* mixed_row, bool valid,
-                                            float (&mx)[16]) {
+                                            bool live, float (&mx)[16]) {
   const int ncols = min(16, N - col0);
   if (!valid || ncols <= 0) return;
+  if (!live) {
+#pragma unroll
+    for (int j = 0; j < 16; ++j) mx[j] = 0.f;
+    return;
+  }
   int f = col0 % e.F;
   if (ncols == 16 && f + 16 <= e.F) {
     const float* mp = mixed_row + static_cast<size_t>(f) * e.T;
@@ -273,7 +281,7 @@ __device__ __forceinline__ void tail_load16(const GemmEpilogue& e, int N, int co
 }
 
 __device__ __forceinline__ void tail_store16(const GemmEpilogue& e, int N, int col0, size_t out_base, bool valid,
-                                             const uint32_t (&v)[16], const float* sb, const float (&mx)[16]) {
+                                             bool live, const uint32_t (&v)[16], const float* sb, const float (&mx)[16]) {
   const int ncols = min(16, N - col0);
   if (!valid || ncols <= 0) return;
   float* mo = e.masks + out_base + static_cast<size_t>(col0) * e.T;
@@ -281,7 +289,7 @@ __device__ __forceinline__ void tail_store16(const GemmEpilogue& e, int N, int c
   if (ncols == 16) {
 #pragma unroll
     for (int j = 0; j < 16; ++j) {
-      const float mk = sigmoid_fast(__uint_as_float(v[j]) + sb[j]);
+      const float mk = live ? sigmoid_fast(__uint_as_float(v[j]) + sb[j]) : 0.f;
       __stcs(mo + static_cast<size_t>(j) * e.T, mk);
       __stcs(so + static_cast<size_t>(j) * e.T, mk * mx[j]);
     }
@@ -289,7 +297,7 @@ __device__ __forceinline__ void tail_store16(const GemmEpilogue& e, int N, int c
 #pragma unroll
     for (int j = 0; j < 16; ++j) {
       if (j < ncols) {
-        const float mk = sigmoid_fast(__uint_as_float(v[j]) + sb[j]);
+        const float mk = live ? sigmoid_fast(__uint_as_float(v[j]) + sb[j]) : 0.f;
         __stcs(mo + static_cast<size_t>(j) * e.T, mk);
         __stcs(so + static_cast<size_t>(j) * e.T, mk * mx[j]);
       }
@@ -453,7 +461,7 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
       }
       // EPI_TAIL: this thread's row of the (B,S,F,T) outputs, its share of the tile's columns, and the mixed_spec
       // values of its first 16 columns - requested now, while the tile's MMAs are still running
-      bool t_valid = false;
+      bool t_valid = false, t_live = true;
       const float* t_mixed_row = nullptr;
       size_t t_out_base = 0;
       int t_cbeg = 0, t_cend = 0;
@@ -465,6 +473,7 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
         t_valid = m < p.M;
         const int tb = m / e.T;
         const int tt = m - tb * e.T;
+        t_live = e.lens == nullptr || (t_valid && tt < utt_len(e.lens, tb, e.T));
         t_mixed_row = e.mixed + static_cast<size_t>(tb) * e.F * e.T + tt;
         t_out_base = static_cast<size_t>(tb) * e.S * e.F * e.T + tt;
         // Each column part takes a contiguous, balanced share of the tile in units of 16 columns (176 columns ->
@@ -473,7 +482,7 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
         const int units = p.n_tile >> 4, ubase = units >> 2, urem = units & 3;
         t_cbeg = (part * ubase + min(part, urem)) << 4;
         t_cend = t_cbeg + ((ubase + (part < urem ? 1 : 0)) << 4);
-        if (t_cbeg < t_cend) tail_load16(e, p.N, n0 + t_cbeg, t_mixed_row, t_valid, mxa);
+        if (t_cbeg < t_cend) tail_load16(e, p.N, n0 + t_cbeg, t_mixed_row, t_valid, t_live, mxa);
         // each column part stages its own bias slice and synchronises only its 4 warps (same columns, same amount
         // of work): with one 512-thread barrier per tile every part waited ~1.2 us for the slowest of the 16 warps
         const int c = t_cbeg + r;
@@ -496,14 +505,14 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
           uint32_t v[16];
           tmem_ld_32x32b_x16(taddr_row + static_cast<uint32_t>(c0), v);
           const bool second = c0 + 16 < t_cend;
-          if (second) tail_load16(e, p.N, n0 + c0 + 16, t_mixed_row, t_valid, mxb);
+          if (second) tail_load16(e, p.N, n0 + c0 + 16, t_mixed_row, t_valid, t_live, mxb);
           tmem_ld_wait();
-          tail_store16(e, p.N, n0 + c0, t_out_base, t_valid, v, sb + c0, mxa);
+          tail_store16(e, p.N, n0 + c0, t_out_base, t_valid, t_live, v, sb + c0, mxa);
           if (second && n0 + c0 + 16 < p.N) {
             tmem_ld_32x32b_x16(taddr_row + static_cast<uint32_t>(c0 + 16), v);
-            if (c0 + 32 < t_cend) tail_load16(e, p.N, n0 + c0 + 32, t_mixed_row, t_valid, mxa);
+            if (c0 + 32 < t_cend) tail_load16(e, p.N, n0 + c0 + 32, t_mixed_row, t_valid, t_live, mxa);
             tmem_ld_wait();
-            tail_store16(e, p.N, n0 + c0 + 16, t_out_base, t_valid, v, sb + c0 + 16, mxb);
+            tail_store16(e, p.N, n0 + c0 + 16, t_out_base, t_valid, t_live, v, sb + c0 + 16, mxb);
           }
         }
       } else if constexpr (EPI == EPI_LN_TMA) {

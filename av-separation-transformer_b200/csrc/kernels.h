@@ -73,7 +73,19 @@ struct GemmEpilogue {
   float* masks = nullptr;
   float* separated = nullptr;
   int F = 0, S = 0, T = 0;
+  // Variable-length batch (null: every utterance has all its rows).  ROW_PAD2PAD: rows t >= lens[b] (t = padded row - 1)
+  // are written as zeros like the halo rows.  EPI_TAIL: masks / separated are 0 for t >= lens[b] and mixed is not read
+  // there.  Values are clamped to [1, rows per utterance].
+  const int* lens = nullptr;
 };
+// Per-utterance length of a variable-length batch: lens[b] clamped to [1, L], or L when lens is null.
+__device__ __forceinline__ int utt_len(const int* lens, int b, int L) {
+  return lens == nullptr ? L : min(max(__ldg(lens + b), 1), L);
+}
+// Frame fr of N-frame utterances lies within the first lens[fr / N] frames of its utterance (always when lens is null).
+__device__ __forceinline__ bool frame_live(const int* lens, int N, int fr) {
+  return lens == nullptr || fr % N < utt_len(lens, fr / N, N);
+}
 
 // Returns nullptr on success or a static error string.
 const char* gemm_init();   // resolves cuTensorMapEncodeTiled, sets smem attributes
@@ -117,6 +129,11 @@ struct StackProblem {
   const float* mixed = nullptr;          // (B, F, L) fp32
   float *masks = nullptr, *separated = nullptr;   // (B, S, F, L) fp32
   int F = 0, S = 0;
+  // Variable-length batch (null: all L).  lens[b]: rows of utterance b that are real; its keys past them are masked,
+  // the fused decoder stores 0 there and the K | V interpolation reads lens[b] source rows.  kvp_lens[b]: the
+  // interpolation target (null: all kvp_L).  L stays the slot pitch; values are clamped to [1, L] / [1, kvp_L].
+  const int* lens = nullptr;
+  const int* kvp_lens = nullptr;
 };
 bool xformer_decoder_usable(int S, int F);
 int xformer_decoder_chunks(int S, int F);
@@ -144,8 +161,10 @@ const char* launch_xformer_stack(cudaStream_t s, const StackProblem& p, int num_
 const char* launch_add_layernorm(cudaStream_t s, int prec, const float* x, const float* y, const float* gamma,
                                  const float* beta, float* x_out, void* out_op, int M, int d);
 
-// mixed (B,F,T) fp32 -> Xp (B, T+2, Fp) operand precision, zero halo rows and zero pad columns.
-const char* launch_prep_audio(cudaStream_t s, int prec, const float* mixed, void* xp, int B, int F, int T, int Fp);
+// mixed (B,F,T) fp32 -> Xp (B, T+2, Fp) operand precision, zero halo rows and zero pad columns; lens (or null):
+// rows t >= lens[b] are zero.
+const char* launch_prep_audio(cudaStream_t s, int prec, const float* mixed, void* xp, int B, int F, int T, int Fp,
+                              const int* lens = nullptr);
 
 // SeparationDecoder.separate (model.py:210-220): out[b,s,f,t] = masks[b,s,f,t] * mixed[b,f,t] (peer_gather.cu).
 const char* launch_separate(cudaStream_t s, const float* masks, const float* mixed, float* out, long long B, int S,
@@ -167,6 +186,11 @@ struct AttnProblem {
   int B, H, hd, Lq, Lk;
   int lerp_src;                    // 0 = plain; >0 = K/V hold lerp_src source rows per utterance, interpolated to Lk rows
   int tc_mode;                     // tcgen05 kernel: 0 = never, 1 = when min(Lq, Lk) >= 96, 2 = whenever usable
+  // Variable-length batch (null: all Lk / all lerp_src).  k_lens[b]: keys of utterance b (the rest are masked; on the
+  // lerp path also the interpolation target); src_lens[b]: its interpolation source rows.  Lk / lerp_src stay the row
+  // pitch of the K/V buffers; values are clamped to [1, Lk] / [1, lerp_src].
+  const int* k_lens = nullptr;
+  const int* src_lens = nullptr;
 };
 const char* launch_attention(cudaStream_t s, int prec, const AttnProblem& p);
 // tcgen05 flash attention (attention_tc.cu): bf16, head dim 64, materialised K/V rows.  launch_attention dispatches
@@ -174,9 +198,11 @@ const char* launch_attention(cudaStream_t s, int prec, const AttnProblem& p);
 bool attention_tc_usable(int prec, const AttnProblem& p);
 bool attention_tc_wanted(int prec, const AttnProblem& p);      // usable and selected by p.tc_mode
 const char* launch_attention_tc(cudaStream_t s, const AttnProblem& p);
-// dst[b*L + t, 0:cols] (bf16) = linear interpolation (align_corners=False) of src rows [b*nsrc + i, 0:cols] (fp32)
+// dst[b*L + t, 0:cols] (bf16) = linear interpolation (align_corners=False) of src rows [b*nsrc + i, 0:cols] (fp32).
+// Variable-length batch: src_lens[b] source rows of utterance b interpolated to dst_lens[b] rows (null: nsrc / L); the
+// rows past dst_lens[b] are finite filler.
 const char* launch_lerp_rows(cudaStream_t s, const float* src, int ld_src, int B, int nsrc, int L, int cols,
-                             void* dst_bf16, int ld_dst);
+                             void* dst_bf16, int ld_dst, const int* src_lens = nullptr, const int* dst_lens = nullptr);
 
 struct CnnWeights {                // BN-folded, fragment-ordered (see visual_cnn.cu)
   const uint32_t* w1; const float* b1;
@@ -184,16 +210,17 @@ struct CnnWeights {                // BN-folded, fragment-ordered (see visual_cn
   const uint32_t* w3; const float* b3;
   const uint32_t *w1l, *w2l, *w3l;   // lo parts (fp32-grade split path), fragment-ordered like w1/w2/w3
 };
-// frames (M,H,W) fp32 -> pooled (M,128) operand precision
+// frames (M,H,W) fp32 -> pooled (M,128) operand precision.  frame_lens (variable-length batch of N-frame utterances, or
+// null): frames past an utterance's length are not read and go through the network as zero frames.
 const char* launch_visual_cnn(cudaStream_t s, int prec, const float* frames, int M, int H, int W, const CnnWeights& w,
-                              void* pooled, int num_sms);
+                              void* pooled, int num_sms, const int* frame_lens = nullptr, int N = 1);
 // tcgen05 fast path for 32x32 frames, bf16 (visual_cnn_tc.cu)
 size_t visual_cnn_tc_w2_bytes();
 size_t visual_cnn_tc_w3_bytes();
 void visual_cnn_tc_pack(const float* w2, const float* w3, uint8_t* w2_slabs, uint8_t* w3_rows);
 const char* launch_visual_cnn_tc(cudaStream_t s, const float* frames, int M, const CnnWeights& w, const uint8_t* w2_slabs,
                                  const uint8_t* w3_rows, void* pooled, int num_sms,
-                                 unsigned long long* trace = nullptr);
+                                 unsigned long long* trace = nullptr, const int* frame_lens = nullptr, int N = 1);
 size_t visual_cnn_pack_sizes(int which);   // elements of packed w1/w2/w3 (uint32)
 void visual_cnn_pack(const float* w1, const float* w2, const float* w3, uint32_t* p1, uint32_t* p2, uint32_t* p3,
                      bool lo_part = false);

@@ -35,6 +35,8 @@ struct CnnDev {
   const uint32_t* w3; const float* b3;
   const uint32_t *w1l, *w2l, *w3l;   // lo parts (w - bf16(w)) for the fp32-grade split path
   int M, H, W, H1, W1, H2, W2, H3, W3, G, num_groups;
+  const int* frame_lens;             // variable-length batch: frames past an utterance's length are staged as zeros
+  int N;                             // frames per utterance (pitch of frame_lens)
 };
 
 __device__ __forceinline__ void mma16816(float (&c)[4], uint32_t a0, uint32_t a1, uint32_t a2, uint32_t a3,
@@ -121,7 +123,7 @@ __global__ void __launch_bounds__(CNN_THREADS, 1) visual_cnn_kernel(const CnnDev
         const int rem = i - g * per;
         const int y = rem / p.W, x = rem - y * p.W;
         const int fr = frame0 + g;
-        const float val = fr < p.M ? __ldg(p.frames + static_cast<size_t>(fr) * per + rem) : 0.f;
+        const float val = fr < p.M && frame_live(p.frame_lens, p.N, fr) ? __ldg(p.frames + static_cast<size_t>(fr) * per + rem) : 0.f;
         sIn[g * in_words + (y + 1) * Wp + (x + 1)] = val;
       }
     }
@@ -436,10 +438,11 @@ void visual_cnn_pack(const float* w1, const float* w2, const float* w3, uint32_t
 }
 
 const char* launch_visual_cnn(cudaStream_t s, int prec, const float* frames, int M, int H, int W, const CnnWeights& w,
-                              void* pooled, int num_sms) {
+                              void* pooled, int num_sms, const int* frame_lens, int N) {
   if (M <= 0 || H <= 0 || W <= 0) return "visual_cnn: empty problem";
   CnnDev d;
   d.frames = frames; d.pooled = pooled;
+  d.frame_lens = frame_lens; d.N = N;
   d.w1 = w.w1; d.b1 = w.b1; d.w2 = w.w2; d.b2 = w.b2; d.w3 = w.w3; d.b3 = w.b3;
   d.w1l = w.w1l; d.w2l = w.w2l; d.w3l = w.w3l;
   const bool split = (prec == PREC_TF32);

@@ -48,6 +48,8 @@ struct CnnTcDev {
   const uint8_t* w2_slabs; const float* b2;
   const float* b3;
   int M, num_groups;
+  const int* frame_lens;       // variable-length batch: frames past an utterance's length are staged as zeros
+  int N;                       // frames per utterance (pitch of frame_lens)
   unsigned long long* trace;   // optional [grid][64] globaltimer stamps of the CTA's 2nd group (debug), else null
 };
 
@@ -238,7 +240,7 @@ visual_cnn_tc_kernel(const __grid_constant__ CUtensorMap tmW3, const CnnTcDev p)
         const int f = id >> 8, rem = id & 255;
         const int fr = first_frame + f;
         pre[i] = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (fr < p.M) pre[i] = __ldg(reinterpret_cast<const float4*>(p.frames + static_cast<size_t>(fr) * 1024) + rem);
+        if (fr < p.M && frame_live(p.frame_lens, p.N, fr)) pre[i] = __ldg(reinterpret_cast<const float4*>(p.frames + static_cast<size_t>(fr) * 1024) + rem);
       }
     };
     // hand a finished slab to the MMA issuer
@@ -485,7 +487,8 @@ void visual_cnn_tc_pack(const float* w2, const float* w3, uint8_t* w2_slabs, uin
 }
 
 const char* launch_visual_cnn_tc(cudaStream_t s, const float* frames, int M, const CnnWeights& w, const uint8_t* w2_slabs,
-                                 const uint8_t* w3_rows, void* pooled, int num_sms, unsigned long long* trace) {
+                                 const uint8_t* w3_rows, void* pooled, int num_sms, unsigned long long* trace,
+                                 const int* frame_lens, int N) {
   if (M <= 0) return "visual_cnn_tc: empty problem";
   static PFN_cuTensorMapEncodeTiled_v12000 encode = nullptr;
   if (encode == nullptr) {
@@ -516,6 +519,7 @@ const char* launch_visual_cnn_tc(cudaStream_t s, const float* frames, int M, con
   d.w1 = w.w1; d.b1 = w.b1; d.w2_slabs = w2_slabs; d.b2 = w.b2; d.b3 = w.b3;
   d.M = M; d.num_groups = (M + GROUP - 1) / GROUP;
   d.trace = trace;
+  d.frame_lens = frame_lens; d.N = N;
   const int grid = d.num_groups < num_sms ? d.num_groups : num_sms;
   launch_pdl(visual_cnn_tc_kernel, dim3(grid), dim3(TC_THREADS), TC_SMEM, s, tm, d);
   return cudaGetLastError() == cudaSuccess ? nullptr : "visual_cnn_tc: launch failed";

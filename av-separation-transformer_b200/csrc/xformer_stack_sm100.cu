@@ -96,6 +96,8 @@ struct StackDev {
   int kvp_chunks, kvp_L, kvp_ld;
   float kvp_scale;              // L / kvp_L
   __nv_bfloat16* kvp_out;
+  // variable-length batch (null: all L / all kvp_L): rows of each utterance that are real, K | V interpolation targets
+  const int *lens, *kvp_lens;
   long long* trace;             // optional [grid][256] clock64 stamps of the CTA's first tile (debug), else null:
                                 //   row thread (warp 2 lane 0) in [0,128), MMA thread in [128,256); see tools/stack_trace.py
 };
@@ -131,11 +133,16 @@ __device__ __forceinline__ float ex2_approx(float x) {
   return y;
 }
 
+// VARLEN = false (no length arrays): every per-utterance length is p.L / p.kvp_L at compile time, so the uniform
+// batch runs exactly the code it ran before variable-length batches existed.
+template <bool VARLEN>
 __global__ void __launch_bounds__(STACK_THREADS, 1)
 xformer_stack_kernel(const __grid_constant__ CUtensorMap tmXin, const __grid_constant__ CUtensorMap tmXout,
                      const __grid_constant__ CUtensorMap tmOp, const __grid_constant__ CUtensorMap tmKV,
                      const StackDev p) {
   extern __shared__ __align__(1024) uint8_t smem_stack[];
+  const int* const lens = VARLEN ? p.lens : nullptr;
+  const int* const kvp_lens = VARLEN ? p.kvp_lens : nullptr;
   uint8_t* const smem = smem_stack;
   if ((smem_u32(smem) & 1023u) != 0) __trap();
   uint64_t* bars = reinterpret_cast<uint64_t*>(smem + OFF_BAR);
@@ -593,11 +600,11 @@ xformer_stack_kernel(const __grid_constant__ CUtensorMap tmXin, const __grid_con
     const int etid = threadIdx.x - 64;                       // 0..511
     const uint32_t lane_sel = static_cast<uint32_t>(q * 32) << 16;
     const bool elected = (warp == 2 + 4 * part) && (lane == 0);
-    // block-diagonal attention: row r attends the keys [klo, klo + L) of its own utterance slot
+    // block-diagonal attention: row r attends the keys [klo, klo + lk) of its own utterance slot (lk: per tile below)
     const int klo = (r / p.stride) * p.stride;
-    const bool row_valid = (r - klo) < p.L;                  // tile rows past the utterance's length are padding
-    // this row's valid score columns within the part: [lo_i, hi_i)
-    const int lo_i = klo - part * 32, hi_i = klo + p.L - part * 32;
+    const bool row_valid = (r - klo) < p.L;                  // tile rows past the slot pitch are padding
+    // this row's valid score columns within the part start at lo_i
+    const int lo_i = klo - part * 32;
     // stream items per tile: input projection | layers | decoder block or K|V projection block
     const uint32_t per_tile = static_cast<uint32_t>(n_pro + p.n_layers * p.items_per_layer + (p.decoder ? 1 + 8 + 4 * p.nc3 : 0) +
                                                     (p.kvp_chunks ? 1 + 2 * p.kvp_chunks : 0));
@@ -688,6 +695,9 @@ xformer_stack_kernel(const __grid_constant__ CUtensorMap tmXin, const __grid_con
     int lt = 0;
     for (int tile = blockIdx.x; tile < p.n_tiles; tile += gridDim.x, ++lt) {
       const int utt0 = tile * p.U;
+      // keys of this row's utterance (p.L unless the batch has per-utterance lengths); the rows of the slot in
+      // [lk, L) are computed like any other row but no row attends to them
+      const int lk = VARLEN ? utt_len(lens, min(utt0 + r / p.stride, p.B - 1), p.L) : p.L;
       // ---- residual tile: staging slabs (fp32, 32 columns each) -> tensor memory ----
       XTRACE(0);
       if (!p.pro_taps) {
@@ -847,8 +857,8 @@ xformer_stack_kernel(const __grid_constant__ CUtensorMap tmXin, const __grid_con
           XTRACE(th + 2);                                    // S complete
           if (p.stride == 64) {
             // two utterance slots of 64 rows: the row's 64 candidate keys split into four 16-column parts, so that all
-            // 16 row warps work (columns klo + 16 part .. +16; valid while < klo + L)
-            const int nval = p.L - part * 16;                // valid columns of this part: [0, nval)
+            // 16 row warps work (columns klo + 16 part .. +16; valid while < klo + lk)
+            const int nval = lk - part * 16;                 // valid columns of this part: [0, nval)
             uint32_t s[16];
             tmem_ld_32x32b_x16(tmW + lane_sel + TW_S + klo + part * 16, s);
             tmem_ld_wait();
@@ -885,6 +895,7 @@ xformer_stack_kernel(const __grid_constant__ CUtensorMap tmXin, const __grid_con
             __syncwarp();
             if (lane == 0) mbar_arrive(p_ready);
           } else {
+            const int hi_i = lo_i + lk;                      // valid score columns within the part: [lo_i, hi_i)
             const bool any = __any_sync(0xffffffffu, (lo_i < 32) && (hi_i > 0));
             float e[32];
             float mx = -INFINITY, sum = 0.f;
@@ -1040,6 +1051,7 @@ xformer_stack_kernel(const __grid_constant__ CUtensorMap tmXin, const __grid_con
         // live set (two mixture buffers, 16 accumulator values, S + S running pointers) stays inside the 96 registers.
         const int utt = utt0 + r / p.stride, t = r - klo;
         const bool out_ok = row_valid && utt < p.B;
+        const bool live = !VARLEN || t < lk;               // past the utterance's length: masks = separated = 0
         const int Lp = p.L;
         const size_t obase = static_cast<size_t>(out_ok ? utt : 0) * p.SF * Lp + t;
         float* const mo_u = p.masks + obase;
@@ -1053,7 +1065,7 @@ xformer_stack_kernel(const __grid_constant__ CUtensorMap tmXin, const __grid_con
           auto load_mx = [&](float (&mx)[G], int f0) {         // mixture values of bins [f0, f0 + G)
             const float* q = mx_u + f0 * Lp;
 #pragma unroll
-            for (int j = 0; j < G; ++j, q += Lp) mx[j] = (out_ok && f0 + j < p.F) ? __ldg(q) : 0.f;
+            for (int j = 0; j < G; ++j, q += Lp) mx[j] = (out_ok && live && f0 + j < p.F) ? __ldg(q) : 0.f;
           };
           auto store_half = [&](const uint32_t (&v)[16], const float (&mx)[G], int f0, int col) {
             if (!out_ok || f0 >= p.F) return;
@@ -1065,7 +1077,7 @@ xformer_stack_kernel(const __grid_constant__ CUtensorMap tmXin, const __grid_con
               for (int j = 0; j < G; ++j, mo += Lp, so += Lp) {
 #pragma unroll
                 for (int sp = 0; sp < S; ++sp) {
-                  const float mk = sigmoid_fast(__uint_as_float(v[j * S + sp]) + b3[j * S + sp]);
+                  const float mk = live ? sigmoid_fast(__uint_as_float(v[j * S + sp]) + b3[j * S + sp]) : 0.f;
                   __stcs(mo + sp * FL, mk);
                   __stcs(so + sp * FL, mk * mx[j]);
                 }
@@ -1076,7 +1088,7 @@ xformer_stack_kernel(const __grid_constant__ CUtensorMap tmXin, const __grid_con
                 if (f0 + j < p.F) {
 #pragma unroll
                   for (int sp = 0; sp < S; ++sp) {
-                    const float mk = sigmoid_fast(__uint_as_float(v[j * S + sp]) + b3[j * S + sp]);
+                    const float mk = live ? sigmoid_fast(__uint_as_float(v[j * S + sp]) + b3[j * S + sp]) : 0.f;
                     __stcs(mo + sp * FL, mk);
                     __stcs(so + sp * FL, mk * mx[j]);
                   }
@@ -1132,10 +1144,16 @@ xformer_stack_kernel(const __grid_constant__ CUtensorMap tmXin, const __grid_con
         {
           const int t = r - klo;
           const bool live = t < p.kvp_L;
-          const float sp = fmaxf(p.kvp_scale * (static_cast<float>(t) + 0.5f) - 0.5f, 0.0f);
+          // a short utterance: lk source rows interpolated to its own target length (the rows past that target are
+          // finite and masked as keys by the fusion stack)
+          const float scale = lens == nullptr && kvp_lens == nullptr
+                                  ? p.kvp_scale
+                                  : static_cast<float>(lk) /
+                                        static_cast<float>(utt_len(kvp_lens, min(utt0 + r / p.stride, p.B - 1), p.kvp_L));
+          const float sp = fmaxf(scale * (static_cast<float>(t) + 0.5f) - 0.5f, 0.0f);
           int i0 = static_cast<int>(sp);
-          if (i0 > p.L - 1) i0 = p.L - 1;
-          const int i1 = min(i0 + 1, p.L - 1);
+          if (i0 > lk - 1) i0 = lk - 1;
+          const int i1 = min(i0 + 1, lk - 1);
           const float w1 = sp - static_cast<float>(i0), w0 = 1.0f - w1;
           const int r0 = klo + i0, r1 = klo + i1;
           uint8_t* slab = smem + OFF_A + part * SLAB;
@@ -1472,7 +1490,8 @@ const char* launch_xformer_stack(cudaStream_t s, const StackProblem& sp, int num
     if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres) != cudaSuccess ||
         qres != cudaDriverEntryPointSuccess || fn == nullptr)
       return "xformer_stack: cuTensorMapEncodeTiled entry point not found";
-    if (cudaFuncSetAttribute(xformer_stack_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, STACK_SMEM) != cudaSuccess)
+    if (cudaFuncSetAttribute(xformer_stack_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, STACK_SMEM) != cudaSuccess ||
+        cudaFuncSetAttribute(xformer_stack_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, STACK_SMEM) != cudaSuccess)
       return "xformer_stack: cudaFuncSetAttribute failed";
     g_enc = reinterpret_cast<PFN_cuTensorMapEncodeTiled_v12000>(fn);
   }
@@ -1510,11 +1529,13 @@ const char* launch_xformer_stack(cudaStream_t s, const StackProblem& sp, int num
   d.kvp_chunks = kvp ? sp.kvp_n / 128 : 0; d.kvp_L = sp.kvp_L; d.kvp_ld = sp.kvp_ld;
   d.kvp_scale = kvp ? static_cast<float>(sp.L) / static_cast<float>(sp.kvp_L) : 0.f;
   d.kvp_out = static_cast<__nv_bfloat16*>(sp.kvp_out);
+  d.lens = sp.lens; d.kvp_lens = kvp ? sp.kvp_lens : nullptr;
   d.decoder = decoder ? 1 : 0;
   d.SF = sp.S * sp.F; d.F = sp.F; d.S = sp.S; d.nc3 = decoder ? xformer_decoder_chunks(sp.S, sp.F) : 0;
   d.mixed = sp.mixed; d.masks = sp.masks; d.separated = sp.separated;
   const int grid = n_tiles < num_sms ? n_tiles : num_sms;
-  if (launch_pdl(xformer_stack_kernel, dim3(grid), dim3(STACK_THREADS), STACK_SMEM, s, tin, tout, top, tkv, d) !=
+  auto kern = (d.lens != nullptr || d.kvp_lens != nullptr) ? xformer_stack_kernel<true> : xformer_stack_kernel<false>;
+  if (launch_pdl(kern, dim3(grid), dim3(STACK_THREADS), STACK_SMEM, s, tin, tout, top, tkv, d) !=
       cudaSuccess) {
     cudaGetLastError();
     return "xformer_stack: launch failed";

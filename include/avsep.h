@@ -75,6 +75,18 @@ AVSEP_API int avsep_forward(avsep_handle* h, const float* mixed_spec, const floa
                   int32_t Hh, int32_t Ww, float* separated, float* masks, void* workspace, size_t workspace_bytes,
                   void* cuda_stream);
 
+/* Variable-length batch.  mixed_spec (B,F,T), lip_frames (B,N,Hh,Ww) hold each utterance left-aligned in the
+ * first lengths[b] frames / frame_lengths[b] lip frames; T and N are the batch maxima.  lengths, frame_lengths:
+ * DEVICE int32 [B], or NULL for "all T" / "all N".  For each b the outputs [b, :, :, :lengths[b]] equal the
+ * outputs of avsep_forward on that utterance alone at (lengths[b], frame_lengths[b]); [b, :, :, lengths[b]:] are 0
+ * in both separated and masks.  Input values past the lengths are never read (NaN there is harmless).
+ * Lengths are read on the device (no host sync; a captured graph replays with whatever the buffers hold then);
+ * values outside [1, T] / [1, N] behave as the nearest bound.  Workspace: avsep_workspace_bytes(B, T, N, Hh, Ww). */
+AVSEP_API int avsep_forward_varlen(avsep_handle* h, const float* mixed_spec, const float* lip_frames,
+                                   const int32_t* lengths, const int32_t* frame_lengths, int32_t B, int32_t T,
+                                   int32_t N, int32_t Hh, int32_t Ww, float* separated, float* masks,
+                                   void* workspace, size_t workspace_bytes, void* cuda_stream);
+
 /* Same call with HOST buffers (pinned memory recommended): H2D copies, forward and D2H copies are issued on
  * the stream and the call returns after the results have landed (the e2e path of bench.py). */
 AVSEP_API int avsep_forward_host(avsep_handle* h, const float* mixed_spec, const float* lip_frames, int32_t B, int32_t T,
