@@ -9,6 +9,7 @@
 #include <stdlib.h>
 #include <string.h>
 
+#include <functional>
 #include <map>
 #include <string>
 #include <vector>
@@ -78,13 +79,11 @@ struct HostTensor {
   std::vector<int64_t> shape;
 };
 
-struct EncLayerW {
-  const void *wqkv, *wo, *w1, *w2;
-  const float *bqkv, *bo, *b1, *b2, *n1g, *n1b, *n2g, *n2b;
-};
-struct FusLayerW {
-  const void *wq, *wo, *w1, *w2;
-  const float *bq, *bo, *b1, *b2, *n1g, *n1b, *n2g, *n2b;
+// One encoder or fusion layer on the device.  w_in / b_in: the attention input projection, Q|K|V rows in an encoder
+// layer, Q rows only in a fusion layer (the K|V rows of all fusion layers are one concatenated matrix).
+struct LayerW {
+  const void *w_in, *wo, *w1, *w2;
+  const float *b_in, *bo, *b1, *b2, *n1g, *n1b, *n2g, *n2b;
 };
 
 struct Workspace {   // carved from one base pointer; all offsets 1 KB aligned
@@ -128,8 +127,7 @@ struct avsep_handle {
   const float *pe_a = nullptr, *pe_v = nullptr, *fng = nullptr, *fnb = nullptr;
   CnnWeights cnn{};
   const uint8_t *cnn_w2_slabs = nullptr, *cnn_w3_rows = nullptr;   // tcgen05 CNN operands
-  std::vector<EncLayerW> enc_a, enc_v;
-  std::vector<FusLayerW> fus;
+  std::vector<LayerW> enc_a, enc_v, fus;
   // prepacked weight streams / vector blocks of the fused transformer-stack kernel (null when the config cannot use it)
   const uint8_t *xs_a = nullptr, *xs_v = nullptr, *xs_f = nullptr;
   bool xs_f_decoder = false;   // the fusion stream continues with the SeparationDecoder block
@@ -311,11 +309,16 @@ const char* run_visual_cnn(avsep_handle* h, cudaStream_t s, const float* frames,
   return launch_visual_cnn(s, h->cfg.precision, frames, M, Hh, Ww, h->cnn, pooled, h->num_sms, frame_lens, N);
 }
 
+// out[M, N] = A[M, K] W[N, K]^T: one tap, densely packed operands
+GemmProblem dense(const void* A, int M, int K, const void* W, int N) {
+  GemmProblem p{};
+  p.A = A; p.lda = K; p.rowsA = M; p.M = M; p.W = W; p.ldw = K; p.N = N; p.K = K; p.taps = 1;
+  return p;
+}
+
 int linear(avsep_handle* h, cudaStream_t s, const char* label, const void* A, int M, int K, const void* W,
            const float* bias, int N, int act, float* out_f32, void* out_op) {
-  GemmProblem p{};
-  p.A = A; p.lda = K; p.rowsA = M; p.M = M; p.W = W; p.ldw = K; p.N = N; p.K = K;
-  p.taps = 1; p.tap_stride = 0; p.row_shift = 0;
+  const GemmProblem p = dense(A, M, K, W, N);
   GemmEpilogue e;
   e.bias = bias; e.act = act;
   // a GELU whose only consumer is a bf16 operand does not need the fp32-grade erf
@@ -359,43 +362,54 @@ int gemm_resid_ln(avsep_handle* h, cudaStream_t s, const char* label, const Gemm
 
 int linear_resid_ln(avsep_handle* h, cudaStream_t s, const char* label, const void* A, int M, int K, const void* W,
                     const float* bias, int N, float* x, const float* g, const float* b, void* out_op, float* y) {
-  GemmProblem p{};
-  p.A = A; p.lda = K; p.rowsA = M; p.M = M; p.W = W; p.ldw = K; p.N = N; p.K = K; p.taps = 1;
   GemmEpilogue e;
   e.bias = bias;
-  return gemm_resid_ln(h, s, label, p, e, x, x, g, b, out_op, M, y);
+  return gemm_resid_ln(h, s, label, dense(A, M, K, W, N), e, x, x, g, b, out_op, M, y);
 }
 
 bool stack_fusable(const avsep_handle* h, int len) {
   return h->xs_a != nullptr && xformer_stack_usable(h->cfg.precision, h->cfg.d_model, h->cfg.nhead, len);
 }
 
-// A whole stack in one kernel (xformer_stack_sm100.cu).  which: 0 audio encoder, 1 visual encoder, 2 fusion.
-int run_stack(avsep_handle* h, cudaStream_t s, int which, const float* x_in, float* out_x, void* out_op,
-              const float* fin_g, const float* fin_b, const void* kv, int kv_ld, int B, int L, long long* trace = nullptr,
-              const float* mixed = nullptr, float* separated = nullptr, float* masks = nullptr, const void* pro_a = nullptr,
-              void* kvp_out = nullptr, int kvp_L = 0, const int* lens = nullptr, const int* kvp_lens = nullptr) {
-  StackProblem sp{};
-  sp.trace = trace;
-  sp.lens = lens; sp.kvp_lens = kvp_lens;
-  if (kvp_out != nullptr) {      // which 1: the fusion layers' K | V rows are produced inside the kernel
-    sp.kvp_out = kvp_out; sp.kvp_L = kvp_L; sp.kvp_n = h->cfg.num_fusion_layers * 2 * h->cfg.d_model; sp.kvp_ld = sp.kvp_n;
-  }
-  if (pro_a != nullptr) {        // x_in is produced inside the kernel (which 0: Conv1d #2 + ReLU + PE; 1: frame_proj + PE)
-    sp.pro_a = pro_a; sp.pro_relu = which == 0;
-    sp.pro_taps = which == 0 ? 3 : 1; sp.pro_k = which == 0 ? h->cfg.d_model : 128;
-    sp.pro_pitch = which == 0 ? L + 2 : L; sp.pro_rows = B * sp.pro_pitch;
-    sp.pe = which == 0 ? h->pe_a : h->pe_v;
-  }
-  sp.mixed = mixed; sp.separated = separated; sp.masks = masks; sp.F = h->cfg.freq_bins; sp.S = h->cfg.num_speakers;
-  sp.x_in = x_in; sp.out_x = out_x; sp.out_op = out_op; sp.fin_gamma = fin_g; sp.fin_beta = fin_b;
-  sp.wstream = which == 0 ? (pro_a ? h->xs_a : h->xs_a_np) : which == 1 ? (pro_a ? h->xs_v : h->xs_v_np) : h->xs_f;
+// Which kernels a forward of T audio and N lip frames per utterance launches.  Computed on every call: set_debug,
+// set_profile and set_option change it.  A default Plan is the per-layer path of the sub-module entry points.
+struct Plan {
+  bool stack_a = false, stack_v = false;   // the audio / visual encoder stack in one kernel, else per-layer kernels
+  bool stack_f = false;   // the fusion stack in one kernel (it reads the fp32 residual rows of both encoders)
+  bool pro = false;       // the encoder stack kernels also run the input projection (Conv1d #2 / frame_proj, + PE)
+  bool kvp = false;       // the visual stack kernel also writes the fusion layers' K|V rows
+  bool dec = false;       // the fusion stack kernel also runs the SeparationDecoder
+  bool fork = false;      // audio and visual branches on two streams (fork / join), so that partial waves overlap
+};
+
+Plan forward_plan(const avsep_handle* h, int T, int N) {
+  Plan p;
+  p.stack_a = stack_fusable(h, T);
+  p.stack_v = stack_fusable(h, N);
+  p.stack_f = p.stack_a && p.stack_v;
+  // stage snapshots (debug) read the embeddings, the K|V rows and the fused rows from memory
+  p.pro = !h->debug;
+  // the fused K|V projection needs the audio frames inside a visual tile slot
+  p.kvp = p.stack_f && h->xs_v_kvp && !h->debug &&
+          xformer_kvp_usable(h->cfg.num_fusion_layers * 2 * h->cfg.d_model, N, T);
+  p.dec = p.stack_f && h->xs_f_decoder && !h->debug;
+  // per-kernel profiling and stage snapshots need a single ordered stream
+  p.fork = h->two_stream && !h->profile && !h->debug;
+  return p;
+}
+
+// A whole stack in one kernel (xformer_stack_sm100.cu).  which: 0 audio encoder, 1 visual encoder, 2 fusion.  The
+// caller sets the buffers and the optional stages of `sp`; this fills what follows from the stack: the weight stream
+// (from the input-projection items on when sp.pro_a is set), layer count, attention kind, activation, decoder geometry.
+int run_stack(avsep_handle* h, cudaStream_t s, int which, StackProblem sp) {
+  const bool pro = sp.pro_a != nullptr;
+  sp.wstream = which == 0 ? (pro ? h->xs_a : h->xs_a_np) : which == 1 ? (pro ? h->xs_v : h->xs_v_np) : h->xs_f;
   sp.n_layers = which == 2 ? h->cfg.num_fusion_layers : h->cfg.num_encoder_layers;
   sp.cross = which == 2;
-  sp.kv = kv; sp.kv_ld = kv_ld;
-  sp.B = B; sp.L = L;
-  sp.act = which == 2 ? ACT_GELU : ACT_RELU;
-  CKL(which == 0 ? "layer.audio_enc" : which == 1 ? "layer.visual_enc" : masks ? "layer.fusion_decoder" : "layer.fusion",
+  if (sp.cross) sp.kv_ld = sp.n_layers * 2 * h->cfg.d_model;
+  sp.act = sp.cross ? ACT_GELU : ACT_RELU;
+  sp.F = h->cfg.freq_bins; sp.S = h->cfg.num_speakers;
+  CKL(which == 0 ? "layer.audio_enc" : which == 1 ? "layer.visual_enc" : sp.masks ? "layer.fusion_decoder" : "layer.fusion",
       launch_xformer_stack(s, sp, h->num_sms));
   return 0;
 }
@@ -404,17 +418,29 @@ int run_stack(avsep_handle* h, cudaStream_t s, int which, const float* x_in, flo
 // pair spreads over more CTAs and wins.
 constexpr int FFN_FUSED_MIN_ROWS = 2048;
 
+// Feed-forward sub-layer of layer w: x += W2 act(W1 a_op + b1) + b2; a_op = LN_{g,b}(x).  ffn [M, 4d], y [M, d]: scratch.
+int ffn_sublayer(avsep_handle* h, cudaStream_t s, const LayerW& w, int act, int M, float* x, void* a_op, void* ffn,
+                 float* y, const float* g, const float* b) {
+  const int d = h->cfg.d_model;
+  if (ffn_fusable(h->cfg.precision, d) && M >= FFN_FUSED_MIN_ROWS) {
+    CKL("ffn.fused", launch_ffn_fused(s, a_op, w.w1, w.b1, w.w2, w.b2, act, x, x, g, b, a_op, M, h->num_sms, nullptr));
+    return 0;
+  }
+  if (linear(h, s, "gemm.ffn1", a_op, M, d, w.w1, w.b1, 4 * d, act, nullptr, ffn)) return 1;
+  return linear_resid_ln(h, s, "gemm.ffn2", ffn, M, 4 * d, w.w2, w.b2, d, x, g, b, a_op, y);
+}
+
 // nn.TransformerEncoderLayer x L (pre-norm, ReLU FFN; model.py:48-52,59; torch transformer.py:946-950).
 // In: x (fp32 residual stream), a_op = LN_{layer0.norm1}(x).  Out: x, a_op = LN_{final}(x) (or cast when final_g == null).
 // lens: keys per utterance of a variable-length batch, or null.
-int encoder_stack(avsep_handle* h, cudaStream_t s, const std::vector<EncLayerW>& layers, int B, int L, float* x,
+int encoder_stack(avsep_handle* h, cudaStream_t s, const std::vector<LayerW>& layers, int B, int L, float* x,
                   float* y, void* a_op, void* qkv, void* attn, void* ffn, const float* final_g, const float* final_b,
                   const int* lens = nullptr) {
   const int d = h->cfg.d_model, H = h->cfg.nhead, M = B * L, prec = h->cfg.precision;
   const size_t os = op_size(h);
   for (size_t l = 0; l < layers.size(); ++l) {
-    const EncLayerW& w = layers[l];
-    if (linear(h, s, "gemm.qkv", a_op, M, d, w.wqkv, w.bqkv, 3 * d, ACT_NONE, nullptr, qkv)) return 1;
+    const LayerW& w = layers[l];
+    if (linear(h, s, "gemm.qkv", a_op, M, d, w.w_in, w.b_in, 3 * d, ACT_NONE, nullptr, qkv)) return 1;
     AttnProblem ap{};
     ap.q = qkv; ap.ldq = 3 * d;
     ap.k = static_cast<const uint8_t*>(qkv) + static_cast<size_t>(d) * os;
@@ -426,24 +452,18 @@ int encoder_stack(avsep_handle* h, cudaStream_t s, const std::vector<EncLayerW>&
     CKL("attn.self", launch_attention(s, prec, ap));
     if (linear_resid_ln(h, s, "gemm.out_proj", attn, M, d, w.wo, w.bo, d, x, w.n2g, w.n2b, a_op, y)) return 1;
     const bool last = (l + 1 == layers.size());
-    const float* g = last ? final_g : layers[l + 1].n1g;
-    const float* b = last ? final_b : layers[l + 1].n1b;
-    if (ffn_fusable(prec, d) && M >= FFN_FUSED_MIN_ROWS) {
-      CKL("ffn.fused", launch_ffn_fused(s, a_op, w.w1, w.b1, w.w2, w.b2, ACT_RELU, x, x,
-                                                                             g, b, a_op, M, h->num_sms, nullptr));
-    } else {
-      if (linear(h, s, "gemm.ffn1", a_op, M, d, w.w1, w.b1, 4 * d, ACT_RELU, nullptr, ffn)) return 1;
-      if (linear_resid_ln(h, s, "gemm.ffn2", ffn, M, 4 * d, w.w2, w.b2, d, x, g, b, a_op, y)) return 1;
-    }
+    if (ffn_sublayer(h, s, w, ACT_RELU, M, x, a_op, ffn, y, last ? final_g : layers[l + 1].n1g,
+                     last ? final_b : layers[l + 1].n1b))
+      return 1;
   }
   return 0;
 }
 
 // AudioEncoder up to (not including) the transformer: Conv1d+ReLU x2, +PE (model.py:56-58), then the first
-// layer's LayerNorm: x_a (fp32) and a_op = LN_{g,b}(x_a).
-// x_only: the fused stack kernel computes the first LayerNorm itself, so only the fp32 residual rows are written.
-int audio_frontend(avsep_handle* h, cudaStream_t s, Workspace& w, const float* mixed, const float* g, const float* b,
-                   bool x_only = false, bool conv1_only = false) {
+// layer's LayerNorm: x_a (fp32) and a_op = LN_{layer0.norm1}(x_a).
+// pl.stack_a: the stack kernel computes the first LayerNorm itself, so only the fp32 residual rows are written, and with
+// pl.pro it runs Conv1d #2 + ReLU + PE too, on h1.
+int audio_frontend(avsep_handle* h, cudaStream_t s, Workspace& w, const float* mixed, const Plan& pl) {
   h->prof_stream = s;
   const int d = h->cfg.d_model, F = h->cfg.freq_bins, B = w.B, T = w.T, prec = h->cfg.precision;
   const int Map = B * (T + 2);
@@ -458,7 +478,7 @@ int audio_frontend(avsep_handle* h, cudaStream_t s, Workspace& w, const float* m
     e.out_op = w.h1; e.ld_op = d;
     CKL("gemm.conv1d_0", launch_gemm(s, prec, p, e));
   }
-  if (conv1_only) return 0;      // Conv1d #2 + ReLU + PE run inside the encoder stack kernel, on h1
+  if (pl.stack_a && pl.pro) return 0;
   {
     GemmProblem p{};
     p.A = w.h1; p.lda = d; p.rowsA = Map; p.M = Map; p.W = h->wc2; p.ldw = 3 * d; p.N = d; p.K = d;
@@ -466,10 +486,11 @@ int audio_frontend(avsep_handle* h, cudaStream_t s, Workspace& w, const float* m
     GemmEpilogue e;
     e.bias = h->bc2; e.act = ACT_RELU; e.rowmap = ROW_PAD2COMPACT; e.Lp = T + 2;
     e.pe = h->pe_a;
-    if (x_only) {
+    if (pl.stack_a) {
       e.out_f32 = w.x_a; e.ld_f32 = d;
       CKL("gemm.conv1d_2", launch_gemm(s, prec, p, e));
-    } else if (gemm_resid_ln(h, s, "gemm.conv1d_2", p, e, nullptr, w.x_a, g, b, w.a_op, B * T, w.y_a)) {
+    } else if (gemm_resid_ln(h, s, "gemm.conv1d_2", p, e, nullptr, w.x_a, h->enc_a[0].n1g, h->enc_a[0].n1b, w.a_op,
+                             B * T, w.y_a)) {
       return 1;
     }
   }
@@ -477,55 +498,55 @@ int audio_frontend(avsep_handle* h, cudaStream_t s, Workspace& w, const float* m
 }
 
 // VisualEncoder up to (not including) the transformer: CNN, pool, frame_proj, +PE (model.py:106-110), then the
-// first layer's LayerNorm: x_v (fp32) and v_op = LN_{g,b}(x_v).
-int visual_frontend(avsep_handle* h, cudaStream_t s, Workspace& w, const float* frames, const float* g, const float* b,
-                    bool x_only = false, bool cnn_only = false) {
+// first layer's LayerNorm: x_v (fp32) and v_op = LN_{layer0.norm1}(x_v).  pl.stack_v / pl.pro as in audio_frontend.
+int visual_frontend(avsep_handle* h, cudaStream_t s, Workspace& w, const float* frames, const Plan& pl) {
   h->prof_stream = s;
   const int d = h->cfg.d_model, B = w.B, N = w.N;
   const int Mv = B * N;
   CKL("visual_cnn", run_visual_cnn(h, s, frames, Mv, w.Hh, w.Ww, w.pooled, nullptr, w.frame_lens, N));
   if (snapshot(h, s, "visual_pool", w.pooled, static_cast<size_t>(Mv) * 128, true)) return 1;
-  if (cnn_only) return 0;        // frame_proj + PE run inside the encoder stack kernel, on the pooled features
-  GemmProblem p{};
-  p.A = w.pooled; p.lda = 128; p.rowsA = Mv; p.M = Mv; p.W = h->wproj; p.ldw = 128; p.N = d; p.K = 128;
-  p.taps = 1;
+  if (pl.stack_v && pl.pro) return 0;
+  const GemmProblem p = dense(w.pooled, Mv, 128, h->wproj, d);
   GemmEpilogue e;
   e.bias = h->bproj; e.pe = h->pe_v; e.pe_period = N;
-  if (x_only) {
+  if (pl.stack_v) {
     e.out_f32 = w.x_v; e.ld_f32 = d;
     CKL("gemm.frame_proj", launch_gemm(s, h->cfg.precision, p, e));
-  } else if (gemm_resid_ln(h, s, "gemm.frame_proj", p, e, nullptr, w.x_v, g, b, w.v_op, Mv, w.y_v)) {
+  } else if (gemm_resid_ln(h, s, "gemm.frame_proj", p, e, nullptr, w.x_v, h->enc_v[0].n1g, h->enc_v[0].n1b, w.v_op, Mv,
+                           w.y_v)) {
     return 1;
   }
   return snapshot(h, s, "visual_embed", w.x_v, static_cast<size_t>(Mv) * d, false);
 }
 
-// CrossModalFusion (model.py:145-149,166-173).  In: x_a residual stream, a_op = LN_{layer0.norm1}(x_a),
-// v_op = visual rows (L_src per utterance).  Out: a_op = fusion.norm(x) in operand precision.
-// Fused variant (stack_fusable(T)): the visual rows are interpolated to the audio frame rate first, exactly where the
-// reference does it (model.py:114-116, before the K/V projection), the K|V rows of every fusion layer come from one GEMM
-// on those T rows (bf16), and the whole fusion stack runs in one kernel.  In: x_a (fp32 residual), x_v (fp32 visual
-// encoder output, L_src rows per utterance).  Out: a_op = fusion.norm(x) in bf16.
-// with_decoder (out: *decoded = true): SeparationDecoder runs inside the same kernel and writes separated / masks.
-int fusion_stack_fused(avsep_handle* h, cudaStream_t s, Workspace& w, int L_src, const float* mixed, float* separated,
-                       float* masks, bool* decoded, bool have_kv = false) {
+// CrossModalFusion (model.py:145-149,166-173) as one kernel: the visual rows are interpolated to the audio frame rate
+// first, exactly where the reference does it (model.py:114-116, before the K/V projection), and the K|V rows of every
+// fusion layer come from one GEMM on those T rows (bf16) unless the visual stack kernel has written them (pl.kvp).
+// In: x_a (fp32 residual), x_v (fp32 visual encoder output, N rows per utterance).  Out: a_op = fusion.norm(x) in bf16,
+// or with pl.dec separated / masks from the SeparationDecoder inside the same kernel.
+int fusion_stack_fused(avsep_handle* h, cudaStream_t s, Workspace& w, const Plan& pl, const float* mixed,
+                       float* separated, float* masks) {
   h->prof_stream = s;
   const int d = h->cfg.d_model, B = w.B, T = w.T;
   const int Ma = B * T, Lf = h->cfg.num_fusion_layers;
-  if (!have_kv) {                // else the visual stack kernel has already written w.kvb
-    CKL("lerp_kv", launch_lerp_rows(s, w.x_v, d, B, L_src, T, d, w.attn_a, d, w.frame_lens, w.lens));
+  if (!pl.kvp) {
+    CKL("lerp_kv", launch_lerp_rows(s, w.x_v, d, B, w.N, T, d, w.attn_a, d, w.frame_lens, w.lens));
     if (linear(h, s, "gemm.cross_kv", w.attn_a, Ma, d, h->wkv_all, h->bkv_all, Lf * 2 * d, ACT_NONE, nullptr, w.kvb)) return 1;
   }
-  *decoded = h->xs_f_decoder && !h->debug && masks != nullptr;
-  if (*decoded)
-    return run_stack(h, s, 2, w.x_a, nullptr, nullptr, h->fng, h->fnb, w.kvb, Lf * 2 * d, B, T, nullptr, mixed, separated, masks,
-                     nullptr, nullptr, 0, w.lens);
-  if (run_stack(h, s, 2, w.x_a, h->debug ? w.x_a : nullptr, w.a_op, h->fng, h->fnb, w.kvb, Lf * 2 * d, B, T, nullptr, nullptr,
-                nullptr, nullptr, nullptr, nullptr, 0, w.lens))
-    return 1;
+  StackProblem sp{};
+  sp.x_in = w.x_a; sp.fin_gamma = h->fng; sp.fin_beta = h->fnb; sp.kv = w.kvb;
+  sp.B = B; sp.L = T; sp.lens = w.lens;
+  if (pl.dec) {
+    sp.mixed = mixed; sp.separated = separated; sp.masks = masks;
+    return run_stack(h, s, 2, sp);
+  }
+  sp.out_x = h->debug ? w.x_a : nullptr; sp.out_op = w.a_op;
+  if (run_stack(h, s, 2, sp)) return 1;
   return snapshot(h, s, "fused", w.a_op, static_cast<size_t>(Ma) * d, true);
 }
 
+// CrossModalFusion, one kernel per layer.  In: x_a residual stream, a_op = LN_{layer0.norm1}(x_a), v_op = visual rows
+// (L_src per utterance).  Out: a_op = fusion.norm(x) in operand precision.
 int fusion_stack(avsep_handle* h, cudaStream_t s, Workspace& w, int L_src) {
   h->prof_stream = s;
   const int d = h->cfg.d_model, H = h->cfg.nhead, B = w.B, T = w.T, prec = h->cfg.precision;
@@ -533,8 +554,8 @@ int fusion_stack(avsep_handle* h, cudaStream_t s, Workspace& w, int L_src) {
   // K/V projection of every fusion layer in one GEMM on the un-interpolated visual rows
   if (linear(h, s, "gemm.cross_kv", w.v_op, Mv, d, h->wkv_all, h->bkv_all, Lf * 2 * d, ACT_NONE, w.kvn, nullptr)) return 1;
   for (int l = 0; l < Lf; ++l) {
-    const FusLayerW& fw = h->fus[l];
-    if (linear(h, s, "gemm.cross_q", w.a_op, Ma, d, fw.wq, fw.bq, d, ACT_NONE, nullptr, w.qkv_a)) return 1;
+    const LayerW& fw = h->fus[l];
+    if (linear(h, s, "gemm.cross_q", w.a_op, Ma, d, fw.w_in, fw.b_in, d, ACT_NONE, nullptr, w.qkv_a)) return 1;
     AttnProblem ap{};
     ap.q = w.qkv_a; ap.ldq = d;
     ap.k = w.kvn + static_cast<size_t>(l) * 2 * d;
@@ -560,16 +581,9 @@ int fusion_stack(avsep_handle* h, cudaStream_t s, Workspace& w, int L_src) {
     if (linear_resid_ln(h, s, "gemm.out_proj", w.attn_a, Ma, d, fw.wo, fw.bo, d, w.x_a, fw.n2g, fw.n2b, w.a_op, w.y_a))
       return 1;
     const bool last = (l + 1 == Lf);
-    const float* g = last ? h->fng : h->fus[l + 1].n1g;
-    const float* b = last ? h->fnb : h->fus[l + 1].n1b;
-    if (ffn_fusable(prec, d) && Ma >= FFN_FUSED_MIN_ROWS) {
-      CKL("ffn.fused", launch_ffn_fused(s, w.a_op, fw.w1, fw.b1, fw.w2, fw.b2, ACT_GELU,
-                                                                             w.x_a, w.x_a, g, b, w.a_op, Ma, h->num_sms,
-                                                                             nullptr));
-    } else {
-      if (linear(h, s, "gemm.ffn1", w.a_op, Ma, d, fw.w1, fw.b1, 4 * d, ACT_GELU, nullptr, w.ffn_a)) return 1;
-      if (linear_resid_ln(h, s, "gemm.ffn2", w.ffn_a, Ma, 4 * d, fw.w2, fw.b2, d, w.x_a, g, b, w.a_op, w.y_a)) return 1;
-    }
+    if (ffn_sublayer(h, s, fw, ACT_GELU, Ma, w.x_a, w.a_op, w.ffn_a, w.y_a, last ? h->fng : h->fus[l + 1].n1g,
+                     last ? h->fnb : h->fus[l + 1].n1b))
+      return 1;
   }
   return snapshot(h, s, "fused", w.a_op, static_cast<size_t>(Ma) * d, true);
 }
@@ -580,15 +594,12 @@ int decoder_stage(avsep_handle* h, cudaStream_t s, Workspace& w, const float* mi
   const int d = h->cfg.d_model, F = h->cfg.freq_bins, S = h->cfg.num_speakers, B = w.B, T = w.T;
   const int Ma = B * T;
   if (linear(h, s, "gemm.dec0", w.a_op, Ma, d, h->wdec0, h->bdec0, 2 * d, ACT_GELU, nullptr, w.ffn_a)) return 1;
-  GemmProblem p{};
-  p.A = w.ffn_a; p.lda = 2 * d; p.rowsA = Ma; p.M = Ma; p.W = h->wdec3; p.ldw = 2 * d; p.N = S * F; p.K = 2 * d;
-  p.taps = 1;
   GemmEpilogue e;
   e.kind = EPI_TAIL;
   e.bias = h->bdec3;
   e.mixed = mixed; e.masks = masks; e.separated = separated; e.F = F; e.S = S; e.T = T;
   e.lens = w.lens;
-  CKL("gemm.dec3_tail", launch_gemm(s, h->cfg.precision, p, e));
+  CKL("gemm.dec3_tail", launch_gemm(s, h->cfg.precision, dense(w.ffn_a, Ma, 2 * d, h->wdec3, S * F), e));
   return 0;
 }
 
@@ -596,13 +607,12 @@ int forward_device(avsep_handle* h, cudaStream_t s, Workspace& w, const float* m
                    float* separated, float* masks) {
   const int d = h->cfg.d_model;
   const int Ma = w.B * w.T, Mv = w.B * w.N;
+  const Plan pl = forward_plan(h, w.T, w.N);
   h->prof_stream = s;
   if (h->profile && h->profile_spin_us > 0) spin_kernel<<<1, 1, 0, s>>>(1000ull * h->profile_spin_us);
-  // The audio and visual branches are independent until the fusion: run them on two streams (fork / join) unless
-  // per-kernel profiling or stage snapshots need a single ordered stream.
+  // The audio and visual branches are independent until the fusion.
   cudaStream_t sv = s;
-  const bool fork = h->two_stream && !h->profile && !h->debug;
-  if (fork) {
+  if (pl.fork) {
     if (h->aux_stream == nullptr) {
       CUDA_OK(cudaStreamCreateWithFlags(&h->aux_stream, cudaStreamNonBlocking));
       CUDA_OK(cudaEventCreateWithFlags(&h->ev_fork, cudaEventDisableTiming));
@@ -612,50 +622,50 @@ int forward_device(avsep_handle* h, cudaStream_t s, Workspace& w, const float* m
     CUDA_OK(cudaEventRecord(h->ev_fork, s));
     CUDA_OK(cudaStreamWaitEvent(sv, h->ev_fork, 0));
   }
-  const bool fa = stack_fusable(h, w.T), fv = stack_fusable(h, w.N);
-  const bool ff = fa && fv;            // the fused fusion stack reads the fp32 residual rows of both encoders
   // --- visual branch (enqueued first: its CNN is the longest kernel) ---
-  const bool fp = !h->debug;     // input projections inside the stack kernels (no stage snapshots then)
-  bool kvp = false;
-  if (visual_frontend(h, sv, w, frames, h->enc_v[0].n1g, h->enc_v[0].n1b, fv, fv && fp)) return 1;
-  if (fv) {
-    // out: x_v (fp32) for the interpolation in front of the K/V projection; v_op (bf16 cast) only for the unfused fusion
-    // fused K | V projection: needs the fused fusion stack behind it and the audio frames inside a visual tile slot
-    kvp = ff && h->xs_v_kvp && !h->debug &&
-          xformer_kvp_usable(h->cfg.num_fusion_layers * 2 * d, w.N, w.T);
-    if (run_stack(h, sv, 1, w.x_v, kvp ? nullptr : w.x_v, (ff || kvp) ? nullptr : w.v_op, nullptr, nullptr, nullptr, 0, w.B,
-                  w.N, nullptr, nullptr, nullptr, nullptr, fp ? w.pooled : nullptr, kvp ? w.kvb : nullptr, w.T, w.frame_lens,
-                  w.lens))
-      return 1;
+  if (visual_frontend(h, sv, w, frames, pl)) return 1;
+  if (pl.stack_v) {
+    // out: x_v (fp32) for the interpolation in front of the K/V projection; v_op (bf16 cast) only for the per-layer fusion
+    StackProblem sp{};
+    sp.x_in = w.x_v; sp.B = w.B; sp.L = w.N; sp.lens = w.frame_lens; sp.kvp_lens = w.lens;
+    if (pl.pro) {
+      sp.pro_a = w.pooled; sp.pro_taps = 1; sp.pro_k = 128; sp.pro_pitch = w.N; sp.pro_rows = Mv; sp.pe = h->pe_v;
+    }
+    if (pl.kvp) {
+      sp.kvp_out = w.kvb; sp.kvp_L = w.T; sp.kvp_n = sp.kvp_ld = h->cfg.num_fusion_layers * 2 * d;
+    } else {
+      sp.out_x = w.x_v; sp.out_op = pl.stack_f ? nullptr : w.v_op;
+    }
+    if (run_stack(h, sv, 1, sp)) return 1;
   } else if (encoder_stack(h, sv, h->enc_v, w.B, w.N, w.x_v, w.y_v, w.v_op, w.qkv_v, w.attn_v, w.ffn_v, nullptr, nullptr,
                            w.frame_lens)) {
     return 1;
   }
   if (snapshot(h, sv, "visual_enc", w.x_v, static_cast<size_t>(Mv) * d, false)) return 1;
   // --- audio branch ---
-  if (audio_frontend(h, s, w, mixed, h->enc_a[0].n1g, h->enc_a[0].n1b, fa, fa && fp)) return 1;
-  if (fa) {
-    if (run_stack(h, s, 0, w.x_a, w.x_a, ff ? nullptr : w.a_op, h->fus[0].n1g, h->fus[0].n1b, nullptr, 0, w.B, w.T, nullptr,
-                  nullptr, nullptr, nullptr, fp ? w.h1 : nullptr, nullptr, 0, w.lens))
-      return 1;
+  if (audio_frontend(h, s, w, mixed, pl)) return 1;
+  if (pl.stack_a) {
+    StackProblem sp{};
+    sp.x_in = w.x_a; sp.out_x = w.x_a; sp.out_op = pl.stack_f ? nullptr : w.a_op;
+    sp.fin_gamma = h->fus[0].n1g; sp.fin_beta = h->fus[0].n1b;
+    sp.B = w.B; sp.L = w.T; sp.lens = w.lens;
+    if (pl.pro) {
+      sp.pro_a = w.h1; sp.pro_relu = 1; sp.pro_taps = 3; sp.pro_k = d; sp.pro_pitch = w.T + 2;
+      sp.pro_rows = w.B * (w.T + 2); sp.pe = h->pe_a;
+    }
+    if (run_stack(h, s, 0, sp)) return 1;
   } else if (encoder_stack(h, s, h->enc_a, w.B, w.T, w.x_a, w.y_a, w.a_op, w.qkv_a, w.attn_a, w.ffn_a, h->fus[0].n1g,
                            h->fus[0].n1b, w.lens)) {
     return 1;
   }
   if (snapshot(h, s, "audio_enc", w.x_a, static_cast<size_t>(Ma) * d, false)) return 1;
-  if (fork) {
+  if (pl.fork) {
     CUDA_OK(cudaEventRecord(h->ev_join, sv));
     CUDA_OK(cudaStreamWaitEvent(s, h->ev_join, 0));
   }
   // --- fusion + decoder ---
-  if (ff) {
-    bool decoded = false;
-    if (fusion_stack_fused(h, s, w, w.N, mixed, separated, masks, &decoded, kvp)) return 1;
-    if (decoded) return 0;
-  } else if (fusion_stack(h, s, w, w.N)) {
-    return 1;
-  }
-  return decoder_stage(h, s, w, mixed, separated, masks);
+  if (pl.stack_f ? fusion_stack_fused(h, s, w, pl, mixed, separated, masks) : fusion_stack(h, s, w, w.N)) return 1;
+  return pl.dec ? 0 : decoder_stage(h, s, w, mixed, separated, masks);
 }
 
 // Eager on the first use of a (shape, buffer set); captured into a CUDA graph on the second; replayed afterwards.
@@ -721,16 +731,37 @@ const HostTensor* find_w(avsep_handle* h, const std::string& key, std::initializ
   return &it->second;
 }
 
+// The 12 tensors of one encoder layer (nn.TransformerEncoderLayer) or fusion layer (model.py:136-149), shape-checked.
+// The two kinds differ only in their key names.
+struct HostLayer {
+  const HostTensor *w_in, *b_in, *wo, *bo, *w1, *b1, *w2, *b2, *n1g, *n1b, *n2g, *n2b;
+};
+bool find_layer(avsep_handle* h, const std::string& p, bool cross, int64_t d, HostLayer& t) {
+  const std::string at = p + (cross ? ".cross_attn." : ".self_attn."), f1 = p + (cross ? ".ff.0." : ".linear1."),
+                    f2 = p + (cross ? ".ff.3." : ".linear2.");
+  return (t.w_in = find_w(h, at + "in_proj_weight", {3 * d, d})) && (t.b_in = find_w(h, at + "in_proj_bias", {3 * d})) &&
+         (t.wo = find_w(h, at + "out_proj.weight", {d, d})) && (t.bo = find_w(h, at + "out_proj.bias", {d})) &&
+         (t.w1 = find_w(h, f1 + "weight", {4 * d, d})) && (t.b1 = find_w(h, f1 + "bias", {4 * d})) &&
+         (t.w2 = find_w(h, f2 + "weight", {d, 4 * d})) && (t.b2 = find_w(h, f2 + "bias", {d})) &&
+         (t.n1g = find_w(h, p + ".norm1.weight", {d})) && (t.n1b = find_w(h, p + ".norm1.bias", {d})) &&
+         (t.n2g = find_w(h, p + ".norm2.weight", {d})) && (t.n2b = find_w(h, p + ".norm2.bias", {d}));
+}
+
+// Host image of the weight arena.  Every item names the device-pointer field that views it; patch() sets those fields
+// once the image is uploaded.
 struct ArenaBuilder {
   std::vector<uint8_t> bytes;
-  size_t add(const void* src, size_t n) {
+  std::vector<std::function<void(const uint8_t*)>> fills;
+  template <typename T>
+  void add(const T*& field, const void* src, size_t n) {
     const size_t off = align_up(bytes.size(), 256);
     bytes.resize(off + n);
-    if (src) memcpy(bytes.data() + off, src, n);
-    return off;
+    memcpy(bytes.data() + off, src, n);
+    fills.push_back([&field, off](const uint8_t* base) { field = reinterpret_cast<const T*>(base + off); });
   }
-  size_t add_f32(const float* src, size_t n) { return add(src, n * 4); }
-  size_t add_op(const float* src, size_t n, bool tf32) {
+  void add_f32(const float*& field, const float* src, size_t n) { add(field, src, n * 4); }
+  void add_f32(const float*& field, const HostTensor* t) { add_f32(field, t->data.data(), t->data.size()); }
+  void add_op(const void*& field, const float* src, size_t n, bool tf32) {
     if (tf32) {   // round to tf32 (10-bit mantissa, nearest, ties away) so the tensor core's truncation is exact
       std::vector<float> tmp(n);
       for (size_t i = 0; i < n; ++i) {
@@ -739,13 +770,44 @@ struct ArenaBuilder {
         if ((u & 0x7f800000u) != 0x7f800000u) u = (u + 0x1000u) & 0xffffe000u;
         memcpy(&tmp[i], &u, 4);
       }
-      return add(tmp.data(), n * 4);
+      return add(field, tmp.data(), n * 4);
     }
     std::vector<uint16_t> tmp(n);
     for (size_t i = 0; i < n; ++i) tmp[i] = f2bf_host(src[i]);
-    return add(tmp.data(), n * 2);
+    add(field, tmp.data(), n * 2);
+  }
+  void add_op(const void*& field, const HostTensor* t, bool tf32) { add_op(field, t->data.data(), t->data.size(), tf32); }
+  void patch(const uint8_t* base) {
+    for (auto& f : fills) f(base);
   }
 };
+
+// Arena items of one layer: the weights, then the vectors.  A fusion layer keeps the Q rows of its input projection
+// (the first d), with their bias right behind them.
+void add_layer(ArenaBuilder& ar, LayerW& w, const HostLayer& t, bool cross, int64_t d, bool tf32) {
+  ar.add_op(w.w_in, t.w_in->data.data(), static_cast<size_t>(cross ? d : 3 * d) * d, tf32);
+  if (cross) ar.add_f32(w.b_in, t.b_in->data.data(), d);
+  ar.add_op(w.wo, t.wo, tf32);
+  ar.add_op(w.w1, t.w1, tf32);
+  ar.add_op(w.w2, t.w2, tf32);
+  if (!cross) ar.add_f32(w.b_in, t.b_in);
+  ar.add_f32(w.bo, t.bo);
+  ar.add_f32(w.b1, t.b1);
+  ar.add_f32(w.b2, t.b2);
+  ar.add_f32(w.n1g, t.n1g);
+  ar.add_f32(w.n1b, t.n1b);
+  ar.add_f32(w.n2g, t.n2g);
+  ar.add_f32(w.n2b, t.n2b);
+}
+
+// One layer of a stack-kernel weight stream: its vector block, then its weight items.  b0: bias of the input
+// projection in front of layer 0, which rides in that layer's vector block (or null).
+void pack_stream_layer(const HostLayer& t, bool cross, int d, const float* b0, std::vector<float>& vecs, uint8_t* dst) {
+  xformer_pack_vecs(t.b_in->data.data(), cross ? d : 3 * d, t.bo->data.data(), t.b1->data.data(), t.b2->data.data(),
+                    t.n1g->data.data(), t.n1b->data.data(), t.n2g->data.data(), t.n2b->data.data(), vecs.data(), b0);
+  (cross ? xformer_pack_cross : xformer_pack_self)(t.w_in->data.data(), t.wo->data.data(), t.w1->data.data(),
+                                                   t.w2->data.data(), vecs.data(), dst);
+}
 
 }  // namespace
 
@@ -861,258 +923,145 @@ int avsep_finalize_weights(avsep_handle* h, void* cuda_stream) {
   const int64_t d = h->cfg.d_model, F = h->cfg.freq_bins, S = h->cfg.num_speakers, Fp = h->Fp;
   const int Le = h->cfg.num_encoder_layers, Lf = h->cfg.num_fusion_layers;
   const bool tf32 = h->cfg.precision == AVSEP_PREC_TF32;
-  ArenaBuilder ar;
-  std::map<std::string, size_t> off;
+  // --- look up every tensor once
 #define GETW(var, key, ...)                                  \
   const HostTensor* var = find_w(h, key, {__VA_ARGS__});     \
   if (!var) return 1;
+  GETW(c0w, "audio_encoder.input_proj.0.weight", d, F, 3);
+  GETW(c0b, "audio_encoder.input_proj.0.bias", d);
+  GETW(c2w, "audio_encoder.input_proj.2.weight", d, d, 3);
+  GETW(c2b, "audio_encoder.input_proj.2.bias", d);
+  GETW(pea, "audio_encoder.pos_enc.pe", 1, 5000, d);
+  GETW(pev, "visual_encoder.pos_enc.pe", 1, 5000, d);
+  GETW(projw, "visual_encoder.frame_proj.weight", d, 128);
+  GETW(projb, "visual_encoder.frame_proj.bias", d);
+  GETW(fng, "fusion.norm.weight", d);
+  GETW(fnb, "fusion.norm.bias", d);
+  GETW(dec0w, "decoder.decoder.0.weight", 2 * d, d);
+  GETW(dec0b, "decoder.decoder.0.bias", 2 * d);
+  GETW(dec3w, "decoder.decoder.3.weight", S * F, 2 * d);
+  GETW(dec3b, "decoder.decoder.3.bias", S * F);
+  std::vector<HostLayer> enc[2] = {std::vector<HostLayer>(Le), std::vector<HostLayer>(Le)}, fus(Lf);
+  for (int l = 0; l < Le; ++l)
+    if (!find_layer(h, "audio_encoder.transformer.layers." + std::to_string(l), false, d, enc[0][l]) ||
+        !find_layer(h, "visual_encoder.transformer.layers." + std::to_string(l), false, d, enc[1][l]))
+      return 1;
+  for (int l = 0; l < Lf; ++l)
+    if (!find_layer(h, "fusion.layers." + std::to_string(l), true, d, fus[l])) return 1;
+  // VisualEncoder CNN: fold BatchNorm (eval) into conv weight/bias, repack tap-major
+  const int cins[3] = {1, 32, 64}, couts[3] = {32, 64, 128}, idx[3] = {0, 3, 6};
+  std::vector<float> folded[3], fbias[3];
+  for (int c = 0; c < 3; ++c) {
+    const std::string cp = "visual_encoder.conv." + std::to_string(idx[c]);
+    const std::string bp = "visual_encoder.conv." + std::to_string(idx[c] + 1);
+    GETW(w, cp + ".weight", couts[c], cins[c], 3, 3);
+    GETW(b, cp + ".bias", couts[c]);
+    GETW(g, bp + ".weight", couts[c]);
+    GETW(be, bp + ".bias", couts[c]);
+    GETW(mu, bp + ".running_mean", couts[c]);
+    GETW(var, bp + ".running_var", couts[c]);
+    const int K = 9 * cins[c];
+    folded[c].assign(static_cast<size_t>(couts[c]) * K, 0.f);
+    fbias[c].assign(couts[c], 0.f);
+    for (int o = 0; o < couts[c]; ++o) {
+      const float scale = g->data[o] / sqrtf(var->data[o] + 1e-5f);
+      fbias[c][o] = (b->data[o] - mu->data[o]) * scale + be->data[o];
+      for (int ci = 0; ci < cins[c]; ++ci)
+        for (int tap = 0; tap < 9; ++tap)
+          folded[c][static_cast<size_t>(o) * K + tap * cins[c] + ci] =
+              w->data[(static_cast<size_t>(o) * cins[c] + ci) * 9 + tap] * scale;
+    }
+  }
+#undef GETW
+  // fusion: the K|V rows of every layer's in_proj, concatenated
+  const int n_kv = static_cast<int>(Lf * 2 * d);
+  std::vector<float> wkv(static_cast<size_t>(n_kv) * d), bkv(n_kv);
+  for (int l = 0; l < Lf; ++l) {
+    memcpy(wkv.data() + static_cast<size_t>(l) * 2 * d * d, fus[l].w_in->data.data() + d * d, sizeof(float) * 2 * d * d);
+    memcpy(bkv.data() + static_cast<size_t>(l) * 2 * d, fus[l].b_in->data.data() + d, sizeof(float) * 2 * d);
+  }
 
-  // --- AudioEncoder Conv1d weights: (Cout, Cin, 3) -> (Cout, 3*Cin_pad), k = tap*Cin_pad + c
+  // --- the GEMM path's arena items
+  ArenaBuilder ar;
+  h->enc_a.assign(Le, LayerW{});
+  h->enc_v.assign(Le, LayerW{});
+  h->fus.assign(Lf, LayerW{});
   {
-    GETW(w0, "audio_encoder.input_proj.0.weight", d, F, 3);
-    GETW(b0, "audio_encoder.input_proj.0.bias", d);
-    GETW(w2, "audio_encoder.input_proj.2.weight", d, d, 3);
-    GETW(b2, "audio_encoder.input_proj.2.bias", d);
+    // AudioEncoder Conv1d weights: (Cout, Cin, 3) -> (Cout, 3*Cin_pad), k = tap*Cin_pad + c
     std::vector<float> p0(static_cast<size_t>(d) * 3 * Fp, 0.f), p2(static_cast<size_t>(d) * 3 * d, 0.f);
     for (int64_t o = 0; o < d; ++o)
       for (int64_t c = 0; c < F; ++c)
-        for (int tap = 0; tap < 3; ++tap) p0[(o * 3 + tap) * Fp + c] = w0->data[(o * F + c) * 3 + tap];
+        for (int tap = 0; tap < 3; ++tap) p0[(o * 3 + tap) * Fp + c] = c0w->data[(o * F + c) * 3 + tap];
     for (int64_t o = 0; o < d; ++o)
       for (int64_t c = 0; c < d; ++c)
-        for (int tap = 0; tap < 3; ++tap) p2[(o * 3 + tap) * d + c] = w2->data[(o * d + c) * 3 + tap];
-    off["wc1"] = ar.add_op(p0.data(), p0.size(), tf32);
-    off["wc2"] = ar.add_op(p2.data(), p2.size(), tf32);
-    off["bc1"] = ar.add_f32(b0->data.data(), d);
-    off["bc2"] = ar.add_f32(b2->data.data(), d);
-    GETW(pea, "audio_encoder.pos_enc.pe", 1, 5000, d);
-    GETW(pev, "visual_encoder.pos_enc.pe", 1, 5000, d);
-    off["pe_a"] = ar.add_f32(pea->data.data(), pea->data.size());
-    off["pe_v"] = ar.add_f32(pev->data.data(), pev->data.size());
+        for (int tap = 0; tap < 3; ++tap) p2[(o * 3 + tap) * d + c] = c2w->data[(o * d + c) * 3 + tap];
+    ar.add_op(h->wc1, p0.data(), p0.size(), tf32);
+    ar.add_op(h->wc2, p2.data(), p2.size(), tf32);
   }
-  // --- encoder stacks
-  for (int stack = 0; stack < 2; ++stack) {
-    const std::string pre = stack == 0 ? "audio_encoder" : "visual_encoder";
-    for (int l = 0; l < Le; ++l) {
-      const std::string p = pre + ".transformer.layers." + std::to_string(l);
-      const std::string t = (stack == 0 ? "a" : "v") + std::to_string(l);
-      GETW(wqkv, p + ".self_attn.in_proj_weight", 3 * d, d);
-      GETW(bqkv, p + ".self_attn.in_proj_bias", 3 * d);
-      GETW(wo, p + ".self_attn.out_proj.weight", d, d);
-      GETW(bo, p + ".self_attn.out_proj.bias", d);
-      GETW(w1, p + ".linear1.weight", 4 * d, d);
-      GETW(b1, p + ".linear1.bias", 4 * d);
-      GETW(w2, p + ".linear2.weight", d, 4 * d);
-      GETW(b2, p + ".linear2.bias", d);
-      GETW(n1g, p + ".norm1.weight", d);
-      GETW(n1b, p + ".norm1.bias", d);
-      GETW(n2g, p + ".norm2.weight", d);
-      GETW(n2b, p + ".norm2.bias", d);
-      off[t + "wqkv"] = ar.add_op(wqkv->data.data(), wqkv->data.size(), tf32);
-      off[t + "wo"] = ar.add_op(wo->data.data(), wo->data.size(), tf32);
-      off[t + "w1"] = ar.add_op(w1->data.data(), w1->data.size(), tf32);
-      off[t + "w2"] = ar.add_op(w2->data.data(), w2->data.size(), tf32);
-      off[t + "bqkv"] = ar.add_f32(bqkv->data.data(), 3 * d);
-      off[t + "bo"] = ar.add_f32(bo->data.data(), d);
-      off[t + "b1"] = ar.add_f32(b1->data.data(), 4 * d);
-      off[t + "b2"] = ar.add_f32(b2->data.data(), d);
-      off[t + "n1g"] = ar.add_f32(n1g->data.data(), d);
-      off[t + "n1b"] = ar.add_f32(n1b->data.data(), d);
-      off[t + "n2g"] = ar.add_f32(n2g->data.data(), d);
-      off[t + "n2b"] = ar.add_f32(n2b->data.data(), d);
-    }
-  }
-  // --- VisualEncoder CNN: fold BatchNorm (eval) into conv weight/bias, repack tap-major, fragment order
+  ar.add_f32(h->bc1, c0b);
+  ar.add_f32(h->bc2, c2b);
+  ar.add_f32(h->pe_a, pea);
+  ar.add_f32(h->pe_v, pev);
+  for (int l = 0; l < Le; ++l) add_layer(ar, h->enc_a[l], enc[0][l], false, d, tf32);
+  for (int l = 0; l < Le; ++l) add_layer(ar, h->enc_v[l], enc[1][l], false, d, tf32);
   {
-    const int cins[3] = {1, 32, 64}, couts[3] = {32, 64, 128}, idx[3] = {0, 3, 6};
-    std::vector<float> folded[3], fbias[3];
-    for (int c = 0; c < 3; ++c) {
-      const std::string cp = "visual_encoder.conv." + std::to_string(idx[c]);
-      const std::string bp = "visual_encoder.conv." + std::to_string(idx[c] + 1);
-      GETW(w, cp + ".weight", couts[c], cins[c], 3, 3);
-      GETW(b, cp + ".bias", couts[c]);
-      GETW(g, bp + ".weight", couts[c]);
-      GETW(be, bp + ".bias", couts[c]);
-      GETW(mu, bp + ".running_mean", couts[c]);
-      GETW(var, bp + ".running_var", couts[c]);
-      const int K = 9 * cins[c];
-      folded[c].assign(static_cast<size_t>(couts[c]) * K, 0.f);
-      fbias[c].assign(couts[c], 0.f);
-      for (int o = 0; o < couts[c]; ++o) {
-        const float scale = g->data[o] / sqrtf(var->data[o] + 1e-5f);
-        fbias[c][o] = (b->data[o] - mu->data[o]) * scale + be->data[o];
-        for (int ci = 0; ci < cins[c]; ++ci)
-          for (int tap = 0; tap < 9; ++tap)
-            folded[c][static_cast<size_t>(o) * K + tap * cins[c] + ci] =
-                w->data[(static_cast<size_t>(o) * cins[c] + ci) * 9 + tap] * scale;
-      }
-    }
+    // CNN operands: tcgen05 slabs, fragment order (hi, then the lo parts of the fp32-grade split path)
     std::vector<uint32_t> p1(visual_cnn_pack_sizes(1)), p2(visual_cnn_pack_sizes(2)), p3(visual_cnn_pack_sizes(3));
     visual_cnn_pack(folded[0].data(), folded[1].data(), folded[2].data(), p1.data(), p2.data(), p3.data());
     std::vector<uint8_t> tc2(visual_cnn_tc_w2_bytes()), tc3(visual_cnn_tc_w3_bytes());
     visual_cnn_tc_pack(folded[1].data(), folded[2].data(), tc2.data(), tc3.data());
-    off["tcw2"] = ar.add(tc2.data(), tc2.size());
-    off["tcw3"] = ar.add(tc3.data(), tc3.size());
-    off["cw1"] = ar.add(p1.data(), p1.size() * 4);
-    off["cw2"] = ar.add(p2.data(), p2.size() * 4);
-    off["cw3"] = ar.add(p3.data(), p3.size() * 4);
+    ar.add(h->cnn_w2_slabs, tc2.data(), tc2.size());
+    ar.add(h->cnn_w3_rows, tc3.data(), tc3.size());
+    ar.add(h->cnn.w1, p1.data(), p1.size() * 4);
+    ar.add(h->cnn.w2, p2.data(), p2.size() * 4);
+    ar.add(h->cnn.w3, p3.data(), p3.size() * 4);
     visual_cnn_pack(folded[0].data(), folded[1].data(), folded[2].data(), p1.data(), p2.data(), p3.data(), true);
-    off["cw1l"] = ar.add(p1.data(), p1.size() * 4);
-    off["cw2l"] = ar.add(p2.data(), p2.size() * 4);
-    off["cw3l"] = ar.add(p3.data(), p3.size() * 4);
-    off["cb1"] = ar.add_f32(fbias[0].data(), 32);
-    off["cb2"] = ar.add_f32(fbias[1].data(), 64);
-    off["cb3"] = ar.add_f32(fbias[2].data(), 128);
-    GETW(wp, "visual_encoder.frame_proj.weight", d, 128);
-    GETW(bp_, "visual_encoder.frame_proj.bias", d);
-    off["wproj"] = ar.add_op(wp->data.data(), wp->data.size(), tf32);
-    off["bproj"] = ar.add_f32(bp_->data.data(), d);
+    ar.add(h->cnn.w1l, p1.data(), p1.size() * 4);
+    ar.add(h->cnn.w2l, p2.data(), p2.size() * 4);
+    ar.add(h->cnn.w3l, p3.data(), p3.size() * 4);
+    ar.add_f32(h->cnn.b1, fbias[0].data(), 32);
+    ar.add_f32(h->cnn.b2, fbias[1].data(), 64);
+    ar.add_f32(h->cnn.b3, fbias[2].data(), 128);
   }
-  // --- fusion: q rows of the packed in_proj per layer; k|v rows of every layer concatenated
-  {
-    std::vector<float> wkv(static_cast<size_t>(Lf) * 2 * d * d), bkv(static_cast<size_t>(Lf) * 2 * d);
-    for (int l = 0; l < Lf; ++l) {
-      const std::string p = "fusion.layers." + std::to_string(l);
-      const std::string t = "f" + std::to_string(l);
-      GETW(win, p + ".cross_attn.in_proj_weight", 3 * d, d);
-      GETW(bin, p + ".cross_attn.in_proj_bias", 3 * d);
-      GETW(wo, p + ".cross_attn.out_proj.weight", d, d);
-      GETW(bo, p + ".cross_attn.out_proj.bias", d);
-      GETW(w1, p + ".ff.0.weight", 4 * d, d);
-      GETW(b1, p + ".ff.0.bias", 4 * d);
-      GETW(w2, p + ".ff.3.weight", d, 4 * d);
-      GETW(b2, p + ".ff.3.bias", d);
-      GETW(n1g, p + ".norm1.weight", d);
-      GETW(n1b, p + ".norm1.bias", d);
-      GETW(n2g, p + ".norm2.weight", d);
-      GETW(n2b, p + ".norm2.bias", d);
-      off[t + "wq"] = ar.add_op(win->data.data(), static_cast<size_t>(d) * d, tf32);
-      off[t + "bq"] = ar.add_f32(bin->data.data(), d);
-      memcpy(wkv.data() + static_cast<size_t>(l) * 2 * d * d, win->data.data() + d * d, sizeof(float) * 2 * d * d);
-      memcpy(bkv.data() + static_cast<size_t>(l) * 2 * d, bin->data.data() + d, sizeof(float) * 2 * d);
-      off[t + "wo"] = ar.add_op(wo->data.data(), wo->data.size(), tf32);
-      off[t + "w1"] = ar.add_op(w1->data.data(), w1->data.size(), tf32);
-      off[t + "w2"] = ar.add_op(w2->data.data(), w2->data.size(), tf32);
-      off[t + "bo"] = ar.add_f32(bo->data.data(), d);
-      off[t + "b1"] = ar.add_f32(b1->data.data(), 4 * d);
-      off[t + "b2"] = ar.add_f32(b2->data.data(), d);
-      off[t + "n1g"] = ar.add_f32(n1g->data.data(), d);
-      off[t + "n1b"] = ar.add_f32(n1b->data.data(), d);
-      off[t + "n2g"] = ar.add_f32(n2g->data.data(), d);
-      off[t + "n2b"] = ar.add_f32(n2b->data.data(), d);
+  ar.add_op(h->wproj, projw, tf32);
+  ar.add_f32(h->bproj, projb);
+  for (int l = 0; l < Lf; ++l) add_layer(ar, h->fus[l], fus[l], true, d, tf32);
+  ar.add_op(h->wkv_all, wkv.data(), wkv.size(), tf32);
+  ar.add_f32(h->bkv_all, bkv.data(), bkv.size());
+  ar.add_f32(h->fng, fng);
+  ar.add_f32(h->fnb, fnb);
+  ar.add_op(h->wdec0, dec0w, tf32);
+  ar.add_op(h->wdec3, dec3w, tf32);
+  ar.add_f32(h->bdec0, dec0b);
+  ar.add_f32(h->bdec3, dec3b);
+
+  // --- fused transformer-stack kernel: weight streams in consumption order + per-layer vector blocks.  The encoder
+  // streams start with the input projection (Conv1d #2 as 3 taps x d / frame_proj as 1 x 128), whose bias rides in
+  // layer 0's vector block; the visual one ends with the fusion K|V projection, the fusion one with the decoder.
+  h->xs_a = h->xs_v = h->xs_f = nullptr;
+  if (xformer_stack_usable(h->cfg.precision, static_cast<int>(d), h->cfg.nhead, 1)) {
+    const size_t sb = xformer_stream_bytes(false), cb = xformer_stream_bytes(true);
+    const size_t pro_a = xformer_pro_bytes(3, static_cast<int>(d)), pro_v = xformer_pro_bytes(1, 128);
+    h->xs_v_kvp = xformer_kvp_usable(n_kv, 1, 1);
+    h->xs_f_decoder = xformer_decoder_usable(static_cast<int>(S), static_cast<int>(F));
+    std::vector<uint8_t> xa(pro_a + Le * sb), xv(pro_v + Le * sb + (h->xs_v_kvp ? xformer_kvp_bytes(n_kv) : 0)),
+        xf(Lf * cb + (h->xs_f_decoder ? xformer_decoder_bytes(static_cast<int>(S), static_cast<int>(F)) : 0));
+    std::vector<float> vecs(xformer_vec_floats());
+    xformer_pack_pro(c2w->data.data(), static_cast<int>(3 * d), 3, 3, static_cast<int>(d), xa.data());
+    xformer_pack_pro(projw->data.data(), 128, 1, 1, 128, xv.data());
+    for (int l = 0; l < Le; ++l) {
+      pack_stream_layer(enc[0][l], false, d, l == 0 ? c2b->data.data() : nullptr, vecs, xa.data() + pro_a + l * sb);
+      pack_stream_layer(enc[1][l], false, d, l == 0 ? projb->data.data() : nullptr, vecs, xv.data() + pro_v + l * sb);
     }
-    off["wkv"] = ar.add_op(wkv.data(), wkv.size(), tf32);
-    off["bkv"] = ar.add_f32(bkv.data(), bkv.size());
-    GETW(fg, "fusion.norm.weight", d);
-    GETW(fb, "fusion.norm.bias", d);
-    off["fng"] = ar.add_f32(fg->data.data(), d);
-    off["fnb"] = ar.add_f32(fb->data.data(), d);
+    if (h->xs_v_kvp) xformer_pack_kvp(wkv.data(), bkv.data(), n_kv, xv.data() + pro_v + Le * sb);
+    for (int l = 0; l < Lf; ++l) pack_stream_layer(fus[l], true, d, nullptr, vecs, xf.data() + l * cb);
+    if (h->xs_f_decoder)
+      xformer_pack_decoder(dec0w->data.data(), dec0b->data.data(), dec3w->data.data(), dec3b->data.data(),
+                           static_cast<int>(S), static_cast<int>(F), xf.data() + Lf * cb);
+    ar.add(h->xs_a, xa.data(), xa.size());
+    ar.add(h->xs_v, xv.data(), xv.size());
+    ar.add(h->xs_f, xf.data(), xf.size());
   }
-  // --- decoder
-  {
-    GETW(w0, "decoder.decoder.0.weight", 2 * d, d);
-    GETW(b0, "decoder.decoder.0.bias", 2 * d);
-    GETW(w3, "decoder.decoder.3.weight", S * F, 2 * d);
-    GETW(b3, "decoder.decoder.3.bias", S * F);
-    off["wdec0"] = ar.add_op(w0->data.data(), w0->data.size(), tf32);
-    off["wdec3"] = ar.add_op(w3->data.data(), w3->data.size(), tf32);
-    off["bdec0"] = ar.add_f32(b0->data.data(), 2 * d);
-    off["bdec3"] = ar.add_f32(b3->data.data(), S * F);
-  }
-  // --- fused transformer-stack kernel: weight streams in consumption order + per-layer vector blocks
-  const bool pack_stacks = xformer_stack_usable(h->cfg.precision, static_cast<int>(d), h->cfg.nhead, 1);
-  if (pack_stacks) {
-    const size_t vf = static_cast<size_t>(xformer_vec_floats());
-    for (int stack = 0; stack < 2; ++stack) {
-      const std::string pre = stack == 0 ? "audio_encoder" : "visual_encoder";
-      // the stream starts with the input projection (Conv1d #2 as 3 taps x 256 / frame_proj as 1 x 128), whose bias
-      // rides in layer 0's vector block
-      const size_t pro_bytes = stack == 0 ? xformer_pro_bytes(3, static_cast<int>(d)) : xformer_pro_bytes(1, 128);
-      const int n_kv = static_cast<int>(Lf * 2 * d);
-      const bool with_kvp = stack == 1 && xformer_kvp_usable(n_kv, 1, 1);
-      std::vector<uint8_t> stream(pro_bytes + static_cast<size_t>(Le) * xformer_stream_bytes(false) +
-                                  (with_kvp ? xformer_kvp_bytes(n_kv) : 0));
-      const HostTensor* b0t = nullptr;
-      if (stack == 0) {
-        GETW(wc, "audio_encoder.input_proj.2.weight", d, d, 3);
-        GETW(bc, "audio_encoder.input_proj.2.bias", d);
-        xformer_pack_pro(wc->data.data(), static_cast<int>(3 * d), 3, 3, static_cast<int>(d), stream.data());
-        b0t = bc;
-      } else {
-        GETW(wc, "visual_encoder.frame_proj.weight", d, 128);
-        GETW(bc, "visual_encoder.frame_proj.bias", d);
-        xformer_pack_pro(wc->data.data(), 128, 1, 1, 128, stream.data());
-        b0t = bc;
-      }
-      std::vector<float> vecs(vf);
-      for (int l = 0; l < Le; ++l) {
-        const std::string p = pre + ".transformer.layers." + std::to_string(l);
-        GETW(wqkv, p + ".self_attn.in_proj_weight", 3 * d, d);
-        GETW(bqkv, p + ".self_attn.in_proj_bias", 3 * d);
-        GETW(wo, p + ".self_attn.out_proj.weight", d, d);
-        GETW(bo, p + ".self_attn.out_proj.bias", d);
-        GETW(w1, p + ".linear1.weight", 4 * d, d);
-        GETW(b1, p + ".linear1.bias", 4 * d);
-        GETW(w2, p + ".linear2.weight", d, 4 * d);
-        GETW(b2, p + ".linear2.bias", d);
-        GETW(n1g, p + ".norm1.weight", d);
-        GETW(n1b, p + ".norm1.bias", d);
-        GETW(n2g, p + ".norm2.weight", d);
-        GETW(n2b, p + ".norm2.bias", d);
-        xformer_pack_vecs(bqkv->data.data(), static_cast<int>(3 * d), bo->data.data(), b1->data.data(), b2->data.data(),
-                          n1g->data.data(), n1b->data.data(), n2g->data.data(), n2b->data.data(), vecs.data(),
-                          l == 0 ? b0t->data.data() : nullptr);
-        xformer_pack_self(wqkv->data.data(), wo->data.data(), w1->data.data(), w2->data.data(), vecs.data(),
-                          stream.data() + pro_bytes + static_cast<size_t>(l) * xformer_stream_bytes(false));
-      }
-      if (with_kvp) {
-        std::vector<float> wkv(static_cast<size_t>(n_kv) * d), bkv(n_kv);
-        for (int l = 0; l < Lf; ++l) {
-          const std::string p = "fusion.layers." + std::to_string(l);
-          GETW(win, p + ".cross_attn.in_proj_weight", 3 * d, d);
-          GETW(bin, p + ".cross_attn.in_proj_bias", 3 * d);
-          memcpy(wkv.data() + static_cast<size_t>(l) * 2 * d * d, win->data.data() + d * d, sizeof(float) * 2 * d * d);
-          memcpy(bkv.data() + static_cast<size_t>(l) * 2 * d, bin->data.data() + d, sizeof(float) * 2 * d);
-        }
-        xformer_pack_kvp(wkv.data(), bkv.data(), n_kv, stream.data() + pro_bytes + static_cast<size_t>(Le) * xformer_stream_bytes(false));
-        h->xs_v_kvp = true;
-      }
-      off[stack == 0 ? "xs_a" : "xs_v"] = ar.add(stream.data(), stream.size());
-    }
-    const bool fuse_dec = xformer_decoder_usable(static_cast<int>(S), static_cast<int>(F));
-    std::vector<uint8_t> stream(static_cast<size_t>(Lf) * xformer_stream_bytes(true) +
-                                (fuse_dec ? xformer_decoder_bytes(static_cast<int>(S), static_cast<int>(F)) : 0));
-    std::vector<float> vecs(vf);
-    for (int l = 0; l < Lf; ++l) {
-      const std::string p = "fusion.layers." + std::to_string(l);
-      GETW(win, p + ".cross_attn.in_proj_weight", 3 * d, d);
-      GETW(bin, p + ".cross_attn.in_proj_bias", 3 * d);
-      GETW(wo, p + ".cross_attn.out_proj.weight", d, d);
-      GETW(bo, p + ".cross_attn.out_proj.bias", d);
-      GETW(w1, p + ".ff.0.weight", 4 * d, d);
-      GETW(b1, p + ".ff.0.bias", 4 * d);
-      GETW(w2, p + ".ff.3.weight", d, 4 * d);
-      GETW(b2, p + ".ff.3.bias", d);
-      GETW(n1g, p + ".norm1.weight", d);
-      GETW(n1b, p + ".norm1.bias", d);
-      GETW(n2g, p + ".norm2.weight", d);
-      GETW(n2b, p + ".norm2.bias", d);
-      xformer_pack_vecs(bin->data.data(), static_cast<int>(d), bo->data.data(), b1->data.data(), b2->data.data(),
-                        n1g->data.data(), n1b->data.data(), n2g->data.data(), n2b->data.data(), vecs.data());
-      xformer_pack_cross(win->data.data(), wo->data.data(), w1->data.data(), w2->data.data(), vecs.data(),
-                         stream.data() + static_cast<size_t>(l) * xformer_stream_bytes(true));
-    }
-    if (fuse_dec) {
-      GETW(w0, "decoder.decoder.0.weight", 2 * d, d);
-      GETW(b0, "decoder.decoder.0.bias", 2 * d);
-      GETW(w3, "decoder.decoder.3.weight", S * F, 2 * d);
-      GETW(b3, "decoder.decoder.3.bias", S * F);
-      xformer_pack_decoder(w0->data.data(), b0->data.data(), w3->data.data(), b3->data.data(), static_cast<int>(S), static_cast<int>(F),
-                           stream.data() + static_cast<size_t>(Lf) * xformer_stream_bytes(true));
-    }
-    h->xs_f_decoder = fuse_dec;
-    off["xs_f"] = ar.add(stream.data(), stream.size());
-  }
-#undef GETW
   // upload
   drop_graphs(h);
   if (h->d_weights) cudaFree(h->d_weights);
@@ -1121,44 +1070,10 @@ int avsep_finalize_weights(avsep_handle* h, void* cuda_stream) {
   h->weight_bytes = ar.bytes.size();
   CUDA_OK(cudaMemcpyAsync(h->d_weights, ar.bytes.data(), ar.bytes.size(), cudaMemcpyHostToDevice, s));
   CUDA_OK(cudaStreamSynchronize(s));
-  auto P = [&](const std::string& k) -> const void* { return h->d_weights + off.at(k); };
-  auto PF = [&](const std::string& k) -> const float* { return reinterpret_cast<const float*>(h->d_weights + off.at(k)); };
-  h->wc1 = P("wc1"); h->wc2 = P("wc2"); h->bc1 = PF("bc1"); h->bc2 = PF("bc2");
-  h->pe_a = PF("pe_a"); h->pe_v = PF("pe_v");
-  h->wproj = P("wproj"); h->bproj = PF("bproj");
-  h->wkv_all = P("wkv"); h->bkv_all = PF("bkv"); h->fng = PF("fng"); h->fnb = PF("fnb");
-  h->wdec0 = P("wdec0"); h->wdec3 = P("wdec3"); h->bdec0 = PF("bdec0"); h->bdec3 = PF("bdec3");
-  h->cnn.w1 = reinterpret_cast<const uint32_t*>(P("cw1")); h->cnn.b1 = PF("cb1");
-  h->cnn.w2 = reinterpret_cast<const uint32_t*>(P("cw2")); h->cnn.b2 = PF("cb2");
-  h->cnn.w3 = reinterpret_cast<const uint32_t*>(P("cw3")); h->cnn.b3 = PF("cb3");
-  h->cnn.w1l = reinterpret_cast<const uint32_t*>(P("cw1l"));
-  h->cnn.w2l = reinterpret_cast<const uint32_t*>(P("cw2l"));
-  h->cnn.w3l = reinterpret_cast<const uint32_t*>(P("cw3l"));
-  h->cnn_w2_slabs = static_cast<const uint8_t*>(P("tcw2"));
-  h->cnn_w3_rows = static_cast<const uint8_t*>(P("tcw3"));
-  h->xs_a = h->xs_v = h->xs_f = nullptr;
-  if (pack_stacks) {
-    h->xs_a = static_cast<const uint8_t*>(P("xs_a")); h->xs_v = static_cast<const uint8_t*>(P("xs_v"));
-    h->xs_a_np = h->xs_a + xformer_pro_bytes(3, h->cfg.d_model); h->xs_v_np = h->xs_v + xformer_pro_bytes(1, 128);
-    h->xs_f = static_cast<const uint8_t*>(P("xs_f"));
-  }
-  h->enc_a.clear(); h->enc_v.clear(); h->fus.clear();
-  for (int stack = 0; stack < 2; ++stack)
-    for (int l = 0; l < Le; ++l) {
-      const std::string t = (stack == 0 ? "a" : "v") + std::to_string(l);
-      EncLayerW w;
-      w.wqkv = P(t + "wqkv"); w.wo = P(t + "wo"); w.w1 = P(t + "w1"); w.w2 = P(t + "w2");
-      w.bqkv = PF(t + "bqkv"); w.bo = PF(t + "bo"); w.b1 = PF(t + "b1"); w.b2 = PF(t + "b2");
-      w.n1g = PF(t + "n1g"); w.n1b = PF(t + "n1b"); w.n2g = PF(t + "n2g"); w.n2b = PF(t + "n2b");
-      (stack == 0 ? h->enc_a : h->enc_v).push_back(w);
-    }
-  for (int l = 0; l < Lf; ++l) {
-    const std::string t = "f" + std::to_string(l);
-    FusLayerW w;
-    w.wq = P(t + "wq"); w.wo = P(t + "wo"); w.w1 = P(t + "w1"); w.w2 = P(t + "w2");
-    w.bq = PF(t + "bq"); w.bo = PF(t + "bo"); w.b1 = PF(t + "b1"); w.b2 = PF(t + "b2");
-    w.n1g = PF(t + "n1g"); w.n1b = PF(t + "n1b"); w.n2g = PF(t + "n2g"); w.n2b = PF(t + "n2b");
-    h->fus.push_back(w);
+  ar.patch(h->d_weights);
+  if (h->xs_a != nullptr) {
+    h->xs_a_np = h->xs_a + xformer_pro_bytes(3, h->cfg.d_model);
+    h->xs_v_np = h->xs_v + xformer_pro_bytes(1, 128);
   }
   h->finalized = true;
   return 0;
@@ -1519,7 +1434,7 @@ int avsep_audio_encoder(avsep_handle* h, const float* mixed_spec, int32_t B, int
   if (get_workspace(h, w, nullptr, 0, B, T, 1, 1, 1)) return 1;
   const int d = h->cfg.d_model, Ma = B * T;
   h->launches = 0;
-  if (audio_frontend(h, s, w, mixed_spec, h->enc_a[0].n1g, h->enc_a[0].n1b)) return 1;
+  if (audio_frontend(h, s, w, mixed_spec, Plan{})) return 1;
   if (encoder_stack(h, s, h->enc_a, B, T, w.x_a, w.y_a, w.a_op, w.qkv_a, w.attn_a, w.ffn_a, nullptr, nullptr)) return 1;
   CUDA_OK(cudaMemcpyAsync(out_BTd, w.x_a, static_cast<size_t>(Ma) * d * 4, cudaMemcpyDeviceToDevice, s));
   return 0;
@@ -1537,7 +1452,7 @@ int avsep_visual_encoder(avsep_handle* h, const float* lip_frames, int32_t B, in
   if (get_workspace(h, w, nullptr, 0, B, 1, N, Hh, Ww)) return 1;
   const int d = h->cfg.d_model;
   h->launches = 0;
-  if (visual_frontend(h, s, w, lip_frames, h->enc_v[0].n1g, h->enc_v[0].n1b)) return 1;
+  if (visual_frontend(h, s, w, lip_frames, Plan{})) return 1;
   if (encoder_stack(h, s, h->enc_v, B, N, w.x_v, w.y_v, w.v_op, w.qkv_v, w.attn_v, w.ffn_v, nullptr, nullptr)) return 1;
   interp_rows_kernel<<<dim3(target_len, B), 128, 0, s>>>(w.x_v, out_BTd, N, target_len, d,
                                                          static_cast<float>(N) / static_cast<float>(target_len));
@@ -1567,9 +1482,7 @@ int avsep_fusion(avsep_handle* h, const float* audio_BTd, const float* visual_BL
   h->debug = dbg;
   if (rc) return 1;
   // fused rows in fp32: recompute the final LayerNorm from the fp32 residual stream straight into the caller's buffer
-  const int save_prec = h->cfg.precision;
   CKL("add_layernorm", launch_add_layernorm(s, PREC_TF32, w.x_a, nullptr, h->fng, h->fnb, nullptr, out_BTd, Ma, d));
-  (void)save_prec;
   return 0;
 }
 
@@ -1645,8 +1558,7 @@ int avsep_profile_report(avsep_handle* h, char* buf, size_t capacity, int32_t re
 int avsep_test_gemm(avsep_handle* h, const void* A, const void* W, const float* bias, float* out, int32_t M, int32_t N,
                     int32_t K, int32_t act, int32_t force_bn, void* cuda_stream) {
   if (!h) return 1;
-  GemmProblem p{};
-  p.A = A; p.lda = K; p.rowsA = M; p.M = M; p.W = W; p.ldw = K; p.N = N; p.K = K; p.taps = 1;
+  const GemmProblem p = dense(A, M, K, W, N);
   GemmEpilogue e;
   e.bias = bias; e.act = act; e.out_f32 = out; e.ld_f32 = N;
   CK(launch_gemm(static_cast<cudaStream_t>(cuda_stream), h->cfg.precision, p, e, force_bn));
@@ -1658,8 +1570,7 @@ int avsep_test_gemm(avsep_handle* h, const void* A, const void* W, const float* 
 int avsep_test_gemm_ln(avsep_handle* h, const void* A, const void* W, const float* bias, float* x, const float* gamma,
                        const float* beta, void* out_op, int32_t M, int32_t N, int32_t K, void* cuda_stream) {
   if (!h) return 1;
-  GemmProblem p{};
-  p.A = A; p.lda = K; p.rowsA = M; p.M = M; p.W = W; p.ldw = K; p.N = N; p.K = K; p.taps = 1;
+  const GemmProblem p = dense(A, M, K, W, N);
   GemmEpilogue e;
   e.kind = EPI_LN;
   e.bias = bias; e.resid = x; e.out_f32 = x; e.ld_f32 = N; e.ln_gamma = gamma; e.ln_beta = beta;
@@ -1675,8 +1586,7 @@ int avsep_test_gemm_trace(avsep_handle* h, const void* A, const void* W, const f
                           const float* gamma, const float* beta, void* out_op, int32_t M, int32_t N, int32_t K,
                           int32_t ln, int32_t act, unsigned long long* trace_dev, void* cuda_stream) {
   if (!h) return 1;
-  GemmProblem p{};
-  p.A = A; p.lda = K; p.rowsA = M; p.M = M; p.W = W; p.ldw = K; p.N = N; p.K = K; p.taps = 1;
+  const GemmProblem p = dense(A, M, K, W, N);
   GemmEpilogue e;
   e.bias = bias; e.act = act;
   if (ln == 7) {
@@ -1734,12 +1644,12 @@ int avsep_test_xformer_stack(avsep_handle* h, int32_t which, const float* x_in, 
   if (which < 0 || which > 2) return fail(h, "test_xformer_stack: which must be 0, 1 or 2");
   if (h->xs_a == nullptr || !xformer_stack_usable(h->cfg.precision, h->cfg.d_model, h->cfg.nhead, L))
     return fail(h, "test_xformer_stack: the fused stack kernel does not support this configuration");
-  const float *g = nullptr, *b = nullptr;
-  if (final_ln && which == 0) { g = h->fus[0].n1g; b = h->fus[0].n1b; }
-  if (final_ln && which == 2) { g = h->fng; b = h->fnb; }
+  StackProblem sp{};
+  sp.x_in = x_in; sp.out_x = out_x; sp.out_op = out_op; sp.kv = kv; sp.B = B; sp.L = L; sp.trace = trace_dev;
+  if (final_ln && which == 0) { sp.fin_gamma = h->fus[0].n1g; sp.fin_beta = h->fus[0].n1b; }
+  if (final_ln && which == 2) { sp.fin_gamma = h->fng; sp.fin_beta = h->fnb; }
   h->prof_stream = static_cast<cudaStream_t>(cuda_stream);
-  return run_stack(h, static_cast<cudaStream_t>(cuda_stream), which, x_in, out_x, out_op, g, b, kv,
-                   h->cfg.num_fusion_layers * 2 * h->cfg.d_model, B, L, trace_dev);
+  return run_stack(h, static_cast<cudaStream_t>(cuda_stream), which, sp);
 }
 
 int avsep_test_fusion_decoder(avsep_handle* h, const float* x_in, const void* kv, int32_t B, int32_t L, const float* mixed,
@@ -1749,9 +1659,11 @@ int avsep_test_fusion_decoder(avsep_handle* h, const float* x_in, const void* kv
   if (h->xs_f == nullptr || !h->xs_f_decoder || !xformer_stack_usable(h->cfg.precision, h->cfg.d_model, h->cfg.nhead, L))
     return fail(h, "test_fusion_decoder: the fused stack kernel does not support this configuration");
   if (!mixed || !separated || !masks) return fail(h, "test_fusion_decoder: null buffer");
+  StackProblem sp{};
+  sp.x_in = x_in; sp.fin_gamma = h->fng; sp.fin_beta = h->fnb; sp.kv = kv; sp.B = B; sp.L = L; sp.trace = trace_dev;
+  sp.mixed = mixed; sp.separated = separated; sp.masks = masks;
   h->prof_stream = static_cast<cudaStream_t>(cuda_stream);
-  return run_stack(h, static_cast<cudaStream_t>(cuda_stream), 2, x_in, nullptr, nullptr, h->fng, h->fnb, kv,
-                   h->cfg.num_fusion_layers * 2 * h->cfg.d_model, B, L, trace_dev, mixed, separated, masks);
+  return run_stack(h, static_cast<cudaStream_t>(cuda_stream), 2, sp);
 }
 
 int avsep_set_option(avsep_handle* h, const char* name, int32_t value) {
