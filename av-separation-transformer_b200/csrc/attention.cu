@@ -44,23 +44,6 @@ __device__ __forceinline__ UttKeys utt_keys(const AttnDev& p, int b) {
   return u;
 }
 
-__device__ __forceinline__ void ldmatrix_x4(uint32_t (&r)[4], uint32_t addr) {
-  asm volatile("ldmatrix.sync.aligned.m8n8.x4.shared.b16 {%0,%1,%2,%3}, [%4];"
-               : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3])
-               : "r"(addr));
-}
-__device__ __forceinline__ void ldmatrix_x4_trans(uint32_t (&r)[4], uint32_t addr) {
-  asm volatile("ldmatrix.sync.aligned.m8n8.x4.trans.shared.b16 {%0,%1,%2,%3}, [%4];"
-               : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3])
-               : "r"(addr));
-}
-__device__ __forceinline__ void mma_bf16_16816(float (&c)[4], const uint32_t (&a)[4], uint32_t b0, uint32_t b1) {
-  asm volatile(
-      "mma.sync.aligned.m16n8k16.row.col.f32.bf16.bf16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
-      : "+f"(c[0]), "+f"(c[1]), "+f"(c[2]), "+f"(c[3])
-      : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
-}
-
 constexpr int QT = 64;   // query rows per CTA
 constexpr int KT = 64;   // key/value rows per tile
 
@@ -479,13 +462,8 @@ const char* launch_small(cudaStream_t s, const AttnDev& d, int B, int H) {
 template <int HD, bool LERP, bool SPLIT>
 const char* launch_t(cudaStream_t s, const AttnDev& d, int B, int H, int Lq) {
   constexpr int SMEM = (SPLIT ? 6 : 3) * 64 * (HD + 8) * 2;
-  static bool attr_done = false;
   auto kern = attention_kernel<HD, LERP, SPLIT>;
-  if (!attr_done && SMEM > 48 * 1024) {
-    if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM) != cudaSuccess)
-      return "attention: cudaFuncSetAttribute failed";
-    attr_done = true;
-  }
+  if (!smem_opt_in(kern, SMEM)) return "attention: cudaFuncSetAttribute failed";
   dim3 grid((Lq + QT - 1) / QT, H, B);
   if (launch_pdl(kern, grid, dim3(128), SMEM, s, d) != cudaSuccess) {
     cudaGetLastError();

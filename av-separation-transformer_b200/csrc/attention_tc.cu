@@ -16,8 +16,6 @@
 #include "common.cuh"
 #include "kernels.h"
 
-#include <cudaTypedefs.h>
-
 namespace avsep {
 
 namespace {
@@ -40,12 +38,6 @@ struct AttnTcDev {
   float scale_log2;
   const int* k_lens;    // variable-length batch: keys of utterance b (null: all Lk)
 };
-
-__device__ __forceinline__ float ex2_approx(float x) {
-  float y;
-  asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
-  return y;
-}
 
 __device__ __forceinline__ void tma_store_3d(const CUtensorMap* m, const void* smem_src, int c0, int c1, int c2) {
   asm volatile("cp.async.bulk.tensor.3d.global.shared::cta.bulk_group [%0, {%2, %3, %4}], [%1];"
@@ -329,22 +321,6 @@ __global__ void lerp_rows_kernel(const float* __restrict__ src, int ld_src, int 
   *reinterpret_cast<uint4*>(dst + rt * ld_dst + c * 8) = val;
 }
 
-PFN_cuTensorMapEncodeTiled_v12000 g_enc = nullptr;
-
-// rows [B, L] x cols, bf16, box = 64 cols x 128 rows of one utterance; rows past L are zero-filled / clipped
-const char* encode_3d(CUtensorMap* map, const void* ptr, int cols, int L, int B, int ld) {
-  if ((reinterpret_cast<uintptr_t>(ptr) & 15) != 0) return "attention_tc: pointer not 16-byte aligned";
-  if ((ld & 7) != 0) return "attention_tc: leading dimension not a multiple of 8";
-  cuuint64_t dims[3] = {static_cast<cuuint64_t>(cols), static_cast<cuuint64_t>(L), static_cast<cuuint64_t>(B)};
-  cuuint64_t strides[2] = {static_cast<cuuint64_t>(ld) * 2, static_cast<cuuint64_t>(L) * ld * 2};
-  cuuint32_t box[3] = {64, 128, 1};
-  cuuint32_t estr[3] = {1, 1, 1};
-  CUresult r = g_enc(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<void*>(ptr), dims, strides, box, estr,
-                     CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                     CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  return r == CUDA_SUCCESS ? nullptr : "attention_tc: cuTensorMapEncodeTiled failed";
-}
-
 }  // namespace
 
 bool attention_tc_usable(int prec, const AttnProblem& p) {
@@ -355,23 +331,14 @@ bool attention_tc_usable(int prec, const AttnProblem& p) {
 const char* launch_attention_tc(cudaStream_t s, const AttnProblem& p) {
   if (p.B <= 0 || p.Lq <= 0 || p.Lk <= 0) return "attention_tc: empty problem";
   if (p.hd != HD || p.lerp_src != 0) return "attention_tc: needs head dim 64 and materialised K/V rows";
-  if (g_enc == nullptr) {
-    void* fn = nullptr;
-    cudaDriverEntryPointQueryResult qres;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres) != cudaSuccess ||
-        qres != cudaDriverEntryPointSuccess || fn == nullptr)
-      return "attention_tc: cuTensorMapEncodeTiled entry point not found";
-    if (cudaFuncSetAttribute(attention_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES) !=
-        cudaSuccess)
-      return "attention_tc: cudaFuncSetAttribute failed";
-    g_enc = reinterpret_cast<PFN_cuTensorMapEncodeTiled_v12000>(fn);
-  }
+  if (!smem_opt_in(attention_tc_kernel, SMEM_BYTES)) return "attention_tc: cudaFuncSetAttribute failed";
   const int cols = p.H * HD;
+  // rows [B, L] x cols, bf16, box = 64 cols x 128 rows of one utterance; rows past L are zero-filled / clipped
   CUtensorMap tq, tk, tv, to;
-  if (const char* e = encode_3d(&tq, p.q, cols, p.Lq, p.B, p.ldq)) return e;
-  if (const char* e = encode_3d(&tk, p.k, cols, p.Lk, p.B, p.ldkv)) return e;
-  if (const char* e = encode_3d(&tv, p.v, cols, p.Lk, p.B, p.ldkv)) return e;
-  if (const char* e = encode_3d(&to, p.out, cols, p.Lq, p.B, p.ldo)) return e;
+  if (const char* e = tma_encode_3d(&tq, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, p.q, cols, p.Lq, p.B, p.ldq, 64, 128)) return e;
+  if (const char* e = tma_encode_3d(&tk, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, p.k, cols, p.Lk, p.B, p.ldkv, 64, 128)) return e;
+  if (const char* e = tma_encode_3d(&tv, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, p.v, cols, p.Lk, p.B, p.ldkv, 64, 128)) return e;
+  if (const char* e = tma_encode_3d(&to, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, p.out, cols, p.Lq, p.B, p.ldo, 64, 128)) return e;
   AttnTcDev d;
   d.Lq = p.Lq; d.Lk = p.Lk;
   d.scale_log2 = 1.4426950408889634f / sqrtf(static_cast<float>(HD));

@@ -20,14 +20,6 @@ namespace {
 
 std::string g_create_error;
 
-inline uint16_t f2bf_host(float f) {
-  uint32_t u;
-  memcpy(&u, &f, 4);
-  if ((u & 0x7fffffffu) > 0x7f800000u) return static_cast<uint16_t>((u >> 16) | 0x40);
-  u += 0x7fffu + ((u >> 16) & 1u);
-  return static_cast<uint16_t>(u >> 16);
-}
-
 __global__ void op_to_f32_kernel(const __nv_bfloat16* in, float* out, size_t n) {
   size_t i = blockIdx.x * static_cast<size_t>(blockDim.x) + threadIdx.x;
   if (i < n) out[i] = __bfloat162float(in[i]);
@@ -325,7 +317,7 @@ int linear(avsep_handle* h, cudaStream_t s, const char* label, const void* A, in
   if (act == ACT_GELU && h->cfg.precision == AVSEP_PREC_BF16 && out_f32 == nullptr) e.act = ACT_GELU_BF16;
   e.out_f32 = out_f32; e.ld_f32 = N;
   e.out_op = out_op; e.ld_op = N;
-  CKL(label, launch_gemm(s, h->cfg.precision, p, e));
+  CKL(label, launch_gemm(s, h->cfg.precision, p, e, h->num_sms));
   return 0;
 }
 
@@ -343,18 +335,18 @@ int gemm_resid_ln(avsep_handle* h, cudaStream_t s, const char* label, const Gemm
     e.out_f32 = x_out; e.ld_f32 = p.N;
     e.ln_gamma = g; e.ln_beta = b;
     e.out_op = out_op; e.ld_op = p.N;
-    CKL(label, launch_gemm(s, prec, p, e));
+    CKL(label, launch_gemm(s, prec, p, e, h->num_sms));
     return 0;
   }
   e.kind = EPI_STD;
   e.out_op = nullptr;
   if (resid != nullptr) {
     e.out_f32 = y; e.ld_f32 = p.N;
-    CKL(label, launch_gemm(s, prec, p, e));
+    CKL(label, launch_gemm(s, prec, p, e, h->num_sms));
     CKL("add_layernorm", launch_add_layernorm(s, prec, resid, y, g, b, x_out, out_op, rows_out, p.N));
   } else {
     e.out_f32 = x_out; e.ld_f32 = p.N;
-    CKL(label, launch_gemm(s, prec, p, e));
+    CKL(label, launch_gemm(s, prec, p, e, h->num_sms));
     CKL("add_layernorm", launch_add_layernorm(s, prec, x_out, nullptr, g, b, nullptr, out_op, rows_out, p.N));
   }
   return 0;
@@ -476,7 +468,7 @@ int audio_frontend(avsep_handle* h, cudaStream_t s, Workspace& w, const float* m
     e.bias = h->bc1; e.act = ACT_RELU; e.rowmap = ROW_PAD2PAD; e.Lp = T + 2;
     e.lens = w.lens;
     e.out_op = w.h1; e.ld_op = d;
-    CKL("gemm.conv1d_0", launch_gemm(s, prec, p, e));
+    CKL("gemm.conv1d_0", launch_gemm(s, prec, p, e, h->num_sms));
   }
   if (pl.stack_a && pl.pro) return 0;
   {
@@ -488,7 +480,7 @@ int audio_frontend(avsep_handle* h, cudaStream_t s, Workspace& w, const float* m
     e.pe = h->pe_a;
     if (pl.stack_a) {
       e.out_f32 = w.x_a; e.ld_f32 = d;
-      CKL("gemm.conv1d_2", launch_gemm(s, prec, p, e));
+      CKL("gemm.conv1d_2", launch_gemm(s, prec, p, e, h->num_sms));
     } else if (gemm_resid_ln(h, s, "gemm.conv1d_2", p, e, nullptr, w.x_a, h->enc_a[0].n1g, h->enc_a[0].n1b, w.a_op,
                              B * T, w.y_a)) {
       return 1;
@@ -511,7 +503,7 @@ int visual_frontend(avsep_handle* h, cudaStream_t s, Workspace& w, const float* 
   e.bias = h->bproj; e.pe = h->pe_v; e.pe_period = N;
   if (pl.stack_v) {
     e.out_f32 = w.x_v; e.ld_f32 = d;
-    CKL("gemm.frame_proj", launch_gemm(s, h->cfg.precision, p, e));
+    CKL("gemm.frame_proj", launch_gemm(s, h->cfg.precision, p, e, h->num_sms));
   } else if (gemm_resid_ln(h, s, "gemm.frame_proj", p, e, nullptr, w.x_v, h->enc_v[0].n1g, h->enc_v[0].n1b, w.v_op, Mv,
                            w.y_v)) {
     return 1;
@@ -599,7 +591,7 @@ int decoder_stage(avsep_handle* h, cudaStream_t s, Workspace& w, const float* mi
   e.bias = h->bdec3;
   e.mixed = mixed; e.masks = masks; e.separated = separated; e.F = F; e.S = S; e.T = T;
   e.lens = w.lens;
-  CKL("gemm.dec3_tail", launch_gemm(s, h->cfg.precision, dense(w.ffn_a, Ma, 2 * d, h->wdec3, S * F), e));
+  CKL("gemm.dec3_tail", launch_gemm(s, h->cfg.precision, dense(w.ffn_a, Ma, 2 * d, h->wdec3, S * F), e, h->num_sms));
   return 0;
 }
 
@@ -773,7 +765,7 @@ struct ArenaBuilder {
       return add(field, tmp.data(), n * 4);
     }
     std::vector<uint16_t> tmp(n);
-    for (size_t i = 0; i < n; ++i) tmp[i] = f2bf_host(src[i]);
+    for (size_t i = 0; i < n; ++i) tmp[i] = f2bf(src[i]);
     add(field, tmp.data(), n * 2);
   }
   void add_op(const void*& field, const HostTensor* t, bool tf32) { add_op(field, t->data.data(), t->data.size(), tf32); }
@@ -838,7 +830,7 @@ int avsep_create(const avsep_config* cfg, avsep_handle** out) {
   if (cudaGetDeviceProperties(&prop, cfg->device) != cudaSuccess) return fail(nullptr, "avsep_create: device query failed");
   if (prop.major != 10) return fail(nullptr, "avsep_create: kernels are built for sm_100a (B200) only");
   if (cudaSetDevice(cfg->device) != cudaSuccess) return fail(nullptr, "avsep_create: cudaSetDevice failed");
-  if (const char* e = gemm_init()) return fail(nullptr, e);
+  if (const char* e = tma_init()) return fail(nullptr, e);
   if (const char* e = fft512_init_tables()) return fail(nullptr, e);
   avsep_handle* h = new avsep_handle();
   h->cfg = *cfg;
@@ -1561,7 +1553,7 @@ int avsep_test_gemm(avsep_handle* h, const void* A, const void* W, const float* 
   const GemmProblem p = dense(A, M, K, W, N);
   GemmEpilogue e;
   e.bias = bias; e.act = act; e.out_f32 = out; e.ld_f32 = N;
-  CK(launch_gemm(static_cast<cudaStream_t>(cuda_stream), h->cfg.precision, p, e, force_bn));
+  CK(launch_gemm(static_cast<cudaStream_t>(cuda_stream), h->cfg.precision, p, e, h->num_sms, force_bn));
   return 0;
 }
 
@@ -1575,7 +1567,7 @@ int avsep_test_gemm_ln(avsep_handle* h, const void* A, const void* W, const floa
   e.kind = EPI_LN;
   e.bias = bias; e.resid = x; e.out_f32 = x; e.ld_f32 = N; e.ln_gamma = gamma; e.ln_beta = beta;
   e.out_op = out_op; e.ld_op = N;
-  CK(launch_gemm(static_cast<cudaStream_t>(cuda_stream), h->cfg.precision, p, e));
+  CK(launch_gemm(static_cast<cudaStream_t>(cuda_stream), h->cfg.precision, p, e, h->num_sms));
   return 0;
 }
 
@@ -1608,7 +1600,7 @@ int avsep_test_gemm_trace(avsep_handle* h, const void* A, const void* W, const f
     e.out_op = out_op; e.ld_op = N;
     e.out_f32 = out_op ? nullptr : x_or_out; e.ld_f32 = N;
   }
-  CK(launch_gemm(static_cast<cudaStream_t>(cuda_stream), h->cfg.precision, p, e, 0, trace_dev));
+  CK(launch_gemm(static_cast<cudaStream_t>(cuda_stream), h->cfg.precision, p, e, h->num_sms, 0, trace_dev));
   return 0;
 }
 
@@ -1687,7 +1679,7 @@ int avsep_test_conv1d(avsep_handle* h, const void* A_padded, const void* W3, con
   p.taps = 3; p.tap_stride = K; p.row_shift = -1;
   GemmEpilogue e;
   e.bias = bias; e.rowmap = ROW_PAD2COMPACT; e.Lp = L + 2; e.out_f32 = out; e.ld_f32 = N;
-  CK(launch_gemm(static_cast<cudaStream_t>(cuda_stream), h->cfg.precision, p, e));
+  CK(launch_gemm(static_cast<cudaStream_t>(cuda_stream), h->cfg.precision, p, e, h->num_sms));
   return 0;
 }
 

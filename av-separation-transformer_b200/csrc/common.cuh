@@ -1,5 +1,7 @@
-// Shared device helpers for the sm_100a kernels: mbarrier, TMA, tcgen05/TMEM wrappers (inline PTX),
-// warp reductions and small math.  Everything here is written for sm_100a only.
+// Device helpers shared by the library's sm_100a kernels (inline PTX): small math, the global timer, the 128-byte
+// swizzle offset, mma.sync / ldmatrix, programmatic dependent launch, mbarrier, TMA and single-CTA tcgen05 / TMEM
+// wrappers.  Only helpers that some library kernel calls live here; the microbenchmarks under tools/ keep their own
+// extras.  Everything here is written for sm_100a only.
 #pragma once
 
 #include <cuda_runtime.h>
@@ -75,13 +77,11 @@ __device__ __forceinline__ float gelu_bf16_grade(float x) {
   return fmaf(hx, xc * p, hx);
 }
 
-// Warpgroup-level register reallocation (all four warps of an aligned warpgroup execute the same instruction).
-template <int N>
-__device__ __forceinline__ void setmaxnreg_inc() { asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(N)); }
-template <int N>
-__device__ __forceinline__ void setmaxnreg_dec() { asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(N)); }
-
-__device__ __forceinline__ float sigmoidf_(float x) { return 1.0f / (1.0f + __expf(-x)); }
+__device__ __forceinline__ float ex2_approx(float x) {
+  float y;
+  asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
+  return y;
+}
 
 // fp32 -> TF32 with round-to-nearest (the tensor core would otherwise truncate the low 13 mantissa bits, which
 // doubles the operand error and biases it towards zero).  Result is an fp32 bit pattern with a 10-bit mantissa.
@@ -94,6 +94,44 @@ __device__ __forceinline__ float round_tf32(float x) {
 __device__ __forceinline__ uint32_t pack_bf16x2(float lo, float hi) {
   __nv_bfloat162 v = __floats2bfloat162_rn(lo, hi);
   return *reinterpret_cast<uint32_t*>(&v);
+}
+
+// Nanoseconds of the GPU's global timer (the debug trace stamps and the flag-wait timeout).
+__device__ __forceinline__ unsigned long long globaltimer() {
+  unsigned long long t;
+  asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t)::"memory");
+  return t;
+}
+
+// Byte offset of 16-byte chunk c of row r in a buffer of 128-byte rows with the 128-byte swizzle (the layout of TMA
+// SWIZZLE_128B boxes and of the UMMA descriptors): the chunk sits at slot c ^ (r & 7).
+__device__ __forceinline__ uint32_t sw128_off(int row, int c) {
+  return static_cast<uint32_t>(row * 128 + ((c ^ (row & 7)) << 4));
+}
+
+// ------------------------------------------------------------------------------------------
+// mma.sync (bf16 operands, fp32 accumulation) and its ldmatrix fragment loads
+// ------------------------------------------------------------------------------------------
+__device__ __forceinline__ void ldmatrix_x4(uint32_t (&r)[4], uint32_t addr) {
+  asm volatile("ldmatrix.sync.aligned.m8n8.x4.shared.b16 {%0,%1,%2,%3}, [%4];"
+               : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3])
+               : "r"(addr));
+}
+__device__ __forceinline__ void ldmatrix_x4_trans(uint32_t (&r)[4], uint32_t addr) {
+  asm volatile("ldmatrix.sync.aligned.m8n8.x4.trans.shared.b16 {%0,%1,%2,%3}, [%4];"
+               : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3])
+               : "r"(addr));
+}
+// c += A (16x16, row) * B (16x8, col)
+__device__ __forceinline__ void mma_bf16_16816(float (&c)[4], uint32_t a0, uint32_t a1, uint32_t a2, uint32_t a3,
+                                               uint32_t b0, uint32_t b1) {
+  asm volatile(
+      "mma.sync.aligned.m16n8k16.row.col.f32.bf16.bf16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
+      : "+f"(c[0]), "+f"(c[1]), "+f"(c[2]), "+f"(c[3])
+      : "r"(a0), "r"(a1), "r"(a2), "r"(a3), "r"(b0), "r"(b1));
+}
+__device__ __forceinline__ void mma_bf16_16816(float (&c)[4], const uint32_t (&a)[4], uint32_t b0, uint32_t b1) {
+  mma_bf16_16816(c, a[0], a[1], a[2], a[3], b0, b1);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -193,38 +231,6 @@ __device__ __forceinline__ void tma_load_3d(void* smem_dst, const CUtensorMap* m
       : "memory");
 }
 
-// Multicast variant: the box lands at the same CTA-relative shared-memory offset in every CTA of the cluster named
-// in cta_mask, and complete_tx is signalled on the mbarrier at the same CTA-relative offset in each of them.
-__device__ __forceinline__ void tma_load_2d_multicast(void* smem_dst, const CUtensorMap* m, uint64_t* bar, int c0,
-                                                      int c1, uint16_t cta_mask) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster"
-      " [%0], [%1, {%4, %5}], [%2], %3;"
-      ::"r"(smem_u32(smem_dst)), "l"(reinterpret_cast<uint64_t>(m)), "r"(smem_u32(bar)), "h"(cta_mask), "r"(c0),
-      "r"(c1)
-      : "memory");
-}
-// TMA load inside a CTA pair (cta_group::2): the box lands in THIS CTA's shared memory, the complete_tx is signalled on
-// the mbarrier at the same CTA-relative offset in CTA `bar_rank` of the cluster (the MMA leader waits for both halves).
-__device__ __forceinline__ void tma_load_2d_cg2(void* smem_dst, const CUtensorMap* m, uint64_t* bar, uint32_t bar_rank,
-                                                int c0, int c1) {
-  uint32_t rbar;
-  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(rbar) : "r"(smem_u32(bar)), "r"(bar_rank));
-  asm volatile(
-      "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
-      ::"r"(smem_u32(smem_dst)), "l"(reinterpret_cast<uint64_t>(m)), "r"(rbar), "r"(c0), "r"(c1)
-      : "memory");
-}
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
-}
-__device__ __forceinline__ void cluster_sync_all() {     // every thread of every CTA in the cluster
-  asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
-  asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-
 // TMA store (shared -> global), bulk-group completion
 __device__ __forceinline__ void tma_store_2d(const CUtensorMap* m, const void* smem_src, int c0, int c1) {
   asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%2, %3}], [%1];"
@@ -234,8 +240,6 @@ __device__ __forceinline__ void tma_store_2d(const CUtensorMap* m, const void* s
 __device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
 // all bulk stores committed by this thread have finished READING their shared-memory source
 __device__ __forceinline__ void bulk_wait_read0() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
-// ... have completed entirely (global writes performed)
-__device__ __forceinline__ void bulk_wait0() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
 __device__ __forceinline__ void named_bar_sync(int id, int nthreads) {
   asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(nthreads) : "memory");
 }
@@ -288,71 +292,6 @@ __device__ __forceinline__ void umma_f16_ts(uint32_t d_tmem, uint32_t a_tmem, ui
 __device__ __forceinline__ void umma_commit(uint64_t* bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar))
                : "memory");
-}
-// Same, arriving on the mbarrier at this CTA-relative offset in every CTA of cta_mask (cluster multicast).
-__device__ __forceinline__ void umma_commit_multicast(uint64_t* bar, uint16_t cta_mask) {
-  asm volatile(
-      "tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-      ::"r"(smem_u32(bar)), "h"(cta_mask)
-      : "memory");
-}
-// ---- cta_group::2: one MMA spans a pair of CTAs (M = 256: 128 rows in each CTA's tensor memory, B split by N halves
-// between the two CTAs' shared memories); issued by one thread of the even-ranked (leader) CTA ----
-__device__ __forceinline__ void tmem_alloc_cg2(uint32_t* smem_result, uint32_t ncols) {   // same warp id in both CTAs
-  asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(smem_result)),
-               "r"(ncols)
-               : "memory");
-  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_dealloc_cg2(uint32_t taddr, uint32_t ncols) {
-  asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
-}
-__device__ __forceinline__ void umma_f16_cg2(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc,
-                                             uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(d_tmem), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-__device__ __forceinline__ void umma_f16_ts_cg2(uint32_t d_tmem, uint32_t a_tmem, uint64_t bdesc, uint32_t idesc,
-                                                uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::2.kind::f16 [%0], [%1], %2, %3, p;\n\t}"
-      ::"r"(d_tmem), "r"(a_tmem), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-// arrive (once all prior MMAs of this thread are complete) on the barrier at this offset in every CTA of cta_mask
-__device__ __forceinline__ void umma_commit_cg2(uint64_t* bar, uint16_t cta_mask) {
-  asm volatile(
-      "tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-      ::"r"(smem_u32(bar)), "h"(cta_mask)
-      : "memory");
-}
-// arrive on the barrier at this CTA-relative offset in CTA `rank` of the cluster
-__device__ __forceinline__ void mbar_arrive_remote(uint64_t* bar, uint32_t rank) {
-  uint32_t raddr;
-  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(raddr) : "r"(smem_u32(bar)), "r"(rank));
-  asm volatile("mbarrier.arrive.shared::cluster.b64 _, [%0];" ::"r"(raddr) : "memory");
-}
-// wait with cluster-scope acquire (the arrivals may come from the peer CTA)
-__device__ __forceinline__ void mbar_wait_cluster(uint64_t* bar, uint32_t parity) {
-  const long long t0 = clock64();
-  for (;;) {
-    uint32_t ok;
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(ok)
-        : "r"(smem_u32(bar)), "r"(parity)
-        : "memory");
-    if (ok) return;
-    if (clock64() - t0 > AVSEP_WATCHDOG_CYCLES) mbar_timeout(bar, parity);
-  }
 }
 __device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
 __device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }

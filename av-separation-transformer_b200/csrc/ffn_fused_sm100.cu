@@ -22,8 +22,6 @@
 #include "common.cuh"
 #include "kernels.h"
 
-#include <cudaTypedefs.h>
-
 namespace avsep {
 
 namespace {
@@ -48,14 +46,7 @@ struct FfnDev {
   unsigned long long* trace;   // optional [grid][64] globaltimer stamps of the CTA's first tile (debug), else null
 };
 
-__device__ __forceinline__ unsigned long long ffn_gtime() {
-  unsigned long long t;
-  asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t)::"memory");
-  return t;
-}
-#define FTRACE(slot) do { if (p.trace != nullptr && lt == 0) p.trace[blockIdx.x * 64 + (slot)] = ffn_gtime(); } while (0)
-
-__device__ __forceinline__ uint32_t soff(int row, int c) { return static_cast<uint32_t>(row * 128 + ((c ^ (row & 7)) << 4)); }
+#define FTRACE(slot) do { if (p.trace != nullptr && lt == 0) p.trace[blockIdx.x * 64 + (slot)] = globaltimer(); } while (0)
 
 __global__ void __launch_bounds__(FFN_THREADS, 1)
 ffn_fused_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmW1,
@@ -85,7 +76,7 @@ ffn_fused_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int m_tiles = (p.M + 127) / 128;
-  if (threadIdx.x == 0 && p.trace != nullptr) p.trace[blockIdx.x * 64] = ffn_gtime();
+  if (threadIdx.x == 0 && p.trace != nullptr) p.trace[blockIdx.x * 64] = globaltimer();
 
   for (int i = threadIdx.x; i < HID; i += FFN_THREADS) sb1[i] = __ldg(p.b1 + i);
   for (int i = threadIdx.x; i < D; i += FFN_THREADS) {
@@ -301,14 +292,14 @@ ffn_fused_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
         if (p.resid != nullptr) {
 #pragma unroll
           for (int c = 0; c < 8; ++c) {
-            const float4 x4 = *reinterpret_cast<const float4*>(sl_q + soff(lane, c));
+            const float4 x4 = *reinterpret_cast<const float4*>(sl_q + sw128_off(lane, c));
             val[ci][4 * c] += x4.x; val[ci][4 * c + 1] += x4.y; val[ci][4 * c + 2] += x4.z; val[ci][4 * c + 3] += x4.w;
           }
         }
         if (p.has_xout) {
 #pragma unroll
           for (int c = 0; c < 8; ++c)
-            *reinterpret_cast<float4*>(sl_q + soff(lane, c)) =
+            *reinterpret_cast<float4*>(sl_q + sw128_off(lane, c)) =
                 make_float4(val[ci][4 * c], val[ci][4 * c + 1], val[ci][4 * c + 2], val[ci][4 * c + 3]);
           fence_proxy_async_smem();
         }
@@ -364,7 +355,7 @@ ffn_fused_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
             u.y = pack_bf16x2(val[ci][8 * c + 2], val[ci][8 * c + 3]);
             u.z = pack_bf16x2(val[ci][8 * c + 4], val[ci][8 * c + 5]);
             u.w = pack_bf16x2(val[ci][8 * c + 6], val[ci][8 * c + 7]);
-            *reinterpret_cast<uint4*>(slab_q + soff(lane, ci * 4 + c)) = u;
+            *reinterpret_cast<uint4*>(slab_q + sw128_off(lane, ci * 4 + c)) = u;
           }
         }
         fence_proxy_async_smem();
@@ -393,22 +384,6 @@ ffn_fused_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
   }
 }
 
-PFN_cuTensorMapEncodeTiled_v12000 g_enc = nullptr;
-
-const char* enc2d(CUtensorMap* map, CUtensorMapDataType dt, int esz, const void* ptr, uint64_t inner, uint64_t outer,
-                  uint64_t ld_elems, uint32_t box_inner, uint32_t box_outer) {
-  if ((reinterpret_cast<uintptr_t>(ptr) & 15) != 0) return "ffn_fused: pointer not 16-byte aligned";
-  cuuint64_t dims[2] = {inner, outer};
-  cuuint64_t strides[1] = {ld_elems * esz};
-  cuuint32_t box[2] = {box_inner, box_outer};
-  cuuint32_t estr[2] = {1, 1};
-  if (g_enc(map, dt, 2, const_cast<void*>(ptr), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-            CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) !=
-      CUDA_SUCCESS)
-    return "ffn_fused: cuTensorMapEncodeTiled failed";
-  return nullptr;
-}
-
 }  // namespace
 
 bool ffn_fusable(int prec, int d_model) { return prec == PREC_BF16 && d_model == D; }
@@ -420,29 +395,16 @@ const char* launch_ffn_fused(cudaStream_t s, const void* a, const void* w1, cons
                              const float* beta, void* out_op, int M, int num_sms, unsigned long long* trace) {
   if (M <= 0) return "ffn_fused: empty problem";
   if (resid != nullptr && resid != x_out) return "ffn_fused: residual must be updated in place";
-  if (g_enc == nullptr) {
-    void* fn = nullptr;
-    cudaDriverEntryPointQueryResult qres;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres) != cudaSuccess ||
-        qres != cudaDriverEntryPointSuccess || fn == nullptr)
-      return "ffn_fused: cuTensorMapEncodeTiled entry point not found";
-    g_enc = reinterpret_cast<PFN_cuTensorMapEncodeTiled_v12000>(fn);
-  }
   CUtensorMap ta, tw1, tw2, tx, top;
-  if (const char* e = enc2d(&ta, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, a, D, M, D, 64, 128)) return e;
-  if (const char* e = enc2d(&tw1, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, w1, D, HID, D, 64, 128)) return e;
-  if (const char* e = enc2d(&tw2, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, w2, HID, D, HID, 64, 128)) return e;
+  if (const char* e = tma_encode_2d(&ta, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, a, D, M, D, 64, 128)) return e;
+  if (const char* e = tma_encode_2d(&tw1, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, w1, D, HID, D, 64, 128)) return e;
+  if (const char* e = tma_encode_2d(&tw2, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, w2, HID, D, HID, 64, 128)) return e;
   tx = ta; top = ta;
   if (x_out != nullptr)
-    if (const char* e = enc2d(&tx, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, x_out, D, M, D, 32, 128)) return e;
+    if (const char* e = tma_encode_2d(&tx, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, x_out, D, M, D, 32, 128)) return e;
   if (out_op != nullptr)
-    if (const char* e = enc2d(&top, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, out_op, D, M, D, 64, 128)) return e;
-  static bool attr_done = false;
-  if (!attr_done) {
-    if (cudaFuncSetAttribute(ffn_fused_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, FFN_SMEM) != cudaSuccess)
-      return "ffn_fused: cudaFuncSetAttribute failed";
-    attr_done = true;
-  }
+    if (const char* e = tma_encode_2d(&top, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, out_op, D, M, D, 64, 128)) return e;
+  if (!smem_opt_in(ffn_fused_kernel, FFN_SMEM)) return "ffn_fused: cudaFuncSetAttribute failed";
   FfnDev d;
   d.b1 = b1; d.b2 = b2; d.gamma = gamma; d.beta = beta; d.resid = resid;
   d.M = M; d.act = act; d.has_xout = x_out != nullptr; d.has_op = out_op != nullptr;

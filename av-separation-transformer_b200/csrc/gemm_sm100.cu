@@ -24,7 +24,6 @@
 #include "common.cuh"
 #include "kernels.h"
 
-#include <cudaTypedefs.h>
 #include <stdio.h>
 
 namespace avsep {
@@ -58,13 +57,8 @@ struct GemmDev {
                                //   (epilogue), +3 epilogue done
 };
 
-__device__ __forceinline__ unsigned long long gtime() {
-  unsigned long long t;
-  asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t)::"memory");
-  return t;
-}
-#define TRACE(slot) do { if (p.trace != nullptr) p.trace[blockIdx.x * 64 + (slot)] = gtime(); } while (0)
-#define TRACE_TILE(lt, k) do { if (p.trace != nullptr && (lt) < 12) p.trace[blockIdx.x * 64 + 8 + 4 * (lt) + (k)] = gtime(); } while (0)
+#define TRACE(slot) do { if (p.trace != nullptr) p.trace[blockIdx.x * 64 + (slot)] = globaltimer(); } while (0)
+#define TRACE_TILE(lt, k) do { if (p.trace != nullptr && (lt) < 12) p.trace[blockIdx.x * 64 + 8 + 4 * (lt) + (k)] = globaltimer(); } while (0)
 
 // 32-byte (full-sector) global store: one request per thread writes a whole sector of its row.
 __device__ __forceinline__ void st_global_v8(void* ptr, uint32_t a, uint32_t b, uint32_t c, uint32_t d, uint32_t e,
@@ -116,7 +110,6 @@ __device__ __forceinline__ void store_op_chunk(void* out_op, size_t off, const f
 // Thread-per-row accesses (lane = row) and row-contiguous cooperative accesses (8 lanes = one 128-byte row) are both
 // bank-conflict free, so the epilogue can read TMEM with thread = row and still move whole 128-byte lines to and
 // from global memory (4 rows per instruction instead of 32 partial lines).
-__device__ __forceinline__ uint32_t stg_off(int row, int c) { return static_cast<uint32_t>(row * 128 + ((c ^ (row & 7)) << 4)); }
 
 // global [32 rows x 128 B] -> buffer.  row_ptr = this lane's row base (already offset to the tile's first column) or 0.
 __device__ __forceinline__ void stg_load_rows(uint8_t* buf, unsigned long long row_ptr, int lane) {
@@ -126,7 +119,7 @@ __device__ __forceinline__ void stg_load_rows(uint8_t* buf, unsigned long long r
     const unsigned long long rp = __shfl_sync(0xffffffffu, row_ptr, row);
     uint4 x = make_uint4(0, 0, 0, 0);
     if (rp != 0) x = *reinterpret_cast<const uint4*>(rp + c * 16);
-    *reinterpret_cast<uint4*>(buf + stg_off(row, c)) = x;
+    *reinterpret_cast<uint4*>(buf + sw128_off(row, c)) = x;
   }
 }
 // buffer -> global [32 rows x 128 B]
@@ -135,26 +128,26 @@ __device__ __forceinline__ void stg_store_rows(const uint8_t* buf, unsigned long
   for (int i = 0; i < 8; ++i) {
     const int row = i * 4 + (lane >> 3), c = lane & 7;
     const unsigned long long rp = __shfl_sync(0xffffffffu, row_ptr, row);
-    if (rp != 0) *reinterpret_cast<uint4*>(rp + c * 16) = *reinterpret_cast<const uint4*>(buf + stg_off(row, c));
+    if (rp != 0) *reinterpret_cast<uint4*>(rp + c * 16) = *reinterpret_cast<const uint4*>(buf + sw128_off(row, c));
   }
 }
 // own row (lane) += 32 fp32 values of the slab
 __device__ __forceinline__ void stg_add_own_f32(const uint8_t* buf, int lane, float (&x)[32]) {
 #pragma unroll
   for (int c = 0; c < 8; ++c) {
-    const float4 v4 = *reinterpret_cast<const float4*>(buf + stg_off(lane, c));
+    const float4 v4 = *reinterpret_cast<const float4*>(buf + sw128_off(lane, c));
     x[4 * c] += v4.x; x[4 * c + 1] += v4.y; x[4 * c + 2] += v4.z; x[4 * c + 3] += v4.w;
   }
 }
 __device__ __forceinline__ void stg_write_own_f32(uint8_t* buf, int lane, const float (&x)[32]) {
 #pragma unroll
   for (int c = 0; c < 8; ++c)
-    *reinterpret_cast<float4*>(buf + stg_off(lane, c)) = make_float4(x[4 * c], x[4 * c + 1], x[4 * c + 2], x[4 * c + 3]);
+    *reinterpret_cast<float4*>(buf + sw128_off(lane, c)) = make_float4(x[4 * c], x[4 * c + 1], x[4 * c + 2], x[4 * c + 3]);
 }
 __device__ __forceinline__ void stg_write_own_tf32(uint8_t* buf, int lane, const float (&x)[32]) {
 #pragma unroll
   for (int c = 0; c < 8; ++c)
-    *reinterpret_cast<float4*>(buf + stg_off(lane, c)) =
+    *reinterpret_cast<float4*>(buf + sw128_off(lane, c)) =
         make_float4(round_tf32(x[4 * c]), round_tf32(x[4 * c + 1]), round_tf32(x[4 * c + 2]), round_tf32(x[4 * c + 3]));
 }
 // own row: 32 values as bf16 into chunk slots [slot0, slot0+4) (two calls fill one 128-byte row of 64 bf16)
@@ -166,7 +159,7 @@ __device__ __forceinline__ void stg_write_own_bf16(uint8_t* buf, int lane, int s
     u.y = pack_bf16x2(x[8 * c + 2], x[8 * c + 3]);
     u.z = pack_bf16x2(x[8 * c + 4], x[8 * c + 5]);
     u.w = pack_bf16x2(x[8 * c + 6], x[8 * c + 7]);
-    *reinterpret_cast<uint4*>(buf + stg_off(lane, slot0 + c)) = u;
+    *reinterpret_cast<uint4*>(buf + sw128_off(lane, slot0 + c)) = u;
   }
 }
 
@@ -917,38 +910,13 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
 // ------------------------------------------------------------------------------------------
 // host side
 // ------------------------------------------------------------------------------------------
-PFN_cuTensorMapEncodeTiled_v12000 g_encode = nullptr;
-int g_num_sms = 0;
-
-const char* encode_2d(CUtensorMap* map, bool tf32, const void* ptr, uint64_t inner, uint64_t outer, uint64_t ld_elems,
-                      uint32_t box_inner, uint32_t box_outer) {
-  const uint64_t esz = tf32 ? 4 : 2;   // tf32 == true also serves plain fp32 tensors (epilogue slabs)
-  if ((reinterpret_cast<uintptr_t>(ptr) & 15) != 0) return "gemm: operand pointer not 16-byte aligned";
-  if (((ld_elems * esz) & 15) != 0) return "gemm: operand leading dimension not a multiple of 16 bytes";
-  cuuint64_t dims[2] = {inner, outer};
-  cuuint64_t strides[1] = {ld_elems * esz};
-  cuuint32_t box[2] = {box_inner, box_outer};
-  cuuint32_t estr[2] = {1, 1};
-  CUresult r = g_encode(map, tf32 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2,
-                        const_cast<void*>(ptr), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                        CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                        CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) return "gemm: cuTensorMapEncodeTiled failed";
-  return nullptr;
-}
-
 template <int EPI, bool TF32>
 const char* launch_cfg(cudaStream_t s, const CUtensorMap& ta, const CUtensorMap& tw, const CUtensorMap& top,
-                       const CUtensorMap& tf32m, const GemmDev& d) {
-  static bool attr_done = false;
+                       const CUtensorMap& tf32m, const GemmDev& d, int num_sms) {
   auto kern = gemm_tcgen05_kernel<EPI, TF32>;
-  if (!attr_done) {
-    if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_TOTAL) != cudaSuccess)
-      return "gemm: cudaFuncSetAttribute(smem) failed";
-    attr_done = true;
-  }
+  if (!smem_opt_in(kern, SMEM_TOTAL)) return "gemm: cudaFuncSetAttribute(smem) failed";
   const int tiles = ((d.M + BM - 1) / BM) * ((d.N + d.n_tile - 1) / d.n_tile);
-  const int grid = tiles < g_num_sms ? tiles : g_num_sms;
+  const int grid = tiles < num_sms ? tiles : num_sms;
   if (launch_pdl(kern, dim3(grid), dim3(NUM_THREADS), SMEM_TOTAL, s, ta, tw, top, tf32m, d) != cudaSuccess) {
     cudaGetLastError();
     return "gemm: kernel launch failed";
@@ -958,27 +926,10 @@ const char* launch_cfg(cudaStream_t s, const CUtensorMap& ta, const CUtensorMap&
 
 }  // namespace
 
-const char* gemm_init() {
-  if (g_encode != nullptr) return nullptr;
-  void* fn = nullptr;
-  cudaDriverEntryPointQueryResult qres;
-  if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres) != cudaSuccess ||
-      qres != cudaDriverEntryPointSuccess || fn == nullptr)
-    return "gemm: cuTensorMapEncodeTiled entry point not found (driver too old?)";
-  int dev = 0;
-  cudaDeviceProp prop;
-  if (cudaGetDevice(&dev) != cudaSuccess || cudaGetDeviceProperties(&prop, dev) != cudaSuccess)
-    return "gemm: device query failed";
-  g_num_sms = prop.multiProcessorCount;
-  g_encode = reinterpret_cast<PFN_cuTensorMapEncodeTiled_v12000>(fn);
-  return nullptr;
-}
-
 bool gemm_ln_fusable(int N) { return N <= BN_MAX && N >= 32 && (N % 32) == 0; }
 
-const char* launch_gemm(cudaStream_t s, int prec, const GemmProblem& p, const GemmEpilogue& e, int force_bn,
-                        unsigned long long* trace) {
-  if (const char* err = gemm_init()) return err;
+const char* launch_gemm(cudaStream_t s, int prec, const GemmProblem& p, const GemmEpilogue& e, int num_sms,
+                        int force_bn, unsigned long long* trace) {
   if (p.M <= 0 || p.N <= 0 || p.K <= 0) return "gemm: empty problem";
   const bool tf32 = (prec == PREC_TF32);
   const int m_tiles = (p.M + BM - 1) / BM;
@@ -998,7 +949,7 @@ const char* launch_gemm(cudaStream_t s, int prec, const GemmProblem& p, const Ge
     for (int bn = BN_MAX; bn >= 64; bn -= 64) {
       const int ntiles = (p.N + bn - 1) / bn;
       const int width = ((p.N + ntiles - 1) / ntiles + 15) / 16 * 16;
-      const long rounds = (static_cast<long>(m_tiles) * ntiles + g_num_sms - 1) / g_num_sms;
+      const long rounds = (static_cast<long>(m_tiles) * ntiles + num_sms - 1) / num_sms;
       const long cost = rounds * (128 + width);
       if (best_cost < 0 || cost < best_cost) { best_cost = cost; best = width; }
     }
@@ -1011,9 +962,11 @@ const char* launch_gemm(cudaStream_t s, int prec, const GemmProblem& p, const Ge
   d.e = e;
   d.trace = trace;
   CUtensorMap ta, tw;
+  const CUtensorMapDataType op_dt = tf32 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
+  const int op_esz = tf32 ? 4 : 2;
   const uint32_t box_k = tf32 ? 32 : 64;
-  if (const char* err = encode_2d(&ta, tf32, p.A, p.K, p.rowsA, p.lda, box_k, BM)) return err;
-  if (const char* err = encode_2d(&tw, tf32, p.W, static_cast<uint64_t>(p.ldw), p.N, p.ldw, box_k, n_tile)) return err;
+  if (const char* err = tma_encode_2d(&ta, op_dt, op_esz, p.A, p.K, p.rowsA, p.lda, box_k, BM)) return err;
+  if (const char* err = tma_encode_2d(&tw, op_dt, op_esz, p.W, p.ldw, p.N, p.ldw, box_k, n_tile)) return err;
   // Epilogue I/O through TMA slabs: rows map one-to-one (no Conv1d halo remap), columns in 64-wide units.
   CUtensorMap top = ta, tf32m = ta;   // placeholders when unused
   bool use_tma = e.kind != EPI_TAIL && e.rowmap == ROW_IDENT && (p.N % 64 == 0) && (n_tile % 64 == 0);
@@ -1024,19 +977,19 @@ const char* launch_gemm(cudaStream_t s, int prec, const GemmProblem& p, const Ge
   }
   if (use_tma) {
     if (e.out_op != nullptr) {
-      if (encode_2d(&top, tf32, e.out_op, p.N, p.M, e.ld_op, tf32 ? 32 : 64, BM)) use_tma = false;
+      if (tma_encode_2d(&top, op_dt, op_esz, e.out_op, p.N, p.M, e.ld_op, box_k, BM)) use_tma = false;
     }
     if (use_tma && e.out_f32 != nullptr) {
-      if (encode_2d(&tf32m, true, e.out_f32, p.N, p.M, e.ld_f32, 32, BM)) use_tma = false;
+      if (tma_encode_2d(&tf32m, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, e.out_f32, p.N, p.M, e.ld_f32, 32, BM)) use_tma = false;
     }
   }
   d.use_tma = use_tma ? 1 : 0;
   switch (e.kind) {
-    case EPI_STD: return tf32 ? launch_cfg<EPI_STD, true>(s, ta, tw, top, tf32m, d) : launch_cfg<EPI_STD, false>(s, ta, tw, top, tf32m, d);
-    case EPI_TAIL: return tf32 ? launch_cfg<EPI_TAIL, true>(s, ta, tw, top, tf32m, d) : launch_cfg<EPI_TAIL, false>(s, ta, tw, top, tf32m, d);
+    case EPI_STD: return tf32 ? launch_cfg<EPI_STD, true>(s, ta, tw, top, tf32m, d, num_sms) : launch_cfg<EPI_STD, false>(s, ta, tw, top, tf32m, d, num_sms);
+    case EPI_TAIL: return tf32 ? launch_cfg<EPI_TAIL, true>(s, ta, tw, top, tf32m, d, num_sms) : launch_cfg<EPI_TAIL, false>(s, ta, tw, top, tf32m, d, num_sms);
     case EPI_LN:
-      if (use_tma) return tf32 ? launch_cfg<EPI_LN_TMA, true>(s, ta, tw, top, tf32m, d) : launch_cfg<EPI_LN_TMA, false>(s, ta, tw, top, tf32m, d);
-      return tf32 ? launch_cfg<EPI_LN, true>(s, ta, tw, top, tf32m, d) : launch_cfg<EPI_LN, false>(s, ta, tw, top, tf32m, d);
+      if (use_tma) return tf32 ? launch_cfg<EPI_LN_TMA, true>(s, ta, tw, top, tf32m, d, num_sms) : launch_cfg<EPI_LN_TMA, false>(s, ta, tw, top, tf32m, d, num_sms);
+      return tf32 ? launch_cfg<EPI_LN, true>(s, ta, tw, top, tf32m, d, num_sms) : launch_cfg<EPI_LN, false>(s, ta, tw, top, tf32m, d, num_sms);
     default: return "gemm: unknown epilogue";
   }
 }

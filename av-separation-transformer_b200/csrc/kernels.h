@@ -1,11 +1,42 @@
 // Internal (C++) interface between the C-ABI layer (avsep_api.cu) and the sm_100a kernels.
 #pragma once
 
+#include <cuda.h>
 #include <cuda_runtime.h>
 #include <cuda_bf16.h>
 #include <stdint.h>
+#include <string.h>
 
 namespace avsep {
+
+// fp32 -> bf16 bit pattern, round to nearest even as __float2bfloat16_rn (NaN stays a quiet NaN): every host-side
+// weight packer rounds through this one function, so all uploaded bf16 weights agree with the device conversion.
+inline uint16_t f2bf(float f) {
+  uint32_t u;
+  memcpy(&u, &f, 4);
+  if ((u & 0x7fffffffu) > 0x7f800000u) return static_cast<uint16_t>((u >> 16) | 0x40);
+  u += 0x7fffu + ((u >> 16) & 1u);
+  return static_cast<uint16_t>(u >> 16);
+}
+
+// ---- host helpers of the launchers (launch_util.cu); the const char* functions return nullptr or a static error ----
+// Resolves cuTensorMapEncodeTiled from the driver; called once by avsep_create before any launcher runs.
+const char* tma_init();
+// TMA descriptor of a row-major [outer, inner] tensor with leading dimension ld_elems (elements of esz bytes), moved in
+// boxes of box_outer rows x box_inner elements: 128-byte swizzle, 256-byte L2 promotion, out-of-range elements read as
+// zero and not written.  The pointer must be 16-byte aligned and the row pitch a multiple of 16 bytes.
+const char* tma_encode_2d(CUtensorMap* map, CUtensorMapDataType dt, int esz, const void* ptr, uint64_t inner,
+                          uint64_t outer, uint64_t ld_elems, uint32_t box_inner, uint32_t box_outer);
+// The same for `batches` such tensors stored back to back ([batches, outer, inner]); a box stays inside one batch.
+const char* tma_encode_3d(CUtensorMap* map, CUtensorMapDataType dt, int esz, const void* ptr, uint64_t inner,
+                          uint64_t outer, uint64_t batches, uint64_t ld_elems, uint32_t box_inner, uint32_t box_outer);
+// Raises the kernel's dynamic shared-memory limit to `bytes` unless this process already set it at least that high (up
+// to 48 KB needs no opt-in).  False when the runtime refuses.
+bool smem_opt_in(const void* kern, int bytes);
+template <typename... KArgs>
+bool smem_opt_in(void (*kern)(KArgs...), int bytes) {
+  return smem_opt_in(reinterpret_cast<const void*>(kern), bytes);
+}
 
 // Programmatic dependent launch (PDL) of the forward-path kernels: every kernel launched through launch_pdl calls
 // griddep_wait() before it touches anything its predecessor wrote.  pdl_set(false) = plain stream order.
@@ -88,9 +119,8 @@ __device__ __forceinline__ bool frame_live(const int* lens, int N, int fr) {
 }
 
 // Returns nullptr on success or a static error string.
-const char* gemm_init();   // resolves cuTensorMapEncodeTiled, sets smem attributes
-const char* launch_gemm(cudaStream_t s, int prec, const GemmProblem& p, const GemmEpilogue& e, int force_bn = 0,
-                        unsigned long long* trace = nullptr);   // trace: [grid][8] globaltimer stamps (debug)
+const char* launch_gemm(cudaStream_t s, int prec, const GemmProblem& p, const GemmEpilogue& e, int num_sms,
+                        int force_bn = 0, unsigned long long* trace = nullptr);   // trace: [grid][8] globaltimer stamps (debug)
 bool gemm_ln_fusable(int N);   // EPI_LN usable for this row width
 
 // Fused FFN sub-layer (d_model = 256, bf16): x += W2 act(W1 a + b1) + b2 ; out_op = LayerNorm(x)  (ffn_fused_sm100.cu)

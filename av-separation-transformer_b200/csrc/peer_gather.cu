@@ -66,11 +66,6 @@ __device__ __forceinline__ unsigned ld_acquire_sys(const unsigned* p) {
 __device__ __forceinline__ void st_release_sys(unsigned* p, unsigned v) {
   asm volatile("st.release.sys.global.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
 }
-__device__ __forceinline__ unsigned long long flag_gtime() {
-  unsigned long long t;
-  asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t)::"memory");
-  return t;
-}
 
 // One CTA, thread i raises flag i (its own memory or a peer's).  Stream order puts it after the copies it announces.
 __global__ void flag_signal_kernel(FlagSet f, unsigned value) {
@@ -87,10 +82,10 @@ __global__ void flag_signal_kernel(FlagSet f, unsigned value) {
 __global__ void flag_wait_kernel(FlagSet f, unsigned value, unsigned long long timeout_ns) {
   const int i = threadIdx.x;
   if (i < f.n) {
-    const unsigned long long t0 = flag_gtime();
+    const unsigned long long t0 = globaltimer();
     while (static_cast<int>(ld_acquire_sys(f.ptr[i]) - value) < 0) {
       __nanosleep(200);
-      if (flag_gtime() - t0 > timeout_ns) {
+      if (globaltimer() - t0 > timeout_ns) {
         printf("avsep flag wait: flag %d stuck at %u, waiting for %u\n", i, ld_acquire_sys(f.ptr[i]), value);
         __trap();
       }

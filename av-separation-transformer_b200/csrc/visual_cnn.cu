@@ -39,14 +39,6 @@ struct CnnDev {
   int N;                             // frames per utterance (pitch of frame_lens)
 };
 
-__device__ __forceinline__ void mma16816(float (&c)[4], uint32_t a0, uint32_t a1, uint32_t a2, uint32_t a3,
-                                         uint32_t b0, uint32_t b1) {
-  asm volatile(
-      "mma.sync.aligned.m16n8k16.row.col.f32.bf16.bf16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
-      : "+f"(c[0]), "+f"(c[1]), "+f"(c[2]), "+f"(c[3])
-      : "r"(a0), "r"(a1), "r"(a2), "r"(a3), "r"(b0), "r"(b1));
-}
-
 // Gather state for one accumulator row of a stride-2 / pad-1 3x3 conv: top-left input coordinate and frame base.
 struct RowRef {
   int base;   // word offset of the frame's activation block (or -1 when the row does not exist)
@@ -171,10 +163,10 @@ __global__ void __launch_bounds__(CNN_THREADS, 1) visual_cnn_kernel(const CnnDev
 #pragma unroll
         for (int nt = 0; nt < 4; ++nt) {
           float c[4] = {0.f, 0.f, 0.f, 0.f};
-          mma16816(c, a[0], a[1], a[2], a[3], bw[nt][0], bw[nt][1]);
+          mma_bf16_16816(c, a[0], a[1], a[2], a[3], bw[nt][0], bw[nt][1]);
           if constexpr (SPLIT) {
-            mma16816(c, al[0], al[1], al[2], al[3], bw[nt][0], bw[nt][1]);
-            mma16816(c, a[0], a[1], a[2], a[3], bwl[nt][0], bwl[nt][1]);
+            mma_bf16_16816(c, al[0], al[1], al[2], al[3], bw[nt][0], bw[nt][1]);
+            mma_bf16_16816(c, a[0], a[1], a[2], a[3], bwl[nt][0], bwl[nt][1]);
           }
           const int ch = nt * 8 + 2 * tig;
           const float bb0 = sB1[ch], bb1 = sB1[ch + 1];
@@ -238,14 +230,14 @@ __global__ void __launch_bounds__(CNN_THREADS, 1) visual_cnn_kernel(const CnnDev
 #pragma unroll
             for (int n = 0; n < 4; ++n) {
               const uint2 bw = *reinterpret_cast<const uint2*>(sW2 + (ks * 8 + ng * 4 + n) * 64 + lane * 2);
-              mma16816(acc[0][n], af[0][0], af[0][1], af[0][2], af[0][3], bw.x, bw.y);
-              mma16816(acc[1][n], af[1][0], af[1][1], af[1][2], af[1][3], bw.x, bw.y);
+              mma_bf16_16816(acc[0][n], af[0][0], af[0][1], af[0][2], af[0][3], bw.x, bw.y);
+              mma_bf16_16816(acc[1][n], af[1][0], af[1][1], af[1][2], af[1][3], bw.x, bw.y);
               if constexpr (SPLIT) {
                 const uint2 bl = *reinterpret_cast<const uint2*>(sW2l + (ks * 8 + ng * 4 + n) * 64 + lane * 2);
-                mma16816(acc[0][n], afl[0][0], afl[0][1], afl[0][2], afl[0][3], bw.x, bw.y);
-                mma16816(acc[1][n], afl[1][0], afl[1][1], afl[1][2], afl[1][3], bw.x, bw.y);
-                mma16816(acc[0][n], af[0][0], af[0][1], af[0][2], af[0][3], bl.x, bl.y);
-                mma16816(acc[1][n], af[1][0], af[1][1], af[1][2], af[1][3], bl.x, bl.y);
+                mma_bf16_16816(acc[0][n], afl[0][0], afl[0][1], afl[0][2], afl[0][3], bw.x, bw.y);
+                mma_bf16_16816(acc[1][n], afl[1][0], afl[1][1], afl[1][2], afl[1][3], bw.x, bw.y);
+                mma_bf16_16816(acc[0][n], af[0][0], af[0][1], af[0][2], af[0][3], bl.x, bl.y);
+                mma_bf16_16816(acc[1][n], af[1][0], af[1][1], af[1][2], af[1][3], bl.x, bl.y);
               }
             }
           }
@@ -316,20 +308,20 @@ __global__ void __launch_bounds__(CNN_THREADS, 1) visual_cnn_kernel(const CnnDev
               const uint32_t a1 = o1 >= 0 ? sA2[o1 + q * 8] : 0u;
               const uint32_t a2 = o0 >= 0 ? sA2[o0 + q * 8 + 4] : 0u;
               const uint32_t a3 = o1 >= 0 ? sA2[o1 + q * 8 + 4] : 0u;
-              mma16816(acc[mt][0], a0, a1, a2, a3, bw[q][0].x, bw[q][0].y);
-              mma16816(acc[mt][1], a0, a1, a2, a3, bw[q][1].x, bw[q][1].y);
+              mma_bf16_16816(acc[mt][0], a0, a1, a2, a3, bw[q][0].x, bw[q][0].y);
+              mma_bf16_16816(acc[mt][1], a0, a1, a2, a3, bw[q][1].x, bw[q][1].y);
               if constexpr (SPLIT) {
                 const uint32_t l0 = o0 >= 0 ? sA2l[o0 + q * 8] : 0u;
                 const uint32_t l1 = o1 >= 0 ? sA2l[o1 + q * 8] : 0u;
                 const uint32_t l2 = o0 >= 0 ? sA2l[o0 + q * 8 + 4] : 0u;
                 const uint32_t l3 = o1 >= 0 ? sA2l[o1 + q * 8 + 4] : 0u;
-                mma16816(acc[mt][0], l0, l1, l2, l3, bw[q][0].x, bw[q][0].y);
-                mma16816(acc[mt][1], l0, l1, l2, l3, bw[q][1].x, bw[q][1].y);
+                mma_bf16_16816(acc[mt][0], l0, l1, l2, l3, bw[q][0].x, bw[q][0].y);
+                mma_bf16_16816(acc[mt][1], l0, l1, l2, l3, bw[q][1].x, bw[q][1].y);
                 const int ksl = tap * 4 + q;
                 const uint2 wl0 = __ldg(wbase_l + (ksl * 16 + np * 2) * 32);
                 const uint2 wl1 = __ldg(wbase_l + (ksl * 16 + np * 2 + 1) * 32);
-                mma16816(acc[mt][0], a0, a1, a2, a3, wl0.x, wl0.y);
-                mma16816(acc[mt][1], a0, a1, a2, a3, wl1.x, wl1.y);
+                mma_bf16_16816(acc[mt][0], a0, a1, a2, a3, wl0.x, wl0.y);
+                mma_bf16_16816(acc[mt][1], a0, a1, a2, a3, wl1.x, wl1.y);
               }
             }
           }
@@ -388,14 +380,6 @@ __global__ void __launch_bounds__(CNN_THREADS, 1) visual_cnn_kernel(const CnnDev
     }
     // sIn interior is overwritten and sA1/sA2 fully rewritten next round; the barrier after staging orders it.
   }
-}
-
-inline uint16_t f2bf(float f) {   // round-to-nearest-even, as __float2bfloat16_rn
-  uint32_t u;
-  memcpy(&u, &f, 4);
-  if ((u & 0x7fffffffu) > 0x7f800000u) return static_cast<uint16_t>((u >> 16) | 0x40);
-  u += 0x7fffu + ((u >> 16) & 1u);
-  return static_cast<uint16_t>(u >> 16);
 }
 
 // Pack a [N][K] fp32 matrix into mma.m16n8k16 B-fragment order: [k-step][n-tile][lane][2 words].
@@ -461,18 +445,10 @@ const char* launch_visual_cnn(cudaStream_t s, int prec, const float* frames, int
   d.G = G;
   d.num_groups = (M + G - 1) / G;
   const size_t smem = fixed + per_frame * G;
-  static size_t attr_set = 0;
-  auto k0 = visual_cnn_kernel<false>;
-  auto k1 = visual_cnn_kernel<true>;
-  if (smem > attr_set) {
-    if (cudaFuncSetAttribute(k0, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(cap)) != cudaSuccess ||
-        cudaFuncSetAttribute(k1, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(cap)) != cudaSuccess)
-      return "visual_cnn: cudaFuncSetAttribute failed";
-    attr_set = cap;
-  }
+  auto kern = split ? visual_cnn_kernel<true> : visual_cnn_kernel<false>;
+  if (!smem_opt_in(kern, static_cast<int>(cap))) return "visual_cnn: cudaFuncSetAttribute failed";
   const int grid = d.num_groups < num_sms ? d.num_groups : num_sms;
-  if (prec == PREC_TF32) k1<<<grid, CNN_THREADS, smem, s>>>(d);
-  else k0<<<grid, CNN_THREADS, smem, s>>>(d);
+  kern<<<grid, CNN_THREADS, smem, s>>>(d);
   return cudaGetLastError() == cudaSuccess ? nullptr : "visual_cnn: launch failed";
 }
 

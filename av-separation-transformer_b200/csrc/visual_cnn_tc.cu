@@ -17,7 +17,6 @@
 #include "common.cuh"
 #include "kernels.h"
 
-#include <cudaTypedefs.h>
 #include <string.h>
 
 namespace avsep {
@@ -53,21 +52,8 @@ struct CnnTcDev {
   unsigned long long* trace;   // optional [grid][64] globaltimer stamps of the CTA's 2nd group (debug), else null
 };
 
-__device__ __forceinline__ unsigned long long cnn_gtime() {
-  unsigned long long t;
-  asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t)::"memory");
-  return t;
-}
 #define CTRACE(slot) do { if (p.trace != nullptr && tid == 0 && grp == static_cast<int>(blockIdx.x + gridDim.x)) \
-    p.trace[blockIdx.x * 64 + (slot)] = cnn_gtime(); } while (0)
-
-__device__ __forceinline__ void mma16816(float (&c)[4], uint32_t a0, uint32_t a1, uint32_t a2, uint32_t a3,
-                                         uint32_t b0, uint32_t b1) {
-  asm volatile(
-      "mma.sync.aligned.m16n8k16.row.col.f32.bf16.bf16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
-      : "+f"(c[0]), "+f"(c[1]), "+f"(c[2]), "+f"(c[3])
-      : "r"(a0), "r"(a1), "r"(a2), "r"(a3), "r"(b0), "r"(b1));
-}
+    p.trace[blockIdx.x * 64 + (slot)] = globaltimer(); } while (0)
 
 // act1: 2 pixels per 128-byte line, 16-byte chunk slot XOR-swizzled by the line index.
 __device__ __forceinline__ int act1_chunk_off(int pixel, int c) {   // pixel = f*256 + y*16 + x, c = 8-channel chunk 0..3
@@ -378,7 +364,7 @@ visual_cnn_tc_kernel(const __grid_constant__ CUtensorMap tmW3, const CnnTcDev p)
 #pragma unroll
           for (int nt = 0; nt < 4; ++nt) {
             float cacc[4] = {0.f, 0.f, 0.f, 0.f};
-            mma16816(cacc, a[0], a[1], a[2], a[3], bw1[nt][0], bw1[nt][1]);
+            mma_bf16_16816(cacc, a[0], a[1], a[2], a[3], bw1[nt][0], bw1[nt][1]);
             const float bb0 = bias1[nt][0], bb1 = bias1[nt][1];
             *reinterpret_cast<uint32_t*>(act1 + act1_chunk_off(pix[0], nt) + tig * 4) =
                 pack_bf16x2(fmaxf(cacc[0] + bb0, 0.f), fmaxf(cacc[1] + bb1, 0.f));
@@ -453,14 +439,6 @@ visual_cnn_tc_kernel(const __grid_constant__ CUtensorMap tmW3, const CnnTcDev p)
   }
 }
 
-inline uint16_t f2bf_tc(float f) {
-  uint32_t u;
-  memcpy(&u, &f, 4);
-  if ((u & 0x7fffffffu) > 0x7f800000u) return static_cast<uint16_t>((u >> 16) | 0x40);
-  u += 0x7fffu + ((u >> 16) & 1u);
-  return static_cast<uint16_t>(u >> 16);
-}
-
 }  // namespace
 
 size_t visual_cnn_tc_w2_bytes() { return W2_SLABS * W2_SLAB_BYTES; }
@@ -478,42 +456,21 @@ void visual_cnn_tc_pack(const float* w2, const float* w3, uint8_t* w2_slabs, uin
         const float val = tap < 9 ? w2[static_cast<size_t>(n) * 288 + tap * 32 + c] : 0.f;
         const int chunk = (k >> 3) ^ (n & 7);
         uint16_t* dst = reinterpret_cast<uint16_t*>(w2_slabs + j * W2_SLAB_BYTES + n * 128 + chunk * 16) + (k & 7);
-        *dst = f2bf_tc(val);
+        *dst = f2bf(val);
       }
   uint16_t* o = reinterpret_cast<uint16_t*>(w3_rows);
   for (int t = 0; t < 9; ++t)
     for (int n = 0; n < 128; ++n)
-      for (int c = 0; c < 64; ++c) o[(static_cast<size_t>(t) * 128 + n) * 64 + c] = f2bf_tc(w3[static_cast<size_t>(n) * 576 + t * 64 + c]);
+      for (int c = 0; c < 64; ++c) o[(static_cast<size_t>(t) * 128 + n) * 64 + c] = f2bf(w3[static_cast<size_t>(n) * 576 + t * 64 + c]);
 }
 
 const char* launch_visual_cnn_tc(cudaStream_t s, const float* frames, int M, const CnnWeights& w, const uint8_t* w2_slabs,
                                  const uint8_t* w3_rows, void* pooled, int num_sms, unsigned long long* trace,
                                  const int* frame_lens, int N) {
   if (M <= 0) return "visual_cnn_tc: empty problem";
-  static PFN_cuTensorMapEncodeTiled_v12000 encode = nullptr;
-  if (encode == nullptr) {
-    void* fn = nullptr;
-    cudaDriverEntryPointQueryResult qres;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres) != cudaSuccess ||
-        qres != cudaDriverEntryPointSuccess || fn == nullptr)
-      return "visual_cnn_tc: cuTensorMapEncodeTiled entry point not found";
-    encode = reinterpret_cast<PFN_cuTensorMapEncodeTiled_v12000>(fn);
-  }
-  CUtensorMap tm;
-  cuuint64_t dims[2] = {64, 9 * 128};
-  cuuint64_t strides[1] = {128};
-  cuuint32_t box[2] = {64, 128};
-  cuuint32_t estr[2] = {1, 1};
-  if (encode(&tm, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<uint8_t*>(w3_rows), dims, strides, box, estr,
-             CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-             CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
-    return "visual_cnn_tc: cuTensorMapEncodeTiled failed";
-  static bool attr_done = false;
-  if (!attr_done) {
-    if (cudaFuncSetAttribute(visual_cnn_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, TC_SMEM) != cudaSuccess)
-      return "visual_cnn_tc: cudaFuncSetAttribute failed";
-    attr_done = true;
-  }
+  CUtensorMap tm;   // w3_rows as [9 * 128 rows][64] bf16
+  if (const char* e = tma_encode_2d(&tm, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, w3_rows, 64, 9 * 128, 64, 64, 128)) return e;
+  if (!smem_opt_in(visual_cnn_tc_kernel, TC_SMEM)) return "visual_cnn_tc: cudaFuncSetAttribute failed";
   CnnTcDev d;
   d.frames = frames; d.pooled = reinterpret_cast<__nv_bfloat16*>(pooled);
   d.w1 = w.w1; d.b1 = w.b1; d.w2_slabs = w2_slabs; d.b2 = w.b2; d.b3 = w.b3;

@@ -34,7 +34,6 @@
 #include "common.cuh"
 #include "kernels.h"
 
-#include <cudaTypedefs.h>
 #include <stdlib.h>
 #include <string.h>
 
@@ -104,8 +103,6 @@ struct StackDev {
 
 #define XTRACE(slot) do { if (p.trace != nullptr && lt == 0 && (slot) < 128) p.trace[blockIdx.x * 256 + trace_base + (slot)] = clock64(); } while (0)
 
-__device__ __forceinline__ uint32_t soff(int row, int c) { return static_cast<uint32_t>(row * 128 + ((c ^ (row & 7)) << 4)); }
-
 // Weight items are read by every CTA of every launch: keep them in L2 (evict_last) against the step's streaming traffic
 __device__ __forceinline__ uint64_t l2_policy_evict_last() {
   uint64_t pol;
@@ -125,12 +122,6 @@ __device__ __forceinline__ void tmem_st_32x32b_x8(uint32_t taddr, const uint32_t
   asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};"
                ::"r"(taddr), "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7])
                : "memory");
-}
-
-__device__ __forceinline__ float ex2_approx(float x) {
-  float y;
-  asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
-  return y;
 }
 
 // VARLEN = false (no length arrays): every per-utterance length is p.L / p.kvp_L at compile time, so the uniform
@@ -676,7 +667,7 @@ xformer_stack_kernel(const __grid_constant__ CUtensorMap tmXin, const __grid_con
         uint4 w;
         w.x = pack_bf16x2(y[0], y[1]); w.y = pack_bf16x2(y[2], y[3]);
         w.z = pack_bf16x2(y[4], y[5]); w.w = pack_bf16x2(y[6], y[7]);
-        *reinterpret_cast<uint4*>(slab + soff(r, c)) = w;
+        *reinterpret_cast<uint4*>(slab + sw128_off(r, c)) = w;
       }
     };
     auto ln_to_a = [&](const float* bias, const float* g, const float* b) {
@@ -711,7 +702,7 @@ xformer_stack_kernel(const __grid_constant__ CUtensorMap tmXin, const __grid_con
           if (row_valid) {
 #pragma unroll
             for (int i = 0; i < 8; ++i) {
-              const uint4 w = *reinterpret_cast<const uint4*>(slab + soff(r, i));
+              const uint4 w = *reinterpret_cast<const uint4*>(slab + sw128_off(r, i));
               u[4 * i] = w.x; u[4 * i + 1] = w.y; u[4 * i + 2] = w.z; u[4 * i + 3] = w.w;
             }
           } else {
@@ -816,7 +807,7 @@ xformer_stack_kernel(const __grid_constant__ CUtensorMap tmXin, const __grid_con
                 w.y = pack_bf16x2(__uint_as_float(a[8 * c + 2]) + bk[8 * c + 2], __uint_as_float(a[8 * c + 3]) + bk[8 * c + 3]);
                 w.z = pack_bf16x2(__uint_as_float(a[8 * c + 4]) + bk[8 * c + 4], __uint_as_float(a[8 * c + 5]) + bk[8 * c + 5]);
                 w.w = pack_bf16x2(__uint_as_float(a[8 * c + 6]) + bk[8 * c + 6], __uint_as_float(a[8 * c + 7]) + bk[8 * c + 7]);
-                *reinterpret_cast<uint4*>(smem + OFF_KT + soff(r, part * 2 + c)) = w;
+                *reinterpret_cast<uint4*>(smem + OFF_KT + sw128_off(r, part * 2 + c)) = w;
               }
               fence_proxy_async_smem();
             }
@@ -841,7 +832,7 @@ xformer_stack_kernel(const __grid_constant__ CUtensorMap tmXin, const __grid_con
               w.y = pack_bf16x2(__uint_as_float(a[8 * c + 2]) + bv[8 * c + 2], __uint_as_float(a[8 * c + 3]) + bv[8 * c + 3]);
               w.z = pack_bf16x2(__uint_as_float(a[8 * c + 4]) + bv[8 * c + 4], __uint_as_float(a[8 * c + 5]) + bv[8 * c + 5]);
               w.w = pack_bf16x2(__uint_as_float(a[8 * c + 6]) + bv[8 * c + 6], __uint_as_float(a[8 * c + 7]) + bv[8 * c + 7]);
-              *reinterpret_cast<uint4*>(smem + OFF_VT + soff(r, part * 2 + c)) = w;
+              *reinterpret_cast<uint4*>(smem + OFF_VT + sw128_off(r, part * 2 + c)) = w;
             }
             fence_proxy_async_smem();
             tc_fence_before();
@@ -1170,7 +1161,7 @@ xformer_stack_kernel(const __grid_constant__ CUtensorMap tmXin, const __grid_con
               w.z = pack_bf16x2(w0 * a1.x + w1 * b1.x, w0 * a1.y + w1 * b1.y);
               w.w = pack_bf16x2(w0 * a1.z + w1 * b1.z, w0 * a1.w + w1 * b1.w);
             }
-            *reinterpret_cast<uint4*>(slab + soff(r, c)) = w;
+            *reinterpret_cast<uint4*>(slab + sw128_off(r, c)) = w;
           }
           fence_proxy_async_smem();
           tc_fence_before();
@@ -1236,7 +1227,7 @@ xformer_stack_kernel(const __grid_constant__ CUtensorMap tmXin, const __grid_con
             uint8_t* slab = smem + OFF_A + (part * 2 + c) * SLAB;
 #pragma unroll
             for (int i = 0; i < 8; ++i)
-              *reinterpret_cast<uint4*>(slab + soff(r, i)) =
+              *reinterpret_cast<uint4*>(slab + sw128_off(r, i)) =
                   make_uint4(vu[c * 32 + 4 * i], vu[c * 32 + 4 * i + 1], vu[c * 32 + 4 * i + 2], vu[c * 32 + 4 * i + 3]);
           }
           fence_proxy_async_smem();
@@ -1280,30 +1271,6 @@ xformer_stack_kernel(const __grid_constant__ CUtensorMap tmXin, const __grid_con
     tc_fence_after();
     tmem_dealloc(tmem_base, 512);
   }
-}
-
-PFN_cuTensorMapEncodeTiled_v12000 g_enc = nullptr;
-
-const char* enc2d(CUtensorMap* map, CUtensorMapDataType dt, int esz, const void* ptr, uint64_t inner, uint64_t outer,
-                  uint64_t ld_elems, uint32_t box_inner, uint32_t box_outer) {
-  if ((reinterpret_cast<uintptr_t>(ptr) & 15) != 0) return "xformer_stack: pointer not 16-byte aligned";
-  cuuint64_t dims[2] = {inner, outer};
-  cuuint64_t strides[1] = {ld_elems * esz};
-  cuuint32_t box[2] = {box_inner, box_outer};
-  cuuint32_t estr[2] = {1, 1};
-  if (g_enc(map, dt, 2, const_cast<void*>(ptr), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-            CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) !=
-      CUDA_SUCCESS)
-    return "xformer_stack: cuTensorMapEncodeTiled failed";
-  return nullptr;
-}
-
-inline uint16_t f2bf(float f) {
-  uint32_t u;
-  memcpy(&u, &f, 4);
-  if ((u & 0x7fffffffu) > 0x7f800000u) return static_cast<uint16_t>((u >> 16) | 0x40);
-  u += 0x7fffu + ((u >> 16) & 1u);
-  return static_cast<uint16_t>(u >> 16);
 }
 
 // [nrows x 64] bf16 tile of W (row-major, leading dimension ld) starting at (row0, col0), written as the 128B-swizzled
@@ -1484,17 +1451,6 @@ const char* launch_xformer_stack(cudaStream_t s, const StackProblem& sp, int num
       return "xformer_stack: the fused decoder follows the fusion stack and replaces its outputs";
     if (!xformer_decoder_usable(sp.S, sp.F)) return "xformer_stack: speaker count / freq_bins not supported by the fused decoder";
   }
-  if (g_enc == nullptr) {
-    void* fn = nullptr;
-    cudaDriverEntryPointQueryResult qres;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres) != cudaSuccess ||
-        qres != cudaDriverEntryPointSuccess || fn == nullptr)
-      return "xformer_stack: cuTensorMapEncodeTiled entry point not found";
-    if (cudaFuncSetAttribute(xformer_stack_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, STACK_SMEM) != cudaSuccess ||
-        cudaFuncSetAttribute(xformer_stack_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, STACK_SMEM) != cudaSuccess)
-      return "xformer_stack: cudaFuncSetAttribute failed";
-    g_enc = reinterpret_cast<PFN_cuTensorMapEncodeTiled_v12000>(fn);
-  }
   int U = 1;                                   // utterances per tile: the largest power of two with U * L <= 128
   while (U < 16 && 2 * U * sp.L <= 128) U *= 2;
   const int stride = 128 / U;
@@ -1502,20 +1458,20 @@ const char* launch_xformer_stack(cudaStream_t s, const StackProblem& sp, int num
   const int n_tiles = (sp.B + U - 1) / U;
   CUtensorMap tin, tout, top, tkv;
   if (pro) {
-    if (const char* e = enc2d(&tkv, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, sp.pro_a, sp.pro_k, sp.pro_rows, sp.pro_k, 64, stride)) return e;
+    if (const char* e = tma_encode_2d(&tkv, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, sp.pro_a, sp.pro_k, sp.pro_rows, sp.pro_k, 64, stride)) return e;
     tin = tkv;
   } else {
-    if (const char* e = enc2d(&tin, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, sp.x_in, D, M, D, 32, sp.L)) return e;
+    if (const char* e = tma_encode_2d(&tin, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, sp.x_in, D, M, D, 32, sp.L)) return e;
     tkv = tin;
   }
   tout = tin; top = tin;
   if (sp.out_x)
-    if (const char* e = enc2d(&tout, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, sp.out_x, D, M, D, 32, sp.L)) return e;
+    if (const char* e = tma_encode_2d(&tout, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, sp.out_x, D, M, D, 32, sp.L)) return e;
   if (sp.out_op)
-    if (const char* e = enc2d(&top, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, sp.out_op, D, M, D, 64, sp.L)) return e;
+    if (const char* e = tma_encode_2d(&top, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, sp.out_op, D, M, D, 64, sp.L)) return e;
   if (sp.cross) {
     if (sp.kv == nullptr || sp.kv_ld < sp.n_layers * 2 * D) return "xformer_stack: cross-attention needs the K|V rows";
-    if (const char* e = enc2d(&tkv, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, sp.kv, sp.kv_ld, M, sp.kv_ld, 64, sp.L)) return e;
+    if (const char* e = tma_encode_2d(&tkv, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, sp.kv, sp.kv_ld, M, sp.kv_ld, 64, sp.L)) return e;
   }
   StackDev d{};
   d.wstream = sp.wstream; d.fin_gamma = sp.fin_gamma; d.fin_beta = sp.fin_beta;
@@ -1535,6 +1491,7 @@ const char* launch_xformer_stack(cudaStream_t s, const StackProblem& sp, int num
   d.mixed = sp.mixed; d.masks = sp.masks; d.separated = sp.separated;
   const int grid = n_tiles < num_sms ? n_tiles : num_sms;
   auto kern = (d.lens != nullptr || d.kvp_lens != nullptr) ? xformer_stack_kernel<true> : xformer_stack_kernel<false>;
+  if (!smem_opt_in(kern, STACK_SMEM)) return "xformer_stack: cudaFuncSetAttribute failed";
   if (launch_pdl(kern, dim3(grid), dim3(STACK_THREADS), STACK_SMEM, s, tin, tout, top, tkv, d) !=
       cudaSuccess) {
     cudaGetLastError();

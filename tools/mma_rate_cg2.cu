@@ -4,6 +4,52 @@
 #include <cstdio>
 using namespace avsep;
 
+// ---- cta_group::2: one MMA spans a pair of CTAs (M = 256: 128 rows in each CTA's tensor memory, B split by N halves
+// between the two CTAs' shared memories); issued by one thread of the even-ranked (leader) CTA ----
+__device__ __forceinline__ void tmem_alloc_cg2(uint32_t* smem_result, uint32_t ncols) {   // same warp id in both CTAs
+  asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(smem_result)),
+               "r"(ncols)
+               : "memory");
+  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
+}
+__device__ __forceinline__ void tmem_dealloc_cg2(uint32_t taddr, uint32_t ncols) {
+  asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
+}
+__device__ __forceinline__ void umma_f16_cg2(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc,
+                                             uint32_t accumulate) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}"
+      ::"r"(d_tmem), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
+__device__ __forceinline__ void umma_f16_ts_cg2(uint32_t d_tmem, uint32_t a_tmem, uint64_t bdesc, uint32_t idesc,
+                                                uint32_t accumulate) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::2.kind::f16 [%0], [%1], %2, %3, p;\n\t}"
+      ::"r"(d_tmem), "r"(a_tmem), "l"(bdesc), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
+// arrive (once all prior MMAs of this thread are complete) on the barrier at this offset in every CTA of cta_mask
+__device__ __forceinline__ void umma_commit_cg2(uint64_t* bar, uint16_t cta_mask) {
+  asm volatile(
+      "tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
+      ::"r"(smem_u32(bar)), "h"(cta_mask)
+      : "memory");
+}
+__device__ __forceinline__ uint32_t cluster_ctarank() {
+  uint32_t r;
+  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
+  return r;
+}
+__device__ __forceinline__ void cluster_sync_all() {     // every thread of every CTA in the cluster
+  asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
+  asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
+}
+
 __global__ void __launch_bounds__(64, 1) mma_rate_cg2_kernel(int N, int a_in_tmem, int reps, long long* out) {
   extern __shared__ __align__(1024) uint8_t smem[];
   __shared__ uint64_t bar;
