@@ -91,7 +91,7 @@ class Engine:
             raise RuntimeError("avsep_create: " + self.lib.avsep_last_error(None).decode())
         self.h = h
         self._keep = []
-        self._len_bufs = {}   # (name, stream) -> engine-owned int32 device buffer (stable graph key per stream)
+        self._len_bufs = {}   # ((method, name), stream) -> engine-owned int32 device buffer (stable graph key)
 
     def close(self):
         if getattr(self, "h", None):
@@ -182,34 +182,40 @@ class Engine:
                     raise ValueError(f"{what}: output buffers must be contiguous float32 {want}, got {tuple(t.shape)}")
         return B, T, N, Hh, Ww
 
-    def _lengths(self, v, name: str, B: int, limit: int):
+    def _lengths(self, v, name: str, B: int, limit: int, what: str = "forward"):
         """Per-utterance lengths -> int32 device tensor (or None).  A list, numpy array or CPU integer tensor is
         validated here (B entries, 1 <= v <= limit) and copied into an engine-owned buffer of the current stream, so
         the pointer - and with it the CUDA-graph key - stays the same from call to call, and the copy is ordered after
-        the previous forward on that stream that read the buffer (one buffer per stream: forwards on two streams never
-        share one).  The copy goes through pinned memory and does not block the host.  An int32 tensor on the engine's
-        device is passed through without reading it: the library clamps its values to [1, limit]."""
+        the previous call on that stream that read the buffer (one buffer per method, name and stream: calls on two
+        streams never share one).  The copy goes through pinned memory and does not block the host.  An int32 tensor
+        on the engine's device is passed through without reading it: the library clamps its values to [1, limit].
+        ``what`` names the calling method in the error messages."""
         if v is None:
             return None
         if isinstance(v, torch.Tensor) and v.is_cuda:
             if v.device.index != self.device or v.dtype != torch.int32 or tuple(v.shape) != (B,) or not v.is_contiguous():
-                raise ValueError(f"forward: a device {name} tensor must be contiguous int32 ({B},) on cuda:{self.device}")
+                raise ValueError(f"{what}: a device {name} tensor must be contiguous int32 ({B},) on cuda:{self.device}")
             return v
         a = v.numpy() if isinstance(v, torch.Tensor) else np.asarray(v)
         if a.shape != (B,):
-            raise ValueError(f"forward: {name} must have one entry per utterance ({B}), got shape {a.shape}")
+            raise ValueError(f"{what}: {name} must have one entry per utterance ({B}), got shape {a.shape}")
         if a.dtype == np.bool_ or not np.issubdtype(a.dtype, np.integer):
-            raise ValueError(f"forward: {name} must hold integers, got {a.dtype}")
+            raise ValueError(f"{what}: {name} must hold integers, got {a.dtype}")
         if a.min() < 1 or a.max() > limit:
-            raise ValueError(f"forward: {name} must lie in [1, {limit}], got [{a.min()}, {a.max()}]")
+            raise ValueError(f"{what}: {name} must lie in [1, {limit}], got [{a.min()}, {a.max()}]")
+        buf = self._stream_buf((what, name), B)
+        # the pinned staging block is not reused before this copy has run (torch's host allocator records the stream)
+        buf[:B].copy_(torch.from_numpy(a.astype(np.int32)).pin_memory(), non_blocking=True)
+        return buf[:B]
+
+    def _stream_buf(self, name, B: int) -> torch.Tensor:
+        """Engine-owned int32 device buffer of at least B entries for ``name`` on the current stream."""
         key = (name, torch.cuda.current_stream(self.device).cuda_stream)
         buf = self._len_bufs.get(key)
         if buf is None or buf.numel() < B:
             buf = torch.empty(max(B, 256), dtype=torch.int32, device=torch.device("cuda", self.device))
             self._len_bufs[key] = buf
-        # the pinned staging block is not reused before this copy has run (torch's host allocator records the stream)
-        buf[:B].copy_(torch.from_numpy(a.astype(np.int32)).pin_memory(), non_blocking=True)
-        return buf[:B]
+        return buf
 
     # ---- forward ---------------------------------------------------------------------------------
     def forward(self, mixed: torch.Tensor, frames: torch.Tensor, out=None, lengths=None, frame_lengths=None):
@@ -414,9 +420,16 @@ class Engine:
         self._check(rc, "avsep_eval_snr")
         return in_snr, out_snr, perm, si
 
-    def stft(self, waves, n_fft: int = 512, hop_length: int = 128, want_mag: bool = True):
+    def stft(self, waves, n_fft: int = 512, hop_length: int = 128, want_mag: bool = True, lengths=None):
         """avsep_stft: (B, L) float32 waveforms -> complex64 (B, F, T) with the framing of the reference's
-        SyntheticAVDataset._stft (dataset.py:122-135) and, optionally, its float32 magnitude (the model input)."""
+        SyntheticAVDataset._stft (dataset.py:122-135) and, optionally, its float32 magnitude (the model input).
+
+        Variable-length batch: ``lengths`` (B,) samples per utterance, each left-aligned in its row (see
+        ``Engine._lengths`` for the accepted forms).  Utterance b's spec / mag [b, :, :T_b] with T_b = 1 + L_b // hop
+        equal this call on ``waves[b, :L_b]`` alone and the rest is 0; samples past L_b are never read.  The call then
+        returns (spec, mag, frame_lengths): frame_lengths is an int32 device tensor of the T_b, ready for
+        ``forward(lengths=...)``.  It lives in an engine-owned buffer of the current stream (a stable pointer keeps the
+        forward's CUDA graph cached) and is overwritten by the next such call on that stream."""
         dev = torch.device("cuda", self.device)
         if waves.device != dev or waves.dtype != torch.float32 or not waves.is_contiguous() or waves.dim() != 2:
             raise ValueError("stft: waves must be a contiguous float32 (B, L) tensor on the engine device")
@@ -425,14 +438,26 @@ class Engine:
         spec = torch.empty(B, F, T, device=dev, dtype=torch.complex64)
         mag = torch.empty(B, F, T, device=dev, dtype=torch.float32) if want_mag else None
         with torch.cuda.device(self.device):
-            rc = self.lib.avsep_stft(self.h, waves.data_ptr(), B, L, n_fft, hop_length, spec.data_ptr(),
-                                     mag.data_ptr() if want_mag else None, self._stream())
-        self._check(rc, "avsep_stft")
-        return spec, mag
+            if lengths is None:
+                rc = self.lib.avsep_stft(self.h, waves.data_ptr(), B, L, n_fft, hop_length, spec.data_ptr(),
+                                         mag.data_ptr() if want_mag else None, self._stream())
+                self._check(rc, "avsep_stft")
+                return spec, mag
+            lens = self._lengths(lengths, "lengths", B, L, "stft")
+            flens = self._stream_buf(("stft", "frame_lengths"), B)[:B]
+            rc = self.lib.avsep_stft_varlen(self.h, waves.data_ptr(), lens.data_ptr(), B, L, n_fft, hop_length,
+                                            spec.data_ptr(), mag.data_ptr() if want_mag else None, flens.data_ptr(),
+                                            self._stream())
+        self._check(rc, "avsep_stft_varlen")
+        return spec, mag, flens
 
-    def istft(self, spec, masks=None, length: int = None, n_fft: int = 512, hop_length: int = 128):
+    def istft(self, spec, masks=None, length: int = None, n_fft: int = 512, hop_length: int = 128, lengths=None):
         """avsep_istft: complex64 (B, F, T) mixture spectrum (+ (B, S, F, T) float32 masks) -> (B, S, L) float32
-        waveforms by weighted overlap-add; without masks the plain inverse, (B, 1, L)."""
+        waveforms by weighted overlap-add; without masks the plain inverse, (B, 1, L).
+
+        Variable-length batch: ``lengths`` (B,) output samples per utterance (forms as for ``stft``).  With
+        T_b = min(T, 1 + L_b // hop), waves[b, :, :L_b] equal this call on spec[b, :, :T_b] and masks[b, :, :, :T_b]
+        alone at length L_b, the rest is 0, and spectrum and mask columns past T_b are never read."""
         dev = torch.device("cuda", self.device)
         if spec.device != dev or spec.dtype != torch.complex64 or not spec.is_contiguous() or spec.dim() != 3:
             raise ValueError("istft: spec must be a contiguous complex64 (B, F, T) tensor on the engine device")
@@ -449,9 +474,16 @@ class Engine:
         L = (T - 1) * hop_length if length is None else int(length)
         waves = torch.empty(B, S, L, device=dev, dtype=torch.float32)
         with torch.cuda.device(self.device):
-            rc = self.lib.avsep_istft(self.h, spec.data_ptr(), masks.data_ptr() if masks is not None else None, B, S,
-                                      T, n_fft, hop_length, L, waves.data_ptr(), self._stream())
-        self._check(rc, "avsep_istft")
+            if lengths is None:
+                rc = self.lib.avsep_istft(self.h, spec.data_ptr(), masks.data_ptr() if masks is not None else None, B,
+                                          S, T, n_fft, hop_length, L, waves.data_ptr(), self._stream())
+                self._check(rc, "avsep_istft")
+                return waves
+            lens = self._lengths(lengths, "lengths", B, L, "istft")
+            rc = self.lib.avsep_istft_varlen(self.h, spec.data_ptr(), masks.data_ptr() if masks is not None else None,
+                                             lens.data_ptr(), B, S, T, n_fft, hop_length, L, waves.data_ptr(),
+                                             self._stream())
+        self._check(rc, "avsep_istft_varlen")
         return waves
 
     def set_option(self, name: str, value: int):

@@ -326,18 +326,40 @@ class AVSeparationTransformer(_InferenceOnly):
         return eng.forward_host(mixed_spec, lip_frames, *(out or ()))
 
     def separate_waveforms(self, mixed_wave: torch.Tensor, lip_frames: torch.Tensor, n_fft: int = None,
-                           hop_length: int = 128):
+                           hop_length: int = 128, *, lengths=None, frame_lengths=None):
         """Waveform in, waveforms out (not a reference method: the reference lists phase / iSTFT reconstruction as
         missing, README.md:140).  mixed_wave (B, L) float32 CUDA -> (B, S, L): complex STFT with the framing of
         SyntheticAVDataset._stft (dataset.py:122-135), forward on its magnitude, masks applied to the complex
-        mixture, weighted overlap-add inverse.  Also returns the masks."""
+        mixture, weighted overlap-add inverse.  Also returns the masks.
+
+        ``lengths`` (B,) samples and ``frame_lengths`` (B,) lip frames per utterance (not reference arguments; forms as
+        for ``forward``): utterance b, left-aligned in its rows, then gives what this method gives on
+        ``mixed_wave[b, :lengths[b]]`` and ``lip_frames[b, :frame_lengths[b]]`` alone, and its waveforms and masks are
+        0 past its lengths.  The per-utterance frame counts go from the analysis to the forward on the device."""
         if not mixed_wave.is_cuda:
             raise ValueError("separate_waveforms: mixed_wave must be a CUDA tensor")
         n_fft = 2 * (self.config.freq_bins - 1) if n_fft is None else n_fft
         eng = self._get_engine(mixed_wave.device)
-        spec, mag = eng.stft(mixed_wave, n_fft, hop_length)
-        _, masks = eng.forward(mag, lip_frames)
-        return eng.istft(spec, masks, mixed_wave.shape[1], n_fft, hop_length), masks
+        if lengths is None and frame_lengths is None:
+            spec, mag = eng.stft(mixed_wave, n_fft, hop_length)
+            _, masks = eng.forward(mag, lip_frames)
+            return eng.istft(spec, masks, mixed_wave.shape[1], n_fft, hop_length), masks
+        if not lip_frames.is_cuda:
+            raise ValueError("separate_waveforms: lengths / frame_lengths need CUDA inputs")
+        if mixed_wave.dim() != 2:
+            raise ValueError(f"separate_waveforms: mixed_wave must be (B, L), got {tuple(mixed_wave.shape)}")
+        B, L = mixed_wave.shape
+        _, _, N, _, _ = eng._check_inputs("separate_waveforms", frames=lip_frames)
+        with torch.cuda.device(eng.device):
+            lens = eng._lengths(lengths, "lengths", B, L, "separate_waveforms")
+            flens = eng._lengths(frame_lengths, "frame_lengths", B, N, "separate_waveforms")
+        if lens is None:
+            spec, mag = eng.stft(mixed_wave, n_fft, hop_length)
+            t_lens = None
+        else:
+            spec, mag, t_lens = eng.stft(mixed_wave, n_fft, hop_length, lengths=lens)
+        _, masks = eng.forward(mag, lip_frames, lengths=t_lens, frame_lengths=flens)
+        return eng.istft(spec, masks, L, n_fft, hop_length, lengths=lens), masks
 
     @property
     def engine(self) -> Engine:

@@ -1285,20 +1285,33 @@ int avsep_eval_snr(avsep_handle* h, const float* separated, const float* targets
 
 int avsep_stft(avsep_handle* h, const float* waves, int32_t B, int32_t L, int32_t n_fft, int32_t hop_length,
                float* spec, float* mag, void* cuda_stream) {
+  return avsep_stft_varlen(h, waves, nullptr, B, L, n_fft, hop_length, spec, mag, nullptr, cuda_stream);
+}
+
+int avsep_stft_varlen(avsep_handle* h, const float* waves, const int32_t* lengths, int32_t B, int32_t L, int32_t n_fft,
+                      int32_t hop_length, float* spec, float* mag, int32_t* frame_lengths_out, void* cuda_stream) {
   if (!h) return 1;
   if (!waves || !spec) return fail(h, "avsep_stft: null argument");
   CUDA_OK(cudaSetDevice(h->cfg.device));
-  CK(launch_stft_complex(static_cast<cudaStream_t>(cuda_stream), waves, B, L, n_fft, hop_length, spec, mag));
+  CK(launch_stft_complex(static_cast<cudaStream_t>(cuda_stream), waves, lengths, B, L, n_fft, hop_length, spec, mag,
+                         frame_lengths_out));
   h->launches = 1;
   return 0;
 }
 
 int avsep_istft(avsep_handle* h, const float* spec, const float* masks, int32_t B, int32_t S, int32_t T,
                 int32_t n_fft, int32_t hop_length, int32_t L, float* waves, void* cuda_stream) {
+  return avsep_istft_varlen(h, spec, masks, nullptr, B, S, T, n_fft, hop_length, L, waves, cuda_stream);
+}
+
+int avsep_istft_varlen(avsep_handle* h, const float* spec, const float* masks, const int32_t* lengths, int32_t B,
+                       int32_t S, int32_t T, int32_t n_fft, int32_t hop_length, int32_t L, float* waves,
+                       void* cuda_stream) {
   if (!h) return 1;
   if (!spec || !waves) return fail(h, "avsep_istft: null argument");
   CUDA_OK(cudaSetDevice(h->cfg.device));
-  CK(launch_istft_masked(static_cast<cudaStream_t>(cuda_stream), spec, masks, B, S, T, n_fft, hop_length, L, waves));
+  CK(launch_istft_masked(static_cast<cudaStream_t>(cuda_stream), spec, masks, lengths, B, S, T, n_fft, hop_length, L,
+                         waves));
   h->launches = 1;
   return 0;
 }

@@ -269,12 +269,14 @@ const char* launch_eval_snr(cudaStream_t s, const float* separated, const float*
                             int S, int FT, double* input_snr, double* output_snr, int* best_perm, double* si_snr);
 
 // ---- waveform side (waveform.cu): complex STFT with the reference's framing, masked inverse STFT ----
-const char* launch_stft_complex(cudaStream_t s, const float* waves, int B, int L, int nfft, int hop, float* spec,
-                                float* mag);
+// lengths: device int32 [B] samples per utterance, or null (all L).  The stft runs its variable-length kernel when
+// lengths or frame_lengths (device int32 [B], receives 1 + length / hop) is given; the istft when lengths is.
+const char* launch_stft_complex(cudaStream_t s, const float* waves, const int* lengths, int B, int L, int nfft, int hop,
+                                float* spec, float* mag, int* frame_lengths);
 const char* fft512_init_tables();   // window + twiddle tables of the n_fft = 512 kernels, once per device (avsep_create)
 const char* launch_stft512_synth(cudaStream_t s, const float* waves, int B, int S, int n, int hop, float* mixed_spec,
                                  float* clean_specs);
-const char* launch_istft_masked(cudaStream_t s, const float* spec, const float* masks, int B, int S, int T, int nfft,
-                                int hop, int L, float* waves);
+const char* launch_istft_masked(cudaStream_t s, const float* spec, const float* masks, const int* lengths, int B, int S,
+                                int T, int nfft, int hop, int L, float* waves);
 
 }  // namespace avsep

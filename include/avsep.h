@@ -233,6 +233,27 @@ AVSEP_API int avsep_stft(avsep_handle* h, const float* waves, int32_t B, int32_t
 AVSEP_API int avsep_istft(avsep_handle* h, const float* spec, const float* masks, int32_t B, int32_t S, int32_t T,
                           int32_t n_fft, int32_t hop_length, int32_t L, float* waves, void* cuda_stream);
 
+/* Variable-length waveform batches (the waveform counterpart of avsep_forward_varlen).  Utterance b sits
+ * left-aligned in its padded row and owns its first L_b = lengths[b] samples; lengths is a DEVICE int32 [B] array in
+ * samples, read on the device only (no host sync; a captured graph replays with whatever it holds then), values
+ * outside [1, L] behave as the nearest bound, and NULL means "all L" (avsep_stft / avsep_istft are these calls with
+ * NULL lengths).  Geometry, checks and errors are those of avsep_stft / avsep_istft; each call is one kernel launch.
+ *   avsep_stft_varlen: T = 1 + L / hop_length is the batch's frame count and T_b = 1 + L_b / hop_length the
+ *     utterance's.  spec / mag [b, :, :T_b] equal avsep_stft of waves[b, :L_b] alone, bit for bit; [b, :, T_b:] are
+ *     0; samples past L_b are never read.  frame_lengths_out: DEVICE int32 [B] receiving T_b (exactly the `lengths`
+ *     argument avsep_forward_varlen takes), or NULL.  With NULL lengths and non-NULL frame_lengths_out every entry is T.
+ *   avsep_istft_varlen: with T_b = min(T, 1 + L_b / hop_length), waves[b, s, :L_b] equal avsep_istft of
+ *     spec[b, :, :T_b] and masks[b, s, :, :T_b] alone at length L_b, bit for bit; waves[b, s, L_b:] are 0; spectrum
+ *     and mask columns at or past T_b are never read.
+ * Both transforms pack two frames into one complex FFT; frames at or past T_b are staged as zeros, so NaN or Inf in
+ * the padding never reaches a valid frame through its pair partner. */
+AVSEP_API int avsep_stft_varlen(avsep_handle* h, const float* waves, const int32_t* lengths, int32_t B, int32_t L,
+                                int32_t n_fft, int32_t hop_length, float* spec, float* mag,
+                                int32_t* frame_lengths_out, void* cuda_stream);
+AVSEP_API int avsep_istft_varlen(avsep_handle* h, const float* spec, const float* masks, const int32_t* lengths,
+                                 int32_t B, int32_t S, int32_t T, int32_t n_fft, int32_t hop_length, int32_t L,
+                                 float* waves, void* cuda_stream);
+
 /* Test hook: one whole transformer stack through the fused kernel (csrc/xformer_stack_sm100.cu) on the handle's
  * weights.  which: 0 = AudioEncoder.transformer (model.py:48-52,59), 1 = VisualEncoder.transformer (model.py:97-101,111),
  * 2 = CrossModalFusion.layers (+ .norm when final_ln) (model.py:145-149,166-173) with kv = bf16 [B*L, Lf*2*d] rows holding
