@@ -80,6 +80,7 @@ SIGNATURES = {
     "avsep_shared_close": (C.c_int, [_P, _P]),
     "avsep_copy_async": (C.c_int, [_P, _P, _P, C.c_size_t, _P]),
     "avsep_separate": (C.c_int, [_P, _P, _P, _I, _I, _P, _P]),
+    "avsep_separate_varlen": (C.c_int, [_P, _P, _P, _P, _I, _I, _P, _P]),
     "avsep_flag_signal": (C.c_int, [_P, C.POINTER(_P), _I, C.c_uint32, _P]),
     "avsep_flag_wait": (C.c_int, [_P, C.POINTER(_P), _I, C.c_uint32, C.c_double, _P]),
 }

@@ -355,15 +355,26 @@ class Engine:
         self._check(rc, "avsep_decoder")
         return sep, masks
 
-    def separate(self, masks, mixed, out=None):
-        """avsep_separate: SeparationDecoder.separate (reference model.py:210-220), masks (B,S,F,T) x mixed (B,F,T)."""
+    def separate(self, masks, mixed, out=None, lengths=None):
+        """avsep_separate: SeparationDecoder.separate (reference model.py:210-220), masks (B,S,F,T) x mixed (B,F,T).
+
+        Variable-length batch: ``lengths`` (B,) frames per utterance (forms as for ``forward``).  sep[b, :, :, :T_b] is
+        the same product, sep[b, :, :, T_b:] is 0, and masks / mixed are never read past T_b: on the masks of
+        ``forward(lengths=...)`` this gives that forward's ``separated`` bit for bit."""
         masks = self._dev_f32(masks, "masks")
         mixed = self._dev_f32(mixed, "mixed_spec")
         B, T, _, _, _ = self._check_inputs("separate", mixed=mixed, out=(masks,) if out is None else (masks, out))
         sep = torch.empty_like(masks) if out is None else out
         with torch.cuda.device(self.device):
-            rc = self.lib.avsep_separate(self.h, masks.data_ptr(), mixed.data_ptr(), B, T, sep.data_ptr(), self._stream())
-        self._check(rc, "avsep_separate")
+            if lengths is None:
+                rc = self.lib.avsep_separate(self.h, masks.data_ptr(), mixed.data_ptr(), B, T, sep.data_ptr(),
+                                             self._stream())
+                self._check(rc, "avsep_separate")
+                return sep
+            lens = self._lengths(lengths, "lengths", B, T, "separate")
+            rc = self.lib.avsep_separate_varlen(self.h, masks.data_ptr(), mixed.data_ptr(), lens.data_ptr(), B, T,
+                                                sep.data_ptr(), self._stream())
+        self._check(rc, "avsep_separate_varlen")
         return sep
 
     # ---- rows either side of the path --------------------------------------------------------------

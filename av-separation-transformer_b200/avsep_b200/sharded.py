@@ -27,6 +27,13 @@ the remote decoder epilogue wrote -- and acknowledges with a ticket in every ran
 waits for before it overwrites that output slot two steps later.  The root ends up with the same bytes in the same
 buffers as with ``gather="both"``.
 
+``varlen=True`` carries per-utterance lengths through the same path (a variable-length batch, avsep_forward_varlen):
+the root holds two more int32 [world*B] buffers per input set, audio frames and lip frames per utterance, which every
+rank pulls with the same copy calls as its inputs; the forward gets them as device tensors, and the masks-only rebuild
+runs avsep_separate_varlen over the remote shards' slice of them, which stores 0 past each length without reading the
+(possibly NaN) padding -- so both wire formats still leave the same bytes on the root.  The scatter and gather still
+move padded tensors.
+
 The memory backend is injected so that the bookkeeping (shard offsets, buffer rotation, ordering) is covered by
 world_size-2 gloo tests on CPU (tests/test_multirank_cpu.py); on a GPU box the backend is the C ABI above.
 """
@@ -50,8 +57,8 @@ def shard_slices(world: int, per_rank_batch: int):
 class _RawCuda:
     """Minimal __cuda_array_interface__ holder so that torch can view memory owned by libavsep."""
 
-    def __init__(self, ptr: int, nfloats: int):
-        self.__cuda_array_interface__ = {"shape": (nfloats,), "typestr": "<f4", "data": (int(ptr), False), "version": 2}
+    def __init__(self, ptr: int, n: int, typestr: str = "<f4"):
+        self.__cuda_array_interface__ = {"shape": (n,), "typestr": typestr, "data": (int(ptr), False), "version": 2}
 
 
 class PeerMemoryCuda:
@@ -77,6 +84,9 @@ class PeerMemoryCuda:
         for s in shape:
             n *= int(s)
         return torch.as_tensor(_RawCuda(ptr, n), device=self.dev).view(*shape)
+
+    def view_i32(self, ptr: int, shape) -> torch.Tensor:
+        return torch.as_tensor(_RawCuda(ptr, _prod(shape), "<i4"), device=self.dev).view(*shape)
 
     def empty(self, shape) -> torch.Tensor:
         return torch.empty(*shape, device=self.dev, dtype=torch.float32)
@@ -106,6 +116,11 @@ class PeerMemoryCuda:
                                                     C.c_void_p(sep_ptr), C.c_void_p(stream.cuda_stream)),
                         "avsep_separate")
 
+    def separate_varlen(self, masks_ptr: int, mixed_ptr: int, lens_ptr: int, n_utt: int, T: int, sep_ptr: int, stream):
+        self.eng._check(self.eng.lib.avsep_separate_varlen(self.eng.h, C.c_void_p(masks_ptr), C.c_void_p(mixed_ptr),
+                                                           C.c_void_p(lens_ptr), n_utt, T, C.c_void_p(sep_ptr),
+                                                           C.c_void_p(stream.cuda_stream)), "avsep_separate_varlen")
+
     # stream / event plumbing (torch is used for streams only)
     def stream(self):
         return torch.cuda.Stream(device=self.dev)
@@ -126,13 +141,19 @@ class ShardedForward:
     forward_fn(mixed, frames, sep, masks): runs the model on one shard (tensors of the backend's device), stream-ordered
     on the backend's current stream.  ``shapes``: dict with the per-utterance shapes ``mixed`` (F, T), ``frames``
     (N, H, W), ``out`` (S, F, T).
+
+    ``varlen=True``: a variable-length batch.  ``root_lens[s] = (lengths, frame_lengths)`` are the root's int32
+    [world*B] views of input set s's audio-frame and lip-frame counts, filled by the producer like ``root_in[s]``, and
+    forward_fn is called as forward_fn(mixed, frames, sep, masks, lengths, frame_lengths) with int32 device tensors of
+    the shard (buffers whose pointers stay fixed, so the forward's CUDA-graph keys do too).  With gather="masks" the
+    root's rebuild of step i reads set s's lengths as it reads its mixture: both stay untouched until that rebuild is done.
     """
 
     def __init__(self, backend, forward_fn, per_rank_batch: int, shapes: dict, rank: int, world: int,
-                 n_input_sets: int = 1, group=None, copy_lanes: int = 1, gather: str = "both"):
+                 n_input_sets: int = 1, group=None, copy_lanes: int = 1, gather: str = "both", varlen: bool = False):
         if gather not in ("both", "masks"):
             raise ValueError("gather must be 'both' (separated + masks on the wire) or 'masks' (the root rebuilds separated)")
-        self.gather = gather
+        self.gather, self.varlen = gather, bool(varlen)
         self.mem, self.fwd = backend, forward_fn
         self.B, self.rank, self.world, self.group = int(per_rank_batch), int(rank), int(world), group
         self.n_sets = int(n_input_sets)
@@ -144,6 +165,10 @@ class ShardedForward:
                 [f"out{o}.{k}" for o in range(2) for k in ("sep", "masks")]
         sizes = {n: G * self.per["mixed" if n.endswith("mixed") else "frames" if n.endswith("frames") else "out"]
                  for n in names}
+        if self.varlen:                  # one int32 per utterance (the backend sizes buffers in 4-byte words)
+            lens_names = [f"in{s}.{k}" for s in range(self.n_sets) for k in ("lens", "frame_lens")]
+            names += lens_names
+            sizes.update({n: G for n in lens_names})
         self.ptr = {}
         if rank == 0:
             handles = {}
@@ -158,11 +183,14 @@ class ShardedForward:
             for n in names:
                 self.ptr[n] = self.mem.open(box[0][n])
         # root: tensor views of the global buffers (what its producer fills / its consumer reads)
-        self.root_in, self.root_out = [], []
+        self.root_in, self.root_out, self.root_lens = [], [], []
         if rank == 0:
             for s in range(self.n_sets):
                 self.root_in.append((self.mem.view(self.ptr[f"in{s}.mixed"], (G,) + self.shapes["mixed"]),
                                      self.mem.view(self.ptr[f"in{s}.frames"], (G,) + self.shapes["frames"])))
+                if self.varlen:
+                    self.root_lens.append((self.mem.view_i32(self.ptr[f"in{s}.lens"], (G,)),
+                                           self.mem.view_i32(self.ptr[f"in{s}.frame_lens"], (G,))))
             for o in range(2):
                 self.root_out.append((self.mem.view(self.ptr[f"out{o}.sep"], (G,) + self.shapes["out"]),
                                       self.mem.view(self.ptr[f"out{o}.masks"], (G,) + self.shapes["out"])))
@@ -172,6 +200,8 @@ class ShardedForward:
                            for _ in range(2)]
             self.loc_out = [(self.mem.empty((B,) + self.shapes["out"]), self.mem.empty((B,) + self.shapes["out"]))
                             for _ in range(2)]
+            if self.varlen:              # (lengths, frame_lengths) per slot: int32 views of one 2B-word buffer
+                self.loc_lens = [tuple(self.mem.empty((2, B)).view(torch.int32)) for _ in range(2)]
             self.s_in, self.s_out = self.mem.stream(), self.mem.stream()
             # copy_lanes > 1: every transfer is cut into that many pieces on extra streams (more copy engines and more
             # requests in flight per rank; tools/nvlink_probe.py: the root's links carry more when both directions run)
@@ -184,7 +214,7 @@ class ShardedForward:
             self.ev_fwd_done = [self.mem.event() for _ in range(2)]
             self.ev_out_free = [self.mem.event() for _ in range(2)]
             self.used = [False, False]
-        self.bytes_in_per_step = 4 * self.B * (self.per["mixed"] + self.per["frames"])     # per non-root rank
+        self.bytes_in_per_step = 4 * self.B * (self.per["mixed"] + self.per["frames"] + (2 if self.varlen else 0))
         self.bytes_out_per_step = 4 * self.B * (1 if gather == "masks" else 2) * self.per["out"]
         self.count, self.last_ticket = 0, [0, 0]
         if gather == "masks" and world > 1:
@@ -223,15 +253,20 @@ class ShardedForward:
         if self.rank == 0:
             m, f = self.root_in[s_set]
             sep, masks = self.root_out[b]
-            self.fwd(m[self.lo:self.hi], f[self.lo:self.hi], sep[self.lo:self.hi], masks[self.lo:self.hi])
+            lens = [t[self.lo:self.hi] for t in self.root_lens[s_set]] if self.varlen else []
+            self.fwd(m[self.lo:self.hi], f[self.lo:self.hi], sep[self.lo:self.hi], masks[self.lo:self.hi], *lens)
             self.count += 1
             if self.gather == "masks" and self.world > 1:
                 # rebuild the remote shards' `separated` once their masks have landed, then free the slot for step + 2
                 ticket, st, B = self.count, 4 * self.FLAG_STRIDE, self.B
                 self.mem.wait([self.arrived + r * st for r in range(1, self.world)], ticket, self.s_rb)
-                self.mem.separate(self.ptr[f"out{b}.masks"] + 4 * B * self.per["out"],
-                                  self.ptr[f"in{s_set}.mixed"] + 4 * B * self.per["mixed"], (self.world - 1) * B,
-                                  self.shapes["mixed"][1], self.ptr[f"out{b}.sep"] + 4 * B * self.per["out"], self.s_rb)
+                args = (self.ptr[f"out{b}.masks"] + 4 * B * self.per["out"],
+                        self.ptr[f"in{s_set}.mixed"] + 4 * B * self.per["mixed"], (self.world - 1) * B,
+                        self.shapes["mixed"][1], self.ptr[f"out{b}.sep"] + 4 * B * self.per["out"], self.s_rb)
+                if self.varlen:          # past its length a remote row is 0, as the rank's decoder wrote it
+                    self.mem.separate_varlen(args[0], args[1], self.ptr[f"in{s_set}.lens"] + 4 * B, *args[2:])
+                else:
+                    self.mem.separate(*args)
                 self.mem.signal(self.peer_ack, ticket, self.s_rb)
                 self.ev_rebuilt[b].record(self.s_rb)
             return
@@ -242,15 +277,18 @@ class ShardedForward:
         if self.used[b]:
             self.s_in.wait_event(self.ev_fwd_done[b])
         off = self.lo
-        self._copy(self.s_in, self.x_in, 0, [
-            (m.data_ptr(), self.ptr[f"in{s_set}.mixed"] + 4 * off * self.per["mixed"], self.B * self.per["mixed"]),
-            (f.data_ptr(), self.ptr[f"in{s_set}.frames"] + 4 * off * self.per["frames"], self.B * self.per["frames"])])
+        jobs = [(m.data_ptr(), self.ptr[f"in{s_set}.mixed"] + 4 * off * self.per["mixed"], self.B * self.per["mixed"]),
+                (f.data_ptr(), self.ptr[f"in{s_set}.frames"] + 4 * off * self.per["frames"], self.B * self.per["frames"])]
+        lens = list(self.loc_lens[b]) if self.varlen else []
+        for t, k in zip(lens, ("lens", "frame_lens")):
+            jobs.append((t.data_ptr(), self.ptr[f"in{s_set}.{k}"] + 4 * off, self.B))
+        self._copy(self.s_in, self.x_in, 0, jobs)
         self.ev_in_ready[b].record(self.s_in)
         # forward on the shard, once its inputs have landed and the push that last read these outputs is done
         comp.wait_event(self.ev_in_ready[b])
         if self.used[b]:
             comp.wait_event(self.ev_out_free[b])
-        self.fwd(m, f, sep, masks)
+        self.fwd(m, f, sep, masks, *lens)
         self.ev_fwd_done[b].record(comp)
         # gather: push the shard's outputs into the root's global buffers
         self.s_out.wait_event(self.ev_fwd_done[b])

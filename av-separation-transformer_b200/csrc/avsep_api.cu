@@ -1386,12 +1386,17 @@ int avsep_copy_async(avsep_handle* h, void* dst, const void* src, size_t bytes, 
 
 int avsep_separate(avsep_handle* h, const float* masks, const float* mixed_spec, int32_t B, int32_t T, float* separated,
                    void* cuda_stream) {
+  return avsep_separate_varlen(h, masks, mixed_spec, nullptr, B, T, separated, cuda_stream);
+}
+
+int avsep_separate_varlen(avsep_handle* h, const float* masks, const float* mixed_spec, const int32_t* lengths,
+                          int32_t B, int32_t T, float* separated, void* cuda_stream) {
   if (!h) return 1;
   if (!masks || !mixed_spec || !separated) return fail(h, "avsep_separate: null buffer");
   if (B < 1 || T < 1) return fail(h, "avsep_separate: B and T must be >= 1");
   CUDA_OK(cudaSetDevice(h->cfg.device));
   const char* e = launch_separate(static_cast<cudaStream_t>(cuda_stream), masks, mixed_spec, separated, B,
-                                  h->cfg.num_speakers, h->cfg.freq_bins, T);
+                                  h->cfg.num_speakers, h->cfg.freq_bins, T, lengths);
   return e ? fail(h, e) : 0;
 }
 

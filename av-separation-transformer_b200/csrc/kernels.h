@@ -197,8 +197,9 @@ const char* launch_prep_audio(cudaStream_t s, int prec, const float* mixed, void
                               const int* lens = nullptr);
 
 // SeparationDecoder.separate (model.py:210-220): out[b,s,f,t] = masks[b,s,f,t] * mixed[b,f,t] (peer_gather.cu).
+// lens (or null): out[b,s,f,t] = 0 for t >= lens[b] (clamped to [1, T]), where masks and mixed are not read.
 const char* launch_separate(cudaStream_t s, const float* masks, const float* mixed, float* out, long long B, int S,
-                            int F, int T);
+                            int F, int T, const int* lens = nullptr);
 // Ticket flags of the masks-only gather: 32-bit words in this GPU's or a peer's memory, raised / awaited in stream order.
 struct FlagSet {
   static constexpr int MAX = 16;

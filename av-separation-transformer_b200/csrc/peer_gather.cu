@@ -16,19 +16,30 @@ namespace {
 // of the first 16-byte boundary (masks and separated share their misalignment, e.g. the two halves of one allocation)
 // and the ragged tail are handled element-wise by the first threads.  HBM-bound: 4 * F * T * (2 S + 1) algorithmic
 // bytes per utterance (masks in, separated out, the mixture once).
+// Variable-length batch (VARLEN): utterance b owns the frames t < T_b = lens[b] clamped to [1, T] (utt_len, as in the
+// forward); there the product is the same single multiply, past T_b the kernel stores 0 and reads neither masks nor
+// mixed, so NaN / Inf in the padding cannot reach the output (0 x NaN would).  A 4-element group can straddle T_b (T is
+// odd at the benchmark shape): its 16-byte masks load is taken only when all four elements are live, else the live
+// ones are loaded one by one.
+template <bool VARLEN>
 __device__ __forceinline__ void separate_one(const float* masks, const float* mixed, float* out, long long i, int plane,
-                                             int S) {
+                                             int S, const int* lens, int T) {
   const long long pbs = i / plane;
-  out[i] = masks[i] * mixed[(pbs / S) * plane + (i - pbs * plane)];
+  if constexpr (VARLEN) {
+    const int r = static_cast<int>(i - pbs * plane);
+    out[i] = r % T < utt_len(lens, static_cast<int>(pbs / S), T) ? masks[i] * mixed[(pbs / S) * plane + r] : 0.f;
+  } else {
+    out[i] = masks[i] * mixed[(pbs / S) * plane + (i - pbs * plane)];
+  }
 }
 
-template <bool VEC>
+template <bool VEC, bool VARLEN>
 __global__ void __launch_bounds__(256)
 separate_kernel(const float* __restrict__ masks, const float* __restrict__ mixed, float* __restrict__ out,
-                long long total, int plane, int S, int head) {
+                long long total, int plane, int S, int head, const int* __restrict__ lens, int T) {
   const long long tid = static_cast<long long>(blockIdx.x) * 256 + threadIdx.x;
   if constexpr (!VEC) {
-    if (tid < total) separate_one(masks, mixed, out, tid, plane, S);
+    if (tid < total) separate_one<VARLEN>(masks, mixed, out, tid, plane, S, lens, T);
     return;
   }
   const long long groups = (total - head) / 4;
@@ -37,24 +48,57 @@ separate_kernel(const float* __restrict__ masks, const float* __restrict__ mixed
     long long bs = i0 / plane;                     // (b, s) plane of the first element
     int r = static_cast<int>(i0 - bs * plane);     // offset inside the plane
     long long mbase = (bs / S) * plane;            // mixture plane of utterance b
-    const float4 m = __ldcs(reinterpret_cast<const float4*>(masks + i0));
-    float v[4] = {m.x, m.y, m.z, m.w};
+    if constexpr (VARLEN) {
+      int t = r % T, tb = utt_len(lens, static_cast<int>(bs / S), T);
+      int live = 0;                                // bit k: element k lies inside its utterance's length
+      long long mi[4];
 #pragma unroll
-    for (int k = 0; k < 4; ++k) {
-      if (r == plane) {                            // crossed into the next (b, s) plane
-        r = 0;
-        ++bs;
-        mbase = (bs / S) * plane;
+      for (int k = 0; k < 4; ++k) {
+        if (r == plane) {                          // crossed into the next (b, s) plane: t restarts, b may change
+          r = 0;
+          t = 0;
+          ++bs;
+          mbase = (bs / S) * plane;
+          tb = utt_len(lens, static_cast<int>(bs / S), T);
+        }
+        if (t < tb) live |= 1 << k;
+        mi[k] = mbase + r;
+        ++r;
+        if (++t == T) t = 0;
       }
-      v[k] *= __ldg(mixed + mbase + r);
-      ++r;
+      float v[4] = {0.f, 0.f, 0.f, 0.f};
+      if (live == 15) {
+        const float4 m = __ldcs(reinterpret_cast<const float4*>(masks + i0));
+        v[0] = m.x; v[1] = m.y; v[2] = m.z; v[3] = m.w;
+      } else {
+#pragma unroll
+        for (int k = 0; k < 4; ++k)
+          if (live >> k & 1) v[k] = __ldcs(masks + i0 + k);
+      }
+#pragma unroll
+      for (int k = 0; k < 4; ++k)
+        if (live >> k & 1) v[k] *= __ldg(mixed + mi[k]);
+      __stcs(reinterpret_cast<float4*>(out + i0), make_float4(v[0], v[1], v[2], v[3]));
+    } else {
+      const float4 m = __ldcs(reinterpret_cast<const float4*>(masks + i0));
+      float v[4] = {m.x, m.y, m.z, m.w};
+#pragma unroll
+      for (int k = 0; k < 4; ++k) {
+        if (r == plane) {                            // crossed into the next (b, s) plane
+          r = 0;
+          ++bs;
+          mbase = (bs / S) * plane;
+        }
+        v[k] *= __ldg(mixed + mbase + r);
+        ++r;
+      }
+      __stcs(reinterpret_cast<float4*>(out + i0), make_float4(v[0], v[1], v[2], v[3]));
     }
-    __stcs(reinterpret_cast<float4*>(out + i0), make_float4(v[0], v[1], v[2], v[3]));
   }
   if (tid < 8) {                                   // <= 3 head + <= 3 tail elements
     const long long tail0 = head + groups * 4;
     const long long i = tid < head ? tid : tail0 + (tid - head);
-    if (i < total && (tid < head || i >= tail0)) separate_one(masks, mixed, out, i, plane, S);
+    if (i < total && (tid < head || i >= tail0)) separate_one<VARLEN>(masks, mixed, out, i, plane, S, lens, T);
   }
 }
 
@@ -105,8 +149,10 @@ const char* preload_kernels() {
   if (done[dev]) return nullptr;
   cudaFuncAttributes a;
   if (cudaFuncGetAttributes(&a, flag_signal_kernel) != cudaSuccess || cudaFuncGetAttributes(&a, flag_wait_kernel) != cudaSuccess ||
-      cudaFuncGetAttributes(&a, separate_kernel<true>) != cudaSuccess ||
-      cudaFuncGetAttributes(&a, separate_kernel<false>) != cudaSuccess)
+      cudaFuncGetAttributes(&a, separate_kernel<true, false>) != cudaSuccess ||
+      cudaFuncGetAttributes(&a, separate_kernel<false, false>) != cudaSuccess ||
+      cudaFuncGetAttributes(&a, separate_kernel<true, true>) != cudaSuccess ||
+      cudaFuncGetAttributes(&a, separate_kernel<false, true>) != cudaSuccess)
     return "peer_gather: kernel image not loadable on this device";
   done[dev] = true;
   return nullptr;
@@ -115,7 +161,7 @@ const char* preload_kernels() {
 }  // namespace
 
 const char* launch_separate(cudaStream_t s, const float* masks, const float* mixed, float* out, long long B, int S,
-                            int F, int T) {
+                            int F, int T, const int* lens) {
   if (B <= 0) return nullptr;
   if (const char* e = preload_kernels()) return e;
   const long long plane = static_cast<long long>(F) * T;
@@ -128,10 +174,9 @@ const char* launch_separate(cudaStream_t s, const float* masks, const float* mix
   const long long threads = vec ? (total - head) / 4 + 8 : total;
   const long long blocks = (threads + 255) / 256;
   if (blocks > 0x7fffffffLL) return "separate: batch too large";
-  if (vec)
-    separate_kernel<true><<<static_cast<unsigned>(blocks), 256, 0, s>>>(masks, mixed, out, total, static_cast<int>(plane), S, head);
-  else
-    separate_kernel<false><<<static_cast<unsigned>(blocks), 256, 0, s>>>(masks, mixed, out, total, static_cast<int>(plane), S, 0);
+  auto kernel = vec ? (lens ? separate_kernel<true, true> : separate_kernel<true, false>)
+                    : (lens ? separate_kernel<false, true> : separate_kernel<false, false>);
+  kernel<<<static_cast<unsigned>(blocks), 256, 0, s>>>(masks, mixed, out, total, static_cast<int>(plane), S, head, lens, T);
   return cudaGetLastError() == cudaSuccess ? nullptr : "separate: launch failed";
 }
 

@@ -296,6 +296,17 @@ AVSEP_API int avsep_copy_async(avsep_handle* h, void* dst, const void* src, size
 AVSEP_API int avsep_separate(avsep_handle* h, const float* masks, const float* mixed_spec, int32_t B, int32_t T,
                              float* separated, void* cuda_stream);
 
+/* Variable-length batch (the counterpart of avsep_forward_varlen's decoder epilogue, used by the masks-only gather on
+ * varlen batches).  Utterance b owns the first lengths[b] frames of its padded rows; lengths is a DEVICE int32 [B]
+ * array read on the device only (no host sync; a captured graph replays with whatever it holds then), values outside
+ * [1, T] behave as the nearest bound, and NULL means "all T" (avsep_separate is this call with NULL lengths).
+ * For t < lengths[b], separated[b, s, f, t] = masks[b, s, f, t] * mixed_spec[b, f, t], the same single fp32 multiply;
+ * separated[b, :, :, lengths[b]:] are 0 and masks / mixed_spec are never read there (NaN or Inf in the padding is
+ * harmless).  So avsep_separate_varlen(masks, mixed_spec, lengths) of avsep_forward_varlen's masks equals its
+ * separated bit for bit.  Alignment rules and errors are those of avsep_separate; one kernel launch. */
+AVSEP_API int avsep_separate_varlen(avsep_handle* h, const float* masks, const float* mixed_spec,
+                                    const int32_t* lengths, int32_t B, int32_t T, float* separated, void* cuda_stream);
+
 /* Masks-only gather (SURVEY.md 8e, "gather only masks: the root recomputes separated = masks x mixed, which it already
  * holds"): a rank pushes its masks shard with avsep_copy_async and then raises a ticket -- a 32-bit word in memory
  * from avsep_shared_alloc, its own or a mapped peer's -- with avsep_flag_signal on the same stream; the consumer
