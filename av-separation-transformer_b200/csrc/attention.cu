@@ -23,13 +23,12 @@ struct AttnDev {
   int ldq, ldkv, ldo;
   int H, Lq, Lk, nsrc;
   float scale_log2;
-  float lerp_scale;   // (float)nsrc / Lk, as ATen computes it
   // variable-length batch (null: all Lk / all nsrc): keys of utterance b, and its interpolation source rows.  Lk and
   // nsrc stay the row pitch of the K/V buffers.
   const int *k_lens, *src_lens;
 };
 
-// Keys of utterance b, its interpolation source rows and scale (ATen: (float)nsrc / (float)Lk).
+// Keys of utterance b, its interpolation source rows and scale.
 struct UttKeys {
   int lk, nsrc;
   float scale;
@@ -39,8 +38,7 @@ __device__ __forceinline__ UttKeys utt_keys(const AttnDev& p, int b) {
   UttKeys u;
   u.lk = utt_len(p.k_lens, b, p.Lk);
   u.nsrc = LERP ? utt_len(p.src_lens, b, p.nsrc) : 0;
-  u.scale = (p.k_lens == nullptr && p.src_lens == nullptr) ? p.lerp_scale
-                                                           : static_cast<float>(u.nsrc) / static_cast<float>(u.lk);
+  u.scale = lerp_scale(u.nsrc, u.lk);
   return u;
 }
 
@@ -61,8 +59,28 @@ __device__ __forceinline__ void load_tile_bf16(__nv_bfloat16* dst, const __nv_bf
   }
 }
 
-// Same, but each output row t is the linear interpolation of two fp32 source rows (ATen upsample_linear1d,
-// align_corners=False: src = max(scale*(t+0.5)-0.5, 0); i0 = floor(src); i1 = min(i0+1, n-1); lam = src-i0).
+// Eight fp32 of tile row t, columns [8c, 8c + 8), from fp32 source rows: with LERP the linear interpolation of the
+// utterance's nsrc source rows to the tile's rows (lerp_tap), else source row t itself; zero for t >= nrows.
+template <bool LERP>
+__device__ __forceinline__ void fetch_row8(const float* src, int ld, int t, int c, int nrows, int nsrc, float scale,
+                                           float4& lo, float4& hi) {
+  lo = hi = make_float4(0.f, 0.f, 0.f, 0.f);
+  if (t >= nrows) return;
+  if constexpr (LERP) {
+    const LerpTap k = lerp_tap(t, nsrc, scale);
+    const float4* p0 = reinterpret_cast<const float4*>(src + static_cast<size_t>(k.i0) * ld + c * 8);
+    const float4* p1 = reinterpret_cast<const float4*>(src + static_cast<size_t>(k.i1) * ld + c * 8);
+    const float4 a0 = __ldg(p0), a1 = __ldg(p0 + 1), b0 = __ldg(p1), b1 = __ldg(p1 + 1);
+    lo = lerp4(a0, b0, k.w0, k.w1);
+    hi = lerp4(a1, b1, k.w0, k.w1);
+  } else {
+    const float4* p0 = reinterpret_cast<const float4*>(src + static_cast<size_t>(t) * ld + c * 8);
+    lo = __ldg(p0);
+    hi = __ldg(p0 + 1);
+  }
+}
+
+// Same as load_tile_bf16, but each output row t is interpolated from the nsrc fp32 source rows.
 template <int HD>
 __device__ __forceinline__ void load_tile_lerp(__nv_bfloat16* dst, const float* src, int ld, int row0, int nrows,
                                                int nsrc, float scale) {
@@ -70,24 +88,9 @@ __device__ __forceinline__ void load_tile_lerp(__nv_bfloat16* dst, const float* 
   constexpr int CH = HD / 8;
   for (int i = threadIdx.x; i < 64 * CH; i += 128) {
     const int r = i / CH, c = i - r * CH;
-    const int t = row0 + r;
-    uint4 val = make_uint4(0, 0, 0, 0);
-    if (t < nrows) {
-      const float sp = fmaxf(scale * (static_cast<float>(t) + 0.5f) - 0.5f, 0.0f);
-      int i0 = static_cast<int>(sp);
-      if (i0 > nsrc - 1) i0 = nsrc - 1;
-      const int i1 = min(i0 + 1, nsrc - 1);
-      const float w1 = sp - static_cast<float>(i0);
-      const float w0 = 1.0f - w1;
-      const float4* p0 = reinterpret_cast<const float4*>(src + static_cast<size_t>(i0) * ld + c * 8);
-      const float4* p1 = reinterpret_cast<const float4*>(src + static_cast<size_t>(i1) * ld + c * 8);
-      const float4 a0 = __ldg(p0), a1 = __ldg(p0 + 1), b0 = __ldg(p1), b1 = __ldg(p1 + 1);
-      val.x = pack_bf16x2(w0 * a0.x + w1 * b0.x, w0 * a0.y + w1 * b0.y);
-      val.y = pack_bf16x2(w0 * a0.z + w1 * b0.z, w0 * a0.w + w1 * b0.w);
-      val.z = pack_bf16x2(w0 * a1.x + w1 * b1.x, w0 * a1.y + w1 * b1.y);
-      val.w = pack_bf16x2(w0 * a1.z + w1 * b1.z, w0 * a1.w + w1 * b1.w);
-    }
-    *reinterpret_cast<uint4*>(dst + r * LDS + c * 8) = val;
+    float4 x0, x1;
+    fetch_row8<true>(src, ld, row0 + r, c, nrows, nsrc, scale, x0, x1);
+    *reinterpret_cast<uint4*>(dst + r * LDS + c * 8) = pack_bf16x8(x0, x1);
   }
 }
 
@@ -100,26 +103,10 @@ __device__ __forceinline__ void load_tile_split(__nv_bfloat16* dst_hi, __nv_bflo
   constexpr int CH = HD / 8;
   for (int i = threadIdx.x; i < 64 * CH; i += 128) {
     const int r = i / CH, c = i - r * CH;
-    const int t = row0 + r;
-    float x[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
-    if (t < nrows) {
-      if (nsrc > 0) {
-        const float sp = fmaxf(scale * (static_cast<float>(t) + 0.5f) - 0.5f, 0.0f);
-        int i0 = static_cast<int>(sp);
-        if (i0 > nsrc - 1) i0 = nsrc - 1;
-        const int i1 = min(i0 + 1, nsrc - 1);
-        const float w1 = sp - static_cast<float>(i0), w0 = 1.0f - w1;
-        const float4* p0 = reinterpret_cast<const float4*>(src + static_cast<size_t>(i0) * ld + c * 8);
-        const float4* p1 = reinterpret_cast<const float4*>(src + static_cast<size_t>(i1) * ld + c * 8);
-        const float4 a0 = __ldg(p0), a1 = __ldg(p0 + 1), b0 = __ldg(p1), b1 = __ldg(p1 + 1);
-        x[0] = w0 * a0.x + w1 * b0.x; x[1] = w0 * a0.y + w1 * b0.y; x[2] = w0 * a0.z + w1 * b0.z; x[3] = w0 * a0.w + w1 * b0.w;
-        x[4] = w0 * a1.x + w1 * b1.x; x[5] = w0 * a1.y + w1 * b1.y; x[6] = w0 * a1.z + w1 * b1.z; x[7] = w0 * a1.w + w1 * b1.w;
-      } else {
-        const float4* p0 = reinterpret_cast<const float4*>(src + static_cast<size_t>(t) * ld + c * 8);
-        const float4 a0 = __ldg(p0), a1 = __ldg(p0 + 1);
-        x[0] = a0.x; x[1] = a0.y; x[2] = a0.z; x[3] = a0.w; x[4] = a1.x; x[5] = a1.y; x[6] = a1.z; x[7] = a1.w;
-      }
-    }
+    float4 x0, x1;
+    if (nsrc > 0) fetch_row8<true>(src, ld, row0 + r, c, nrows, nsrc, scale, x0, x1);
+    else fetch_row8<false>(src, ld, row0 + r, c, nrows, nsrc, scale, x0, x1);
+    const float x[8] = {x0.x, x0.y, x0.z, x0.w, x1.x, x1.y, x1.z, x1.w};
     uint32_t hi[4], lo[4];
 #pragma unroll
     for (int j = 0; j < 4; ++j) {
@@ -493,7 +480,6 @@ const char* launch_attention(cudaStream_t s, int prec, const AttnProblem& p) {
   d.ldq = p.ldq; d.ldkv = p.ldkv; d.ldo = p.ldo;
   d.H = p.H; d.Lq = p.Lq; d.Lk = p.Lk; d.nsrc = p.lerp_src;
   d.scale_log2 = 1.4426950408889634f / sqrtf(static_cast<float>(p.hd));
-  d.lerp_scale = p.lerp_src > 0 ? static_cast<float>(p.lerp_src) / static_cast<float>(p.Lk) : 0.f;
   d.k_lens = p.k_lens; d.src_lens = p.lerp_src > 0 ? p.src_lens : nullptr;
   const bool lerp = p.lerp_src > 0;
   if (split) {

@@ -289,7 +289,7 @@ attention_tc_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_consta
 // out[b*L + t, :] = lerp of two fp32 source rows (ATen upsample_linear1d, align_corners=False; model.py:114-116).
 // src_lens / dst_lens (variable-length batch, else null): utterance b interpolates its first src_lens[b] source rows
 // to dst_lens[b] rows; the rows past dst_lens[b] take the same formula (finite filler for masked keys).
-__global__ void lerp_rows_kernel(const float* __restrict__ src, int ld_src, int nsrc, int L, int chunks, float scale,
+__global__ void lerp_rows_kernel(const float* __restrict__ src, int ld_src, int nsrc, int L, int chunks,
                                  __nv_bfloat16* __restrict__ dst, int ld_dst, long long total,
                                  const int* __restrict__ src_lens, const int* __restrict__ dst_lens) {
   griddep_launch_dependents();
@@ -300,25 +300,12 @@ __global__ void lerp_rows_kernel(const float* __restrict__ src, int ld_src, int 
   const long long rt = i / chunks;
   const int t = static_cast<int>(rt % L);
   const long long bb = rt / L;
-  int ns = nsrc;
-  if (src_lens != nullptr || dst_lens != nullptr) {
-    ns = utt_len(src_lens, static_cast<int>(bb), nsrc);
-    scale = static_cast<float>(ns) / static_cast<float>(utt_len(dst_lens, static_cast<int>(bb), L));
-  }
-  const float sp = fmaxf(scale * (static_cast<float>(t) + 0.5f) - 0.5f, 0.0f);
-  int i0 = static_cast<int>(sp);
-  if (i0 > ns - 1) i0 = ns - 1;
-  const int i1 = min(i0 + 1, ns - 1);
-  const float w1 = sp - static_cast<float>(i0), w0 = 1.0f - w1;
-  const float4* p0 = reinterpret_cast<const float4*>(src + (bb * nsrc + i0) * ld_src + c * 8);
-  const float4* p1 = reinterpret_cast<const float4*>(src + (bb * nsrc + i1) * ld_src + c * 8);
+  const int ns = utt_len(src_lens, static_cast<int>(bb), nsrc);
+  const LerpTap k = lerp_tap(t, ns, lerp_scale(ns, utt_len(dst_lens, static_cast<int>(bb), L)));
+  const float4* p0 = reinterpret_cast<const float4*>(src + (bb * nsrc + k.i0) * ld_src + c * 8);
+  const float4* p1 = reinterpret_cast<const float4*>(src + (bb * nsrc + k.i1) * ld_src + c * 8);
   const float4 a0 = __ldg(p0), a1 = __ldg(p0 + 1), b0 = __ldg(p1), b1 = __ldg(p1 + 1);
-  uint4 val;
-  val.x = pack_bf16x2(w0 * a0.x + w1 * b0.x, w0 * a0.y + w1 * b0.y);
-  val.y = pack_bf16x2(w0 * a0.z + w1 * b0.z, w0 * a0.w + w1 * b0.w);
-  val.z = pack_bf16x2(w0 * a1.x + w1 * b1.x, w0 * a1.y + w1 * b1.y);
-  val.w = pack_bf16x2(w0 * a1.z + w1 * b1.z, w0 * a1.w + w1 * b1.w);
-  *reinterpret_cast<uint4*>(dst + rt * ld_dst + c * 8) = val;
+  *reinterpret_cast<uint4*>(dst + rt * ld_dst + c * 8) = pack_bf16x8(lerp4(a0, b0, k.w0, k.w1), lerp4(a1, b1, k.w0, k.w1));
 }
 
 }  // namespace
@@ -359,8 +346,7 @@ const char* launch_lerp_rows(cudaStream_t s, const float* src, int ld_src, int B
   const int threads = 256;
   const long long blocks = (total + threads - 1) / threads;
   launch_pdl(lerp_rows_kernel, dim3(static_cast<unsigned>(blocks)), dim3(threads), 0, s, src, ld_src, nsrc, L, chunks,
-             static_cast<float>(nsrc) / static_cast<float>(L), reinterpret_cast<__nv_bfloat16*>(dst_bf16), ld_dst, total,
-             src_lens, dst_lens);
+             reinterpret_cast<__nv_bfloat16*>(dst_bf16), ld_dst, total, src_lens, dst_lens);
   return cudaGetLastError() == cudaSuccess ? nullptr : "lerp_rows: launch failed";
 }
 

@@ -26,18 +26,13 @@ __global__ void op_to_f32_kernel(const __nv_bfloat16* in, float* out, size_t n) 
 }
 
 // out[b, t, :] = lerp of x[b, i0(t), :], x[b, i1(t), :]   (F.interpolate linear, align_corners=False; model.py:115)
-__global__ void interp_rows_kernel(const float* __restrict__ x, float* __restrict__ out, int N, int T, int d,
-                                   float scale) {
+__global__ void interp_rows_kernel(const float* __restrict__ x, float* __restrict__ out, int N, int T, int d) {
   const int t = blockIdx.x, b = blockIdx.y;
-  const float sp = fmaxf(scale * (static_cast<float>(t) + 0.5f) - 0.5f, 0.0f);
-  int i0 = static_cast<int>(sp);
-  if (i0 > N - 1) i0 = N - 1;
-  const int i1 = min(i0 + 1, N - 1);
-  const float w1 = sp - static_cast<float>(i0), w0 = 1.0f - w1;
-  const float* r0 = x + (static_cast<size_t>(b) * N + i0) * d;
-  const float* r1 = x + (static_cast<size_t>(b) * N + i1) * d;
+  const LerpTap k = lerp_tap(t, N, lerp_scale(N, T));
+  const float* r0 = x + (static_cast<size_t>(b) * N + k.i0) * d;
+  const float* r1 = x + (static_cast<size_t>(b) * N + k.i1) * d;
   float* o = out + (static_cast<size_t>(b) * T + t) * d;
-  for (int c = threadIdx.x; c < d; c += blockDim.x) o[c] = w0 * r0[c] + w1 * r1[c];
+  for (int c = threadIdx.x; c < d; c += blockDim.x) o[c] = k.w0 * r0[c] + k.w1 * r1[c];
 }
 
 // Profiling aid: keeps the GPU busy while the host enqueues a whole forward, so that the per-kernel event pairs
@@ -1464,8 +1459,7 @@ int avsep_visual_encoder(avsep_handle* h, const float* lip_frames, int32_t B, in
   h->launches = 0;
   if (visual_frontend(h, s, w, lip_frames, Plan{})) return 1;
   if (encoder_stack(h, s, h->enc_v, B, N, w.x_v, w.y_v, w.v_op, w.qkv_v, w.attn_v, w.ffn_v, nullptr, nullptr)) return 1;
-  interp_rows_kernel<<<dim3(target_len, B), 128, 0, s>>>(w.x_v, out_BTd, N, target_len, d,
-                                                         static_cast<float>(N) / static_cast<float>(target_len));
+  interp_rows_kernel<<<dim3(target_len, B), 128, 0, s>>>(w.x_v, out_BTd, N, target_len, d);
   CUDA_OK(cudaGetLastError());
   ++h->launches;
   return 0;

@@ -95,6 +95,13 @@ __device__ __forceinline__ uint32_t pack_bf16x2(float lo, float hi) {
   __nv_bfloat162 v = __floats2bfloat162_rn(lo, hi);
   return *reinterpret_cast<uint32_t*>(&v);
 }
+__device__ __forceinline__ uint4 pack_bf16x8(float4 lo, float4 hi) {
+  return make_uint4(pack_bf16x2(lo.x, lo.y), pack_bf16x2(lo.z, lo.w), pack_bf16x2(hi.x, hi.y), pack_bf16x2(hi.z, hi.w));
+}
+// w0 * a + w1 * b: four columns of a linearly interpolated row (see lerp_tap in kernels.h).
+__device__ __forceinline__ float4 lerp4(float4 a, float4 b, float w0, float w1) {
+  return make_float4(w0 * a.x + w1 * b.x, w0 * a.y + w1 * b.y, w0 * a.z + w1 * b.z, w0 * a.w + w1 * b.w);
+}
 
 // Nanoseconds of the GPU's global timer (the debug trace stamps and the flag-wait timeout).
 __device__ __forceinline__ unsigned long long globaltimer() {

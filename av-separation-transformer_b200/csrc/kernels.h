@@ -118,6 +118,27 @@ __device__ __forceinline__ bool frame_live(const int* lens, int N, int fr) {
   return lens == nullptr || fr % N < utt_len(lens, fr / N, N);
 }
 
+// Linear interpolation of nsrc rows to ndst rows along time: F.interpolate(mode='linear', align_corners=False), i.e.
+// ATen upsample_linear1d (model.py:114-116).  Every kernel that stretches rows takes its source rows and weights from
+// lerp_tap, with the scale from lerp_scale resolved once per utterance, outside the per-element loops.
+__host__ __device__ __forceinline__ float lerp_scale(int nsrc, int ndst) {
+  return static_cast<float>(nsrc) / static_cast<float>(ndst);   // as ATen computes it
+}
+struct LerpTap {
+  int i0, i1;       // target row = w0 * source row i0 + w1 * source row i1
+  float w0, w1;
+};
+__device__ __forceinline__ LerpTap lerp_tap(int t, int nsrc, float scale) {
+  const float sp = fmaxf(scale * (static_cast<float>(t) + 0.5f) - 0.5f, 0.0f);
+  LerpTap k;
+  k.i0 = static_cast<int>(sp);
+  if (k.i0 > nsrc - 1) k.i0 = nsrc - 1;
+  k.i1 = min(k.i0 + 1, nsrc - 1);
+  k.w1 = sp - static_cast<float>(k.i0);
+  k.w0 = 1.0f - k.w1;
+  return k;
+}
+
 // Returns nullptr on success or a static error string.
 const char* launch_gemm(cudaStream_t s, int prec, const GemmProblem& p, const GemmEpilogue& e, int num_sms,
                         int force_bn = 0, unsigned long long* trace = nullptr);   // trace: [grid][8] globaltimer stamps (debug)
@@ -229,9 +250,9 @@ const char* launch_attention(cudaStream_t s, int prec, const AttnProblem& p);
 bool attention_tc_usable(int prec, const AttnProblem& p);
 bool attention_tc_wanted(int prec, const AttnProblem& p);      // usable and selected by p.tc_mode
 const char* launch_attention_tc(cudaStream_t s, const AttnProblem& p);
-// dst[b*L + t, 0:cols] (bf16) = linear interpolation (align_corners=False) of src rows [b*nsrc + i, 0:cols] (fp32).
-// Variable-length batch: src_lens[b] source rows of utterance b interpolated to dst_lens[b] rows (null: nsrc / L); the
-// rows past dst_lens[b] are finite filler.
+// dst[b*L + t, 0:cols] (bf16) = linear interpolation (lerp_tap) of src rows [b*nsrc + i, 0:cols] (fp32), with the
+// scale of each utterance's own lengths: src_lens[b] source rows interpolated to dst_lens[b] rows (null: nsrc / L).
+// The rows past dst_lens[b] are finite filler.
 const char* launch_lerp_rows(cudaStream_t s, const float* src, int ld_src, int B, int nsrc, int L, int cols,
                              void* dst_bf16, int ld_dst, const int* src_lens = nullptr, const int* dst_lens = nullptr);
 

@@ -93,7 +93,7 @@ struct StackDev {
   // model.py:114-116) and multiplied by the kvp_chunks * 128 stacked K | V weight rows of every fusion layer
   // (model.py:155,169; functional.py:5847-5865): out = bf16 [B * kvp_L, kvp_ld].  kvp_chunks == 0: off.
   int kvp_chunks, kvp_L, kvp_ld;
-  float kvp_scale;              // L / kvp_L
+  float kvp_scale;              // lerp_scale(L, kvp_L), from the host so that the uniform kernel has no division
   __nv_bfloat16* kvp_out;
   // variable-length batch (null: all L / all kvp_L): rows of each utterance that are real, K | V interpolation targets
   const int *lens, *kvp_lens;
@@ -1137,16 +1137,10 @@ xformer_stack_kernel(const __grid_constant__ CUtensorMap tmXin, const __grid_con
           const bool live = t < p.kvp_L;
           // a short utterance: lk source rows interpolated to its own target length (the rows past that target are
           // finite and masked as keys by the fusion stack)
-          const float scale = lens == nullptr && kvp_lens == nullptr
-                                  ? p.kvp_scale
-                                  : static_cast<float>(lk) /
-                                        static_cast<float>(utt_len(kvp_lens, min(utt0 + r / p.stride, p.B - 1), p.kvp_L));
-          const float sp = fmaxf(scale * (static_cast<float>(t) + 0.5f) - 0.5f, 0.0f);
-          int i0 = static_cast<int>(sp);
-          if (i0 > lk - 1) i0 = lk - 1;
-          const int i1 = min(i0 + 1, lk - 1);
-          const float w1 = sp - static_cast<float>(i0), w0 = 1.0f - w1;
-          const int r0 = klo + i0, r1 = klo + i1;
+          const float scale =
+              VARLEN ? lerp_scale(lk, utt_len(kvp_lens, min(utt0 + r / p.stride, p.B - 1), p.kvp_L)) : p.kvp_scale;
+          const LerpTap k = lerp_tap(t, lk, scale);
+          const int r0 = klo + k.i0, r1 = klo + k.i1;
           uint8_t* slab = smem + OFF_A + part * SLAB;
 #pragma unroll
           for (int c = 0; c < 8; ++c) {
@@ -1156,10 +1150,7 @@ xformer_stack_kernel(const __grid_constant__ CUtensorMap tmXin, const __grid_con
               const float4 a1 = *reinterpret_cast<const float4*>(stg + r0 * 1024 + (((part * 16 + 2 * c + 1) ^ (r0 & 7)) << 4));
               const float4 b0 = *reinterpret_cast<const float4*>(stg + r1 * 1024 + (((part * 16 + 2 * c) ^ (r1 & 7)) << 4));
               const float4 b1 = *reinterpret_cast<const float4*>(stg + r1 * 1024 + (((part * 16 + 2 * c + 1) ^ (r1 & 7)) << 4));
-              w.x = pack_bf16x2(w0 * a0.x + w1 * b0.x, w0 * a0.y + w1 * b0.y);
-              w.y = pack_bf16x2(w0 * a0.z + w1 * b0.z, w0 * a0.w + w1 * b0.w);
-              w.z = pack_bf16x2(w0 * a1.x + w1 * b1.x, w0 * a1.y + w1 * b1.y);
-              w.w = pack_bf16x2(w0 * a1.z + w1 * b1.z, w0 * a1.w + w1 * b1.w);
+              w = pack_bf16x8(lerp4(a0, b0, k.w0, k.w1), lerp4(a1, b1, k.w0, k.w1));
             }
             *reinterpret_cast<uint4*>(slab + sw128_off(r, c)) = w;
           }
@@ -1483,7 +1474,7 @@ const char* launch_xformer_stack(cudaStream_t s, const StackProblem& sp, int num
   d.trace = sp.trace;
   d.pro_taps = pro ? sp.pro_taps : 0; d.pro_ks = sp.pro_k / 64; d.pro_pitch = sp.pro_pitch; d.pro_relu = sp.pro_relu; d.pe = sp.pe;
   d.kvp_chunks = kvp ? sp.kvp_n / 128 : 0; d.kvp_L = sp.kvp_L; d.kvp_ld = sp.kvp_ld;
-  d.kvp_scale = kvp ? static_cast<float>(sp.L) / static_cast<float>(sp.kvp_L) : 0.f;
+  d.kvp_scale = kvp ? lerp_scale(sp.L, sp.kvp_L) : 0.f;
   d.kvp_out = static_cast<__nv_bfloat16*>(sp.kvp_out);
   d.lens = sp.lens; d.kvp_lens = kvp ? sp.kvp_lens : nullptr;
   d.decoder = decoder ? 1 : 0;
