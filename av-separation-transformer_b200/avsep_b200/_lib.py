@@ -46,6 +46,10 @@ SIGNATURES = {
     "avsep_forward_host": (C.c_int, [_P, _P, _P, _I, _I, _I, _I, _I, _P, _P, _P]),
     "avsep_forward_host_async": (C.c_int, [_P, _P, _P, _I, _I, _I, _I, _I, _P, _P, _I, _P]),
     "avsep_host_wait": (C.c_int, [_P, _I]),
+    "avsep_packed_workspace_bytes": (C.c_size_t, [_P, _I, _I, _I, _I, _I]),
+    "avsep_forward_packed": (C.c_int, [_P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _P, _P, _P, C.c_size_t, _P]),
+    "avsep_forward_host_packed": (C.c_int, [_P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _P, _P, _P]),
+    "avsep_forward_host_packed_async": (C.c_int, [_P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _P, _P, _I, _P]),
     "avsep_last_launch_count": (C.c_int64, [_P]),
     "avsep_audio_encoder": (C.c_int, [_P, _P, _I, _I, _P, _P]),
     "avsep_visual_encoder": (C.c_int, [_P, _P, _I, _I, _I, _I, _I, _P, _P]),

@@ -196,17 +196,24 @@ class Engine:
             if v.device.index != self.device or v.dtype != torch.int32 or tuple(v.shape) != (B,) or not v.is_contiguous():
                 raise ValueError(f"{what}: a device {name} tensor must be contiguous int32 ({B},) on cuda:{self.device}")
             return v
+        a = self._host_lengths(v, name, B, limit, what)
+        buf = self._stream_buf((what, name), B)
+        # the pinned staging block is not reused before this copy has run (torch's host allocator records the stream)
+        buf[:B].copy_(torch.from_numpy(a.astype(np.int32)).pin_memory(), non_blocking=True)
+        return buf[:B]
+
+    @staticmethod
+    def _host_lengths(v, name: str, B: int, limit, what: str) -> np.ndarray:
+        """A list, numpy array or CPU integer tensor of B lengths in [1, limit] (limit None: no upper bound) ->
+        contiguous int32 numpy array.  Raises ValueError."""
         a = v.numpy() if isinstance(v, torch.Tensor) else np.asarray(v)
         if a.shape != (B,):
             raise ValueError(f"{what}: {name} must have one entry per utterance ({B}), got shape {a.shape}")
         if a.dtype == np.bool_ or not np.issubdtype(a.dtype, np.integer):
             raise ValueError(f"{what}: {name} must hold integers, got {a.dtype}")
-        if a.min() < 1 or a.max() > limit:
+        if a.min() < 1 or (limit is not None and a.max() > limit):
             raise ValueError(f"{what}: {name} must lie in [1, {limit}], got [{a.min()}, {a.max()}]")
-        buf = self._stream_buf((what, name), B)
-        # the pinned staging block is not reused before this copy has run (torch's host allocator records the stream)
-        buf[:B].copy_(torch.from_numpy(a.astype(np.int32)).pin_memory(), non_blocking=True)
-        return buf[:B]
+        return np.ascontiguousarray(a, dtype=np.int32)
 
     def _stream_buf(self, name, B: int) -> torch.Tensor:
         """Engine-owned int32 device buffer of at least B entries for ``name`` on the current stream."""
@@ -297,6 +304,112 @@ class Engine:
             rc = self.lib.avsep_forward_host_async(self.h, mixed.data_ptr(), frames.data_ptr(), B, T, N, Hh, Ww,
                                                    sep.data_ptr(), masks.data_ptr(), int(slot), self._stream())
         self._check(rc, "avsep_forward_host_async")
+
+    # ---- packed variable-length batches (include/avsep.h: utterances back to back, no padding) ------------------
+    def _packed_plan(self, what, mixed_p, frames_p, lengths, frame_lengths, max_len, max_frames, out, cuda):
+        """Validates a packed batch before a pointer reaches the library, which sizes its copies and offsets from the
+        lengths.  Returns (B, T, N, Hh, Ww, lens, flens, out): lens / flens are validated int32 numpy arrays, or int32
+        device tensors (cuda only; their sum is not read, so out= and max_len / max_frames must be given and every
+        buffer must hold the padded batch, the largest one such lengths can describe); out = (separated, masks), 1-D,
+        allocated when None (pinned CPU memory for the host path)."""
+        F, S = self.cfg.freq_bins, self.cfg.num_speakers
+        if mixed_p.dim() != 1:
+            raise ValueError(f"{what}: mixed_packed must be 1-D (freq_bins * sum T_b), got {tuple(mixed_p.shape)}")
+        if frames_p.dim() != 3:
+            raise ValueError(f"{what}: frames_packed must be (sum N_b, H, W), got {tuple(frames_p.shape)}")
+        Hh, Ww = int(frames_p.shape[1]), int(frames_p.shape[2])
+        if lengths is None or frame_lengths is None:
+            raise ValueError(f"{what}: lengths and frame_lengths are required")
+        on_dev = [isinstance(v, torch.Tensor) and v.is_cuda for v in (lengths, frame_lengths)]
+        if any(on_dev):
+            if not cuda:
+                raise ValueError(f"{what}: the host-buffer path takes host lengths (they size its copies)")
+            if out is None or max_len is None or max_frames is None:
+                raise ValueError(f"{what}: device lengths need out=, max_len and max_frames (their sum cannot be read "
+                                 "without a synchronise)")
+        B = int(lengths.shape[0]) if on_dev[0] else len(np.asarray(lengths).reshape(-1))
+        if B < 1:
+            raise ValueError(f"{what}: empty batch")
+        lens = lengths if on_dev[0] else self._host_lengths(lengths, "lengths", B, max_len, what)
+        flens = frame_lengths if on_dev[1] else self._host_lengths(frame_lengths, "frame_lengths", B, max_frames, what)
+        T = int(max_len) if max_len is not None else int(lens.max())
+        N = int(max_frames) if max_frames is not None else int(flens.max())
+        if T < 1 or N < 1:
+            raise ValueError(f"{what}: max_len and max_frames must be >= 1")
+        for v, name in ((lens, "lengths"), (flens, "frame_lengths")):
+            if isinstance(v, torch.Tensor) and (v.dtype != torch.int32 or tuple(v.shape) != (B,) or
+                                                not v.is_contiguous() or v.device.index != self.device):
+                raise ValueError(f"{what}: a device {name} tensor must be contiguous int32 ({B},) on cuda:{self.device}")
+        st = B * T if on_dev[0] else int(lens.sum())
+        sn = B * N if on_dev[1] else int(flens.sum())
+
+        def fits(n, want, exact):
+            return n == want if exact else n >= want
+        if not fits(mixed_p.numel(), F * st, not on_dev[0]):
+            raise ValueError(f"{what}: mixed_packed holds {mixed_p.numel()} floats, the lengths need {F * st}")
+        if not fits(int(frames_p.shape[0]), sn, not on_dev[1]):
+            raise ValueError(f"{what}: frames_packed holds {frames_p.shape[0]} frames, the frame lengths need {sn}")
+        if out is None:
+            both = torch.empty((2, S * F * st), dtype=torch.float32,
+                               device=torch.device("cuda", self.device) if cuda else None)
+            out = (both[0], both[1]) if cuda else (both[0].pin_memory(), both[1].pin_memory())
+        for t in out:
+            if (not isinstance(t, torch.Tensor) or t.dim() != 1 or t.dtype != torch.float32 or not t.is_contiguous() or
+                    not fits(t.numel(), S * F * st, not on_dev[0])):
+                raise ValueError(f"{what}: output buffers must be contiguous 1-D float32 of {S * F * st} floats")
+            if t.is_cuda != cuda or (cuda and t.device.index != self.device):
+                raise ValueError(f"{what}: output buffers must live " + (f"on cuda:{self.device}" if cuda else "on the CPU"))
+        return B, T, N, Hh, Ww, lens, flens, tuple(out)
+
+    def forward_packed(self, mixed_p, frames_p, lengths, frame_lengths, max_len=None, max_frames=None, out=None):
+        """avsep_forward_packed: device tensors in the packed layout (see AVSeparationTransformer.forward_packed).
+        Host-form lengths go through engine-owned device buffers of the current stream (stable graph keys)."""
+        what = "forward_packed"
+        mixed_p = self._dev_f32(mixed_p, "mixed_packed")
+        frames_p = self._dev_f32(frames_p, "frames_packed")
+        B, T, N, Hh, Ww, lens, flens, (sep, masks) = self._packed_plan(what, mixed_p, frames_p, lengths, frame_lengths,
+                                                                       max_len, max_frames, out, True)
+        with torch.cuda.device(self.device):
+            lens = self._lengths(lens, "lengths", B, T, what)
+            flens = self._lengths(flens, "frame_lengths", B, N, what)
+            rc = self.lib.avsep_forward_packed(self.h, mixed_p.data_ptr(), frames_p.data_ptr(), lens.data_ptr(),
+                                               flens.data_ptr(), B, T, N, Hh, Ww, sep.data_ptr(), masks.data_ptr(),
+                                               None, 0, self._stream())
+        self._check(rc, "avsep_forward_packed")
+        return sep, masks
+
+    def forward_host_packed(self, mixed_p, frames_p, lengths, frame_lengths, max_len=None, max_frames=None, out=None):
+        """avsep_forward_host_packed: CPU tensors in the packed layout in and out (pinned memory for overlap); only each
+        utterance's own frames cross the link."""
+        what = "forward_host_packed"
+        mixed_p = self._host_f32(mixed_p, "mixed_packed")
+        frames_p = self._host_f32(frames_p, "frames_packed")
+        B, T, N, Hh, Ww, lens, flens, (sep, masks) = self._packed_plan(what, mixed_p, frames_p, lengths, frame_lengths,
+                                                                       max_len, max_frames, out, False)
+        with torch.cuda.device(self.device):
+            rc = self.lib.avsep_forward_host_packed(self.h, mixed_p.data_ptr(), frames_p.data_ptr(), lens.ctypes.data,
+                                                    flens.ctypes.data, B, T, N, Hh, Ww, sep.data_ptr(), masks.data_ptr(),
+                                                    self._stream())
+        self._check(rc, "avsep_forward_host_packed")
+        return sep, masks
+
+    def forward_host_packed_async(self, mixed_p, frames_p, lengths, frame_lengths, out, slot: int, max_len=None,
+                                  max_frames=None):
+        """Streaming form of ``forward_host_packed`` on I/O slot 0 .. 3; ``host_wait(slot)`` completes it.  The four
+        tensors must be contiguous float32 CPU tensors (pinned for overlap) that outlive the wait; the lengths are read
+        before the call returns.  Pass fixed max_len / max_frames so that the graph keys stay the same from batch to
+        batch."""
+        what = "forward_host_packed_async"
+        for t in (mixed_p, frames_p) + tuple(out):
+            if t.is_cuda or t.dtype != torch.float32 or not t.is_contiguous():
+                raise ValueError(f"{what}: contiguous float32 CPU tensors required")
+        B, T, N, Hh, Ww, lens, flens, (sep, masks) = self._packed_plan(what, mixed_p, frames_p, lengths, frame_lengths,
+                                                                       max_len, max_frames, out, False)
+        with torch.cuda.device(self.device):
+            rc = self.lib.avsep_forward_host_packed_async(self.h, mixed_p.data_ptr(), frames_p.data_ptr(),
+                                                          lens.ctypes.data, flens.ctypes.data, B, T, N, Hh, Ww,
+                                                          sep.data_ptr(), masks.data_ptr(), int(slot), self._stream())
+        self._check(rc, "avsep_forward_host_packed_async")
 
     def host_wait(self, slot: int):
         self._check(self.lib.avsep_host_wait(self.h, int(slot)), "avsep_host_wait")

@@ -325,6 +325,34 @@ class AVSeparationTransformer(_InferenceOnly):
         eng = self._get_engine(torch.device(self.host_device))
         return eng.forward_host(mixed_spec, lip_frames, *(out or ()))
 
+    def forward_packed(self, mixed_packed: torch.Tensor, frames_packed: torch.Tensor, lengths, frame_lengths, *,
+                       max_len=None, max_frames=None, out=None):
+        """A variable-length batch with no padding (not a reference method): utterances back to back, each as one
+        contiguous block (include/avsep.h).  ``mixed_packed`` is 1-D, (F * sum T_b); ``frames_packed`` is
+        (sum N_b, H, W); the outputs ``(separated, masks)`` are 1-D, (S * F * sum T_b).  Built and split in torch::
+
+            mixed_packed = torch.cat([m.reshape(-1) for m in specs])      # specs[b]: (F, T_b)
+            frames_packed = torch.cat(frame_list)                          # frame_list[b]: (N_b, H, W)
+            seps = [x.view(S, F, t) for x, t in zip(torch.split(sep, [S * F * t for t in lengths]), lengths)]
+
+        Utterance b's block equals ``forward(..., lengths=, frame_lengths=)`` on the padded batch at [b, :, :, :T_b],
+        bit for bit.  CUDA tensors run on the device (``avsep_forward_packed``); CPU tensors through the host-buffer
+        pipeline (``avsep_forward_host_packed``), where only each utterance's own frames cross the link (pinned memory
+        for overlap).
+
+        ``lengths`` / ``frame_lengths``: (B,) audio / lip frames per utterance as a list, numpy array or CPU integer
+        tensor, validated, and the packed sizes are checked against them.  For CUDA inputs, int32 CUDA tensors are
+        accepted too, with ``out=`` (and max_len / max_frames): their sum cannot be read without a synchronise, so
+        every buffer must then hold the padded batch.  ``max_len`` / ``max_frames`` (default: the batch maxima) are the
+        shapes the library's CUDA graphs are keyed on: a streaming caller passes fixed maxima, so that every batch
+        replays the same graphs instead of capturing new ones."""
+        if mixed_packed.is_cuda:
+            return self._get_engine(mixed_packed.device).forward_packed(
+                mixed_packed, frames_packed, lengths, frame_lengths, max_len=max_len, max_frames=max_frames, out=out)
+        eng = self._get_engine(torch.device(self.host_device))
+        return eng.forward_host_packed(mixed_packed, frames_packed, lengths, frame_lengths, max_len=max_len,
+                                       max_frames=max_frames, out=out)
+
     def separate_waveforms(self, mixed_wave: torch.Tensor, lip_frames: torch.Tensor, n_fft: int = None,
                            hop_length: int = 128, *, lengths=None, frame_lengths=None):
         """Waveform in, waveforms out (not a reference method: the reference lists phase / iSTFT reconstruction as

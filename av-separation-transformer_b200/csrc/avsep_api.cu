@@ -132,6 +132,11 @@ struct avsep_handle {
     std::vector<cudaEvent_t> ev;                            // 2 per chunk: copy-in done, kernels done
     cudaEvent_t ev_start = nullptr, ev_end = nullptr;       // ev_end: last copy-out done
     cudaEvent_t ev_lane[3] = {nullptr, nullptr, nullptr};   // last kernels of this slot on each compute lane
+    // packed batches (avsep_forward_host_packed*): the call's lengths, then its frame lengths, uploaded once per call
+    int32_t* lens_host = nullptr;                           // pinned
+    int32_t* lens_dev = nullptr;
+    int lens_cap = 0;                                       // utterances each array holds
+    cudaEvent_t ev_lens = nullptr;                          // upload of lens_host done
   } slot[AVSEP_HOST_SLOTS];
   std::vector<void*> shared_owned, shared_mapped;   // avsep_shared_alloc / avsep_shared_open
   float* synth_waves = nullptr;   // scratch of avsep_synth_batch
@@ -246,11 +251,10 @@ int check_shape(avsep_handle* h, int B, int T, int N, int Hh, int Ww) {
   return 0;
 }
 
-int get_workspace(avsep_handle* h, Workspace& w, void* user_ws, size_t user_bytes, int B, int T, int N, int Hh, int Ww) {
-  const size_t need = carve_workspace(h, w, nullptr, B, T, N, Hh, Ww);
-  uint8_t* base = nullptr;
+// The caller's workspace when given (checked against `need`), else the library-owned one grown to `need`.
+int workspace_base(avsep_handle* h, void* user_ws, size_t user_bytes, size_t need, const char* sizer, uint8_t*& base) {
   if (user_ws != nullptr) {
-    if (user_bytes < need) return fail(h, "workspace too small: see avsep_workspace_bytes");
+    if (user_bytes < need) return fail(h, std::string("workspace too small: see ") + sizer);
     if ((reinterpret_cast<uintptr_t>(user_ws) & 1023) != 0) return fail(h, "workspace must be 1024-byte aligned");
     base = static_cast<uint8_t*>(user_ws);
   } else {
@@ -264,8 +268,37 @@ int get_workspace(avsep_handle* h, Workspace& w, void* user_ws, size_t user_byte
     }
     base = static_cast<uint8_t*>(h->own_ws);
   }
+  return 0;
+}
+
+int get_workspace(avsep_handle* h, Workspace& w, void* user_ws, size_t user_bytes, int B, int T, int N, int Hh, int Ww) {
+  uint8_t* base = nullptr;
+  if (workspace_base(h, user_ws, user_bytes, carve_workspace(h, w, nullptr, B, T, N, Hh, Ww), "avsep_workspace_bytes",
+                     base))
+    return 1;
   carve_workspace(h, w, base, B, T, N, Hh, Ww);
   return 0;
+}
+
+// Padded staging of a packed batch: the varlen forward's inputs and outputs, (B, F, T), (B, N, Hh, Ww) and 2 x
+// (B, S, F, T), carved behind the forward's own workspace.  Returns the bytes of both.
+struct Staging {
+  float *mixed, *frames, *sep, *masks;
+};
+size_t carve_packed(const avsep_handle* h, Workspace& w, Staging& st, uint8_t* base, int B, int T, int N, int Hh,
+                    int Ww) {
+  size_t off = carve_workspace(h, w, base, B, T, N, Hh, Ww);
+  auto take = [&](size_t floats) {
+    float* p = base ? reinterpret_cast<float*>(base + off) : nullptr;
+    off += align_up(floats * 4, 1024);
+    return p;
+  };
+  const size_t F = h->cfg.freq_bins, S = h->cfg.num_speakers;
+  st.mixed = take(B * F * T);
+  st.frames = take(static_cast<size_t>(B) * N * Hh * Ww);
+  st.sep = take(B * S * F * T);
+  st.masks = take(B * S * F * T);
+  return off;
 }
 
 // ---- debug snapshots ---------------------------------------------------------------------------
@@ -703,6 +736,26 @@ int forward_cached(avsep_handle* h, cudaStream_t s, Workspace& w, const void* ws
   return 0;
 }
 
+// Utterances b0 .. b0 + w.B - 1 of a packed batch (include/avsep.h) through the staging: unpack, the varlen forward
+// (cached graph) on the staging, pack.  lens / flens: DEVICE lengths of the whole packed batch (or null), from whose
+// first b0 entries the kernels find the chunk's packed offsets.  Sets w.lens / w.frame_lens.
+int forward_packed_run(avsep_handle* h, cudaStream_t s, Workspace& w, const Staging& st, const void* ws_base,
+                       const float* mixed_p, const float* frames_p, const int* lens, const int* flens, int b0,
+                       float* sep_p, float* masks_p) {
+  const int F = h->cfg.freq_bins, S = h->cfg.num_speakers;
+  h->prof_stream = s;
+  CKL("unpack", launch_unpack(s, mixed_p, frames_p, lens, flens, b0, w.B, F, w.T, w.N, w.Hh * w.Ww, st.mixed,
+                              st.frames));
+  w.lens = lens ? lens + b0 : nullptr;
+  w.frame_lens = flens ? flens + b0 : nullptr;
+  h->launches = 0;   // a graph replay sets the forward's own count
+  if (forward_cached(h, s, w, ws_base, st.mixed, st.frames, st.sep, st.masks)) return 1;
+  h->prof_stream = s;
+  CKL("pack", launch_pack(s, st.sep, st.masks, lens, b0, w.B, S, F, w.T, sep_p, masks_p));
+  ++h->launches;     // the unpack
+  return 0;
+}
+
 // ---- weight access helpers ---------------------------------------------------------------------
 const HostTensor* find_w(avsep_handle* h, const std::string& key, std::initializer_list<int64_t> shape) {
   auto it = h->host_w.find(key);
@@ -862,6 +915,9 @@ void avsep_destroy(avsep_handle* h) {
     if (sl.ev_end) cudaEventDestroy(sl.ev_end);
     for (cudaEvent_t e : sl.ev_lane)
       if (e) cudaEventDestroy(e);
+    if (sl.ev_lens) cudaEventDestroy(sl.ev_lens);
+    if (sl.lens_dev) cudaFree(sl.lens_dev);
+    if (sl.lens_host) cudaFreeHost(sl.lens_host);
   }
   for (void* ptr : h->shared_mapped) cudaIpcCloseMemHandle(ptr);
   for (void* ptr : h->shared_owned) cudaFree(ptr);
@@ -1094,15 +1150,67 @@ int avsep_forward_varlen(avsep_handle* h, const float* mixed_spec, const float* 
                         lip_frames, separated, masks);
 }
 
+size_t avsep_packed_workspace_bytes(avsep_handle* h, int32_t B, int32_t T, int32_t N, int32_t Hh, int32_t Ww) {
+  if (!h || B < 1 || T < 1 || N < 1 || Hh < 1 || Ww < 1) return 0;
+  Workspace w;
+  Staging st;
+  return carve_packed(h, w, st, nullptr, B, T, N, Hh, Ww);
+}
+
+int avsep_forward_packed(avsep_handle* h, const float* mixed_packed, const float* frames_packed, const int32_t* lengths,
+                         const int32_t* frame_lengths, int32_t B, int32_t T, int32_t N, int32_t Hh, int32_t Ww,
+                         float* separated_packed, float* masks_packed, void* workspace, size_t workspace_bytes,
+                         void* cuda_stream) {
+  if (!h) return 1;
+  if (!mixed_packed || !frames_packed || !separated_packed || !masks_packed)
+    return fail(h, "avsep_forward_packed: null buffer");
+  if ((reinterpret_cast<uintptr_t>(mixed_packed) | reinterpret_cast<uintptr_t>(frames_packed) |
+       reinterpret_cast<uintptr_t>(separated_packed) | reinterpret_cast<uintptr_t>(masks_packed)) & 3)
+    return fail(h, "avsep_forward_packed: buffers must be 4-byte aligned");
+  if (check_shape(h, B, T, N, Hh, Ww)) return 1;
+  CUDA_OK(cudaSetDevice(h->cfg.device));
+  Workspace w;
+  Staging st;
+  uint8_t* base = nullptr;
+  if (workspace_base(h, workspace, workspace_bytes, carve_packed(h, w, st, nullptr, B, T, N, Hh, Ww),
+                     "avsep_packed_workspace_bytes", base))
+    return 1;
+  carve_packed(h, w, st, base, B, T, N, Hh, Ww);
+  h->launches = 0;
+  return forward_packed_run(h, static_cast<cudaStream_t>(cuda_stream), w, st, base, mixed_packed, frames_packed,
+                            lengths, frame_lengths, 0, separated_packed, masks_packed);
+}
+
 namespace {
+// packed: the buffers hold packed batches (include/avsep.h) with HOST lengths lens / flens (null: all T / all N); each
+// chunk's copies then cover its packed span and its kernels are forward_packed_run's.
 int host_submit(avsep_handle* h, const float* mixed_spec, const float* lip_frames, int B, int T, int N, int Hh, int Ww,
-                float* separated, float* masks, int slot_id, cudaStream_t s, bool streaming) {
+                float* separated, float* masks, int slot_id, cudaStream_t s, bool streaming, bool packed = false,
+                const int32_t* lens = nullptr, const int32_t* flens = nullptr) {
   // Software pipeline over chunks of the batch: H2D of chunk i+1, kernels of chunk i and D2H of chunk i-1 run
   // concurrently on separate streams (PCIe is full duplex), so a call costs ~max(copy-in, compute, copy-out); the
   // two slots extend the same pipeline across consecutive calls.
-  if (!mixed_spec || !lip_frames || !separated || !masks) return fail(h, "avsep_forward_host: null buffer");
-  if (slot_id < 0 || slot_id >= AVSEP_HOST_SLOTS) return fail(h, "avsep_forward_host_async: slot must be 0 .. AVSEP_HOST_SLOTS - 1");
+  const std::string who = packed ? "avsep_forward_host_packed" : "avsep_forward_host";
+  if (!mixed_spec || !lip_frames || !separated || !masks) return fail(h, who + ": null buffer");
+  if (slot_id < 0 || slot_id >= AVSEP_HOST_SLOTS) return fail(h, who + "_async: slot must be 0 .. AVSEP_HOST_SLOTS - 1");
   if (check_shape(h, B, T, N, Hh, Ww)) return 1;
+  // packed spans: utterances [0, b) hold t_at(b) audio and n_at(b) lip frames; host lengths size the copies, so a
+  // value out of range is an error here, not clamped
+  std::vector<size_t> pt, pn;
+  if (packed) {
+    pt.assign(B + 1, 0);
+    pn.assign(B + 1, 0);
+    for (int b = 0; b < B; ++b) {
+      const int tb = lens ? lens[b] : T, nb = flens ? flens[b] : N;
+      if (tb < 1 || tb > T || nb < 1 || nb > N)
+        return fail(h, who + ": lengths[" + std::to_string(b) + "] = " + std::to_string(tb) + ", frame_lengths[" +
+                           std::to_string(b) + "] = " + std::to_string(nb) + " outside [1, T] / [1, N]");
+      pt[b + 1] = pt[b] + tb;
+      pn[b + 1] = pn[b] + nb;
+    }
+  }
+  auto t_at = [&](size_t b) { return packed ? pt[b] : b * T; };
+  auto n_at = [&](size_t b) { return packed ? pn[b] : b * N; };
   CUDA_OK(cudaSetDevice(h->cfg.device));
   avsep_handle::HostSlot& sl = h->slot[slot_id];
   const size_t F = h->cfg.freq_bins, S = h->cfg.num_speakers;
@@ -1127,6 +1235,28 @@ int host_submit(avsep_handle* h, const float* mixed_spec, const float* lip_frame
     return 0;
   };
   if (make_event(sl.ev_start) || make_event(sl.ev_end)) return 1;
+  const bool upload = packed && (lens || flens);
+  if (upload) {
+    if (sl.lens_cap < B) {
+      CUDA_OK(cudaEventSynchronize(sl.ev_end));     // the slot's previous call still reads them
+      if (sl.lens_dev) cudaFree(sl.lens_dev);
+      if (sl.lens_host) cudaFreeHost(sl.lens_host);
+      sl.lens_dev = nullptr;
+      sl.lens_host = nullptr;
+      sl.lens_cap = 0;
+      CUDA_OK(cudaMalloc(&sl.lens_dev, 2 * sizeof(int32_t) * B));
+      CUDA_OK(cudaMallocHost(&sl.lens_host, 2 * sizeof(int32_t) * B));
+      sl.lens_cap = B;
+    }
+    if (make_event(sl.ev_lens)) return 1;
+    CUDA_OK(cudaEventSynchronize(sl.ev_lens));      // the previous upload from lens_host has been read
+    for (int b = 0; b < B; ++b) {
+      sl.lens_host[b] = lens ? lens[b] : T;
+      sl.lens_host[B + b] = flens ? flens[b] : N;
+    }
+  }
+  const int32_t* d_lens = upload && lens ? sl.lens_dev : nullptr;
+  const int32_t* d_flens = upload && flens ? sl.lens_dev + B : nullptr;
   // Chunk size: a stack kernel takes as long for 64 utterances as for 256 (one tile per CTA either way), so chunks are
   // a trade between pipelining inside one call and kernel time.  Measured at B = 256 (tools/e2e_probe.py): the one-call
   // form is fastest with ~56-utterance chunks on two compute lanes (copy-in of chunk i+1 under the kernels of chunk i),
@@ -1151,7 +1281,9 @@ int host_submit(avsep_handle* h, const float* mixed_spec, const float* lip_frame
   const int want_lanes = h->host_lanes > 0 ? h->host_lanes : (streaming ? 1 : 2);
   const int lanes = want_lanes > 3 ? 3 : want_lanes;
   Workspace wl[3];
-  const size_t per_lane = carve_workspace(h, wl[0], nullptr, Bc, T, N, Hh, Ww);
+  Staging stl[3];
+  const size_t per_lane = packed ? carve_packed(h, wl[0], stl[0], nullptr, Bc, T, N, Hh, Ww)
+                                 : carve_workspace(h, wl[0], nullptr, Bc, T, N, Hh, Ww);
   if (h->host_ws_bytes < per_lane * lanes) {
     CUDA_OK(cudaDeviceSynchronize());          // the other slot may still be using the old workspace
     drop_graphs(h);
@@ -1162,7 +1294,11 @@ int host_submit(avsep_handle* h, const float* mixed_spec, const float* lip_frame
     h->host_ws_bytes = per_lane * lanes;
   }
   for (int l = 0; l < lanes; ++l) {
-    carve_workspace(h, wl[l], static_cast<uint8_t*>(h->host_ws) + l * per_lane, Bc, T, N, Hh, Ww);
+    uint8_t* lane_base = static_cast<uint8_t*>(h->host_ws) + l * per_lane;
+    if (packed)
+      carve_packed(h, wl[l], stl[l], lane_base, Bc, T, N, Hh, Ww);
+    else
+      carve_workspace(h, wl[l], lane_base, Bc, T, N, Hh, Ww);
     if (h->host_comp[l] == nullptr) CUDA_OK(cudaStreamCreateWithFlags(&h->host_comp[l], cudaStreamNonBlocking));
     if (make_event(sl.ev_lane[l])) return 1;
   }
@@ -1178,30 +1314,37 @@ int host_submit(avsep_handle* h, const float* mixed_spec, const float* lip_frame
     CUDA_OK(cudaStreamWaitEvent(h->host_comp[l], sl.ev_end, 0));
   }
   CUDA_OK(cudaStreamWaitEvent(s_out, sl.ev_start, 0));
+  if (upload) {
+    CUDA_OK(cudaMemcpyAsync(sl.lens_dev, sl.lens_host, 2 * sizeof(int32_t) * B, cudaMemcpyHostToDevice, s_in));
+    CUDA_OK(cudaEventRecord(sl.ev_lens, s_in));
+  }
+  const size_t HW = static_cast<size_t>(Hh) * Ww, SF = S * F;
   int64_t launches = 0;
   for (int c = 0; c < nchunks; ++c) {
     const size_t b0 = starts[c];
     const int bc = sizes[c];
     const int lane = c % lanes;
     cudaStream_t s_comp = h->host_comp[lane];
-    CUDA_OK(cudaMemcpyAsync(io_mixed + b0 * mixed_per, mixed_spec + b0 * mixed_per, bc * mixed_per * 4,
-                            cudaMemcpyHostToDevice, s_in));
-    CUDA_OK(cudaMemcpyAsync(io_frames + b0 * frames_per, lip_frames + b0 * frames_per, bc * frames_per * 4,
-                            cudaMemcpyHostToDevice, s_in));
+    // element offsets and counts of the chunk's span in each tensor (packed or padded)
+    const size_t m0 = F * t_at(b0), mn = F * (t_at(b0 + bc) - t_at(b0));
+    const size_t f0 = HW * n_at(b0), fn = HW * (n_at(b0 + bc) - n_at(b0));
+    const size_t o0 = SF * t_at(b0), on = SF * (t_at(b0 + bc) - t_at(b0));
+    CUDA_OK(cudaMemcpyAsync(io_mixed + m0, mixed_spec + m0, mn * 4, cudaMemcpyHostToDevice, s_in));
+    CUDA_OK(cudaMemcpyAsync(io_frames + f0, lip_frames + f0, fn * 4, cudaMemcpyHostToDevice, s_in));
     CUDA_OK(cudaEventRecord(sl.ev[2 * c], s_in));
     CUDA_OK(cudaStreamWaitEvent(s_comp, sl.ev[2 * c], 0));
     Workspace wc = wl[lane];
     wc.B = bc;
-    if (forward_cached(h, s_comp, wc, static_cast<uint8_t*>(h->host_ws) + lane * per_lane, io_mixed + b0 * mixed_per,
-                       io_frames + b0 * frames_per, io_sep + b0 * out_per, io_masks + b0 * out_per))
+    const uint8_t* ws_lane = static_cast<uint8_t*>(h->host_ws) + lane * per_lane;
+    if (packed ? forward_packed_run(h, s_comp, wc, stl[lane], ws_lane, io_mixed, io_frames, d_lens, d_flens,
+                                    static_cast<int>(b0), io_sep, io_masks)
+               : forward_cached(h, s_comp, wc, ws_lane, io_mixed + m0, io_frames + f0, io_sep + o0, io_masks + o0))
       return 1;
     launches += h->launches;
     CUDA_OK(cudaEventRecord(sl.ev[2 * c + 1], s_comp));
     CUDA_OK(cudaStreamWaitEvent(s_out, sl.ev[2 * c + 1], 0));
-    CUDA_OK(cudaMemcpyAsync(separated + b0 * out_per, io_sep + b0 * out_per, bc * out_per * 4,
-                            cudaMemcpyDeviceToHost, s_out));
-    CUDA_OK(cudaMemcpyAsync(masks + b0 * out_per, io_masks + b0 * out_per, bc * out_per * 4,
-                            cudaMemcpyDeviceToHost, s_out));
+    CUDA_OK(cudaMemcpyAsync(separated + o0, io_sep + o0, on * 4, cudaMemcpyDeviceToHost, s_out));
+    CUDA_OK(cudaMemcpyAsync(masks + o0, io_masks + o0, on * 4, cudaMemcpyDeviceToHost, s_out));
   }
   h->launches = launches;
   for (int l = 0; l < lanes; ++l) CUDA_OK(cudaEventRecord(sl.ev_lane[l], h->host_comp[l]));
@@ -1227,6 +1370,26 @@ int avsep_forward_host_async(avsep_handle* h, const float* mixed_spec, const flo
   if (!h) return 1;
   return host_submit(h, mixed_spec, lip_frames, B, T, N, Hh, Ww, separated, masks, slot,
                      static_cast<cudaStream_t>(cuda_stream), true);
+}
+
+int avsep_forward_host_packed(avsep_handle* h, const float* mixed_packed, const float* frames_packed,
+                              const int32_t* lengths, const int32_t* frame_lengths, int32_t B, int32_t T, int32_t N,
+                              int32_t Hh, int32_t Ww, float* separated_packed, float* masks_packed, void* cuda_stream) {
+  if (!h) return 1;
+  if (host_submit(h, mixed_packed, frames_packed, B, T, N, Hh, Ww, separated_packed, masks_packed, 0,
+                  static_cast<cudaStream_t>(cuda_stream), false, true, lengths, frame_lengths))
+    return 1;
+  CUDA_OK(cudaEventSynchronize(h->slot[0].ev_end));
+  return 0;
+}
+
+int avsep_forward_host_packed_async(avsep_handle* h, const float* mixed_packed, const float* frames_packed,
+                                    const int32_t* lengths, const int32_t* frame_lengths, int32_t B, int32_t T,
+                                    int32_t N, int32_t Hh, int32_t Ww, float* separated_packed, float* masks_packed,
+                                    int32_t slot, void* cuda_stream) {
+  if (!h) return 1;
+  return host_submit(h, mixed_packed, frames_packed, B, T, N, Hh, Ww, separated_packed, masks_packed, slot,
+                     static_cast<cudaStream_t>(cuda_stream), true, true, lengths, frame_lengths);
 }
 
 int avsep_host_wait(avsep_handle* h, int32_t slot) {

@@ -221,6 +221,15 @@ const char* launch_prep_audio(cudaStream_t s, int prec, const float* mixed, void
 // lens (or null): out[b,s,f,t] = 0 for t >= lens[b] (clamped to [1, T]), where masks and mixed are not read.
 const char* launch_separate(cudaStream_t s, const float* masks, const float* mixed, float* out, long long B, int S,
                             int F, int T, const int* lens = nullptr);
+// Packed variable-length batches (packed_io.cu): utterances b0 .. b0 + B - 1 of a packed batch, whose blocks sit back to
+// back behind those of utterances 0 .. b0 - 1 (offsets summed on the device from lens / flens, clamped as utt_len
+// clamps; null = all T / all N).  unpack: mixed_p (F, T_b) and frames_p (N_b, hw) blocks -> the valid regions of the
+// padded (B, F, T) / (B, N, hw) staging; pack: the valid regions of the padded (B, S, F, T) sep / masks -> their
+// (S, F, T_b) blocks.  Nothing past the lengths is read or written.
+const char* launch_unpack(cudaStream_t s, const float* mixed_p, const float* frames_p, const int* lens,
+                          const int* flens, int b0, int B, int F, int T, int N, int hw, float* mixed, float* frames);
+const char* launch_pack(cudaStream_t s, const float* sep, const float* masks, const int* lens, int b0, int B, int S,
+                        int F, int T, float* sep_p, float* masks_p);
 // Ticket flags of the masks-only gather: 32-bit words in this GPU's or a peer's memory, raised / awaited in stream order.
 struct FlagSet {
   static constexpr int MAX = 16;

@@ -105,6 +105,49 @@ AVSEP_API int avsep_forward_host_async(avsep_handle* h, const float* mixed_spec,
                                        int32_t slot, void* cuda_stream);
 AVSEP_API int avsep_host_wait(avsep_handle* h, int32_t slot);
 
+/* Packed variable-length batches: the batch holds no padding.  Utterances sit back to back in batch order, each as one
+ * contiguous block, so a range of utterances is one contiguous span of every tensor:
+ *   mixed_packed      utterance b's mixed_spec[b, :, :T_b] as an (F, T_b) block, f-major      F * sum T_b floats
+ *   frames_packed     its lip_frames[b, :N_b] as an (N_b, Hh, Ww) block                       sum N_b * Hh * Ww floats
+ *   separated_packed, masks_packed   its outputs [b, :, :, :T_b] as an (S, F, T_b) block       S * F * sum T_b floats
+ * In torch terms the inputs are torch.cat([m.reshape(-1) for m in specs]) and torch.cat(frame_lists), and
+ * torch.split(out, [S * F * t for t in lengths]) followed by .view(S, F, t) gives per-utterance outputs without a copy.
+ * Each utterance's outputs are what avsep_forward_varlen gives in its valid region [b, :, :, :T_b] (bit for bit).
+ * T and N are the maxima the call is shaped for (the CUDA-graph keys): every T_b <= T, N_b <= N.  With every length
+ * full (or NULL lengths) the packed layout is the padded contiguous one, and the results are avsep_forward's. */
+
+/* Workspace of avsep_forward_packed: the forward's (avsep_workspace_bytes) plus the padded input and output staging
+ * (0 on error). */
+AVSEP_API size_t avsep_packed_workspace_bytes(avsep_handle* h, int32_t B, int32_t T, int32_t N, int32_t Hh, int32_t Ww);
+
+/* DEVICE buffers in the packed layout.  lengths, frame_lengths: DEVICE int32 [B] read on the device only, clamped to
+ * [1, T] / [1, N] (the layout is defined by the clamped values), NULL = all T / all N.  One launch expands the packed
+ * inputs into the padded staging, the varlen forward runs on it, one launch gathers the packed outputs: the forward's
+ * launches + 2.  Packed offsets are summed from the lengths on the device, so the call neither synchronises nor depends
+ * on the length values, can be captured in a graph, and a new ragged batch in the same buffers replays the cached
+ * forward graph.  Buffers need only 4-byte alignment.  workspace may be NULL (library-owned, cached per shape), else
+ * avsep_packed_workspace_bytes(B, T, N, Hh, Ww) bytes, 1024-byte aligned. */
+AVSEP_API int avsep_forward_packed(avsep_handle* h, const float* mixed_packed, const float* frames_packed,
+                                   const int32_t* lengths, const int32_t* frame_lengths, int32_t B, int32_t T,
+                                   int32_t N, int32_t Hh, int32_t Ww, float* separated_packed, float* masks_packed,
+                                   void* workspace, size_t workspace_bytes, void* cuda_stream);
+
+/* avsep_forward_packed with HOST buffers: the pipeline of avsep_forward_host / avsep_forward_host_async (chunks of
+ * "host_chunk" utterances on "host_lanes" compute lanes, one H2D copy per input and one D2H copy per output per chunk),
+ * where a chunk's copies cover its packed span, so only each utterance's own frames cross the link.  lengths,
+ * frame_lengths: HOST int32 [B] (NULL = all T / all N); they size the copies, so a value outside [1, T] / [1, N] is an
+ * error and nothing is enqueued.  They are read before the call returns (into a slot-owned pinned buffer uploaded once
+ * per call).  Pinned buffers are needed for overlap; pageable ones give the same results.  The async form uses the
+ * I/O slots and avsep_host_wait of avsep_forward_host_async, with the same rules. */
+AVSEP_API int avsep_forward_host_packed(avsep_handle* h, const float* mixed_packed, const float* frames_packed,
+                                        const int32_t* lengths, const int32_t* frame_lengths, int32_t B, int32_t T,
+                                        int32_t N, int32_t Hh, int32_t Ww, float* separated_packed,
+                                        float* masks_packed, void* cuda_stream);
+AVSEP_API int avsep_forward_host_packed_async(avsep_handle* h, const float* mixed_packed, const float* frames_packed,
+                                              const int32_t* lengths, const int32_t* frame_lengths, int32_t B,
+                                              int32_t T, int32_t N, int32_t Hh, int32_t Ww, float* separated_packed,
+                                              float* masks_packed, int32_t slot, void* cuda_stream);
+
 /* Number of kernels the last avsep_forward on this handle launched. */
 AVSEP_API int64_t avsep_last_launch_count(const avsep_handle* h);
 
