@@ -450,7 +450,7 @@ template <int HD, bool LERP, bool SPLIT>
 const char* launch_t(cudaStream_t s, const AttnDev& d, int B, int H, int Lq) {
   constexpr int SMEM = (SPLIT ? 6 : 3) * 64 * (HD + 8) * 2;
   auto kern = attention_kernel<HD, LERP, SPLIT>;
-  if (!smem_opt_in(kern, SMEM)) return "attention: cudaFuncSetAttribute failed";
+  if (!smem_opt_in(kern, SMEM)) return "attention: cannot raise the shared-memory limit";
   dim3 grid((Lq + QT - 1) / QT, H, B);
   if (launch_pdl(kern, grid, dim3(128), SMEM, s, d) != cudaSuccess) {
     cudaGetLastError();

@@ -318,7 +318,7 @@ bool attention_tc_usable(int prec, const AttnProblem& p) {
 const char* launch_attention_tc(cudaStream_t s, const AttnProblem& p) {
   if (p.B <= 0 || p.Lq <= 0 || p.Lk <= 0) return "attention_tc: empty problem";
   if (p.hd != HD || p.lerp_src != 0) return "attention_tc: needs head dim 64 and materialised K/V rows";
-  if (!smem_opt_in(attention_tc_kernel, SMEM_BYTES)) return "attention_tc: cudaFuncSetAttribute failed";
+  if (!smem_opt_in(attention_tc_kernel, SMEM_BYTES)) return "attention_tc: cannot raise the shared-memory limit";
   const int cols = p.H * HD;
   // rows [B, L] x cols, bf16, box = 64 cols x 128 rows of one utterance; rows past L are zero-filled / clipped
   CUtensorMap tq, tk, tv, to;

@@ -1450,9 +1450,12 @@ int avsep_stft_varlen(avsep_handle* h, const float* waves, const int32_t* length
                       int32_t hop_length, float* spec, float* mag, int32_t* frame_lengths_out, void* cuda_stream) {
   if (!h) return 1;
   if (!waves || !spec) return fail(h, "avsep_stft: null argument");
+  if (B <= 0 || L <= 0) return fail(h, "stft: empty problem");
+  if (!fft_geometry_ok(n_fft, hop_length))
+    return fail(h, "stft: n_fft must be a power of two in [8, 2048], 1 <= hop <= n_fft");
   CUDA_OK(cudaSetDevice(h->cfg.device));
-  CK(launch_stft_complex(static_cast<cudaStream_t>(cuda_stream), waves, lengths, B, L, n_fft, hop_length, spec, mag,
-                         frame_lengths_out));
+  CK(launch_stft(static_cast<cudaStream_t>(cuda_stream), waves, lengths, B, 0, L, n_fft, hop_length, spec, mag, nullptr,
+                 frame_lengths_out));
   h->launches = 1;
   return 0;
 }

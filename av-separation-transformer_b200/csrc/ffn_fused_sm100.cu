@@ -404,7 +404,7 @@ const char* launch_ffn_fused(cudaStream_t s, const void* a, const void* w1, cons
     if (const char* e = tma_encode_2d(&tx, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, x_out, D, M, D, 32, 128)) return e;
   if (out_op != nullptr)
     if (const char* e = tma_encode_2d(&top, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, out_op, D, M, D, 64, 128)) return e;
-  if (!smem_opt_in(ffn_fused_kernel, FFN_SMEM)) return "ffn_fused: cudaFuncSetAttribute failed";
+  if (!smem_opt_in(ffn_fused_kernel, FFN_SMEM)) return "ffn_fused: cannot raise the shared-memory limit";
   FfnDev d;
   d.b1 = b1; d.b2 = b2; d.gamma = gamma; d.beta = beta; d.resid = resid;
   d.M = M; d.act = act; d.has_xout = x_out != nullptr; d.has_op = out_op != nullptr;

@@ -914,7 +914,7 @@ template <int EPI, bool TF32>
 const char* launch_cfg(cudaStream_t s, const CUtensorMap& ta, const CUtensorMap& tw, const CUtensorMap& top,
                        const CUtensorMap& tf32m, const GemmDev& d, int num_sms) {
   auto kern = gemm_tcgen05_kernel<EPI, TF32>;
-  if (!smem_opt_in(kern, SMEM_TOTAL)) return "gemm: cudaFuncSetAttribute(smem) failed";
+  if (!smem_opt_in(kern, SMEM_TOTAL)) return "gemm: cannot raise the shared-memory limit";
   const int tiles = ((d.M + BM - 1) / BM) * ((d.N + d.n_tile - 1) / d.n_tile);
   const int grid = tiles < num_sms ? tiles : num_sms;
   if (launch_pdl(kern, dim3(grid), dim3(NUM_THREADS), SMEM_TOTAL, s, ta, tw, top, tf32m, d) != cudaSuccess) {

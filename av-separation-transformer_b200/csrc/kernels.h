@@ -30,8 +30,8 @@ const char* tma_encode_2d(CUtensorMap* map, CUtensorMapDataType dt, int esz, con
 // The same for `batches` such tensors stored back to back ([batches, outer, inner]); a box stays inside one batch.
 const char* tma_encode_3d(CUtensorMap* map, CUtensorMapDataType dt, int esz, const void* ptr, uint64_t inner,
                           uint64_t outer, uint64_t batches, uint64_t ld_elems, uint32_t box_inner, uint32_t box_outer);
-// Raises the kernel's dynamic shared-memory limit to `bytes` unless this process already set it at least that high (up
-// to 48 KB needs no opt-in).  False when the runtime refuses.
+// Raises the kernel's dynamic shared-memory limit on the current device to `bytes` unless this process already set it
+// at least that high there (up to 48 KB needs no opt-in).  False when the runtime refuses.
 bool smem_opt_in(const void* kern, int bytes);
 template <typename... KArgs>
 bool smem_opt_in(void (*kern)(KArgs...), int bytes) {
@@ -299,14 +299,21 @@ const char* launch_synth(cudaStream_t s, const SynthProblem& p);
 const char* launch_eval_snr(cudaStream_t s, const float* separated, const float* targets, const float* mixed, int B,
                             int S, int FT, double* input_snr, double* output_snr, int* best_perm, double* si_snr);
 
-// ---- waveform side (waveform.cu): complex STFT with the reference's framing, masked inverse STFT ----
-// lengths: device int32 [B] samples per utterance, or null (all L).  The stft runs its variable-length kernel when
-// lengths or frame_lengths (device int32 [B], receives 1 + length / hop) is given; the istft when lengths is.
-const char* launch_stft_complex(cudaStream_t s, const float* waves, const int* lengths, int B, int L, int nfft, int hop,
-                                float* spec, float* mag, int* frame_lengths);
+// ---- waveform side (waveform.cu): STFT analysis with the reference's framing, masked inverse STFT ----
+bool fft_size_ok(int nfft);               // a power of two in [8, 2048]: the sizes the transforms take
+bool fft_geometry_ok(int nfft, int hop);  // fft_size_ok and 1 <= hop <= nfft: frames that leave no sample out
 const char* fft512_init_tables();   // window + twiddle tables of the n_fft = 512 kernels, once per device (avsep_create)
-const char* launch_stft512_synth(cudaStream_t s, const float* waves, int B, int S, int n, int hop, float* mixed_spec,
-                                 float* clean_specs);
+// STFT analysis of signals of L samples: T = 1 + L / hop frames, F = nfft / 2 + 1 bins; a radix-8 register transform for
+// nfft = 512, a shared-memory radix-2 one otherwise.  The caller checks fft_size_ok(nfft), hop >= 1 and B, L >= 1.
+//   S1 = 0: waves (B, L) -> spec (B, F, T) complex64 and mag (B, F, T) float, either may be null.  lengths: device
+//           int32 [B] samples per utterance, or null (all L); the variable-length kernel runs when lengths or
+//           frame_lengths (device int32 [B], receives 1 + length / hop) is given.
+//   S1 > 0: the synthesis layout, waves (B, S1, L) with the mixture as signal 0 -> magnitudes only: mag (B, F, T) of
+//           the mixture, mag2 (B, S1 - 1, F, T) of the other signals or null.  spec, lengths, frame_lengths null.
+// B * max(S1, 1) above 65535 is "stft: launch failed".
+const char* launch_stft(cudaStream_t s, const float* waves, const int* lengths, int B, int S1, int L, int nfft, int hop,
+                        float* spec, float* mag, float* mag2, int* frame_lengths);
+// lengths as for launch_stft: the istft runs its variable-length kernel when it is given.
 const char* launch_istft_masked(cudaStream_t s, const float* spec, const float* masks, const int* lengths, int B, int S,
                                 int T, int nfft, int hop, int L, float* waves);
 

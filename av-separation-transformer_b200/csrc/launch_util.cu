@@ -3,8 +3,9 @@
 
 #include <cudaTypedefs.h>
 
+#include <map>
 #include <mutex>
-#include <unordered_map>
+#include <utility>
 
 namespace avsep {
 
@@ -55,11 +56,16 @@ const char* tma_encode_3d(CUtensorMap* map, CUtensorMapDataType dt, int esz, con
 }
 
 bool smem_opt_in(const void* kern, int bytes) {
+  if (bytes <= 48 * 1024) return true;
+  int dev;
+  if (cudaGetDevice(&dev) != cudaSuccess) return false;
   static std::mutex mu;
-  static std::unordered_map<const void*, int> limit;   // per kernel: the largest limit set so far
+  // per (device, kernel): the largest limit set so far.  The attribute belongs to the kernel's image on the current
+  // device, so a kernel opted in on one device still has the 48 KB default on the next.
+  static std::map<std::pair<int, const void*>, int> limit;
   std::lock_guard<std::mutex> lock(mu);
-  int& cur = limit[kern];
-  if (bytes <= 48 * 1024 || bytes <= cur) return true;
+  int& cur = limit[{dev, kern}];
+  if (bytes <= cur) return true;
   if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes) != cudaSuccess) return false;
   cur = bytes;
   return true;

@@ -6,10 +6,10 @@
 // The reference draws a handful of random numbers per item from numpy's PCG64 and then spends its time in a Python
 // loop of 3 x 63 windowed rFFTs and 50 frame paintings per item.  Here the draws stay on the host (they are inputs:
 // amplitudes, jittered frequencies, phases, patch noise) and the arithmetic runs on the device: fp64 waveform
-// synthesis rounded to fp32 exactly where the reference rounds, Hann window in fp64, a shared-memory radix-2 FFT per
-// frame (fp32, like numpy's single-precision pocketfft), magnitudes written in the (B, F, T) layout the forward
-// consumes; frame energies by block reduction; patches painted with the clip.  All HBM-bound / latency-bound
-// CUDA-core work: no tensor cores.
+// synthesis rounded to fp32 exactly where the reference rounds; the STFT of waveform.cu's analysis kernels (launch_stft:
+// Hann window in fp64, fp32 FFT like numpy's single-precision pocketfft), magnitudes written in the (B, F, T) layout
+// the forward consumes; frame energies by block reduction; patches painted with the clip.  All HBM-bound /
+// latency-bound CUDA-core work: no tensor cores.
 #include "common.cuh"
 #include "kernels.h"
 
@@ -38,86 +38,6 @@ __global__ void synth_wave_kernel(const double* __restrict__ amps, const double*
     mix = __fadd_rn(mix, x);
   }
   waves[static_cast<size_t>(b) * (S + 1) * n + i] = mix;
-}
-
-// One CTA = TG consecutive STFT frames of one signal, N/2 threads (one butterfly per stage).  Two real frames share
-// one complex transform (frame A in the real part, frame B in the imaginary part; A[k] = (Z[k] + conj Z[N-k]) / 2,
-// B[k] = (Z[k] - conj Z[N-k]) / 2i), the fp64 Hann window is evaluated once per CTA.
-constexpr int TG = 8;
-
-__global__ void stft_mag_kernel(const float* __restrict__ waves, int n, int nfft, int log2n, int hop, int T, int F,
-                                int S, float* __restrict__ mixed_spec, float* __restrict__ clean_specs) {
-  extern __shared__ __align__(16) uint8_t sm_raw[];
-  double* win = reinterpret_cast<double*>(sm_raw);          // [nfft]
-  float* re = reinterpret_cast<float*>(win + nfft);         // [nfft]
-  float* im = re + nfft;                                    // [nfft]
-  float* twr = im + nfft;                                   // [nfft/2]
-  float* twi = twr + nfft / 2;                              // [nfft/2]
-  float* stage = twi + nfft / 2;                            // [F][TG]
-  const int sig = blockIdx.y;     // b * (S+1) + j
-  const int b = sig / (S + 1), j = sig - b * (S + 1);
-  const int t0 = blockIdx.x * TG;
-  const int tid = threadIdx.x;    // 0 .. nfft/2-1
-  const float* x = waves + static_cast<size_t>(sig) * n;
-  {
-    float sv, cv;
-    sincospif(-2.0f * static_cast<float>(tid) / static_cast<float>(nfft), &sv, &cv);
-    twr[tid] = cv; twi[tid] = sv;
-    // np.hanning(M): 0.5 + 0.5*cos(pi*(1-M+2k)/(M-1)), fp64
-#pragma unroll
-    for (int h = 0; h < 2; ++h) {
-      const int k = tid + h * (nfft / 2);
-      win[k] = 0.5 + 0.5 * cos(kPi * static_cast<double>(1 - nfft + 2 * k) / static_cast<double>(nfft - 1));
-    }
-  }
-  const int ng = min(TG, T - t0);
-  for (int g = 0; g < ng; g += 2) {
-    const int ta = t0 + g;
-    const bool has_b = g + 1 < ng;
-    __syncthreads();
-    // windowed product rounded to fp32 (in-place `frame *= window` on a float32 array, dataset.py:131), frames
-    // zero-padded past the end of the signal, bit-reversed placement for the in-place DIT transform
-#pragma unroll
-    for (int h = 0; h < 2; ++h) {
-      const int k = tid + h * (nfft / 2);
-      const int sa = ta * hop + k, sb = sa + hop;
-      const float va = sa < n ? x[sa] : 0.f;
-      const float vb = (has_b && sb < n) ? x[sb] : 0.f;
-      const double w = win[k];
-      const int r = static_cast<int>(__brev(static_cast<unsigned>(k)) >> (32 - log2n));
-      re[r] = static_cast<float>(static_cast<double>(va) * w);
-      im[r] = static_cast<float>(static_cast<double>(vb) * w);
-    }
-    for (int s = 1; s <= log2n; ++s) {
-      __syncthreads();
-      const int half = 1 << (s - 1);
-      const int pos = tid & (half - 1);
-      const int i0 = ((tid >> (s - 1)) << s) + pos;
-      const int i1 = i0 + half;
-      const int tw = pos << (log2n - s);
-      const float wr = twr[tw], wi = twi[tw];
-      const float xr = re[i1], xi = im[i1];
-      const float pr = wr * xr - wi * xi, pi = wr * xi + wi * xr;
-      const float ar = re[i0], ai = im[i0];
-      re[i0] = ar + pr; im[i0] = ai + pi;
-      re[i1] = ar - pr; im[i1] = ai - pi;
-    }
-    __syncthreads();
-    for (int f = tid; f < F; f += blockDim.x) {
-      const int fn = (nfft - f) & (nfft - 1);
-      const float zr = re[f], zi = im[f], yr = re[fn], yi = im[fn];
-      stage[f * TG + g] = 0.5f * hypotf(zr + yr, zi - yi);
-      if (has_b) stage[f * TG + g + 1] = 0.5f * hypotf(zi + yi, yr - zr);
-    }
-  }
-  __syncthreads();
-  float* out = j == 0 ? mixed_spec + static_cast<size_t>(b) * F * T
-                      : (clean_specs ? clean_specs + (static_cast<size_t>(b) * S + (j - 1)) * F * T : nullptr);
-  if (out == nullptr) return;
-  for (int e = tid; e < F * TG; e += blockDim.x) {
-    const int f = e / TG, g = e - f * TG;
-    if (g < ng) out[static_cast<size_t>(f) * T + t0 + g] = stage[e];
-  }
 }
 
 // One warp per (b, speaker, video frame), no block-level synchronisation: energy = fp32 mean of x^2 over the frame's
@@ -285,22 +205,15 @@ __global__ void eval_snr_kernel(const float* __restrict__ separated, const float
 const char* launch_synth(cudaStream_t s, const SynthProblem& p) {
   if (p.B <= 0) return "synth: empty batch";
   if (p.S < 1 || p.S > 8) return "synth: num_speakers must be 1..8";
-  if (p.nfft < 8 || p.nfft > 2048 || (p.nfft & (p.nfft - 1))) return "synth: n_fft must be a power of two in [8, 2048]";
+  if (!fft_size_ok(p.nfft)) return "synth: n_fft must be a power of two in [8, 2048]";
   if (p.n < 1 || p.hop < 1 || p.nf < 1 || p.Hh < 1 || p.Ww < 1) return "synth: bad geometry";
   if (p.nf > p.n) return "synth: more video frames than audio samples";
-  int log2n = 0;
-  while ((1 << log2n) < p.nfft) ++log2n;
-  const int T = 1 + p.n / p.hop, F = p.nfft / 2 + 1;
+  if (static_cast<long long>(p.B) * (p.S + 1) > 65535) return "synth: batch * (speakers + 1) above 65535";
   synth_wave_kernel<<<dim3((p.n + 255) / 256, p.B), 256, 0, s>>>(p.amps, p.freqs, p.phases, p.S, p.n,
                                                                  p.duration / static_cast<double>(p.n), p.waves);
-  const size_t smem = static_cast<size_t>(p.nfft) * sizeof(double) +
-                      (3 * static_cast<size_t>(p.nfft) + static_cast<size_t>(F) * TG) * sizeof(float);
-  if (p.nfft == 512 && p.B * (p.S + 1) <= 65535) {   // the reference's default geometry: register radix-8 transform
-    if (const char* e = launch_stft512_synth(s, p.waves, p.B, p.S, p.n, p.hop, p.mixed_spec, p.clean_specs)) return e;
-  } else {
-    stft_mag_kernel<<<dim3((T + TG - 1) / TG, p.B * (p.S + 1)), p.nfft / 2, smem, s>>>(
-        p.waves, p.n, p.nfft, log2n, p.hop, T, F, p.S, p.mixed_spec, p.clean_specs);
-  }
+  if (const char* e = launch_stft(s, p.waves, nullptr, p.B, p.S + 1, p.n, p.nfft, p.hop, nullptr, p.mixed_spec,
+                                  p.clean_specs, nullptr))
+    return e;
   const long long lip_warps = static_cast<long long>(p.B) * p.S * p.nf;
   lip_frames_kernel<<<static_cast<unsigned>((lip_warps + 7) / 8), 256, 0, s>>>(p.waves, p.noise, p.B, p.S, p.n, p.nf,
                                                                               p.Hh, p.Ww, p.lip_frames);

@@ -446,7 +446,7 @@ const char* launch_visual_cnn(cudaStream_t s, int prec, const float* frames, int
   d.num_groups = (M + G - 1) / G;
   const size_t smem = fixed + per_frame * G;
   auto kern = split ? visual_cnn_kernel<true> : visual_cnn_kernel<false>;
-  if (!smem_opt_in(kern, static_cast<int>(cap))) return "visual_cnn: cudaFuncSetAttribute failed";
+  if (!smem_opt_in(kern, static_cast<int>(cap))) return "visual_cnn: cannot raise the shared-memory limit";
   const int grid = d.num_groups < num_sms ? d.num_groups : num_sms;
   kern<<<grid, CNN_THREADS, smem, s>>>(d);
   return cudaGetLastError() == cudaSuccess ? nullptr : "visual_cnn: launch failed";

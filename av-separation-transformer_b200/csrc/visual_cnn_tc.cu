@@ -470,7 +470,7 @@ const char* launch_visual_cnn_tc(cudaStream_t s, const float* frames, int M, con
   if (M <= 0) return "visual_cnn_tc: empty problem";
   CUtensorMap tm;   // w3_rows as [9 * 128 rows][64] bf16
   if (const char* e = tma_encode_2d(&tm, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, w3_rows, 64, 9 * 128, 64, 64, 128)) return e;
-  if (!smem_opt_in(visual_cnn_tc_kernel, TC_SMEM)) return "visual_cnn_tc: cudaFuncSetAttribute failed";
+  if (!smem_opt_in(visual_cnn_tc_kernel, TC_SMEM)) return "visual_cnn_tc: cannot raise the shared-memory limit";
   CnnTcDev d;
   d.frames = frames; d.pooled = reinterpret_cast<__nv_bfloat16*>(pooled);
   d.w1 = w.w1; d.b1 = w.b1; d.w2_slabs = w2_slabs; d.b2 = w.b2; d.b3 = w.b3;

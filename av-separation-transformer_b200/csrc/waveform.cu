@@ -4,7 +4,8 @@
 //
 //   stft_complex_kernel   the framing of SyntheticAVDataset._stft (dataset.py:122-135: frame i starts at i*hop, no
 //                         centring, zero-padded past the end, np.hanning window, rfft) keeping the phase: complex64
-//                         (B, F, T); |.| is bit-identical to the magnitudes of synth.cu's stft_mag_kernel.
+//                         (B, F, T), and/or the float32 magnitudes.  It is also the analysis of input synthesis
+//                         (synth.cu), whose (B, S+1, n) signals it reads in place and whose magnitudes it writes.
 //   istft_masked_kernel   y[b,s,n] = sum_i w[n-i*hop] * irfft(mask[b,s,:,i] * X[b,:,i])[n-i*hop] / sum_i w^2[n-i*hop]
 //                         (weighted overlap-add, the least-squares inverse of that analysis; samples no window
 //                         reaches with non-zero weight - n = 0 for a Hann window - come out 0).
@@ -48,35 +49,52 @@ __device__ __forceinline__ double hann(int k, int nfft) {
   return 0.5 + 0.5 * cos(kPi * static_cast<double>(1 - nfft + 2 * k) / static_cast<double>(nfft - 1));
 }
 
+// Output selection of the analysis kernels.  S1 == 0: signal sig's (F, T) plane of spec / mag.  S1 > 0 (the synthesis
+// layout, signals (B, S1) with the mixture first): magnitudes only, the mixture's plane of mag (B, F, T) or speaker
+// j - 1's plane of mag2 (B, S1-1, F, T), which may be null.  Returns the plane's offset and sets *m_out.
+__device__ __forceinline__ size_t stft_out_plane(int sig, int S1, int F, int T, float* mag, float* mag2,
+                                                 float** m_out) {
+  *m_out = mag;
+  size_t base = static_cast<size_t>(sig) * F * T;
+  if (S1 > 0) {
+    const int b = sig / S1, j = sig - b * S1;
+    *m_out = j == 0 ? mag : mag2;
+    base = j == 0 ? static_cast<size_t>(b) * F * T : (static_cast<size_t>(b) * (S1 - 1) + (j - 1)) * F * T;
+  }
+  return base;
+}
+
+// |X[f]| of a staged half-spectrum value z = X[f] = (Z[f] + conj Z[N-f]) / 2 (or the / 2i partner): half the hypot of
+// the unscaled sums, the one magnitude expression of every analysis kernel and every layout.
+__device__ __forceinline__ float stft_mag(float2 z) { return 0.5f * hypotf(2.0f * z.x, 2.0f * z.y); }
+
 // Variable-length batch (VARLEN): utterance b owns the first nb = clamp(lengths[b], 1, n) samples of its row (all n
 // when lengths is null) and the first Tb = 1 + nb / hop frames.  Samples at or past nb are never read, frames at or
 // past Tb are neither staged nor transformed, and their outputs are stored as 0.  Frames are paired by absolute index
 // (t0 + g, t0 + g + 1) whatever T is, so frame Tb - 1 has the partner (or the zero partner) it has in a stand-alone
 // call at (nb, Tb): the valid frames are bit-identical to that call.  CTA (0, b) writes Tb to frame_lengths[b].
-// The uniform instantiation ignores the two trailing parameters and compiles as before they existed.
-__device__ __forceinline__ int clamp_len(const int* lengths, int b, int n) {
-  return lengths ? min(max(lengths[b], 1), n) : n;
-}
-
-// grid (ceil(T/TGA), B), nfft/2 threads.  spec: (B, F, T) float2; mag: (B, F, T) float or null.
+// The uniform instantiation ignores the two trailing parameters.
+//
+// grid (ceil(T/TGA), number of signals), nfft/2 threads.  Outputs as stft_out_plane: spec (float2) and mag (float)
+// may each be null.  VARLEN is for the plain layout (S1 == 0) only.
 template <bool VARLEN>
 __global__ void stft_complex_kernel(const float* __restrict__ waves, int n, int nfft, int log2n, int hop, int T, int F,
-                                    float2* __restrict__ spec, float* __restrict__ mag,
-                                    const int* __restrict__ lengths, int* __restrict__ frame_lengths) {
+                                    float2* __restrict__ spec, float* __restrict__ mag, float* __restrict__ mag2,
+                                    int S1, const int* __restrict__ lengths, int* __restrict__ frame_lengths) {
   extern __shared__ __align__(16) uint8_t sm_raw[];
   double* win = reinterpret_cast<double*>(sm_raw);          // [nfft]
   float* re = reinterpret_cast<float*>(win + nfft);         // [nfft]
   float* im = re + nfft;                                    // [nfft]
   float* twr = im + nfft;                                   // [nfft/2]
   float* twi = twr + nfft / 2;                              // [nfft/2]
-  float2* stage = reinterpret_cast<float2*>(twi + nfft / 2);  // [F][TGA]
-  const int b = blockIdx.y;
+  float2* stage = reinterpret_cast<float2*>(twi + nfft / 2);  // [F][TGA + 1]: padded for conflict-free column writes
+  const int sig = blockIdx.y;
   const int t0 = blockIdx.x * TGA;
   const int tid = threadIdx.x;
-  const float* x = waves + static_cast<size_t>(b) * n;
-  const int nb = VARLEN ? clamp_len(lengths, b, n) : n;   // this utterance's samples and frames
+  const float* x = waves + static_cast<size_t>(sig) * n;
+  const int nb = VARLEN ? utt_len(lengths, sig, n) : n;   // this utterance's samples and frames
   const int Tb = VARLEN ? 1 + nb / hop : T;
-  if (VARLEN && frame_lengths && blockIdx.x == 0 && tid == 0) frame_lengths[b] = Tb;
+  if (VARLEN && frame_lengths && blockIdx.x == 0 && tid == 0) frame_lengths[sig] = Tb;
   if (!VARLEN || t0 < Tb) {
     float sv, cv;
     sincospif(-2.0f * static_cast<float>(tid) / static_cast<float>(nfft), &sv, &cv);
@@ -104,19 +122,20 @@ __global__ void stft_complex_kernel(const float* __restrict__ waves, int n, int 
     for (int f = tid; f < F; f += blockDim.x) {
       const int fn = (nfft - f) & (nfft - 1);
       const float zr = re[f], zi = im[f], yr = re[fn], yi = im[fn];
-      stage[f * TGA + g] = make_float2(0.5f * (zr + yr), 0.5f * (zi - yi));                 // A = (Z + conj Z~)/2
-      if (has_b) stage[f * TGA + g + 1] = make_float2(0.5f * (zi + yi), 0.5f * (yr - zr));  // B = (Z - conj Z~)/2i
+      stage[f * (TGA + 1) + g] = make_float2(0.5f * (zr + yr), 0.5f * (zi - yi));             // A = (Z + conj Z~)/2
+      if (has_b) stage[f * (TGA + 1) + g + 1] = make_float2(0.5f * (zi + yi), 0.5f * (yr - zr));  // B = (Z - conj Z~)/2i
     }
   }
   __syncthreads();
+  float* m_out;
+  const size_t base = stft_out_plane(sig, S1, F, T, mag, mag2, &m_out);
   for (int e = tid; e < F * TGA; e += blockDim.x) {
     const int f = e / TGA, g = e - f * TGA;
     if (g >= (VARLEN ? T - t0 : ng)) continue;
-    const size_t o = (static_cast<size_t>(b) * F + f) * T + t0 + g;
-    const float2 v = (!VARLEN || g < ng) ? stage[e] : make_float2(0.f, 0.f);
-    spec[o] = v;
-    // same expression as stft_mag_kernel (0.5 * hypot of the unscaled sums) so the magnitudes agree bit for bit
-    if (mag) mag[o] = 0.5f * hypotf(2.0f * v.x, 2.0f * v.y);
+    const size_t o = base + static_cast<size_t>(f) * T + t0 + g;
+    const float2 v = (!VARLEN || g < ng) ? stage[f * (TGA + 1) + g] : make_float2(0.f, 0.f);
+    if (spec) spec[o] = v;
+    if (m_out) m_out[o] = stft_mag(v);
   }
 }
 
@@ -148,7 +167,7 @@ __global__ void istft_masked_kernel(const float2* __restrict__ spec, const float
   float* twi = twr + nfft / 2;                              // [nfft/2]
   const int b = blockIdx.z, s = blockIdx.y;
   const int n0 = blockIdx.x * CH;
-  const int Lb = VARLEN ? clamp_len(lengths, b, L) : L;
+  const int Lb = VARLEN ? utt_len(lengths, b, L) : L;
   const int Tb = VARLEN ? min(T, 1 + Lb / hop) : T;
   const int n1 = min(n0 + CH, Lb);
   const int tid = threadIdx.x;
@@ -254,10 +273,8 @@ __device__ __forceinline__ void fft512_load_twiddles(float2* tw, int tid) {
   for (int m = tid; m < FFT512_TW; m += 256) tw[m] = g_tw512[m];
 }
 
-// grid (ceil(T/8), number of signals).  Output selection: S1 == 0 -> spec / mag indexed by signal; S1 > 0 (the
-// synthesis layout, signals (B, S1) with the mixture first) -> magnitudes only, mag = mixed_spec (B, F, T) and
-// mag2 = clean_specs (B, S1-1, F, T) or null.  VARLEN (S1 == 0 only): the variable-length rule of
-// stft_complex_kernel; pairs are (t0 + 2g, t0 + 2g + 1), again fixed by absolute frame index.
+// grid (ceil(T/8), number of signals).  Outputs as stft_out_plane.  VARLEN (S1 == 0 only): the variable-length rule
+// of stft_complex_kernel; pairs are (t0 + 2g, t0 + 2g + 1), again fixed by absolute frame index.
 template <bool VARLEN>
 __global__ void __launch_bounds__(256) stft512_kernel(const float* __restrict__ waves, int n, int hop, int T,
                                                       float2* __restrict__ spec, float* __restrict__ mag,
@@ -272,7 +289,7 @@ __global__ void __launch_bounds__(256) stft512_kernel(const float* __restrict__ 
   const int t0 = blockIdx.x * 8;
   const int tid = threadIdx.x, g = tid >> 6, t = tid & 63;
   const float* x = waves + static_cast<size_t>(sig) * n;
-  const int nb = VARLEN ? clamp_len(lengths, sig, n) : n;          // this utterance's samples and frames
+  const int nb = VARLEN ? utt_len(lengths, sig, n) : n;            // this utterance's samples and frames
   const int Tb = VARLEN ? 1 + nb / hop : T;
   if (VARLEN && frame_lengths && blockIdx.x == 0 && tid == 0) frame_lengths[sig] = Tb;
   if (!VARLEN || t0 < Tb) {             // CTA-uniform: a CTA wholly past Tb only stores zeros
@@ -311,20 +328,15 @@ __global__ void __launch_bounds__(256) stft512_kernel(const float* __restrict__ 
     __syncthreads();
   }
   const int ng = min(8, Tb - t0);
-  float* m_out = mag;
-  size_t base = static_cast<size_t>(sig) * F * T;
-  if (S1 > 0) {
-    const int b = sig / S1, j = sig - b * S1;
-    m_out = j == 0 ? mag : mag2;
-    base = j == 0 ? static_cast<size_t>(b) * F * T : (static_cast<size_t>(b) * (S1 - 1) + (j - 1)) * F * T;
-  }
+  float* m_out;
+  const size_t base = stft_out_plane(sig, S1, F, T, mag, mag2, &m_out);
   for (int e = tid; e < F * 8; e += 256) {
     const int f = e >> 3, gg = e & 7;
     if (gg >= (VARLEN ? T - t0 : ng)) continue;
     const size_t o = base + static_cast<size_t>(f) * T + t0 + gg;
     const float2 z = (!VARLEN || gg < ng) ? stage[f * 9 + gg] : make_float2(0.f, 0.f);
     if (spec) spec[o] = z;
-    if (m_out) m_out[o] = 0.5f * hypotf(2.0f * z.x, 2.0f * z.y);
+    if (m_out) m_out[o] = stft_mag(z);
   }
 }
 
@@ -344,7 +356,7 @@ __global__ void __launch_bounds__(256) istft512_kernel(const float2* __restrict_
   float* frames = reinterpret_cast<float*>(tile);
   const int b = blockIdx.z, s = blockIdx.y;
   const int n0 = blockIdx.x * CH;
-  const int Lb = VARLEN ? clamp_len(lengths, b, L) : L;
+  const int Lb = VARLEN ? utt_len(lengths, b, L) : L;
   const int Tb = VARLEN ? min(T, 1 + Lb / hop) : T;
   const int n1 = min(n0 + CH, Lb);
   const int tid = threadIdx.x, g = tid >> 6, t = tid & 63;
@@ -431,14 +443,11 @@ constexpr size_t kIstft512Smem = FFT512_TW * sizeof(float2) + 8 * FFT512_XCH * s
 static_assert(257 * 9 * sizeof(float2) >= 8 * FFT512_XCH * sizeof(float), "the time frames must fit in the staged tile");
 static_assert(kStft512Smem <= 48 * 1024 && kIstft512Smem <= 48 * 1024, "no opt-in shared memory needed");
 
-bool fft_geometry_ok(int nfft, int hop, int* log2n) {
-  if (nfft < 8 || nfft > 2048 || (nfft & (nfft - 1)) || hop < 1 || hop > nfft) return false;
-  *log2n = 0;
-  while ((1 << *log2n) < nfft) ++*log2n;
-  return true;
-}
-
 }  // namespace
+
+bool fft_size_ok(int nfft) { return nfft >= 8 && nfft <= 2048 && (nfft & (nfft - 1)) == 0; }
+
+bool fft_geometry_ok(int nfft, int hop) { return fft_size_ok(nfft) && hop >= 1 && hop <= nfft; }
 
 const char* fft512_init_tables() {
   fft512_tables_kernel<<<1, 256>>>();
@@ -446,46 +455,30 @@ const char* fft512_init_tables() {
   return cudaDeviceSynchronize() == cudaSuccess ? nullptr : "fft512: table kernel failed";
 }
 
-const char* launch_stft_complex(cudaStream_t s, const float* waves, const int* lengths, int B, int L, int nfft, int hop,
-                                float* spec, float* mag, int* frame_lengths) {
-  int log2n;
-  if (B <= 0 || L <= 0) return "stft: empty problem";
-  if (!fft_geometry_ok(nfft, hop, &log2n)) return "stft: n_fft must be a power of two in [8, 2048], 1 <= hop <= n_fft";
+const char* launch_stft(cudaStream_t s, const float* waves, const int* lengths, int B, int S1, int L, int nfft, int hop,
+                        float* spec, float* mag, float* mag2, int* frame_lengths) {
   const int T = 1 + L / hop, F = nfft / 2 + 1;
+  const dim3 grid((T + TGA - 1) / TGA, B * (S1 > 0 ? S1 : 1));
   const bool varlen = lengths || frame_lengths;
-  if (nfft == 512 && B <= 65535) {
+  float2* spec2 = reinterpret_cast<float2*>(spec);
+  if (nfft == 512) {
     auto kern = varlen ? stft512_kernel<true> : stft512_kernel<false>;
-    kern<<<dim3((T + 7) / 8, B), 256, kStft512Smem, s>>>(waves, L, hop, T, reinterpret_cast<float2*>(spec), mag,
-                                                         nullptr, 0, lengths, frame_lengths);
-    return cudaGetLastError() == cudaSuccess ? nullptr : "stft: launch failed";
+    kern<<<grid, 256, kStft512Smem, s>>>(waves, L, hop, T, spec2, mag, mag2, S1, lengths, frame_lengths);
+  } else {
+    const size_t smem = static_cast<size_t>(nfft) * sizeof(double) + 3 * static_cast<size_t>(nfft) * sizeof(float) +
+                        static_cast<size_t>(F) * (TGA + 1) * sizeof(float2);
+    auto kern = varlen ? stft_complex_kernel<true> : stft_complex_kernel<false>;
+    if (!smem_opt_in(kern, static_cast<int>(smem))) return "stft: cannot raise the shared-memory limit";
+    kern<<<grid, nfft / 2, smem, s>>>(waves, L, nfft, __builtin_ctz(nfft), hop, T, F, spec2, mag, mag2, S1, lengths,
+                                      frame_lengths);
   }
-  const size_t smem = static_cast<size_t>(nfft) * sizeof(double) + 3 * static_cast<size_t>(nfft) * sizeof(float) +
-                      static_cast<size_t>(F) * TGA * sizeof(float2);
-  auto kern = varlen ? stft_complex_kernel<true> : stft_complex_kernel<false>;
-  if (smem > 48 * 1024 &&
-      cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024) != cudaSuccess)
-    return "stft: cannot raise the shared-memory limit";
-  kern<<<dim3((T + TGA - 1) / TGA, B), nfft / 2, smem, s>>>(waves, L, nfft, log2n, hop, T, F,
-                                                           reinterpret_cast<float2*>(spec), mag, lengths, frame_lengths);
   return cudaGetLastError() == cudaSuccess ? nullptr : "stft: launch failed";
-}
-
-// Magnitude-only analysis of the synthesis layout (signals (B, S+1, n), mixture first) for n_fft = 512: used by
-// launch_synth instead of its radix-2 kernel.
-const char* launch_stft512_synth(cudaStream_t s, const float* waves, int B, int S, int n, int hop, float* mixed_spec,
-                                 float* clean_specs) {
-  const int T = 1 + n / hop;
-  if (static_cast<long long>(B) * (S + 1) > 65535) return "synth: batch * (speakers + 1) above 65535";
-  stft512_kernel<false><<<dim3((T + 7) / 8, B * (S + 1)), 256, kStft512Smem, s>>>(waves, n, hop, T, nullptr, mixed_spec,
-                                                                                  clean_specs, S + 1, nullptr, nullptr);
-  return cudaGetLastError() == cudaSuccess ? nullptr : "synth: stft launch failed";
 }
 
 const char* launch_istft_masked(cudaStream_t s, const float* spec, const float* masks, const int* lengths, int B, int S,
                                 int T, int nfft, int hop, int L, float* waves) {
-  int log2n;
   if (B <= 0 || S <= 0 || T <= 0 || L <= 0) return "istft: empty problem";
-  if (!fft_geometry_ok(nfft, hop, &log2n)) return "istft: n_fft must be a power of two in [8, 2048], 1 <= hop <= n_fft";
+  if (!fft_geometry_ok(nfft, hop)) return "istft: n_fft must be a power of two in [8, 2048], 1 <= hop <= n_fft";
   if (S > 65535 || B > 65535) return "istft: batch or speaker count above 65535";
   if (masks == nullptr && S != 1) return "istft: without masks there is one output per utterance (S = 1)";
   if (static_cast<long long>(T - 1) * hop + nfft < L) return "istft: the frames do not reach the requested length";
@@ -504,12 +497,9 @@ const char* launch_istft_masked(cudaStream_t s, const float* spec, const float* 
                       3 * static_cast<size_t>(nfft) * sizeof(float);
   if (smem > 227 * 1024) return "istft: geometry needs more than 227 KB of shared memory";
   auto kern = lengths ? istft_masked_kernel<true> : istft_masked_kernel<false>;
-  // per call, not cached: the attribute is per device and a process may hold engines on several
-  if (smem > 48 * 1024 &&
-      cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024) != cudaSuccess)
-    return "istft: cannot raise the shared-memory limit";
+  if (!smem_opt_in(kern, static_cast<int>(smem))) return "istft: cannot raise the shared-memory limit";
   kern<<<dim3((L + CH - 1) / CH, S, B), nfft / 2, smem, s>>>(reinterpret_cast<const float2*>(spec), masks, S, nfft,
-                                                             log2n, hop, T, F, L, CH, waves, lengths);
+                                                             __builtin_ctz(nfft), hop, T, F, L, CH, waves, lengths);
   return cudaGetLastError() == cudaSuccess ? nullptr : "istft: launch failed";
 }
 

@@ -1482,7 +1482,7 @@ const char* launch_xformer_stack(cudaStream_t s, const StackProblem& sp, int num
   d.mixed = sp.mixed; d.masks = sp.masks; d.separated = sp.separated;
   const int grid = n_tiles < num_sms ? n_tiles : num_sms;
   auto kern = (d.lens != nullptr || d.kvp_lens != nullptr) ? xformer_stack_kernel<true> : xformer_stack_kernel<false>;
-  if (!smem_opt_in(kern, STACK_SMEM)) return "xformer_stack: cudaFuncSetAttribute failed";
+  if (!smem_opt_in(kern, STACK_SMEM)) return "xformer_stack: cannot raise the shared-memory limit";
   if (launch_pdl(kern, dim3(grid), dim3(STACK_THREADS), STACK_SMEM, s, tin, tout, top, tkv, d) !=
       cudaSuccess) {
     cudaGetLastError();

@@ -127,20 +127,25 @@ def test_evaluate_separation_mirror_runs_on_device():
     assert np.isfinite(out_snr)
 
 
-def test_synth_and_snr_edge_geometries():
-    """Single speaker, tiny FFT, one item, more video frames than fit evenly; SNR with one speaker."""
-    from avsep_b200.engine import Engine, EngineConfig
-    kw = dict(sample_rate=4000, duration=0.25, n_fft=64, hop_length=16, num_frames=7, frame_h=8, frame_w=12,
-              speaker_freqs=(300.0,))
+def _synth_item_matches_oracle(kw, idx):
+    """One item of the device synthesis at geometry kw against the synthesis oracle; returns (dataset, batch)."""
     cfg = so.SynthConfig(**kw)
     ds = _ds(**kw)
-    b = ds.batch([11])
+    b = ds.batch([idx])
     torch.cuda.synchronize()
-    ref = so.synth_item(cfg, 11)
+    ref = so.synth_item(cfg, idx)
     for k in ("mixed_spec", "lip_frames", "clean_specs"):
         got = b[k][0].cpu().numpy()
         assert got.shape == ref[k].shape, k
         assert np.abs(got - ref[k]).max() <= 2e-6 * max(1.0, np.abs(ref[k]).max()) + 2e-5, k
+    return ds, b
+
+
+def test_synth_and_snr_edge_geometries():
+    """Single speaker, tiny FFT, one item, more video frames than fit evenly; SNR with one speaker."""
+    kw = dict(sample_rate=4000, duration=0.25, n_fft=64, hop_length=16, num_frames=7, frame_h=8, frame_w=12,
+              speaker_freqs=(300.0,))
+    ds, b = _synth_item_matches_oracle(kw, 11)
     eng = ds.engine
     tg = b["clean_specs"]
     sep = (tg * 0.9).contiguous()
@@ -148,6 +153,12 @@ def test_synth_and_snr_edge_geometries():
     assert abs(float(o_snr[0]) - so.permutation_snr(sep[0].cpu().numpy(), tg[0].cpu().numpy())) < 2e-5
     assert int(perm[0]) == 0
     assert abs(float(i_snr[0, 0]) - so.input_snrs(b["mixed_spec"][0].cpu().numpy(), tg[0].cpu().numpy())[0]) < 2e-5
+
+
+def test_synth_at_the_largest_transform():
+    """n_fft = 2048, whose analysis needs more than the default 48 KB of shared memory."""
+    _synth_item_matches_oracle(dict(sample_rate=8000, duration=1.0, n_fft=2048, hop_length=512, num_frames=7,
+                                    frame_h=8, frame_w=12, speaker_freqs=(300.0,)), 11)
 
 
 def test_synth_scratch_growth_leaves_the_host_workspace_alone():

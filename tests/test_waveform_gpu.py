@@ -59,13 +59,11 @@ def test_stft_matches_reference_magnitudes_and_oracle_phase(eng, name):
     assert torch.equal(mag, spec.abs()) or (mag - spec.abs()).abs().max().item() <= 1e-6 * scale
 
 
-def test_stft_magnitude_agrees_with_the_synthesis_path():
-    """avsep_stft on the mixture waveform of dataset items reproduces the mixed_spec avsep_synth_batch makes (same
-    framing and transform; the waveform here comes from the synthesis oracle, so allow the fp32 transform tolerance)."""
+def _stft_matches_synthesis(kw):
     from avsep_b200.dataset import SyntheticAVDataset
     from oracle import synth_oracle as so
-    ds = SyntheticAVDataset()
-    cfg = so.SynthConfig()
+    ds = SyntheticAVDataset(**kw)
+    cfg = so.SynthConfig(**kw)
     idxs = (0, 1, 2, 3)
     waves = []
     for i in idxs:
@@ -76,6 +74,18 @@ def test_stft_magnitude_agrees_with_the_synthesis_path():
     _, mag = ds.engine.stft(x, cfg.n_fft, cfg.hop_length)
     scale = b["mixed_spec"].abs().max().item()
     assert (mag - b["mixed_spec"]).abs().max().item() <= TOL_SPEC_REL * scale
+
+
+def test_stft_magnitude_agrees_with_the_synthesis_path():
+    """avsep_stft on the mixture waveform of dataset items reproduces the mixed_spec avsep_synth_batch makes (same
+    framing and transform; the waveform here comes from the synthesis oracle, so allow the fp32 transform tolerance)."""
+    _stft_matches_synthesis({})
+
+
+def test_stft_magnitude_agrees_with_the_synthesis_path_radix2():
+    """The same at n_fft = 256, where both run the radix-2 analysis kernel."""
+    _stft_matches_synthesis(dict(sample_rate=16000, duration=0.5, n_fft=256, hop_length=64, num_frames=10, frame_h=16,
+                                 frame_w=24, speaker_freqs=(200.0, 330.0, 512.0)))
 
 
 @pytest.mark.parametrize("name", ("default", "short", "ragged"))
@@ -155,6 +165,37 @@ def test_istft_rejects_bad_geometry(eng):
         eng.istft(torch.zeros(1, 151, 4, dtype=torch.complex64, device="cuda"), None, 100, 300, 100)
     with pytest.raises(ValueError):
         eng.istft(spec.cpu(), None, 100, 512, 128)
+
+
+def _forward_and_wide_stft(dev):
+    """A default-model forward and an n_fft = 2048 STFT on cuda:dev (both launch kernels that need more than 48 KB of
+    shared memory)."""
+    from avsep_b200 import AVSeparationTransformer
+    torch.manual_seed(0)
+    model = AVSeparationTransformer().eval()
+    g = torch.Generator().manual_seed(6)
+    mixed, lips = torch.rand(2, 257, 63, generator=g), torch.rand(2, 50, 32, 32, generator=g)
+    x = torch.randn(3, 6000, generator=g)
+    sep, masks = model(mixed.to(dev), lips.to(dev))
+    spec, mag = model.engine.stft(x.to(dev), 2048, 512)
+    torch.cuda.synchronize(dev)
+    return [t.cpu() for t in (sep, masks, spec, mag)]
+
+
+def test_second_device_after_the_first_matches_a_fresh_process(tmp_path):
+    """The shared-memory opt-in is per device: a process that ran on cuda:0 must still opt in on cuda:1."""
+    if torch.cuda.device_count() < 2:
+        pytest.skip("needs two GPUs")
+    import subprocess
+    here = [_forward_and_wide_stft(0), _forward_and_wide_stft(1)]
+    for dev in (0, 1):
+        out = tmp_path / f"fresh{dev}.pt"
+        code = (f"import sys; sys.path[:0] = {[ROOT, os.path.join(ROOT, 'av-separation-transformer_b200')]!r}; "
+                f"import torch; from tests.test_waveform_gpu import _forward_and_wide_stft as f; "
+                f"torch.save(f({dev}), {str(out)!r})")
+        subprocess.run([sys.executable, "-c", code], check=True, cwd=ROOT)
+        fresh = torch.load(out)
+        assert all(torch.equal(a, b) for a, b in zip(here[dev], fresh)), dev
 
 
 def test_separate_waveforms_end_to_end():
