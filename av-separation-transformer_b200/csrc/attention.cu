@@ -436,10 +436,10 @@ __global__ void __launch_bounds__(128, 7) attention_small_kernel(const AttnDev p
 }
 
 template <bool LERP>
-const char* launch_small(cudaStream_t s, const AttnDev& d, int B, int H) {
+const char* launch_small(LaunchCtx lc, const AttnDev& d, int B, int H) {
   constexpr int SMEM = 3 * 64 * (64 + 8) * 2;
   dim3 grid(1, H, B);
-  if (launch_pdl(attention_small_kernel<LERP>, grid, dim3(128), SMEM, s, d) != cudaSuccess) {
+  if (launch_pdl(attention_small_kernel<LERP>, grid, dim3(128), SMEM, lc, d) != cudaSuccess) {
     cudaGetLastError();
     return "attention: launch failed";
   }
@@ -447,12 +447,12 @@ const char* launch_small(cudaStream_t s, const AttnDev& d, int B, int H) {
 }
 
 template <int HD, bool LERP, bool SPLIT>
-const char* launch_t(cudaStream_t s, const AttnDev& d, int B, int H, int Lq) {
+const char* launch_t(LaunchCtx lc, const AttnDev& d, int B, int H, int Lq) {
   constexpr int SMEM = (SPLIT ? 6 : 3) * 64 * (HD + 8) * 2;
   auto kern = attention_kernel<HD, LERP, SPLIT>;
   if (!smem_opt_in(kern, SMEM)) return "attention: cannot raise the shared-memory limit";
   dim3 grid((Lq + QT - 1) / QT, H, B);
-  if (launch_pdl(kern, grid, dim3(128), SMEM, s, d) != cudaSuccess) {
+  if (launch_pdl(kern, grid, dim3(128), SMEM, lc, d) != cudaSuccess) {
     cudaGetLastError();
     return "attention: launch failed";
   }
@@ -469,9 +469,9 @@ bool attention_tc_wanted(int prec, const AttnProblem& p) {
   return p.tc_mode == 2 || (p.Lq < p.Lk ? p.Lq : p.Lk) >= ATTN_TC_MIN_LEN;
 }
 
-const char* launch_attention(cudaStream_t s, int prec, const AttnProblem& p) {
+const char* launch_attention(LaunchCtx lc, int prec, const AttnProblem& p) {
   if (p.B <= 0 || p.Lq <= 0 || p.Lk <= 0) return "attention: empty problem";
-  if (attention_tc_wanted(prec, p)) return launch_attention_tc(s, p);
+  if (attention_tc_wanted(prec, p)) return launch_attention_tc(lc, p);
   const bool split = (prec == PREC_TF32);     // fp32 operands, bf16 hi/lo split contractions, fp32 output
   AttnDev d;
   d.q = p.q;
@@ -486,15 +486,15 @@ const char* launch_attention(cudaStream_t s, int prec, const AttnProblem& p) {
     if ((p.ldq & 3) || (p.ldo & 1) || (p.ldkv & 3)) return "attention: misaligned leading dimension";
   } else {
     if (p.hd == 64 && p.Lq <= QT && p.Lk <= KT && !(p.ldq & 7) && !(p.ldo & 1) && !(lerp ? (p.ldkv & 3) : (p.ldkv & 7)))
-      return lerp ? launch_small<true>(s, d, p.B, p.H) : launch_small<false>(s, d, p.B, p.H);
+      return lerp ? launch_small<true>(lc, d, p.B, p.H) : launch_small<false>(lc, d, p.B, p.H);
   }
   if (!split) {
     if ((p.ldq & 7) || (p.ldo & 1) || (lerp ? (p.ldkv & 3) : (p.ldkv & 7))) return "attention: misaligned leading dimension";
   }
 #define AVSEP_ATTN_CASE(HDV)                                                                              \
   case HDV:                                                                                               \
-    if (split) return lerp ? launch_t<HDV, true, true>(s, d, p.B, p.H, p.Lq) : launch_t<HDV, false, true>(s, d, p.B, p.H, p.Lq); \
-    return lerp ? launch_t<HDV, true, false>(s, d, p.B, p.H, p.Lq) : launch_t<HDV, false, false>(s, d, p.B, p.H, p.Lq);
+    if (split) return lerp ? launch_t<HDV, true, true>(lc, d, p.B, p.H, p.Lq) : launch_t<HDV, false, true>(lc, d, p.B, p.H, p.Lq); \
+    return lerp ? launch_t<HDV, true, false>(lc, d, p.B, p.H, p.Lq) : launch_t<HDV, false, false>(lc, d, p.B, p.H, p.Lq);
   switch (p.hd) {
     AVSEP_ATTN_CASE(16)
     AVSEP_ATTN_CASE(32)

@@ -315,7 +315,7 @@ bool attention_tc_usable(int prec, const AttnProblem& p) {
          (p.ldo & 7) == 0;
 }
 
-const char* launch_attention_tc(cudaStream_t s, const AttnProblem& p) {
+const char* launch_attention_tc(LaunchCtx lc, const AttnProblem& p) {
   if (p.B <= 0 || p.Lq <= 0 || p.Lk <= 0) return "attention_tc: empty problem";
   if (p.hd != HD || p.lerp_src != 0) return "attention_tc: needs head dim 64 and materialised K/V rows";
   if (!smem_opt_in(attention_tc_kernel, SMEM_BYTES)) return "attention_tc: cannot raise the shared-memory limit";
@@ -331,21 +331,21 @@ const char* launch_attention_tc(cudaStream_t s, const AttnProblem& p) {
   d.scale_log2 = 1.4426950408889634f / sqrtf(static_cast<float>(HD));
   d.k_lens = p.k_lens;
   dim3 grid((p.Lq + QT - 1) / QT, p.H, p.B);
-  if (launch_pdl(attention_tc_kernel, grid, dim3(NTHREADS), SMEM_BYTES, s, tq, tk, tv, to, d) != cudaSuccess) {
+  if (launch_pdl(attention_tc_kernel, grid, dim3(NTHREADS), SMEM_BYTES, lc, tq, tk, tv, to, d) != cudaSuccess) {
     cudaGetLastError();
     return "attention_tc: launch failed";
   }
   return nullptr;
 }
 
-const char* launch_lerp_rows(cudaStream_t s, const float* src, int ld_src, int B, int nsrc, int L, int cols,
+const char* launch_lerp_rows(LaunchCtx lc, const float* src, int ld_src, int B, int nsrc, int L, int cols,
                              void* dst_bf16, int ld_dst, const int* src_lens, const int* dst_lens) {
   if ((cols & 7) || (ld_src & 3) || (ld_dst & 7)) return "lerp_rows: misaligned";
   const int chunks = cols / 8;
   const long long total = static_cast<long long>(B) * L * chunks;
   const int threads = 256;
   const long long blocks = (total + threads - 1) / threads;
-  launch_pdl(lerp_rows_kernel, dim3(static_cast<unsigned>(blocks)), dim3(threads), 0, s, src, ld_src, nsrc, L, chunks,
+  launch_pdl(lerp_rows_kernel, dim3(static_cast<unsigned>(blocks)), dim3(threads), 0, lc, src, ld_src, nsrc, L, chunks,
              reinterpret_cast<__nv_bfloat16*>(dst_bf16), ld_dst, total, src_lens, dst_lens);
   return cudaGetLastError() == cudaSuccess ? nullptr : "lerp_rows: launch failed";
 }

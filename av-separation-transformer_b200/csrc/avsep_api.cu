@@ -11,7 +11,9 @@
 
 #include <functional>
 #include <map>
+#include <memory>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 using namespace avsep;
@@ -45,6 +47,53 @@ __global__ void spin_kernel(unsigned long long ns) {
   } while (t - t0 < ns);
 }
 
+// ---- owners of the handle's CUDA resources: each releases its resource when it is replaced or destroyed ----
+template <typename H, cudaError_t (*Release)(H)>
+struct Releaser {
+  void operator()(H x) const { Release(x); }
+};
+template <typename H, cudaError_t (*Release)(H)>
+using Owned = std::unique_ptr<std::remove_pointer_t<H>, Releaser<H, Release>>;
+using Stream = Owned<cudaStream_t, cudaStreamDestroy>;
+using Event = Owned<cudaEvent_t, cudaEventDestroy>;
+using GraphExec = Owned<cudaGraphExec_t, cudaGraphExecDestroy>;
+
+// Creates the (non-blocking) stream or the event unless it exists.
+cudaError_t make_stream(Stream& s) {
+  if (s) return cudaSuccess;
+  cudaStream_t x;
+  const cudaError_t e = cudaStreamCreateWithFlags(&x, cudaStreamNonBlocking);
+  if (e == cudaSuccess) s.reset(x);
+  return e;
+}
+cudaError_t make_event(Event& ev, unsigned flags = cudaEventDisableTiming) {
+  if (ev) return cudaSuccess;
+  cudaEvent_t x;
+  const cudaError_t e = cudaEventCreateWithFlags(&x, flags);
+  if (e == cudaSuccess) ev.reset(x);
+  return e;
+}
+
+// cap elements of device memory (PINNED: page-locked host memory).  alloc() frees the current block before it makes the
+// new one, so its caller first makes sure that no queued work and no cached graph still uses the old one.
+template <typename T, bool PINNED = false>
+struct Buf {
+  struct Free {
+    void operator()(T* p) const { PINNED ? cudaFreeHost(p) : cudaFree(p); }
+  };
+  std::unique_ptr<T, Free> ptr;
+  size_t cap = 0;
+  T* get() const { return ptr.get(); }
+  cudaError_t alloc(size_t n) {
+    ptr.reset();
+    T* p = nullptr;
+    const cudaError_t e = PINNED ? cudaMallocHost(&p, n * sizeof(T)) : cudaMalloc(&p, n * sizeof(T));
+    ptr.reset(e == cudaSuccess ? p : nullptr);
+    cap = e == cudaSuccess ? n : 0;
+    return e;
+  }
+};
+
 struct GraphKey {
   int B, T, N, Hh, Ww;
   const void *mixed, *frames, *sep, *masks, *ws;
@@ -56,7 +105,7 @@ struct GraphKey {
 };
 struct GraphEntry {
   GraphKey key;
-  cudaGraphExec_t exec = nullptr;
+  GraphExec exec;
   int64_t launches = 0;
   uint64_t last_use = 0;
 };
@@ -100,15 +149,14 @@ struct avsep_handle {
   bool use_graph = true; // replay the forward as a CUDA graph (captured per shape + buffer set on its 2nd use)
   int attn_tc = 1;       // AttnProblem::tc_mode of every attention launch
   bool two_stream = true; // audio and visual branches on two streams (fork/join), so partial waves overlap
-  cudaStream_t aux_stream = nullptr;
-  cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
+  Stream aux_stream;
+  Event ev_fork, ev_join;
   std::vector<GraphEntry> graphs;
   uint64_t graph_clock = 0;
-  cudaStream_t cap_stream = nullptr;
+  Stream cap_stream;
   int profile_spin_us = 3000;
-  uint8_t* d_weights = nullptr;
-  size_t weight_bytes = 0;
-  // device views into d_weights
+  Buf<uint8_t> weights;
+  // device views into weights
   const void *wc1 = nullptr, *wc2 = nullptr, *wproj = nullptr, *wkv_all = nullptr, *wdec0 = nullptr, *wdec3 = nullptr;
   const float *bc1 = nullptr, *bc2 = nullptr, *bproj = nullptr, *bkv_all = nullptr, *bdec0 = nullptr, *bdec3 = nullptr;
   const float *pe_a = nullptr, *pe_v = nullptr, *fng = nullptr, *fnb = nullptr;
@@ -121,44 +169,48 @@ struct avsep_handle {
   const uint8_t *xs_a_np = nullptr, *xs_v_np = nullptr;   // encoder streams past their input-projection items
   bool xs_v_kvp = false;       // the visual stream ends with the fusion layers' K | V projection block
   // cached library-owned workspace
-  void* own_ws = nullptr;
-  size_t own_ws_bytes = 0;
+  Buf<uint8_t> own_ws;
   // host-path staging
   // host-buffer entry point: two independent I/O slots so that consecutive calls can overlap (copy-in of call i+1
   // with the kernels and copy-out of call i); slot 0 serves the synchronous avsep_forward_host
   struct HostSlot {
-    float* io[4] = {nullptr, nullptr, nullptr, nullptr};   // mixed, frames, separated, masks (device)
-    size_t cap[4] = {0, 0, 0, 0};
-    std::vector<cudaEvent_t> ev;                            // 2 per chunk: copy-in done, kernels done
-    cudaEvent_t ev_start = nullptr, ev_end = nullptr;       // ev_end: last copy-out done
-    cudaEvent_t ev_lane[3] = {nullptr, nullptr, nullptr};   // last kernels of this slot on each compute lane
+    Buf<float> io[4];                // mixed, frames, separated, masks (device)
+    std::vector<Event> ev;           // 2 per chunk: copy-in done, kernels done
+    Event ev_start, ev_end;          // ev_end: last copy-out done
+    Event ev_lane[3];                // last kernels of this slot on each compute lane
     // packed batches (avsep_forward_host_packed*): the call's lengths, then its frame lengths, uploaded once per call
-    int32_t* lens_host = nullptr;                           // pinned
-    int32_t* lens_dev = nullptr;
-    int lens_cap = 0;                                       // utterances each array holds
-    cudaEvent_t ev_lens = nullptr;                          // upload of lens_host done
+    Buf<int32_t, true> lens_host;
+    Buf<int32_t> lens_dev;
+    Event ev_lens;                   // upload of lens_host done
   } slot[AVSEP_HOST_SLOTS];
   std::vector<void*> shared_owned, shared_mapped;   // avsep_shared_alloc / avsep_shared_open
-  float* synth_waves = nullptr;   // scratch of avsep_synth_batch
-  size_t synth_cap = 0;
-  cudaStream_t hs[3] = {nullptr, nullptr, nullptr};
+  Buf<float> synth_waves;   // scratch of avsep_synth_batch
+  Stream hs[3];
   int host_chunk = 0;    // utterances per pipeline chunk of the host path; 0 = auto (see host_submit)
   bool pdl = true;       // programmatic dependent launch between consecutive kernels of a stream
   int host_lanes = 0;    // chunks whose kernels may be in flight at once (own stream + workspace each); 0 = auto
-  void* host_ws = nullptr;
-  size_t host_ws_bytes = 0;
-  cudaStream_t host_comp[3] = {nullptr, nullptr, nullptr};
+  Buf<uint8_t> host_ws;
+  Stream host_comp[3];
   // debug
   bool debug = false;
-  std::map<std::string, std::pair<float*, size_t>> snaps;
+  struct Snapshot {
+    Buf<float> buf;
+    size_t count = 0;
+  };
+  std::map<std::string, Snapshot> snaps;
   int64_t launches = 0;
   // per-launch profiling (cudaEvent pairs on the launching stream)
   bool profile = false;
-  cudaStream_t prof_stream = nullptr;
-  std::vector<cudaEvent_t> ev_pool;
+  std::vector<Event> ev_pool;
   size_t ev_used = 0;
   std::vector<std::pair<const char*, size_t>> ev_marks;   // label, index of the start event (stop = +1)
   std::map<std::string, std::pair<int64_t, double>> prof;  // label -> (launches, total ms)
+
+  // every other resource has an owner above; the buffers shared with other processes are released here at the latest
+  ~avsep_handle() {
+    for (void* ptr : shared_mapped) cudaIpcCloseMemHandle(ptr);
+    for (void* ptr : shared_owned) cudaFree(ptr);
+  }
 };
 
 namespace {
@@ -168,32 +220,38 @@ int fail(avsep_handle* h, const std::string& msg) {
   return 1;
 }
 
-int prof_begin(avsep_handle* h, const char* label) {
+int prof_begin(avsep_handle* h, const char* label, cudaStream_t s) {
   if (h->ev_used + 2 > h->ev_pool.size()) {
     for (int i = 0; i < 64; ++i) {
-      cudaEvent_t e;
-      if (cudaEventCreate(&e) != cudaSuccess) return 1;
-      h->ev_pool.push_back(e);
+      Event e;
+      if (make_event(e, cudaEventDefault) != cudaSuccess) return 1;
+      h->ev_pool.push_back(std::move(e));
     }
   }
   h->ev_marks.emplace_back(label, h->ev_used);
-  cudaEventRecord(h->ev_pool[h->ev_used], h->prof_stream);
+  cudaEventRecord(h->ev_pool[h->ev_used].get(), s);
   return 0;
 }
-void prof_end(avsep_handle* h) {
-  cudaEventRecord(h->ev_pool[h->ev_used + 1], h->prof_stream);
+void prof_end(avsep_handle* h, cudaStream_t s) {
+  cudaEventRecord(h->ev_pool[h->ev_used + 1].get(), s);
   h->ev_used += 2;
 }
 
-#define CKL(label, expr)                                                \
+cudaStream_t stream_of(LaunchCtx lc) { return lc.stream; }
+cudaStream_t stream_of(cudaStream_t s) { return s; }
+
+// Launcher call fn(on, ...), where `on` is the LaunchCtx of a launch_pdl launcher or the stream of a <<<>>> one.  With
+// profiling on, the call is bracketed by an event pair on that same stream.
+#define CKL(label, on, fn, ...)                                         \
   do {                                                                  \
-    if (h->profile && prof_begin(h, label)) return fail(h, "profiling: cudaEventCreate failed"); \
-    const char* _e = (expr);                                            \
-    if (_e != nullptr) return fail(h, std::string(_e) + " [" #expr "]"); \
-    if (h->profile) prof_end(h);                                        \
+    const cudaStream_t _s = stream_of(on);                              \
+    if (h->profile && prof_begin(h, label, _s)) return fail(h, "profiling: cudaEventCreate failed"); \
+    const char* _e = fn(on, __VA_ARGS__);                               \
+    if (_e != nullptr) return fail(h, std::string(_e) + " [" #fn "(" #on ", " #__VA_ARGS__ ")]"); \
+    if (h->profile) prof_end(h, _s);                                    \
     ++h->launches;                                                      \
   } while (0)
-#define CK(expr) CKL("other", expr)
+#define CK(on, fn, ...) CKL("other", on, fn, __VA_ARGS__)
 
 #define CUDA_OK(expr)                                                                           \
   do {                                                                                          \
@@ -203,11 +261,11 @@ void prof_end(avsep_handle* h) {
 
 size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
-void drop_graphs(avsep_handle* h) {   // cached graphs hold raw pointers to weights / workspace
-  for (auto& g : h->graphs)
-    if (g.exec) cudaGraphExecDestroy(g.exec);
-  h->graphs.clear();
-}
+void drop_graphs(avsep_handle* h) { h->graphs.clear(); }   // cached graphs hold raw pointers to weights / workspace
+
+// The launch settings of h's forward-path kernels on stream s: per-launch event pairs (profiling) must time the kernels
+// one at a time, so profiling turns PDL off.
+LaunchCtx launch_ctx(const avsep_handle* h, cudaStream_t s) { return {s, h->pdl && !h->profile}; }
 
 size_t op_size(const avsep_handle* h) { return h->cfg.precision == AVSEP_PREC_TF32 ? 4 : 2; }
 
@@ -258,15 +316,11 @@ int workspace_base(avsep_handle* h, void* user_ws, size_t user_bytes, size_t nee
     if ((reinterpret_cast<uintptr_t>(user_ws) & 1023) != 0) return fail(h, "workspace must be 1024-byte aligned");
     base = static_cast<uint8_t*>(user_ws);
   } else {
-    if (h->own_ws_bytes < need) {
-      drop_graphs(h);
-      if (h->own_ws) cudaFree(h->own_ws);
-      h->own_ws = nullptr;
-      h->own_ws_bytes = 0;
-      CUDA_OK(cudaMalloc(&h->own_ws, need));
-      h->own_ws_bytes = need;
+    if (h->own_ws.cap < need) {
+      drop_graphs(h);   // the cached graphs hold pointers into the old workspace
+      CUDA_OK(h->own_ws.alloc(need));
     }
-    base = static_cast<uint8_t*>(h->own_ws);
+    base = h->own_ws.get();
   }
   return 0;
 }
@@ -304,29 +358,26 @@ size_t carve_packed(const avsep_handle* h, Workspace& w, Staging& st, uint8_t* b
 // ---- debug snapshots ---------------------------------------------------------------------------
 int snapshot(avsep_handle* h, cudaStream_t s, const char* name, const void* ptr, size_t count, bool is_op) {
   if (!h->debug) return 0;
-  auto& slot = h->snaps[name];
-  if (slot.second < count) {
-    if (slot.first) cudaFree(slot.first);
-    slot.first = nullptr;
-    CUDA_OK(cudaMalloc(&slot.first, count * sizeof(float)));
-  }
-  slot.second = count;
+  auto& snap = h->snaps[name];
+  if (snap.buf.cap < count) CUDA_OK(snap.buf.alloc(count));
+  snap.count = count;
   if (is_op && h->cfg.precision == AVSEP_PREC_BF16) {
     op_to_f32_kernel<<<static_cast<unsigned>((count + 255) / 256), 256, 0, s>>>(
-        static_cast<const __nv_bfloat16*>(ptr), slot.first, count);
+        static_cast<const __nv_bfloat16*>(ptr), snap.buf.get(), count);
   } else {
-    CUDA_OK(cudaMemcpyAsync(slot.first, ptr, count * sizeof(float), cudaMemcpyDeviceToDevice, s));
+    CUDA_OK(cudaMemcpyAsync(snap.buf.get(), ptr, count * sizeof(float), cudaMemcpyDeviceToDevice, s));
   }
   return 0;
 }
 
 // ---- stage helpers -----------------------------------------------------------------------------
-const char* run_visual_cnn(avsep_handle* h, cudaStream_t s, const float* frames, int M, int Hh, int Ww, void* pooled,
-                           unsigned long long* trace = nullptr, const int* frame_lens = nullptr, int N = 1) {
+const char* run_visual_cnn(LaunchCtx lc, const avsep_handle* h, const float* frames, int M, int Hh, int Ww,
+                           void* pooled, unsigned long long* trace = nullptr, const int* frame_lens = nullptr,
+                           int N = 1) {
   if (Hh == 32 && Ww == 32 && h->cfg.precision == AVSEP_PREC_BF16)
-    return launch_visual_cnn_tc(s, frames, M, h->cnn, h->cnn_w2_slabs, h->cnn_w3_rows, pooled, h->num_sms, trace,
+    return launch_visual_cnn_tc(lc, frames, M, h->cnn, h->cnn_w2_slabs, h->cnn_w3_rows, pooled, h->num_sms, trace,
                                 frame_lens, N);
-  return launch_visual_cnn(s, h->cfg.precision, frames, M, Hh, Ww, h->cnn, pooled, h->num_sms, frame_lens, N);
+  return launch_visual_cnn(lc.stream, h->cfg.precision, frames, M, Hh, Ww, h->cnn, pooled, h->num_sms, frame_lens, N);
 }
 
 // out[M, N] = A[M, K] W[N, K]^T: one tap, densely packed operands
@@ -336,7 +387,7 @@ GemmProblem dense(const void* A, int M, int K, const void* W, int N) {
   return p;
 }
 
-int linear(avsep_handle* h, cudaStream_t s, const char* label, const void* A, int M, int K, const void* W,
+int linear(avsep_handle* h, LaunchCtx lc, const char* label, const void* A, int M, int K, const void* W,
            const float* bias, int N, int act, float* out_f32, void* out_op) {
   const GemmProblem p = dense(A, M, K, W, N);
   GemmEpilogue e;
@@ -345,7 +396,7 @@ int linear(avsep_handle* h, cudaStream_t s, const char* label, const void* A, in
   if (act == ACT_GELU && h->cfg.precision == AVSEP_PREC_BF16 && out_f32 == nullptr) e.act = ACT_GELU_BF16;
   e.out_f32 = out_f32; e.ld_f32 = N;
   e.out_op = out_op; e.ld_op = N;
-  CKL(label, launch_gemm(s, h->cfg.precision, p, e, h->num_sms));
+  CKL(label, lc, launch_gemm, h->cfg.precision, p, e, h->num_sms);
   return 0;
 }
 
@@ -353,7 +404,7 @@ int linear(avsep_handle* h, cudaStream_t s, const char* label, const void* A, in
 //   x_out = value (+ resid);  out_op = LayerNorm_{g,b}(x_out)   (g == null: out_op = cast(x_out))
 // Fused into the GEMM epilogue when the row fits one tile (EPI_LN), otherwise GEMM -> y, then the warp-shuffle
 // add+LayerNorm kernel.  rows_out = number of output rows; y = scratch [rows_out, N] fp32.
-int gemm_resid_ln(avsep_handle* h, cudaStream_t s, const char* label, const GemmProblem& p, GemmEpilogue e,
+int gemm_resid_ln(avsep_handle* h, LaunchCtx lc, const char* label, const GemmProblem& p, GemmEpilogue e,
                   const float* resid, float* x_out, const float* g, const float* b, void* out_op, int rows_out,
                   float* y) {
   const int prec = h->cfg.precision;
@@ -363,28 +414,28 @@ int gemm_resid_ln(avsep_handle* h, cudaStream_t s, const char* label, const Gemm
     e.out_f32 = x_out; e.ld_f32 = p.N;
     e.ln_gamma = g; e.ln_beta = b;
     e.out_op = out_op; e.ld_op = p.N;
-    CKL(label, launch_gemm(s, prec, p, e, h->num_sms));
+    CKL(label, lc, launch_gemm, prec, p, e, h->num_sms);
     return 0;
   }
   e.kind = EPI_STD;
   e.out_op = nullptr;
   if (resid != nullptr) {
     e.out_f32 = y; e.ld_f32 = p.N;
-    CKL(label, launch_gemm(s, prec, p, e, h->num_sms));
-    CKL("add_layernorm", launch_add_layernorm(s, prec, resid, y, g, b, x_out, out_op, rows_out, p.N));
+    CKL(label, lc, launch_gemm, prec, p, e, h->num_sms);
+    CKL("add_layernorm", lc, launch_add_layernorm, prec, resid, y, g, b, x_out, out_op, rows_out, p.N);
   } else {
     e.out_f32 = x_out; e.ld_f32 = p.N;
-    CKL(label, launch_gemm(s, prec, p, e, h->num_sms));
-    CKL("add_layernorm", launch_add_layernorm(s, prec, x_out, nullptr, g, b, nullptr, out_op, rows_out, p.N));
+    CKL(label, lc, launch_gemm, prec, p, e, h->num_sms);
+    CKL("add_layernorm", lc, launch_add_layernorm, prec, x_out, nullptr, g, b, nullptr, out_op, rows_out, p.N);
   }
   return 0;
 }
 
-int linear_resid_ln(avsep_handle* h, cudaStream_t s, const char* label, const void* A, int M, int K, const void* W,
+int linear_resid_ln(avsep_handle* h, LaunchCtx lc, const char* label, const void* A, int M, int K, const void* W,
                     const float* bias, int N, float* x, const float* g, const float* b, void* out_op, float* y) {
   GemmEpilogue e;
   e.bias = bias;
-  return gemm_resid_ln(h, s, label, dense(A, M, K, W, N), e, x, x, g, b, out_op, M, y);
+  return gemm_resid_ln(h, lc, label, dense(A, M, K, W, N), e, x, x, g, b, out_op, M, y);
 }
 
 bool stack_fusable(const avsep_handle* h, int len) {
@@ -421,7 +472,7 @@ Plan forward_plan(const avsep_handle* h, int T, int N) {
 // A whole stack in one kernel (xformer_stack_sm100.cu).  which: 0 audio encoder, 1 visual encoder, 2 fusion.  The
 // caller sets the buffers and the optional stages of `sp`; this fills what follows from the stack: the weight stream
 // (from the input-projection items on when sp.pro_a is set), layer count, attention kind, activation, decoder geometry.
-int run_stack(avsep_handle* h, cudaStream_t s, int which, StackProblem sp) {
+int run_stack(avsep_handle* h, LaunchCtx lc, int which, StackProblem sp) {
   const bool pro = sp.pro_a != nullptr;
   sp.wstream = which == 0 ? (pro ? h->xs_a : h->xs_a_np) : which == 1 ? (pro ? h->xs_v : h->xs_v_np) : h->xs_f;
   sp.n_layers = which == 2 ? h->cfg.num_fusion_layers : h->cfg.num_encoder_layers;
@@ -430,7 +481,7 @@ int run_stack(avsep_handle* h, cudaStream_t s, int which, StackProblem sp) {
   sp.act = sp.cross ? ACT_GELU : ACT_RELU;
   sp.F = h->cfg.freq_bins; sp.S = h->cfg.num_speakers;
   CKL(which == 0 ? "layer.audio_enc" : which == 1 ? "layer.visual_enc" : sp.masks ? "layer.fusion_decoder" : "layer.fusion",
-      launch_xformer_stack(s, sp, h->num_sms));
+      lc, launch_xformer_stack, sp, h->num_sms);
   return 0;
 }
 
@@ -439,28 +490,29 @@ int run_stack(avsep_handle* h, cudaStream_t s, int which, StackProblem sp) {
 constexpr int FFN_FUSED_MIN_ROWS = 2048;
 
 // Feed-forward sub-layer of layer w: x += W2 act(W1 a_op + b1) + b2; a_op = LN_{g,b}(x).  ffn [M, 4d], y [M, d]: scratch.
-int ffn_sublayer(avsep_handle* h, cudaStream_t s, const LayerW& w, int act, int M, float* x, void* a_op, void* ffn,
+int ffn_sublayer(avsep_handle* h, LaunchCtx lc, const LayerW& w, int act, int M, float* x, void* a_op, void* ffn,
                  float* y, const float* g, const float* b) {
   const int d = h->cfg.d_model;
   if (ffn_fusable(h->cfg.precision, d) && M >= FFN_FUSED_MIN_ROWS) {
-    CKL("ffn.fused", launch_ffn_fused(s, a_op, w.w1, w.b1, w.w2, w.b2, act, x, x, g, b, a_op, M, h->num_sms, nullptr));
+    CKL("ffn.fused", lc, launch_ffn_fused, a_op, w.w1, w.b1, w.w2, w.b2, act, x, x, g, b, a_op, M, h->num_sms,
+        nullptr);
     return 0;
   }
-  if (linear(h, s, "gemm.ffn1", a_op, M, d, w.w1, w.b1, 4 * d, act, nullptr, ffn)) return 1;
-  return linear_resid_ln(h, s, "gemm.ffn2", ffn, M, 4 * d, w.w2, w.b2, d, x, g, b, a_op, y);
+  if (linear(h, lc, "gemm.ffn1", a_op, M, d, w.w1, w.b1, 4 * d, act, nullptr, ffn)) return 1;
+  return linear_resid_ln(h, lc, "gemm.ffn2", ffn, M, 4 * d, w.w2, w.b2, d, x, g, b, a_op, y);
 }
 
 // nn.TransformerEncoderLayer x L (pre-norm, ReLU FFN; model.py:48-52,59; torch transformer.py:946-950).
 // In: x (fp32 residual stream), a_op = LN_{layer0.norm1}(x).  Out: x, a_op = LN_{final}(x) (or cast when final_g == null).
 // lens: keys per utterance of a variable-length batch, or null.
-int encoder_stack(avsep_handle* h, cudaStream_t s, const std::vector<LayerW>& layers, int B, int L, float* x,
+int encoder_stack(avsep_handle* h, LaunchCtx lc, const std::vector<LayerW>& layers, int B, int L, float* x,
                   float* y, void* a_op, void* qkv, void* attn, void* ffn, const float* final_g, const float* final_b,
                   const int* lens = nullptr) {
   const int d = h->cfg.d_model, H = h->cfg.nhead, M = B * L, prec = h->cfg.precision;
   const size_t os = op_size(h);
   for (size_t l = 0; l < layers.size(); ++l) {
     const LayerW& w = layers[l];
-    if (linear(h, s, "gemm.qkv", a_op, M, d, w.w_in, w.b_in, 3 * d, ACT_NONE, nullptr, qkv)) return 1;
+    if (linear(h, lc, "gemm.qkv", a_op, M, d, w.w_in, w.b_in, 3 * d, ACT_NONE, nullptr, qkv)) return 1;
     AttnProblem ap{};
     ap.q = qkv; ap.ldq = 3 * d;
     ap.k = static_cast<const uint8_t*>(qkv) + static_cast<size_t>(d) * os;
@@ -469,10 +521,10 @@ int encoder_stack(avsep_handle* h, cudaStream_t s, const std::vector<LayerW>& la
     ap.out = attn; ap.ldo = d;
     ap.B = B; ap.H = H; ap.hd = d / H; ap.Lq = L; ap.Lk = L; ap.lerp_src = 0; ap.tc_mode = h->attn_tc;
     ap.k_lens = lens;
-    CKL("attn.self", launch_attention(s, prec, ap));
-    if (linear_resid_ln(h, s, "gemm.out_proj", attn, M, d, w.wo, w.bo, d, x, w.n2g, w.n2b, a_op, y)) return 1;
+    CKL("attn.self", lc, launch_attention, prec, ap);
+    if (linear_resid_ln(h, lc, "gemm.out_proj", attn, M, d, w.wo, w.bo, d, x, w.n2g, w.n2b, a_op, y)) return 1;
     const bool last = (l + 1 == layers.size());
-    if (ffn_sublayer(h, s, w, ACT_RELU, M, x, a_op, ffn, y, last ? final_g : layers[l + 1].n1g,
+    if (ffn_sublayer(h, lc, w, ACT_RELU, M, x, a_op, ffn, y, last ? final_g : layers[l + 1].n1g,
                      last ? final_b : layers[l + 1].n1b))
       return 1;
   }
@@ -483,11 +535,10 @@ int encoder_stack(avsep_handle* h, cudaStream_t s, const std::vector<LayerW>& la
 // layer's LayerNorm: x_a (fp32) and a_op = LN_{layer0.norm1}(x_a).
 // pl.stack_a: the stack kernel computes the first LayerNorm itself, so only the fp32 residual rows are written, and with
 // pl.pro it runs Conv1d #2 + ReLU + PE too, on h1.
-int audio_frontend(avsep_handle* h, cudaStream_t s, Workspace& w, const float* mixed, const Plan& pl) {
-  h->prof_stream = s;
+int audio_frontend(avsep_handle* h, LaunchCtx lc, Workspace& w, const float* mixed, const Plan& pl) {
   const int d = h->cfg.d_model, F = h->cfg.freq_bins, B = w.B, T = w.T, prec = h->cfg.precision;
   const int Map = B * (T + 2);
-  CKL("prep_audio", launch_prep_audio(s, prec, mixed, w.xp, B, F, T, h->Fp, w.lens));
+  CKL("prep_audio", lc, launch_prep_audio, prec, mixed, w.xp, B, F, T, h->Fp, w.lens);
   {
     GemmProblem p{};
     p.A = w.xp; p.lda = h->Fp; p.rowsA = Map; p.M = Map; p.W = h->wc1; p.ldw = 3 * h->Fp; p.N = d; p.K = h->Fp;
@@ -496,7 +547,7 @@ int audio_frontend(avsep_handle* h, cudaStream_t s, Workspace& w, const float* m
     e.bias = h->bc1; e.act = ACT_RELU; e.rowmap = ROW_PAD2PAD; e.Lp = T + 2;
     e.lens = w.lens;
     e.out_op = w.h1; e.ld_op = d;
-    CKL("gemm.conv1d_0", launch_gemm(s, prec, p, e, h->num_sms));
+    CKL("gemm.conv1d_0", lc, launch_gemm, prec, p, e, h->num_sms);
   }
   if (pl.stack_a && pl.pro) return 0;
   {
@@ -508,35 +559,34 @@ int audio_frontend(avsep_handle* h, cudaStream_t s, Workspace& w, const float* m
     e.pe = h->pe_a;
     if (pl.stack_a) {
       e.out_f32 = w.x_a; e.ld_f32 = d;
-      CKL("gemm.conv1d_2", launch_gemm(s, prec, p, e, h->num_sms));
-    } else if (gemm_resid_ln(h, s, "gemm.conv1d_2", p, e, nullptr, w.x_a, h->enc_a[0].n1g, h->enc_a[0].n1b, w.a_op,
+      CKL("gemm.conv1d_2", lc, launch_gemm, prec, p, e, h->num_sms);
+    } else if (gemm_resid_ln(h, lc, "gemm.conv1d_2", p, e, nullptr, w.x_a, h->enc_a[0].n1g, h->enc_a[0].n1b, w.a_op,
                              B * T, w.y_a)) {
       return 1;
     }
   }
-  return snapshot(h, s, "audio_embed", w.x_a, static_cast<size_t>(B) * T * d, false);
+  return snapshot(h, lc.stream, "audio_embed", w.x_a, static_cast<size_t>(B) * T * d, false);
 }
 
 // VisualEncoder up to (not including) the transformer: CNN, pool, frame_proj, +PE (model.py:106-110), then the
 // first layer's LayerNorm: x_v (fp32) and v_op = LN_{layer0.norm1}(x_v).  pl.stack_v / pl.pro as in audio_frontend.
-int visual_frontend(avsep_handle* h, cudaStream_t s, Workspace& w, const float* frames, const Plan& pl) {
-  h->prof_stream = s;
+int visual_frontend(avsep_handle* h, LaunchCtx lc, Workspace& w, const float* frames, const Plan& pl) {
   const int d = h->cfg.d_model, B = w.B, N = w.N;
   const int Mv = B * N;
-  CKL("visual_cnn", run_visual_cnn(h, s, frames, Mv, w.Hh, w.Ww, w.pooled, nullptr, w.frame_lens, N));
-  if (snapshot(h, s, "visual_pool", w.pooled, static_cast<size_t>(Mv) * 128, true)) return 1;
+  CKL("visual_cnn", lc, run_visual_cnn, h, frames, Mv, w.Hh, w.Ww, w.pooled, nullptr, w.frame_lens, N);
+  if (snapshot(h, lc.stream, "visual_pool", w.pooled, static_cast<size_t>(Mv) * 128, true)) return 1;
   if (pl.stack_v && pl.pro) return 0;
   const GemmProblem p = dense(w.pooled, Mv, 128, h->wproj, d);
   GemmEpilogue e;
   e.bias = h->bproj; e.pe = h->pe_v; e.pe_period = N;
   if (pl.stack_v) {
     e.out_f32 = w.x_v; e.ld_f32 = d;
-    CKL("gemm.frame_proj", launch_gemm(s, h->cfg.precision, p, e, h->num_sms));
-  } else if (gemm_resid_ln(h, s, "gemm.frame_proj", p, e, nullptr, w.x_v, h->enc_v[0].n1g, h->enc_v[0].n1b, w.v_op, Mv,
+    CKL("gemm.frame_proj", lc, launch_gemm, h->cfg.precision, p, e, h->num_sms);
+  } else if (gemm_resid_ln(h, lc, "gemm.frame_proj", p, e, nullptr, w.x_v, h->enc_v[0].n1g, h->enc_v[0].n1b, w.v_op, Mv,
                            w.y_v)) {
     return 1;
   }
-  return snapshot(h, s, "visual_embed", w.x_v, static_cast<size_t>(Mv) * d, false);
+  return snapshot(h, lc.stream, "visual_embed", w.x_v, static_cast<size_t>(Mv) * d, false);
 }
 
 // CrossModalFusion (model.py:145-149,166-173) as one kernel: the visual rows are interpolated to the audio frame rate
@@ -544,38 +594,36 @@ int visual_frontend(avsep_handle* h, cudaStream_t s, Workspace& w, const float* 
 // fusion layer come from one GEMM on those T rows (bf16) unless the visual stack kernel has written them (pl.kvp).
 // In: x_a (fp32 residual), x_v (fp32 visual encoder output, N rows per utterance).  Out: a_op = fusion.norm(x) in bf16,
 // or with pl.dec separated / masks from the SeparationDecoder inside the same kernel.
-int fusion_stack_fused(avsep_handle* h, cudaStream_t s, Workspace& w, const Plan& pl, const float* mixed,
+int fusion_stack_fused(avsep_handle* h, LaunchCtx lc, Workspace& w, const Plan& pl, const float* mixed,
                        float* separated, float* masks) {
-  h->prof_stream = s;
   const int d = h->cfg.d_model, B = w.B, T = w.T;
   const int Ma = B * T, Lf = h->cfg.num_fusion_layers;
   if (!pl.kvp) {
-    CKL("lerp_kv", launch_lerp_rows(s, w.x_v, d, B, w.N, T, d, w.attn_a, d, w.frame_lens, w.lens));
-    if (linear(h, s, "gemm.cross_kv", w.attn_a, Ma, d, h->wkv_all, h->bkv_all, Lf * 2 * d, ACT_NONE, nullptr, w.kvb)) return 1;
+    CKL("lerp_kv", lc, launch_lerp_rows, w.x_v, d, B, w.N, T, d, w.attn_a, d, w.frame_lens, w.lens);
+    if (linear(h, lc, "gemm.cross_kv", w.attn_a, Ma, d, h->wkv_all, h->bkv_all, Lf * 2 * d, ACT_NONE, nullptr, w.kvb)) return 1;
   }
   StackProblem sp{};
   sp.x_in = w.x_a; sp.fin_gamma = h->fng; sp.fin_beta = h->fnb; sp.kv = w.kvb;
   sp.B = B; sp.L = T; sp.lens = w.lens;
   if (pl.dec) {
     sp.mixed = mixed; sp.separated = separated; sp.masks = masks;
-    return run_stack(h, s, 2, sp);
+    return run_stack(h, lc, 2, sp);
   }
   sp.out_x = h->debug ? w.x_a : nullptr; sp.out_op = w.a_op;
-  if (run_stack(h, s, 2, sp)) return 1;
-  return snapshot(h, s, "fused", w.a_op, static_cast<size_t>(Ma) * d, true);
+  if (run_stack(h, lc, 2, sp)) return 1;
+  return snapshot(h, lc.stream, "fused", w.a_op, static_cast<size_t>(Ma) * d, true);
 }
 
 // CrossModalFusion, one kernel per layer.  In: x_a residual stream, a_op = LN_{layer0.norm1}(x_a), v_op = visual rows
 // (L_src per utterance).  Out: a_op = fusion.norm(x) in operand precision.
-int fusion_stack(avsep_handle* h, cudaStream_t s, Workspace& w, int L_src) {
-  h->prof_stream = s;
+int fusion_stack(avsep_handle* h, LaunchCtx lc, Workspace& w, int L_src) {
   const int d = h->cfg.d_model, H = h->cfg.nhead, B = w.B, T = w.T, prec = h->cfg.precision;
   const int Ma = B * T, Mv = B * L_src, Lf = h->cfg.num_fusion_layers;
   // K/V projection of every fusion layer in one GEMM on the un-interpolated visual rows
-  if (linear(h, s, "gemm.cross_kv", w.v_op, Mv, d, h->wkv_all, h->bkv_all, Lf * 2 * d, ACT_NONE, w.kvn, nullptr)) return 1;
+  if (linear(h, lc, "gemm.cross_kv", w.v_op, Mv, d, h->wkv_all, h->bkv_all, Lf * 2 * d, ACT_NONE, w.kvn, nullptr)) return 1;
   for (int l = 0; l < Lf; ++l) {
     const LayerW& fw = h->fus[l];
-    if (linear(h, s, "gemm.cross_q", w.a_op, Ma, d, fw.w_in, fw.b_in, d, ACT_NONE, nullptr, w.qkv_a)) return 1;
+    if (linear(h, lc, "gemm.cross_q", w.a_op, Ma, d, fw.w_in, fw.b_in, d, ACT_NONE, nullptr, w.qkv_a)) return 1;
     AttnProblem ap{};
     ap.q = w.qkv_a; ap.ldq = d;
     ap.k = w.kvn + static_cast<size_t>(l) * 2 * d;
@@ -592,55 +640,52 @@ int fusion_stack(avsep_handle* h, cudaStream_t s, Workspace& w, int L_src) {
       __nv_bfloat16* kvi = static_cast<__nv_bfloat16*>(w.qkv_a) + static_cast<size_t>(Ma) * d;
       tp.k = kvi; tp.v = kvi + d; tp.ldkv = 2 * d;
       if (attention_tc_wanted(prec, tp)) {
-        CKL("lerp_kv", launch_lerp_rows(s, w.kvn + static_cast<size_t>(l) * 2 * d, Lf * 2 * d, B, L_src, T, 2 * d, kvi, 2 * d,
-                                        w.frame_lens, w.lens));
+        CKL("lerp_kv", lc, launch_lerp_rows, w.kvn + static_cast<size_t>(l) * 2 * d, Lf * 2 * d, B, L_src, T, 2 * d,
+            kvi, 2 * d, w.frame_lens, w.lens);
         ap = tp;
       }
     }
-    CKL("attn.cross", launch_attention(s, prec, ap));
-    if (linear_resid_ln(h, s, "gemm.out_proj", w.attn_a, Ma, d, fw.wo, fw.bo, d, w.x_a, fw.n2g, fw.n2b, w.a_op, w.y_a))
+    CKL("attn.cross", lc, launch_attention, prec, ap);
+    if (linear_resid_ln(h, lc, "gemm.out_proj", w.attn_a, Ma, d, fw.wo, fw.bo, d, w.x_a, fw.n2g, fw.n2b, w.a_op, w.y_a))
       return 1;
     const bool last = (l + 1 == Lf);
-    if (ffn_sublayer(h, s, fw, ACT_GELU, Ma, w.x_a, w.a_op, w.ffn_a, w.y_a, last ? h->fng : h->fus[l + 1].n1g,
+    if (ffn_sublayer(h, lc, fw, ACT_GELU, Ma, w.x_a, w.a_op, w.ffn_a, w.y_a, last ? h->fng : h->fus[l + 1].n1g,
                      last ? h->fnb : h->fus[l + 1].n1b))
       return 1;
   }
-  return snapshot(h, s, "fused", w.a_op, static_cast<size_t>(Ma) * d, true);
+  return snapshot(h, lc.stream, "fused", w.a_op, static_cast<size_t>(Ma) * d, true);
 }
 
 // SeparationDecoder.forward + .separate (model.py:201-220): a_op = fused rows in operand precision.
-int decoder_stage(avsep_handle* h, cudaStream_t s, Workspace& w, const float* mixed, float* separated, float* masks) {
-  h->prof_stream = s;
+int decoder_stage(avsep_handle* h, LaunchCtx lc, Workspace& w, const float* mixed, float* separated, float* masks) {
   const int d = h->cfg.d_model, F = h->cfg.freq_bins, S = h->cfg.num_speakers, B = w.B, T = w.T;
   const int Ma = B * T;
-  if (linear(h, s, "gemm.dec0", w.a_op, Ma, d, h->wdec0, h->bdec0, 2 * d, ACT_GELU, nullptr, w.ffn_a)) return 1;
+  if (linear(h, lc, "gemm.dec0", w.a_op, Ma, d, h->wdec0, h->bdec0, 2 * d, ACT_GELU, nullptr, w.ffn_a)) return 1;
   GemmEpilogue e;
   e.kind = EPI_TAIL;
   e.bias = h->bdec3;
   e.mixed = mixed; e.masks = masks; e.separated = separated; e.F = F; e.S = S; e.T = T;
   e.lens = w.lens;
-  CKL("gemm.dec3_tail", launch_gemm(s, h->cfg.precision, dense(w.ffn_a, Ma, 2 * d, h->wdec3, S * F), e, h->num_sms));
+  CKL("gemm.dec3_tail", lc, launch_gemm, h->cfg.precision, dense(w.ffn_a, Ma, 2 * d, h->wdec3, S * F), e,
+      h->num_sms);
   return 0;
 }
 
-int forward_device(avsep_handle* h, cudaStream_t s, Workspace& w, const float* mixed, const float* frames,
+int forward_device(avsep_handle* h, LaunchCtx lc, Workspace& w, const float* mixed, const float* frames,
                    float* separated, float* masks) {
   const int d = h->cfg.d_model;
   const int Ma = w.B * w.T, Mv = w.B * w.N;
   const Plan pl = forward_plan(h, w.T, w.N);
-  h->prof_stream = s;
-  if (h->profile && h->profile_spin_us > 0) spin_kernel<<<1, 1, 0, s>>>(1000ull * h->profile_spin_us);
+  if (h->profile && h->profile_spin_us > 0) spin_kernel<<<1, 1, 0, lc.stream>>>(1000ull * h->profile_spin_us);
   // The audio and visual branches are independent until the fusion.
-  cudaStream_t sv = s;
+  LaunchCtx sv = lc;
   if (pl.fork) {
-    if (h->aux_stream == nullptr) {
-      CUDA_OK(cudaStreamCreateWithFlags(&h->aux_stream, cudaStreamNonBlocking));
-      CUDA_OK(cudaEventCreateWithFlags(&h->ev_fork, cudaEventDisableTiming));
-      CUDA_OK(cudaEventCreateWithFlags(&h->ev_join, cudaEventDisableTiming));
-    }
-    sv = h->aux_stream;
-    CUDA_OK(cudaEventRecord(h->ev_fork, s));
-    CUDA_OK(cudaStreamWaitEvent(sv, h->ev_fork, 0));
+    CUDA_OK(make_stream(h->aux_stream));
+    CUDA_OK(make_event(h->ev_fork));
+    CUDA_OK(make_event(h->ev_join));
+    sv.stream = h->aux_stream.get();
+    CUDA_OK(cudaEventRecord(h->ev_fork.get(), lc.stream));
+    CUDA_OK(cudaStreamWaitEvent(sv.stream, h->ev_fork.get(), 0));
   }
   // --- visual branch (enqueued first: its CNN is the longest kernel) ---
   if (visual_frontend(h, sv, w, frames, pl)) return 1;
@@ -661,9 +706,9 @@ int forward_device(avsep_handle* h, cudaStream_t s, Workspace& w, const float* m
                            w.frame_lens)) {
     return 1;
   }
-  if (snapshot(h, sv, "visual_enc", w.x_v, static_cast<size_t>(Mv) * d, false)) return 1;
+  if (snapshot(h, sv.stream, "visual_enc", w.x_v, static_cast<size_t>(Mv) * d, false)) return 1;
   // --- audio branch ---
-  if (audio_frontend(h, s, w, mixed, pl)) return 1;
+  if (audio_frontend(h, lc, w, mixed, pl)) return 1;
   if (pl.stack_a) {
     StackProblem sp{};
     sp.x_in = w.x_a; sp.out_x = w.x_a; sp.out_op = pl.stack_f ? nullptr : w.a_op;
@@ -673,26 +718,26 @@ int forward_device(avsep_handle* h, cudaStream_t s, Workspace& w, const float* m
       sp.pro_a = w.h1; sp.pro_relu = 1; sp.pro_taps = 3; sp.pro_k = d; sp.pro_pitch = w.T + 2;
       sp.pro_rows = w.B * (w.T + 2); sp.pe = h->pe_a;
     }
-    if (run_stack(h, s, 0, sp)) return 1;
-  } else if (encoder_stack(h, s, h->enc_a, w.B, w.T, w.x_a, w.y_a, w.a_op, w.qkv_a, w.attn_a, w.ffn_a, h->fus[0].n1g,
+    if (run_stack(h, lc, 0, sp)) return 1;
+  } else if (encoder_stack(h, lc, h->enc_a, w.B, w.T, w.x_a, w.y_a, w.a_op, w.qkv_a, w.attn_a, w.ffn_a, h->fus[0].n1g,
                            h->fus[0].n1b, w.lens)) {
     return 1;
   }
-  if (snapshot(h, s, "audio_enc", w.x_a, static_cast<size_t>(Ma) * d, false)) return 1;
+  if (snapshot(h, lc.stream, "audio_enc", w.x_a, static_cast<size_t>(Ma) * d, false)) return 1;
   if (pl.fork) {
-    CUDA_OK(cudaEventRecord(h->ev_join, sv));
-    CUDA_OK(cudaStreamWaitEvent(s, h->ev_join, 0));
+    CUDA_OK(cudaEventRecord(h->ev_join.get(), sv.stream));
+    CUDA_OK(cudaStreamWaitEvent(lc.stream, h->ev_join.get(), 0));
   }
   // --- fusion + decoder ---
-  if (pl.stack_f ? fusion_stack_fused(h, s, w, pl, mixed, separated, masks) : fusion_stack(h, s, w, w.N)) return 1;
-  return pl.dec ? 0 : decoder_stage(h, s, w, mixed, separated, masks);
+  if (pl.stack_f ? fusion_stack_fused(h, lc, w, pl, mixed, separated, masks) : fusion_stack(h, lc, w, w.N)) return 1;
+  return pl.dec ? 0 : decoder_stage(h, lc, w, mixed, separated, masks);
 }
 
 // Eager on the first use of a (shape, buffer set); captured into a CUDA graph on the second; replayed afterwards.
 // The graph bakes in the kernel parameters (tensor maps included), so a replay costs one host call.
-int forward_cached(avsep_handle* h, cudaStream_t s, Workspace& w, const void* ws_base, const float* mixed,
+int forward_cached(avsep_handle* h, LaunchCtx lc, Workspace& w, const void* ws_base, const float* mixed,
                    const float* frames, float* separated, float* masks) {
-  if (!h->use_graph || h->profile || h->debug) return forward_device(h, s, w, mixed, frames, separated, masks);
+  if (!h->use_graph || h->profile || h->debug) return forward_device(h, lc, w, mixed, frames, separated, masks);
   const GraphKey key{w.B, w.T, w.N, w.Hh, w.Ww, mixed, frames, separated, masks, ws_base, w.lens, w.frame_lens};
   GraphEntry* ent = nullptr;
   for (auto& g : h->graphs)
@@ -702,56 +747,52 @@ int forward_cached(avsep_handle* h, cudaStream_t s, Workspace& w, const void* ws
       size_t victim = 0;
       for (size_t i = 1; i < h->graphs.size(); ++i)
         if (h->graphs[i].last_use < h->graphs[victim].last_use) victim = i;
-      if (h->graphs[victim].exec) cudaGraphExecDestroy(h->graphs[victim].exec);
       h->graphs.erase(h->graphs.begin() + victim);
     }
     GraphEntry g;
     g.key = key;
     g.last_use = ++h->graph_clock;
-    h->graphs.push_back(g);
-    return forward_device(h, s, w, mixed, frames, separated, masks);   // warm-up, also sets kernel attributes
+    h->graphs.push_back(std::move(g));
+    return forward_device(h, lc, w, mixed, frames, separated, masks);   // warm-up, also sets kernel attributes
   }
   ent->last_use = ++h->graph_clock;
   if (ent->exec == nullptr) {
-    if (h->cap_stream == nullptr) CUDA_OK(cudaStreamCreateWithFlags(&h->cap_stream, cudaStreamNonBlocking));
-    CUDA_OK(cudaStreamBeginCapture(h->cap_stream, cudaStreamCaptureModeRelaxed));
-    const int rc = forward_device(h, h->cap_stream, w, mixed, frames, separated, masks);
+    CUDA_OK(make_stream(h->cap_stream));
+    CUDA_OK(cudaStreamBeginCapture(h->cap_stream.get(), cudaStreamCaptureModeRelaxed));
+    const int rc = forward_device(h, {h->cap_stream.get(), lc.pdl}, w, mixed, frames, separated, masks);
     cudaGraph_t graph = nullptr;
-    const cudaError_t ce = cudaStreamEndCapture(h->cap_stream, &graph);
+    const cudaError_t ce = cudaStreamEndCapture(h->cap_stream.get(), &graph);
     if (rc != 0) {
       if (graph) cudaGraphDestroy(graph);
       return 1;
     }
     if (ce != cudaSuccess) return fail(h, std::string("cudaStreamEndCapture: ") + cudaGetErrorString(ce));
-    const cudaError_t ci = cudaGraphInstantiate(&ent->exec, graph, 0);
+    cudaGraphExec_t exec = nullptr;
+    const cudaError_t ci = cudaGraphInstantiate(&exec, graph, 0);
     cudaGraphDestroy(graph);
-    if (ci != cudaSuccess) {
-      ent->exec = nullptr;
-      return fail(h, std::string("cudaGraphInstantiate: ") + cudaGetErrorString(ci));
-    }
+    if (ci != cudaSuccess) return fail(h, std::string("cudaGraphInstantiate: ") + cudaGetErrorString(ci));
+    ent->exec.reset(exec);
     ent->launches = h->launches;
   }
   h->launches = ent->launches;
-  CUDA_OK(cudaGraphLaunch(ent->exec, s));
+  CUDA_OK(cudaGraphLaunch(ent->exec.get(), lc.stream));
   return 0;
 }
 
 // Utterances b0 .. b0 + w.B - 1 of a packed batch (include/avsep.h) through the staging: unpack, the varlen forward
 // (cached graph) on the staging, pack.  lens / flens: DEVICE lengths of the whole packed batch (or null), from whose
 // first b0 entries the kernels find the chunk's packed offsets.  Sets w.lens / w.frame_lens.
-int forward_packed_run(avsep_handle* h, cudaStream_t s, Workspace& w, const Staging& st, const void* ws_base,
+int forward_packed_run(avsep_handle* h, LaunchCtx lc, Workspace& w, const Staging& st, const void* ws_base,
                        const float* mixed_p, const float* frames_p, const int* lens, const int* flens, int b0,
                        float* sep_p, float* masks_p) {
   const int F = h->cfg.freq_bins, S = h->cfg.num_speakers;
-  h->prof_stream = s;
-  CKL("unpack", launch_unpack(s, mixed_p, frames_p, lens, flens, b0, w.B, F, w.T, w.N, w.Hh * w.Ww, st.mixed,
-                              st.frames));
+  CKL("unpack", lc, launch_unpack, mixed_p, frames_p, lens, flens, b0, w.B, F, w.T, w.N, w.Hh * w.Ww, st.mixed,
+      st.frames);
   w.lens = lens ? lens + b0 : nullptr;
   w.frame_lens = flens ? flens + b0 : nullptr;
   h->launches = 0;   // a graph replay sets the forward's own count
-  if (forward_cached(h, s, w, ws_base, st.mixed, st.frames, st.sep, st.masks)) return 1;
-  h->prof_stream = s;
-  CKL("pack", launch_pack(s, st.sep, st.masks, lens, b0, w.B, S, F, w.T, sep_p, masks_p));
+  if (forward_cached(h, lc, w, ws_base, st.mixed, st.frames, st.sep, st.masks)) return 1;
+  CKL("pack", lc, launch_pack, st.sep, st.masks, lens, b0, w.B, S, F, w.T, sep_p, masks_p);
   ++h->launches;     // the unpack
   return 0;
 }
@@ -904,38 +945,7 @@ int avsep_create(const avsep_config* cfg, avsep_handle** out) {
 
 void avsep_destroy(avsep_handle* h) {
   if (!h) return;
-  cudaSetDevice(h->cfg.device);
-  if (h->d_weights) cudaFree(h->d_weights);
-  if (h->own_ws) cudaFree(h->own_ws);
-  for (auto& sl : h->slot) {
-    for (float* ptr : sl.io)
-      if (ptr) cudaFree(ptr);
-    for (cudaEvent_t e : sl.ev) cudaEventDestroy(e);
-    if (sl.ev_start) cudaEventDestroy(sl.ev_start);
-    if (sl.ev_end) cudaEventDestroy(sl.ev_end);
-    for (cudaEvent_t e : sl.ev_lane)
-      if (e) cudaEventDestroy(e);
-    if (sl.ev_lens) cudaEventDestroy(sl.ev_lens);
-    if (sl.lens_dev) cudaFree(sl.lens_dev);
-    if (sl.lens_host) cudaFreeHost(sl.lens_host);
-  }
-  for (void* ptr : h->shared_mapped) cudaIpcCloseMemHandle(ptr);
-  for (void* ptr : h->shared_owned) cudaFree(ptr);
-  if (h->synth_waves) cudaFree(h->synth_waves);
-  if (h->host_ws) cudaFree(h->host_ws);
-  for (auto& kv : h->snaps)
-    if (kv.second.first) cudaFree(kv.second.first);
-  for (cudaEvent_t e : h->ev_pool) cudaEventDestroy(e);
-  for (auto& g : h->graphs)
-    if (g.exec) cudaGraphExecDestroy(g.exec);
-  if (h->cap_stream) cudaStreamDestroy(h->cap_stream);
-  if (h->aux_stream) cudaStreamDestroy(h->aux_stream);
-  if (h->ev_fork) cudaEventDestroy(h->ev_fork);
-  if (h->ev_join) cudaEventDestroy(h->ev_join);
-  for (int i = 0; i < 3; ++i) {
-    if (h->hs[i]) cudaStreamDestroy(h->hs[i]);
-    if (h->host_comp[i]) cudaStreamDestroy(h->host_comp[i]);
-  }
+  cudaSetDevice(h->cfg.device);   // the handle's resources belong to its device
   delete h;
 }
 
@@ -1107,13 +1117,10 @@ int avsep_finalize_weights(avsep_handle* h, void* cuda_stream) {
   }
   // upload
   drop_graphs(h);
-  if (h->d_weights) cudaFree(h->d_weights);
-  h->d_weights = nullptr;
-  CUDA_OK(cudaMalloc(&h->d_weights, ar.bytes.size()));
-  h->weight_bytes = ar.bytes.size();
-  CUDA_OK(cudaMemcpyAsync(h->d_weights, ar.bytes.data(), ar.bytes.size(), cudaMemcpyHostToDevice, s));
+  CUDA_OK(h->weights.alloc(ar.bytes.size()));
+  CUDA_OK(cudaMemcpyAsync(h->weights.get(), ar.bytes.data(), ar.bytes.size(), cudaMemcpyHostToDevice, s));
   CUDA_OK(cudaStreamSynchronize(s));
-  ar.patch(h->d_weights);
+  ar.patch(h->weights.get());
   if (h->xs_a != nullptr) {
     h->xs_a_np = h->xs_a + xformer_pro_bytes(3, h->cfg.d_model);
     h->xs_v_np = h->xs_v + xformer_pro_bytes(1, 128);
@@ -1146,8 +1153,8 @@ int avsep_forward_varlen(avsep_handle* h, const float* mixed_spec, const float* 
   if (get_workspace(h, w, workspace, workspace_bytes, B, T, N, Hh, Ww)) return 1;
   w.lens = lengths; w.frame_lens = frame_lengths;
   h->launches = 0;
-  return forward_cached(h, static_cast<cudaStream_t>(cuda_stream), w, workspace ? workspace : h->own_ws, mixed_spec,
-                        lip_frames, separated, masks);
+  return forward_cached(h, launch_ctx(h, static_cast<cudaStream_t>(cuda_stream)), w,
+                        workspace ? workspace : h->own_ws.get(), mixed_spec, lip_frames, separated, masks);
 }
 
 size_t avsep_packed_workspace_bytes(avsep_handle* h, int32_t B, int32_t T, int32_t N, int32_t Hh, int32_t Ww) {
@@ -1177,8 +1184,8 @@ int avsep_forward_packed(avsep_handle* h, const float* mixed_packed, const float
     return 1;
   carve_packed(h, w, st, base, B, T, N, Hh, Ww);
   h->launches = 0;
-  return forward_packed_run(h, static_cast<cudaStream_t>(cuda_stream), w, st, base, mixed_packed, frames_packed,
-                            lengths, frame_lengths, 0, separated_packed, masks_packed);
+  return forward_packed_run(h, launch_ctx(h, static_cast<cudaStream_t>(cuda_stream)), w, st, base, mixed_packed,
+                            frames_packed, lengths, frame_lengths, 0, separated_packed, masks_packed);
 }
 
 namespace {
@@ -1217,46 +1224,32 @@ int host_submit(avsep_handle* h, const float* mixed_spec, const float* lip_frame
   const size_t mixed_per = F * T, frames_per = static_cast<size_t>(N) * Hh * Ww, out_per = S * F * T;
   const size_t need[4] = {B * mixed_per, B * frames_per, B * out_per, B * out_per};
   for (int i = 0; i < 4; ++i) {
-    if (sl.cap[i] < need[i]) {
-      if (sl.ev_end) CUDA_OK(cudaEventSynchronize(sl.ev_end));     // the slot's previous call still owns the buffer
-      if (sl.io[i]) cudaFree(sl.io[i]);
-      sl.io[i] = nullptr;
-      sl.cap[i] = 0;
-      CUDA_OK(cudaMalloc(&sl.io[i], need[i] * sizeof(float)));
-      sl.cap[i] = need[i];
+    if (sl.io[i].cap < need[i]) {
+      if (sl.ev_end) CUDA_OK(cudaEventSynchronize(sl.ev_end.get()));   // the slot's previous call still owns the buffer
+      CUDA_OK(sl.io[i].alloc(need[i]));
     }
   }
-  float *io_mixed = sl.io[0], *io_frames = sl.io[1], *io_sep = sl.io[2], *io_masks = sl.io[3];
-  if (h->hs[0] == nullptr) {
-    for (int i = 0; i < 3; ++i) CUDA_OK(cudaStreamCreateWithFlags(&h->hs[i], cudaStreamNonBlocking));
-  }
-  auto make_event = [&](cudaEvent_t& e) -> int {
-    if (e == nullptr) CUDA_OK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-    return 0;
-  };
-  if (make_event(sl.ev_start) || make_event(sl.ev_end)) return 1;
+  float *io_mixed = sl.io[0].get(), *io_frames = sl.io[1].get(), *io_sep = sl.io[2].get(), *io_masks = sl.io[3].get();
+  for (Stream& st : h->hs) CUDA_OK(make_stream(st));
+  CUDA_OK(make_event(sl.ev_start));
+  CUDA_OK(make_event(sl.ev_end));
   const bool upload = packed && (lens || flens);
   if (upload) {
-    if (sl.lens_cap < B) {
-      CUDA_OK(cudaEventSynchronize(sl.ev_end));     // the slot's previous call still reads them
-      if (sl.lens_dev) cudaFree(sl.lens_dev);
-      if (sl.lens_host) cudaFreeHost(sl.lens_host);
-      sl.lens_dev = nullptr;
-      sl.lens_host = nullptr;
-      sl.lens_cap = 0;
-      CUDA_OK(cudaMalloc(&sl.lens_dev, 2 * sizeof(int32_t) * B));
-      CUDA_OK(cudaMallocHost(&sl.lens_host, 2 * sizeof(int32_t) * B));
-      sl.lens_cap = B;
+    const size_t n = 2 * static_cast<size_t>(B);   // the call's lengths, then its frame lengths
+    if (sl.lens_dev.cap < n || sl.lens_host.cap < n) {
+      CUDA_OK(cudaEventSynchronize(sl.ev_end.get()));     // the slot's previous call still reads them
+      CUDA_OK(sl.lens_dev.alloc(n));
+      CUDA_OK(sl.lens_host.alloc(n));
     }
-    if (make_event(sl.ev_lens)) return 1;
-    CUDA_OK(cudaEventSynchronize(sl.ev_lens));      // the previous upload from lens_host has been read
+    CUDA_OK(make_event(sl.ev_lens));
+    CUDA_OK(cudaEventSynchronize(sl.ev_lens.get()));      // the previous upload from lens_host has been read
     for (int b = 0; b < B; ++b) {
-      sl.lens_host[b] = lens ? lens[b] : T;
-      sl.lens_host[B + b] = flens ? flens[b] : N;
+      sl.lens_host.get()[b] = lens ? lens[b] : T;
+      sl.lens_host.get()[B + b] = flens ? flens[b] : N;
     }
   }
-  const int32_t* d_lens = upload && lens ? sl.lens_dev : nullptr;
-  const int32_t* d_flens = upload && flens ? sl.lens_dev + B : nullptr;
+  const int32_t* d_lens = upload && lens ? sl.lens_dev.get() : nullptr;
+  const int32_t* d_flens = upload && flens ? sl.lens_dev.get() + B : nullptr;
   // Chunk size: a stack kernel takes as long for 64 utterances as for 256 (one tile per CTA either way), so chunks are
   // a trade between pipelining inside one call and kernel time.  Measured at B = 256 (tools/e2e_probe.py): the one-call
   // form is fastest with ~56-utterance chunks on two compute lanes (copy-in of chunk i+1 under the kernels of chunk i),
@@ -1272,9 +1265,9 @@ int host_submit(avsep_handle* h, const float* mixed_spec, const float* lip_frame
   }
   const int nchunks = static_cast<int>(starts.size());
   while (static_cast<int>(sl.ev.size()) < 2 * nchunks) {
-    cudaEvent_t e;
-    CUDA_OK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-    sl.ev.push_back(e);
+    Event e;
+    CUDA_OK(make_event(e));
+    sl.ev.push_back(std::move(e));
   }
   // one workspace + compute stream per lane: with small chunks a single forward cannot fill the GPU, so the kernels
   // of consecutive chunks are allowed to overlap
@@ -1284,39 +1277,36 @@ int host_submit(avsep_handle* h, const float* mixed_spec, const float* lip_frame
   Staging stl[3];
   const size_t per_lane = packed ? carve_packed(h, wl[0], stl[0], nullptr, Bc, T, N, Hh, Ww)
                                  : carve_workspace(h, wl[0], nullptr, Bc, T, N, Hh, Ww);
-  if (h->host_ws_bytes < per_lane * lanes) {
+  if (h->host_ws.cap < per_lane * lanes) {
     CUDA_OK(cudaDeviceSynchronize());          // the other slot may still be using the old workspace
-    drop_graphs(h);
-    if (h->host_ws) cudaFree(h->host_ws);
-    h->host_ws = nullptr;
-    h->host_ws_bytes = 0;
-    CUDA_OK(cudaMalloc(&h->host_ws, per_lane * lanes));
-    h->host_ws_bytes = per_lane * lanes;
+    drop_graphs(h);                            // the cached graphs hold pointers into it
+    CUDA_OK(h->host_ws.alloc(per_lane * lanes));
   }
   for (int l = 0; l < lanes; ++l) {
-    uint8_t* lane_base = static_cast<uint8_t*>(h->host_ws) + l * per_lane;
+    uint8_t* lane_base = h->host_ws.get() + l * per_lane;
     if (packed)
       carve_packed(h, wl[l], stl[l], lane_base, Bc, T, N, Hh, Ww);
     else
       carve_workspace(h, wl[l], lane_base, Bc, T, N, Hh, Ww);
-    if (h->host_comp[l] == nullptr) CUDA_OK(cudaStreamCreateWithFlags(&h->host_comp[l], cudaStreamNonBlocking));
-    if (make_event(sl.ev_lane[l])) return 1;
+    CUDA_OK(make_stream(h->host_comp[l]));
+    CUDA_OK(make_event(sl.ev_lane[l]));
   }
-  cudaStream_t s_in = h->hs[0], s_out = h->hs[2];
+  cudaStream_t s_in = h->hs[0].get(), s_out = h->hs[2].get();
   // order after whatever the caller queued on its stream, and after this slot's previous use: its kernels have read
   // the input buffers (before they are overwritten) and its copy-out has read the output buffers
-  CUDA_OK(cudaEventRecord(sl.ev_start, s));
-  CUDA_OK(cudaStreamWaitEvent(s_in, sl.ev_start, 0));
-  for (int l = 0; l < 3; ++l)
-    if (sl.ev_lane[l]) CUDA_OK(cudaStreamWaitEvent(s_in, sl.ev_lane[l], 0));
+  CUDA_OK(cudaEventRecord(sl.ev_start.get(), s));
+  CUDA_OK(cudaStreamWaitEvent(s_in, sl.ev_start.get(), 0));
+  for (const Event& e : sl.ev_lane)
+    if (e) CUDA_OK(cudaStreamWaitEvent(s_in, e.get(), 0));
   for (int l = 0; l < lanes; ++l) {
-    CUDA_OK(cudaStreamWaitEvent(h->host_comp[l], sl.ev_start, 0));
-    CUDA_OK(cudaStreamWaitEvent(h->host_comp[l], sl.ev_end, 0));
+    CUDA_OK(cudaStreamWaitEvent(h->host_comp[l].get(), sl.ev_start.get(), 0));
+    CUDA_OK(cudaStreamWaitEvent(h->host_comp[l].get(), sl.ev_end.get(), 0));
   }
-  CUDA_OK(cudaStreamWaitEvent(s_out, sl.ev_start, 0));
+  CUDA_OK(cudaStreamWaitEvent(s_out, sl.ev_start.get(), 0));
   if (upload) {
-    CUDA_OK(cudaMemcpyAsync(sl.lens_dev, sl.lens_host, 2 * sizeof(int32_t) * B, cudaMemcpyHostToDevice, s_in));
-    CUDA_OK(cudaEventRecord(sl.ev_lens, s_in));
+    CUDA_OK(cudaMemcpyAsync(sl.lens_dev.get(), sl.lens_host.get(), 2 * sizeof(int32_t) * B, cudaMemcpyHostToDevice,
+                            s_in));
+    CUDA_OK(cudaEventRecord(sl.ev_lens.get(), s_in));
   }
   const size_t HW = static_cast<size_t>(Hh) * Ww, SF = S * F;
   int64_t launches = 0;
@@ -1324,33 +1314,33 @@ int host_submit(avsep_handle* h, const float* mixed_spec, const float* lip_frame
     const size_t b0 = starts[c];
     const int bc = sizes[c];
     const int lane = c % lanes;
-    cudaStream_t s_comp = h->host_comp[lane];
+    const LaunchCtx comp = launch_ctx(h, h->host_comp[lane].get());
     // element offsets and counts of the chunk's span in each tensor (packed or padded)
     const size_t m0 = F * t_at(b0), mn = F * (t_at(b0 + bc) - t_at(b0));
     const size_t f0 = HW * n_at(b0), fn = HW * (n_at(b0 + bc) - n_at(b0));
     const size_t o0 = SF * t_at(b0), on = SF * (t_at(b0 + bc) - t_at(b0));
     CUDA_OK(cudaMemcpyAsync(io_mixed + m0, mixed_spec + m0, mn * 4, cudaMemcpyHostToDevice, s_in));
     CUDA_OK(cudaMemcpyAsync(io_frames + f0, lip_frames + f0, fn * 4, cudaMemcpyHostToDevice, s_in));
-    CUDA_OK(cudaEventRecord(sl.ev[2 * c], s_in));
-    CUDA_OK(cudaStreamWaitEvent(s_comp, sl.ev[2 * c], 0));
+    CUDA_OK(cudaEventRecord(sl.ev[2 * c].get(), s_in));
+    CUDA_OK(cudaStreamWaitEvent(comp.stream, sl.ev[2 * c].get(), 0));
     Workspace wc = wl[lane];
     wc.B = bc;
-    const uint8_t* ws_lane = static_cast<uint8_t*>(h->host_ws) + lane * per_lane;
-    if (packed ? forward_packed_run(h, s_comp, wc, stl[lane], ws_lane, io_mixed, io_frames, d_lens, d_flens,
+    const uint8_t* ws_lane = h->host_ws.get() + lane * per_lane;
+    if (packed ? forward_packed_run(h, comp, wc, stl[lane], ws_lane, io_mixed, io_frames, d_lens, d_flens,
                                     static_cast<int>(b0), io_sep, io_masks)
-               : forward_cached(h, s_comp, wc, ws_lane, io_mixed + m0, io_frames + f0, io_sep + o0, io_masks + o0))
+               : forward_cached(h, comp, wc, ws_lane, io_mixed + m0, io_frames + f0, io_sep + o0, io_masks + o0))
       return 1;
     launches += h->launches;
-    CUDA_OK(cudaEventRecord(sl.ev[2 * c + 1], s_comp));
-    CUDA_OK(cudaStreamWaitEvent(s_out, sl.ev[2 * c + 1], 0));
+    CUDA_OK(cudaEventRecord(sl.ev[2 * c + 1].get(), comp.stream));
+    CUDA_OK(cudaStreamWaitEvent(s_out, sl.ev[2 * c + 1].get(), 0));
     CUDA_OK(cudaMemcpyAsync(separated + o0, io_sep + o0, on * 4, cudaMemcpyDeviceToHost, s_out));
     CUDA_OK(cudaMemcpyAsync(masks + o0, io_masks + o0, on * 4, cudaMemcpyDeviceToHost, s_out));
   }
   h->launches = launches;
-  for (int l = 0; l < lanes; ++l) CUDA_OK(cudaEventRecord(sl.ev_lane[l], h->host_comp[l]));
+  for (int l = 0; l < lanes; ++l) CUDA_OK(cudaEventRecord(sl.ev_lane[l].get(), h->host_comp[l].get()));
   // The caller's stream is deliberately NOT made to wait for the results: that would chain call i+1 (which is ordered
   // after the caller's stream) behind call i's copy-out.  Results are consumed on the host after avsep_host_wait.
-  CUDA_OK(cudaEventRecord(sl.ev_end, s_out));
+  CUDA_OK(cudaEventRecord(sl.ev_end.get(), s_out));
   return 0;
 }
 }  // namespace
@@ -1360,7 +1350,7 @@ int avsep_forward_host(avsep_handle* h, const float* mixed_spec, const float* li
   if (!h) return 1;
   if (host_submit(h, mixed_spec, lip_frames, B, T, N, Hh, Ww, separated, masks, 0, static_cast<cudaStream_t>(cuda_stream), false))
     return 1;
-  CUDA_OK(cudaEventSynchronize(h->slot[0].ev_end));
+  CUDA_OK(cudaEventSynchronize(h->slot[0].ev_end.get()));
   return 0;
 }
 
@@ -1379,7 +1369,7 @@ int avsep_forward_host_packed(avsep_handle* h, const float* mixed_packed, const 
   if (host_submit(h, mixed_packed, frames_packed, B, T, N, Hh, Ww, separated_packed, masks_packed, 0,
                   static_cast<cudaStream_t>(cuda_stream), false, true, lengths, frame_lengths))
     return 1;
-  CUDA_OK(cudaEventSynchronize(h->slot[0].ev_end));
+  CUDA_OK(cudaEventSynchronize(h->slot[0].ev_end.get()));
   return 0;
 }
 
@@ -1395,9 +1385,9 @@ int avsep_forward_host_packed_async(avsep_handle* h, const float* mixed_packed, 
 int avsep_host_wait(avsep_handle* h, int32_t slot) {
   if (!h) return 1;
   if (slot < 0 || slot >= AVSEP_HOST_SLOTS) return fail(h, "avsep_host_wait: slot must be 0 .. AVSEP_HOST_SLOTS - 1");
-  if (h->slot[slot].ev_end == nullptr) return 0;       // nothing was ever submitted on this slot
+  if (!h->slot[slot].ev_end) return 0;       // nothing was ever submitted on this slot
   CUDA_OK(cudaSetDevice(h->cfg.device));
-  CUDA_OK(cudaEventSynchronize(h->slot[slot].ev_end));
+  CUDA_OK(cudaEventSynchronize(h->slot[slot].ev_end.get()));
   return 0;
 }
 
@@ -1415,15 +1405,11 @@ int avsep_synth_batch(avsep_handle* h, const avsep_synth_config* cfg, int32_t B,
   p.mixed_spec = mixed_spec; p.lip_frames = lip_frames; p.clean_specs = clean_specs;
   if (p.S < 1 || p.n < 1) return fail(h, "avsep_synth_batch: bad geometry");
   const size_t need = static_cast<size_t>(B) * (p.S + 1) * p.n;
-  if (h->synth_cap < need) {
-    if (h->synth_waves) cudaFree(h->synth_waves);
-    h->synth_waves = nullptr; h->synth_cap = 0;
-    CUDA_OK(cudaMalloc(&h->synth_waves, need * sizeof(float)));
-    h->synth_cap = need;
-  }
-  p.waves = h->synth_waves;
+  if (h->synth_waves.cap < need) CUDA_OK(h->synth_waves.alloc(need));
+  p.waves = h->synth_waves.get();
   h->launches = 0;
-  CK(launch_synth(static_cast<cudaStream_t>(cuda_stream), p));
+  const cudaStream_t s = static_cast<cudaStream_t>(cuda_stream);
+  CK(s, launch_synth, p);
   h->launches = 3;
   return 0;
 }
@@ -1435,8 +1421,8 @@ int avsep_eval_snr(avsep_handle* h, const float* separated, const float* targets
   if (!separated || !targets) return fail(h, "avsep_eval_snr: null argument");
   if (B < 1 || F < 1 || T < 1) return fail(h, "avsep_eval_snr: empty problem");
   CUDA_OK(cudaSetDevice(h->cfg.device));
-  CK(launch_eval_snr(static_cast<cudaStream_t>(cuda_stream), separated, targets, mixed, B, S, F * T, input_snr,
-                     output_snr, best_perm, si_snr));
+  const cudaStream_t s = static_cast<cudaStream_t>(cuda_stream);
+  CK(s, launch_eval_snr, separated, targets, mixed, B, S, F * T, input_snr, output_snr, best_perm, si_snr);
   h->launches = 1;
   return 0;
 }
@@ -1454,8 +1440,8 @@ int avsep_stft_varlen(avsep_handle* h, const float* waves, const int32_t* length
   if (!fft_geometry_ok(n_fft, hop_length))
     return fail(h, "stft: n_fft must be a power of two in [8, 2048], 1 <= hop <= n_fft");
   CUDA_OK(cudaSetDevice(h->cfg.device));
-  CK(launch_stft(static_cast<cudaStream_t>(cuda_stream), waves, lengths, B, 0, L, n_fft, hop_length, spec, mag, nullptr,
-                 frame_lengths_out));
+  const cudaStream_t s = static_cast<cudaStream_t>(cuda_stream);
+  CK(s, launch_stft, waves, lengths, B, 0, L, n_fft, hop_length, spec, mag, nullptr, frame_lengths_out);
   h->launches = 1;
   return 0;
 }
@@ -1471,8 +1457,8 @@ int avsep_istft_varlen(avsep_handle* h, const float* spec, const float* masks, c
   if (!h) return 1;
   if (!spec || !waves) return fail(h, "avsep_istft: null argument");
   CUDA_OK(cudaSetDevice(h->cfg.device));
-  CK(launch_istft_masked(static_cast<cudaStream_t>(cuda_stream), spec, masks, lengths, B, S, T, n_fft, hop_length, L,
-                         waves));
+  const cudaStream_t s = static_cast<cudaStream_t>(cuda_stream);
+  CK(s, launch_istft_masked, spec, masks, lengths, B, S, T, n_fft, hop_length, L, waves);
   h->launches = 1;
   return 0;
 }
@@ -1600,14 +1586,14 @@ int avsep_audio_encoder(avsep_handle* h, const float* mixed_spec, int32_t B, int
   if (!mixed_spec || !out_BTd) return fail(h, "avsep_audio_encoder: null buffer");
   if (check_shape(h, B, T, 1, 1, 1)) return 1;
   CUDA_OK(cudaSetDevice(h->cfg.device));
-  cudaStream_t s = static_cast<cudaStream_t>(cuda_stream);
+  const LaunchCtx lc = launch_ctx(h, static_cast<cudaStream_t>(cuda_stream));
   Workspace w;
   if (get_workspace(h, w, nullptr, 0, B, T, 1, 1, 1)) return 1;
   const int d = h->cfg.d_model, Ma = B * T;
   h->launches = 0;
-  if (audio_frontend(h, s, w, mixed_spec, Plan{})) return 1;
-  if (encoder_stack(h, s, h->enc_a, B, T, w.x_a, w.y_a, w.a_op, w.qkv_a, w.attn_a, w.ffn_a, nullptr, nullptr)) return 1;
-  CUDA_OK(cudaMemcpyAsync(out_BTd, w.x_a, static_cast<size_t>(Ma) * d * 4, cudaMemcpyDeviceToDevice, s));
+  if (audio_frontend(h, lc, w, mixed_spec, Plan{})) return 1;
+  if (encoder_stack(h, lc, h->enc_a, B, T, w.x_a, w.y_a, w.a_op, w.qkv_a, w.attn_a, w.ffn_a, nullptr, nullptr)) return 1;
+  CUDA_OK(cudaMemcpyAsync(out_BTd, w.x_a, static_cast<size_t>(Ma) * d * 4, cudaMemcpyDeviceToDevice, lc.stream));
   return 0;
 }
 
@@ -1618,14 +1604,14 @@ int avsep_visual_encoder(avsep_handle* h, const float* lip_frames, int32_t B, in
   if (check_shape(h, B, 1, N, Hh, Ww)) return 1;
   if (target_len < 1) return fail(h, "avsep_visual_encoder: target_len must be >= 1");
   CUDA_OK(cudaSetDevice(h->cfg.device));
-  cudaStream_t s = static_cast<cudaStream_t>(cuda_stream);
+  const LaunchCtx lc = launch_ctx(h, static_cast<cudaStream_t>(cuda_stream));
   Workspace w;
   if (get_workspace(h, w, nullptr, 0, B, 1, N, Hh, Ww)) return 1;
   const int d = h->cfg.d_model;
   h->launches = 0;
-  if (visual_frontend(h, s, w, lip_frames, Plan{})) return 1;
-  if (encoder_stack(h, s, h->enc_v, B, N, w.x_v, w.y_v, w.v_op, w.qkv_v, w.attn_v, w.ffn_v, nullptr, nullptr)) return 1;
-  interp_rows_kernel<<<dim3(target_len, B), 128, 0, s>>>(w.x_v, out_BTd, N, target_len, d);
+  if (visual_frontend(h, lc, w, lip_frames, Plan{})) return 1;
+  if (encoder_stack(h, lc, h->enc_v, B, N, w.x_v, w.y_v, w.v_op, w.qkv_v, w.attn_v, w.ffn_v, nullptr, nullptr)) return 1;
+  interp_rows_kernel<<<dim3(target_len, B), 128, 0, lc.stream>>>(w.x_v, out_BTd, N, target_len, d);
   CUDA_OK(cudaGetLastError());
   ++h->launches;
   return 0;
@@ -1638,21 +1624,23 @@ int avsep_fusion(avsep_handle* h, const float* audio_BTd, const float* visual_BL
   if (check_shape(h, B, T, L, 1, 1)) return 1;
   if (L != T) return fail(h, "avsep_fusion: audio and visual must have the same length (model.py:131-133)");
   CUDA_OK(cudaSetDevice(h->cfg.device));
-  cudaStream_t s = static_cast<cudaStream_t>(cuda_stream);
+  const LaunchCtx lc = launch_ctx(h, static_cast<cudaStream_t>(cuda_stream));
   Workspace w;
   if (get_workspace(h, w, nullptr, 0, B, T, L, 1, 1)) return 1;
   const int d = h->cfg.d_model, Ma = B * T, Mv = B * L, prec = h->cfg.precision;
   h->launches = 0;
-  CUDA_OK(cudaMemcpyAsync(w.x_a, audio_BTd, static_cast<size_t>(Ma) * d * 4, cudaMemcpyDeviceToDevice, s));
-  CKL("add_layernorm", launch_add_layernorm(s, prec, w.x_a, nullptr, h->fus[0].n1g, h->fus[0].n1b, nullptr, w.a_op, Ma, d));
-  CKL("add_layernorm", launch_add_layernorm(s, prec, visual_BLd, nullptr, nullptr, nullptr, nullptr, w.v_op, Mv, d));   // cast only
+  CUDA_OK(cudaMemcpyAsync(w.x_a, audio_BTd, static_cast<size_t>(Ma) * d * 4, cudaMemcpyDeviceToDevice, lc.stream));
+  CKL("add_layernorm", lc, launch_add_layernorm, prec, w.x_a, nullptr, h->fus[0].n1g, h->fus[0].n1b, nullptr, w.a_op,
+      Ma, d);
+  // cast only
+  CKL("add_layernorm", lc, launch_add_layernorm, prec, visual_BLd, nullptr, nullptr, nullptr, nullptr, w.v_op, Mv, d);
   const bool dbg = h->debug;
   h->debug = false;
-  const int rc = fusion_stack(h, s, w, L);   // identity interpolation (L == T)
+  const int rc = fusion_stack(h, lc, w, L);   // identity interpolation (L == T)
   h->debug = dbg;
   if (rc) return 1;
   // fused rows in fp32: recompute the final LayerNorm from the fp32 residual stream straight into the caller's buffer
-  CKL("add_layernorm", launch_add_layernorm(s, PREC_TF32, w.x_a, nullptr, h->fng, h->fnb, nullptr, out_BTd, Ma, d));
+  CKL("add_layernorm", lc, launch_add_layernorm, PREC_TF32, w.x_a, nullptr, h->fng, h->fnb, nullptr, out_BTd, Ma, d);
   return 0;
 }
 
@@ -1662,13 +1650,14 @@ int avsep_decoder(avsep_handle* h, const float* fused_BTd, const float* mixed_sp
   if (!fused_BTd || !mixed_spec || !separated || !masks) return fail(h, "avsep_decoder: null buffer");
   if (check_shape(h, B, T, 1, 1, 1)) return 1;
   CUDA_OK(cudaSetDevice(h->cfg.device));
-  cudaStream_t s = static_cast<cudaStream_t>(cuda_stream);
+  const LaunchCtx lc = launch_ctx(h, static_cast<cudaStream_t>(cuda_stream));
   Workspace w;
   if (get_workspace(h, w, nullptr, 0, B, T, 1, 1, 1)) return 1;
   const int d = h->cfg.d_model, Ma = B * T;
   h->launches = 0;
-  CKL("add_layernorm", launch_add_layernorm(s, h->cfg.precision, fused_BTd, nullptr, nullptr, nullptr, nullptr, w.a_op, Ma, d));
-  return decoder_stage(h, s, w, mixed_spec, separated, masks);
+  CKL("add_layernorm", lc, launch_add_layernorm, h->cfg.precision, fused_BTd, nullptr, nullptr, nullptr, nullptr,
+      w.a_op, Ma, d);
+  return decoder_stage(h, lc, w, mixed_spec, separated, masks);
 }
 
 // ---- debug ---------------------------------------------------------------------------------------
@@ -1682,18 +1671,18 @@ int avsep_debug_get_stage(avsep_handle* h, const char* name, float* host_out, si
   if (!h || !name || !count) return fail(h, "avsep_debug_get_stage: bad argument");
   auto it = h->snaps.find(name);
   if (it == h->snaps.end()) return fail(h, std::string("no snapshot named ") + name);
-  *count = it->second.second;
+  const auto& snap = it->second;
+  *count = snap.count;
   if (host_out == nullptr) return 0;
-  if (capacity < it->second.second) return fail(h, "avsep_debug_get_stage: buffer too small");
+  if (capacity < snap.count) return fail(h, "avsep_debug_get_stage: buffer too small");
   CUDA_OK(cudaDeviceSynchronize());
-  CUDA_OK(cudaMemcpy(host_out, it->second.first, it->second.second * sizeof(float), cudaMemcpyDeviceToHost));
+  CUDA_OK(cudaMemcpy(host_out, snap.buf.get(), snap.count * sizeof(float), cudaMemcpyDeviceToHost));
   return 0;
 }
 
 int avsep_set_profile(avsep_handle* h, int32_t enable) {
   if (!h) return 1;
   h->profile = enable != 0;
-  pdl_set(h->pdl && !h->profile);   // per-launch event pairs measure kernels one at a time
   return 0;
 }
 
@@ -1704,7 +1693,7 @@ int avsep_profile_report(avsep_handle* h, char* buf, size_t capacity, int32_t re
   CUDA_OK(cudaDeviceSynchronize());
   for (auto& mk : h->ev_marks) {
     float ms = 0.f;
-    if (cudaEventElapsedTime(&ms, h->ev_pool[mk.second], h->ev_pool[mk.second + 1]) == cudaSuccess) {
+    if (cudaEventElapsedTime(&ms, h->ev_pool[mk.second].get(), h->ev_pool[mk.second + 1].get()) == cudaSuccess) {
       auto& slot = h->prof[mk.first];
       slot.first += 1;
       slot.second += ms;
@@ -1731,7 +1720,8 @@ int avsep_test_gemm(avsep_handle* h, const void* A, const void* W, const float* 
   const GemmProblem p = dense(A, M, K, W, N);
   GemmEpilogue e;
   e.bias = bias; e.act = act; e.out_f32 = out; e.ld_f32 = N;
-  CK(launch_gemm(static_cast<cudaStream_t>(cuda_stream), h->cfg.precision, p, e, h->num_sms, force_bn));
+  const LaunchCtx lc = launch_ctx(h, static_cast<cudaStream_t>(cuda_stream));
+  CK(lc, launch_gemm, h->cfg.precision, p, e, h->num_sms, force_bn);
   return 0;
 }
 
@@ -1745,7 +1735,8 @@ int avsep_test_gemm_ln(avsep_handle* h, const void* A, const void* W, const floa
   e.kind = EPI_LN;
   e.bias = bias; e.resid = x; e.out_f32 = x; e.ld_f32 = N; e.ln_gamma = gamma; e.ln_beta = beta;
   e.out_op = out_op; e.ld_op = N;
-  CK(launch_gemm(static_cast<cudaStream_t>(cuda_stream), h->cfg.precision, p, e, h->num_sms));
+  const LaunchCtx lc = launch_ctx(h, static_cast<cudaStream_t>(cuda_stream));
+  CK(lc, launch_gemm, h->cfg.precision, p, e, h->num_sms);
   return 0;
 }
 
@@ -1778,7 +1769,8 @@ int avsep_test_gemm_trace(avsep_handle* h, const void* A, const void* W, const f
     e.out_op = out_op; e.ld_op = N;
     e.out_f32 = out_op ? nullptr : x_or_out; e.ld_f32 = N;
   }
-  CK(launch_gemm(static_cast<cudaStream_t>(cuda_stream), h->cfg.precision, p, e, h->num_sms, 0, trace_dev));
+  const LaunchCtx lc = launch_ctx(h, static_cast<cudaStream_t>(cuda_stream));
+  CK(lc, launch_gemm, h->cfg.precision, p, e, h->num_sms, 0, trace_dev);
   return 0;
 }
 
@@ -1787,8 +1779,8 @@ int avsep_test_ffn_fused(avsep_handle* h, const void* a, const void* w1, const f
                          const float* b2, int32_t act, float* x_inout, const float* gamma, const float* beta,
                          void* out_op, int32_t M, void* cuda_stream) {
   if (!h) return 1;
-  CK(launch_ffn_fused(static_cast<cudaStream_t>(cuda_stream), a, w1, b1, w2, b2, act,
-                                                             x_inout, x_inout, gamma, beta, out_op, M, h->num_sms, nullptr));
+  const LaunchCtx lc = launch_ctx(h, static_cast<cudaStream_t>(cuda_stream));
+  CK(lc, launch_ffn_fused, a, w1, b1, w2, b2, act, x_inout, x_inout, gamma, beta, out_op, M, h->num_sms, nullptr);
   return 0;
 }
 
@@ -1798,8 +1790,8 @@ int avsep_test_ffn_fused_trace(avsep_handle* h, const void* a, const void* w1, c
                                const float* b2, int32_t act, float* x_inout, const float* gamma, const float* beta,
                                void* out_op, int32_t M, unsigned long long* trace_dev, void* cuda_stream) {
   if (!h) return 1;
-  CK(launch_ffn_fused(static_cast<cudaStream_t>(cuda_stream), a, w1, b1, w2, b2, act,
-                                                             x_inout, x_inout, gamma, beta, out_op, M, h->num_sms, trace_dev));
+  const LaunchCtx lc = launch_ctx(h, static_cast<cudaStream_t>(cuda_stream));
+  CK(lc, launch_ffn_fused, a, w1, b1, w2, b2, act, x_inout, x_inout, gamma, beta, out_op, M, h->num_sms, trace_dev);
   return 0;
 }
 
@@ -1818,8 +1810,7 @@ int avsep_test_xformer_stack(avsep_handle* h, int32_t which, const float* x_in, 
   sp.x_in = x_in; sp.out_x = out_x; sp.out_op = out_op; sp.kv = kv; sp.B = B; sp.L = L; sp.trace = trace_dev;
   if (final_ln && which == 0) { sp.fin_gamma = h->fus[0].n1g; sp.fin_beta = h->fus[0].n1b; }
   if (final_ln && which == 2) { sp.fin_gamma = h->fng; sp.fin_beta = h->fnb; }
-  h->prof_stream = static_cast<cudaStream_t>(cuda_stream);
-  return run_stack(h, static_cast<cudaStream_t>(cuda_stream), which, sp);
+  return run_stack(h, launch_ctx(h, static_cast<cudaStream_t>(cuda_stream)), which, sp);
 }
 
 int avsep_test_fusion_decoder(avsep_handle* h, const float* x_in, const void* kv, int32_t B, int32_t L, const float* mixed,
@@ -1832,15 +1823,14 @@ int avsep_test_fusion_decoder(avsep_handle* h, const float* x_in, const void* kv
   StackProblem sp{};
   sp.x_in = x_in; sp.fin_gamma = h->fng; sp.fin_beta = h->fnb; sp.kv = kv; sp.B = B; sp.L = L; sp.trace = trace_dev;
   sp.mixed = mixed; sp.separated = separated; sp.masks = masks;
-  h->prof_stream = static_cast<cudaStream_t>(cuda_stream);
-  return run_stack(h, static_cast<cudaStream_t>(cuda_stream), 2, sp);
+  return run_stack(h, launch_ctx(h, static_cast<cudaStream_t>(cuda_stream)), 2, sp);
 }
 
 int avsep_set_option(avsep_handle* h, const char* name, int32_t value) {
   if (!h || !name) return 1;
   if (strcmp(name, "host_chunk") == 0) { h->host_chunk = value; return 0; }
   if (strcmp(name, "host_lanes") == 0) { h->host_lanes = value; return 0; }
-  if (strcmp(name, "pdl") == 0) { h->pdl = value != 0; pdl_set(h->pdl && !h->profile); drop_graphs(h); return 0; }
+  if (strcmp(name, "pdl") == 0) { h->pdl = value != 0; drop_graphs(h); return 0; }
   if (strcmp(name, "use_graph") == 0) { h->use_graph = value != 0; return 0; }
   if (strcmp(name, "two_stream") == 0) { h->two_stream = value != 0; drop_graphs(h); return 0; }
   if (strcmp(name, "attn_tc") == 0) { h->attn_tc = value; drop_graphs(h); return 0; }
@@ -1857,7 +1847,8 @@ int avsep_test_conv1d(avsep_handle* h, const void* A_padded, const void* W3, con
   p.taps = 3; p.tap_stride = K; p.row_shift = -1;
   GemmEpilogue e;
   e.bias = bias; e.rowmap = ROW_PAD2COMPACT; e.Lp = L + 2; e.out_f32 = out; e.ld_f32 = N;
-  CK(launch_gemm(static_cast<cudaStream_t>(cuda_stream), h->cfg.precision, p, e, h->num_sms));
+  const LaunchCtx lc = launch_ctx(h, static_cast<cudaStream_t>(cuda_stream));
+  CK(lc, launch_gemm, h->cfg.precision, p, e, h->num_sms);
   return 0;
 }
 
@@ -1867,22 +1858,23 @@ int avsep_test_attention(avsep_handle* h, const void* q, const void* k, const vo
   AttnProblem ap{};
   ap.q = q; ap.ldq = H * hd; ap.k = k; ap.v = v; ap.ldkv = H * hd; ap.out = out; ap.ldo = H * hd;
   ap.B = B; ap.H = H; ap.hd = hd; ap.Lq = Lq; ap.Lk = Lk; ap.lerp_src = lerp_src; ap.tc_mode = h->attn_tc;
-  cudaStream_t s = static_cast<cudaStream_t>(cuda_stream);
-  void* scratch = nullptr;
+  const LaunchCtx lc = launch_ctx(h, static_cast<cudaStream_t>(cuda_stream));
+  Buf<__nv_bfloat16> scratch;
   if (lerp_src > 0) {   // same routing as fusion_stack: K then V columns side by side in one interpolated buffer
     AttnProblem tp = ap;
     tp.lerp_src = 0; tp.ldkv = 2 * H * hd;
     if (attention_tc_wanted(h->cfg.precision, tp)) {
       const int dm = H * hd;
-      if (cudaMalloc(&scratch, static_cast<size_t>(B) * Lk * 2 * dm * 2) != cudaSuccess) return fail(h, "test_attention: cudaMalloc failed");
-      tp.k = scratch; tp.v = static_cast<__nv_bfloat16*>(scratch) + dm;
-      CK(launch_lerp_rows(s, static_cast<const float*>(k), dm, B, lerp_src, Lk, dm, scratch, 2 * dm));
-      CK(launch_lerp_rows(s, static_cast<const float*>(v), dm, B, lerp_src, Lk, dm, static_cast<__nv_bfloat16*>(scratch) + dm, 2 * dm));
+      if (scratch.alloc(static_cast<size_t>(B) * Lk * 2 * dm) != cudaSuccess)
+        return fail(h, "test_attention: cudaMalloc failed");
+      tp.k = scratch.get(); tp.v = scratch.get() + dm;
+      CK(lc, launch_lerp_rows, static_cast<const float*>(k), dm, B, lerp_src, Lk, dm, scratch.get(), 2 * dm);
+      CK(lc, launch_lerp_rows, static_cast<const float*>(v), dm, B, lerp_src, Lk, dm, scratch.get() + dm, 2 * dm);
       ap = tp;
     }
   }
-  const char* err = launch_attention(s, h->cfg.precision, ap);
-  if (scratch) { cudaStreamSynchronize(s); cudaFree(scratch); }
+  const char* err = launch_attention(lc, h->cfg.precision, ap);
+  if (scratch.get()) cudaStreamSynchronize(lc.stream);   // before scratch is freed
   if (err) return fail(h, err);
   return 0;
 }
@@ -1890,7 +1882,8 @@ int avsep_test_attention(avsep_handle* h, const void* q, const void* k, const vo
 int avsep_test_add_layernorm(avsep_handle* h, const float* x, const float* y, const float* gamma, const float* beta,
                              float* x_out, void* out_op, int32_t M, int32_t d, void* cuda_stream) {
   if (!h) return 1;
-  CKL("add_layernorm", launch_add_layernorm(static_cast<cudaStream_t>(cuda_stream), h->cfg.precision, x, y, gamma, beta, x_out, out_op, M, d));
+  const LaunchCtx lc = launch_ctx(h, static_cast<cudaStream_t>(cuda_stream));
+  CKL("add_layernorm", lc, launch_add_layernorm, h->cfg.precision, x, y, gamma, beta, x_out, out_op, M, d);
   return 0;
 }
 
@@ -1898,7 +1891,8 @@ int avsep_test_visual_cnn(avsep_handle* h, const float* frames, int32_t M, int32
                           void* cuda_stream) {
   if (!h) return 1;
   if (!h->finalized) return fail(h, "weights not finalized");
-  CK(run_visual_cnn(h, static_cast<cudaStream_t>(cuda_stream), frames, M, Hh, Ww, pooled));
+  const LaunchCtx lc = launch_ctx(h, static_cast<cudaStream_t>(cuda_stream));
+  CK(lc, run_visual_cnn, h, frames, M, Hh, Ww, pooled);
   return 0;
 }
 
@@ -1907,7 +1901,8 @@ int avsep_test_visual_cnn_trace(avsep_handle* h, const float* frames, int32_t M,
                                 unsigned long long* trace_dev, void* cuda_stream) {
   if (!h) return 1;
   if (!h->finalized) return fail(h, "weights not finalized");
-  CK(run_visual_cnn(h, static_cast<cudaStream_t>(cuda_stream), frames, M, 32, 32, pooled, trace_dev));
+  const LaunchCtx lc = launch_ctx(h, static_cast<cudaStream_t>(cuda_stream));
+  CK(lc, run_visual_cnn, h, frames, M, 32, 32, pooled, trace_dev);
   return 0;
 }
 

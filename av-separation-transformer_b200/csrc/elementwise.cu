@@ -6,13 +6,6 @@
 namespace avsep {
 
 namespace {
-bool g_pdl = true;
-}
-void pdl_set(bool on) { g_pdl = on; }
-bool pdl_enabled() { return g_pdl; }
-
-
-namespace {
 
 constexpr int LN_WARPS = 8;
 constexpr int LN_MAX_V4 = 8;   // float4 chunks cached per lane: d <= 8*32*4 = 1024
@@ -150,23 +143,23 @@ prep_audio_kernel(const float* __restrict__ mixed, void* __restrict__ xp, int F,
 
 }  // namespace
 
-const char* launch_add_layernorm(cudaStream_t s, int prec, const float* x, const float* y, const float* gamma,
+const char* launch_add_layernorm(LaunchCtx lc, int prec, const float* x, const float* y, const float* gamma,
                                  const float* beta, float* x_out, void* out_op, int M, int d) {
   if ((d & 3) != 0 || d > LN_MAX_V4 * 128) return "layernorm: d_model must be a multiple of 4 and <= 1024";
   if (M <= 0) return "layernorm: empty";
   dim3 grid((M + LN_WARPS - 1) / LN_WARPS);
   if (prec == PREC_TF32)
-    launch_pdl(add_layernorm_kernel<true>, dim3(grid), dim3(LN_WARPS * 32), 0, s, x, y, gamma, beta, x_out, out_op, M, d);
+    launch_pdl(add_layernorm_kernel<true>, dim3(grid), dim3(LN_WARPS * 32), 0, lc, x, y, gamma, beta, x_out, out_op, M, d);
   else
-    launch_pdl(add_layernorm_kernel<false>, dim3(grid), dim3(LN_WARPS * 32), 0, s, x, y, gamma, beta, x_out, out_op, M, d);
+    launch_pdl(add_layernorm_kernel<false>, dim3(grid), dim3(LN_WARPS * 32), 0, lc, x, y, gamma, beta, x_out, out_op, M, d);
   return cudaGetLastError() == cudaSuccess ? nullptr : "layernorm: launch failed";
 }
 
-const char* launch_prep_audio(cudaStream_t s, int prec, const float* mixed, void* xp, int B, int F, int T, int Fp,
+const char* launch_prep_audio(LaunchCtx lc, int prec, const float* mixed, void* xp, int B, int F, int T, int Fp,
                               const int* lens) {
   dim3 grid((T + 31) / 32, (Fp + 31) / 32, B);
-  if (prec == PREC_TF32) launch_pdl(prep_audio_kernel<true>, grid, dim3(256), 0, s, mixed, xp, F, T, Fp, lens);
-  else launch_pdl(prep_audio_kernel<false>, grid, dim3(256), 0, s, mixed, xp, F, T, Fp, lens);
+  if (prec == PREC_TF32) launch_pdl(prep_audio_kernel<true>, grid, dim3(256), 0, lc, mixed, xp, F, T, Fp, lens);
+  else launch_pdl(prep_audio_kernel<false>, grid, dim3(256), 0, lc, mixed, xp, F, T, Fp, lens);
   return cudaGetLastError() == cudaSuccess ? nullptr : "prep_audio: launch failed";
 }
 

@@ -390,7 +390,7 @@ bool ffn_fusable(int prec, int d_model) { return prec == PREC_BF16 && d_model ==
 
 // a [M,256] bf16; w1 [1024,256] bf16; w2 [256,1024] bf16; x [M,256] fp32 (residual in, x' out, in place) or null
 // residual with x_out; out_op [M,256] bf16 (LayerNorm(x') or cast when gamma == null).
-const char* launch_ffn_fused(cudaStream_t s, const void* a, const void* w1, const float* b1, const void* w2,
+const char* launch_ffn_fused(LaunchCtx lc, const void* a, const void* w1, const float* b1, const void* w2,
                              const float* b2, int act, const float* resid, float* x_out, const float* gamma,
                              const float* beta, void* out_op, int M, int num_sms, unsigned long long* trace) {
   if (M <= 0) return "ffn_fused: empty problem";
@@ -411,7 +411,7 @@ const char* launch_ffn_fused(cudaStream_t s, const void* a, const void* w1, cons
   d.trace = trace;
   const int m_tiles = (M + 127) / 128;
   const int grid = m_tiles < num_sms ? m_tiles : num_sms;
-  if (launch_pdl(ffn_fused_kernel, dim3(grid), dim3(FFN_THREADS), FFN_SMEM, s, ta, tw1, tw2, tx, top, d) != cudaSuccess) {
+  if (launch_pdl(ffn_fused_kernel, dim3(grid), dim3(FFN_THREADS), FFN_SMEM, lc, ta, tw1, tw2, tx, top, d) != cudaSuccess) {
     cudaGetLastError();
     return "ffn_fused: launch failed";
   }

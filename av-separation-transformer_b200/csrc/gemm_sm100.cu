@@ -911,13 +911,13 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
 // host side
 // ------------------------------------------------------------------------------------------
 template <int EPI, bool TF32>
-const char* launch_cfg(cudaStream_t s, const CUtensorMap& ta, const CUtensorMap& tw, const CUtensorMap& top,
+const char* launch_cfg(LaunchCtx lc, const CUtensorMap& ta, const CUtensorMap& tw, const CUtensorMap& top,
                        const CUtensorMap& tf32m, const GemmDev& d, int num_sms) {
   auto kern = gemm_tcgen05_kernel<EPI, TF32>;
   if (!smem_opt_in(kern, SMEM_TOTAL)) return "gemm: cannot raise the shared-memory limit";
   const int tiles = ((d.M + BM - 1) / BM) * ((d.N + d.n_tile - 1) / d.n_tile);
   const int grid = tiles < num_sms ? tiles : num_sms;
-  if (launch_pdl(kern, dim3(grid), dim3(NUM_THREADS), SMEM_TOTAL, s, ta, tw, top, tf32m, d) != cudaSuccess) {
+  if (launch_pdl(kern, dim3(grid), dim3(NUM_THREADS), SMEM_TOTAL, lc, ta, tw, top, tf32m, d) != cudaSuccess) {
     cudaGetLastError();
     return "gemm: kernel launch failed";
   }
@@ -928,7 +928,7 @@ const char* launch_cfg(cudaStream_t s, const CUtensorMap& ta, const CUtensorMap&
 
 bool gemm_ln_fusable(int N) { return N <= BN_MAX && N >= 32 && (N % 32) == 0; }
 
-const char* launch_gemm(cudaStream_t s, int prec, const GemmProblem& p, const GemmEpilogue& e, int num_sms,
+const char* launch_gemm(LaunchCtx lc, int prec, const GemmProblem& p, const GemmEpilogue& e, int num_sms,
                         int force_bn, unsigned long long* trace) {
   if (p.M <= 0 || p.N <= 0 || p.K <= 0) return "gemm: empty problem";
   const bool tf32 = (prec == PREC_TF32);
@@ -985,11 +985,11 @@ const char* launch_gemm(cudaStream_t s, int prec, const GemmProblem& p, const Ge
   }
   d.use_tma = use_tma ? 1 : 0;
   switch (e.kind) {
-    case EPI_STD: return tf32 ? launch_cfg<EPI_STD, true>(s, ta, tw, top, tf32m, d, num_sms) : launch_cfg<EPI_STD, false>(s, ta, tw, top, tf32m, d, num_sms);
-    case EPI_TAIL: return tf32 ? launch_cfg<EPI_TAIL, true>(s, ta, tw, top, tf32m, d, num_sms) : launch_cfg<EPI_TAIL, false>(s, ta, tw, top, tf32m, d, num_sms);
+    case EPI_STD: return tf32 ? launch_cfg<EPI_STD, true>(lc, ta, tw, top, tf32m, d, num_sms) : launch_cfg<EPI_STD, false>(lc, ta, tw, top, tf32m, d, num_sms);
+    case EPI_TAIL: return tf32 ? launch_cfg<EPI_TAIL, true>(lc, ta, tw, top, tf32m, d, num_sms) : launch_cfg<EPI_TAIL, false>(lc, ta, tw, top, tf32m, d, num_sms);
     case EPI_LN:
-      if (use_tma) return tf32 ? launch_cfg<EPI_LN_TMA, true>(s, ta, tw, top, tf32m, d, num_sms) : launch_cfg<EPI_LN_TMA, false>(s, ta, tw, top, tf32m, d, num_sms);
-      return tf32 ? launch_cfg<EPI_LN, true>(s, ta, tw, top, tf32m, d, num_sms) : launch_cfg<EPI_LN, false>(s, ta, tw, top, tf32m, d, num_sms);
+      if (use_tma) return tf32 ? launch_cfg<EPI_LN_TMA, true>(lc, ta, tw, top, tf32m, d, num_sms) : launch_cfg<EPI_LN_TMA, false>(lc, ta, tw, top, tf32m, d, num_sms);
+      return tf32 ? launch_cfg<EPI_LN, true>(lc, ta, tw, top, tf32m, d, num_sms) : launch_cfg<EPI_LN, false>(lc, ta, tw, top, tf32m, d, num_sms);
     default: return "gemm: unknown epilogue";
   }
 }

@@ -38,22 +38,25 @@ bool smem_opt_in(void (*kern)(KArgs...), int bytes) {
   return smem_opt_in(reinterpret_cast<const void*>(kern), bytes);
 }
 
-// Programmatic dependent launch (PDL) of the forward-path kernels: every kernel launched through launch_pdl calls
-// griddep_wait() before it touches anything its predecessor wrote.  pdl_set(false) = plain stream order.
-void pdl_set(bool on);
-bool pdl_enabled();
+// Where a forward-path kernel runs: its stream, and whether it may use programmatic dependent launch (PDL).  Every
+// kernel launched through launch_pdl calls griddep_wait() before it touches anything its predecessor wrote, so
+// pdl = false only means plain stream order.  The launching handle decides (its "pdl" option, off while it profiles).
+struct LaunchCtx {
+  cudaStream_t stream;
+  bool pdl;
+};
 template <typename... KArgs, typename... Args>
-inline cudaError_t launch_pdl(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t s, Args... args) {
+inline cudaError_t launch_pdl(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, LaunchCtx lc, Args... args) {
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = grid;
   cfg.blockDim = block;
   cfg.dynamicSmemBytes = smem;
-  cfg.stream = s;
+  cfg.stream = lc.stream;
   cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = pdl_enabled() ? 1 : 0;
+  cfg.numAttrs = lc.pdl ? 1 : 0;
   return cudaLaunchKernelEx(&cfg, kern, KArgs(args)...);
 }
 
@@ -140,13 +143,13 @@ __device__ __forceinline__ LerpTap lerp_tap(int t, int nsrc, float scale) {
 }
 
 // Returns nullptr on success or a static error string.
-const char* launch_gemm(cudaStream_t s, int prec, const GemmProblem& p, const GemmEpilogue& e, int num_sms,
+const char* launch_gemm(LaunchCtx lc, int prec, const GemmProblem& p, const GemmEpilogue& e, int num_sms,
                         int force_bn = 0, unsigned long long* trace = nullptr);   // trace: [grid][8] globaltimer stamps (debug)
 bool gemm_ln_fusable(int N);   // EPI_LN usable for this row width
 
 // Fused FFN sub-layer (d_model = 256, bf16): x += W2 act(W1 a + b1) + b2 ; out_op = LayerNorm(x)  (ffn_fused_sm100.cu)
 bool ffn_fusable(int prec, int d_model);
-const char* launch_ffn_fused(cudaStream_t s, const void* a, const void* w1, const float* b1, const void* w2,
+const char* launch_ffn_fused(LaunchCtx lc, const void* a, const void* w1, const float* b1, const void* w2,
                              const float* b2, int act, const float* resid, float* x_out, const float* gamma,
                              const float* beta, void* out_op, int M, int num_sms,
                              unsigned long long* trace = nullptr);
@@ -205,16 +208,16 @@ void xformer_pack_cross(const float* wq, const float* wo, const float* w1, const
                         uint8_t* dst);
 void xformer_pack_vecs(const float* bqkv, int n_bqkv, const float* bo, const float* b1, const float* b2, const float* n1g,
                        const float* n1b, const float* n2g, const float* n2b, float* dst, const float* b0 = nullptr);
-const char* launch_xformer_stack(cudaStream_t s, const StackProblem& p, int num_sms);
+const char* launch_xformer_stack(LaunchCtx lc, const StackProblem& p, int num_sms);
 
 // x_out = x + y (y may be null); out = LayerNorm(x_out) * gamma + beta (skipped when gamma == null, then out = x_out).
 // out_op is bf16 (PREC_BF16) or fp32 (PREC_TF32).
-const char* launch_add_layernorm(cudaStream_t s, int prec, const float* x, const float* y, const float* gamma,
+const char* launch_add_layernorm(LaunchCtx lc, int prec, const float* x, const float* y, const float* gamma,
                                  const float* beta, float* x_out, void* out_op, int M, int d);
 
 // mixed (B,F,T) fp32 -> Xp (B, T+2, Fp) operand precision, zero halo rows and zero pad columns; lens (or null):
 // rows t >= lens[b] are zero.
-const char* launch_prep_audio(cudaStream_t s, int prec, const float* mixed, void* xp, int B, int F, int T, int Fp,
+const char* launch_prep_audio(LaunchCtx lc, int prec, const float* mixed, void* xp, int B, int F, int T, int Fp,
                               const int* lens = nullptr);
 
 // SeparationDecoder.separate (model.py:210-220): out[b,s,f,t] = masks[b,s,f,t] * mixed[b,f,t] (peer_gather.cu).
@@ -226,9 +229,9 @@ const char* launch_separate(cudaStream_t s, const float* masks, const float* mix
 // clamps; null = all T / all N).  unpack: mixed_p (F, T_b) and frames_p (N_b, hw) blocks -> the valid regions of the
 // padded (B, F, T) / (B, N, hw) staging; pack: the valid regions of the padded (B, S, F, T) sep / masks -> their
 // (S, F, T_b) blocks.  Nothing past the lengths is read or written.
-const char* launch_unpack(cudaStream_t s, const float* mixed_p, const float* frames_p, const int* lens,
+const char* launch_unpack(LaunchCtx lc, const float* mixed_p, const float* frames_p, const int* lens,
                           const int* flens, int b0, int B, int F, int T, int N, int hw, float* mixed, float* frames);
-const char* launch_pack(cudaStream_t s, const float* sep, const float* masks, const int* lens, int b0, int B, int S,
+const char* launch_pack(LaunchCtx lc, const float* sep, const float* masks, const int* lens, int b0, int B, int S,
                         int F, int T, float* sep_p, float* masks_p);
 // Ticket flags of the masks-only gather: 32-bit words in this GPU's or a peer's memory, raised / awaited in stream order.
 struct FlagSet {
@@ -253,16 +256,16 @@ struct AttnProblem {
   const int* k_lens = nullptr;
   const int* src_lens = nullptr;
 };
-const char* launch_attention(cudaStream_t s, int prec, const AttnProblem& p);
+const char* launch_attention(LaunchCtx lc, int prec, const AttnProblem& p);
 // tcgen05 flash attention (attention_tc.cu): bf16, head dim 64, materialised K/V rows.  launch_attention dispatches
 // to it by itself when attention_tc_wanted.
 bool attention_tc_usable(int prec, const AttnProblem& p);
 bool attention_tc_wanted(int prec, const AttnProblem& p);      // usable and selected by p.tc_mode
-const char* launch_attention_tc(cudaStream_t s, const AttnProblem& p);
+const char* launch_attention_tc(LaunchCtx lc, const AttnProblem& p);
 // dst[b*L + t, 0:cols] (bf16) = linear interpolation (lerp_tap) of src rows [b*nsrc + i, 0:cols] (fp32), with the
 // scale of each utterance's own lengths: src_lens[b] source rows interpolated to dst_lens[b] rows (null: nsrc / L).
 // The rows past dst_lens[b] are finite filler.
-const char* launch_lerp_rows(cudaStream_t s, const float* src, int ld_src, int B, int nsrc, int L, int cols,
+const char* launch_lerp_rows(LaunchCtx lc, const float* src, int ld_src, int B, int nsrc, int L, int cols,
                              void* dst_bf16, int ld_dst, const int* src_lens = nullptr, const int* dst_lens = nullptr);
 
 struct CnnWeights {                // BN-folded, fragment-ordered (see visual_cnn.cu)
@@ -279,7 +282,7 @@ const char* launch_visual_cnn(cudaStream_t s, int prec, const float* frames, int
 size_t visual_cnn_tc_w2_bytes();
 size_t visual_cnn_tc_w3_bytes();
 void visual_cnn_tc_pack(const float* w2, const float* w3, uint8_t* w2_slabs, uint8_t* w3_rows);
-const char* launch_visual_cnn_tc(cudaStream_t s, const float* frames, int M, const CnnWeights& w, const uint8_t* w2_slabs,
+const char* launch_visual_cnn_tc(LaunchCtx lc, const float* frames, int M, const CnnWeights& w, const uint8_t* w2_slabs,
                                  const uint8_t* w3_rows, void* pooled, int num_sms,
                                  unsigned long long* trace = nullptr, const int* frame_lens = nullptr, int N = 1);
 size_t visual_cnn_pack_sizes(int which);   // elements of packed w1/w2/w3 (uint32)

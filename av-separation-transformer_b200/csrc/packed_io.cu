@@ -131,7 +131,7 @@ unsigned ctas_for(long long elems) { return static_cast<unsigned>((elems + PK_SP
 
 }  // namespace
 
-const char* launch_unpack(cudaStream_t s, const float* mixed_p, const float* frames_p, const int* lens,
+const char* launch_unpack(LaunchCtx lc, const float* mixed_p, const float* frames_p, const int* lens,
                           const int* flens, int b0, int B, int F, int T, int N, int hw, float* mixed, float* frames) {
   if (B <= 0) return nullptr;
   if (static_cast<long long>(F) * T > 0x7fffffffLL || static_cast<long long>(N) * hw > 0x7fffffffLL)
@@ -140,18 +140,18 @@ const char* launch_unpack(cudaStream_t s, const float* mixed_p, const float* fra
                    (reinterpret_cast<uintptr_t>(frames) & 15) == 0;
   const long long fr = static_cast<long long>(N) * hw / (vec ? 4 : 1);
   const dim3 grid(std::max(ctas_for(static_cast<long long>(F) * T), ctas_for(fr)), B);
-  const cudaError_t e = launch_pdl(vec ? unpack_kernel<true> : unpack_kernel<false>, grid, dim3(PK_THREADS), 0, s,
+  const cudaError_t e = launch_pdl(vec ? unpack_kernel<true> : unpack_kernel<false>, grid, dim3(PK_THREADS), 0, lc,
                                    mixed_p, frames_p, lens, flens, b0, F, T, N, hw, mixed, frames);
   return e == cudaSuccess ? nullptr : "unpack: launch failed";
 }
 
-const char* launch_pack(cudaStream_t s, const float* sep, const float* masks, const int* lens, int b0, int B, int S,
+const char* launch_pack(LaunchCtx lc, const float* sep, const float* masks, const int* lens, int b0, int B, int S,
                         int F, int T, float* sep_p, float* masks_p) {
   if (B <= 0) return nullptr;
   const long long SF = static_cast<long long>(S) * F;
   if (SF * T > 0x7fffffffLL) return "pack: utterance too large";
   const dim3 grid(ctas_for(SF * T), B);
-  const cudaError_t e = launch_pdl(pack_kernel, grid, dim3(PK_THREADS), 0, s, sep, masks, lens, b0,
+  const cudaError_t e = launch_pdl(pack_kernel, grid, dim3(PK_THREADS), 0, lc, sep, masks, lens, b0,
                                    static_cast<int>(SF), T, sep_p, masks_p);
   return e == cudaSuccess ? nullptr : "pack: launch failed";
 }

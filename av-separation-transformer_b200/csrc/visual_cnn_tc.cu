@@ -464,7 +464,7 @@ void visual_cnn_tc_pack(const float* w2, const float* w3, uint8_t* w2_slabs, uin
       for (int c = 0; c < 64; ++c) o[(static_cast<size_t>(t) * 128 + n) * 64 + c] = f2bf(w3[static_cast<size_t>(n) * 576 + t * 64 + c]);
 }
 
-const char* launch_visual_cnn_tc(cudaStream_t s, const float* frames, int M, const CnnWeights& w, const uint8_t* w2_slabs,
+const char* launch_visual_cnn_tc(LaunchCtx lc, const float* frames, int M, const CnnWeights& w, const uint8_t* w2_slabs,
                                  const uint8_t* w3_rows, void* pooled, int num_sms, unsigned long long* trace,
                                  const int* frame_lens, int N) {
   if (M <= 0) return "visual_cnn_tc: empty problem";
@@ -478,7 +478,7 @@ const char* launch_visual_cnn_tc(cudaStream_t s, const float* frames, int M, con
   d.trace = trace;
   d.frame_lens = frame_lens; d.N = N;
   const int grid = d.num_groups < num_sms ? d.num_groups : num_sms;
-  launch_pdl(visual_cnn_tc_kernel, dim3(grid), dim3(TC_THREADS), TC_SMEM, s, tm, d);
+  launch_pdl(visual_cnn_tc_kernel, dim3(grid), dim3(TC_THREADS), TC_SMEM, lc, tm, d);
   return cudaGetLastError() == cudaSuccess ? nullptr : "visual_cnn_tc: launch failed";
 }
 

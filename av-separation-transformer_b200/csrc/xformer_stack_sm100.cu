@@ -1424,7 +1424,7 @@ bool xformer_stack_usable(int prec, int d_model, int nhead, int len) {
   return prec == PREC_BF16 && d_model == D && nhead == NH && len >= 1 && len <= 128;
 }
 
-const char* launch_xformer_stack(cudaStream_t s, const StackProblem& sp, int num_sms) {
+const char* launch_xformer_stack(LaunchCtx lc, const StackProblem& sp, int num_sms) {
   if (sp.B <= 0 || sp.L <= 0 || sp.L > 128 || sp.n_layers <= 0) return "xformer_stack: bad problem";
   const bool decoder = sp.masks != nullptr;
   const bool pro = sp.pro_a != nullptr;
@@ -1483,7 +1483,7 @@ const char* launch_xformer_stack(cudaStream_t s, const StackProblem& sp, int num
   const int grid = n_tiles < num_sms ? n_tiles : num_sms;
   auto kern = (d.lens != nullptr || d.kvp_lens != nullptr) ? xformer_stack_kernel<true> : xformer_stack_kernel<false>;
   if (!smem_opt_in(kern, STACK_SMEM)) return "xformer_stack: cannot raise the shared-memory limit";
-  if (launch_pdl(kern, dim3(grid), dim3(STACK_THREADS), STACK_SMEM, s, tin, tout, top, tkv, d) !=
+  if (launch_pdl(kern, dim3(grid), dim3(STACK_THREADS), STACK_SMEM, lc, tin, tout, top, tkv, d) !=
       cudaSuccess) {
     cudaGetLastError();
     return "xformer_stack: launch failed";

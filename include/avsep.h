@@ -179,12 +179,12 @@ AVSEP_API int avsep_debug_get_stage(avsep_handle* h, const char* name, float* ho
  *                            (56 x 2 lanes for avsep_forward_host, 128 x 1 lane for avsep_forward_host_async)
  *   "profile_spin_us"        length of the GPU spin kernel that precedes a profiled forward
  * Any other name is an error.  The environment variable AVSEP_OPTS="name=value,name=value" applies options at
- * avsep_create (measurement runs).  "pdl" is process-wide: it applies to every handle of the process, not only to `h`;
- * every other option applies to `h` alone. */
+ * avsep_create (measurement runs).  Every option applies to `h` alone. */
 AVSEP_API int avsep_set_option(avsep_handle* h, const char* name, int32_t value);
 
-/* Per-kernel timing: when enabled every launch of the forward is bracketed by a cudaEvent pair on the launching
- * stream.  avsep_profile_report synchronises and writes one "label launches total_ms" line per kernel class. */
+/* Per-kernel timing of `h` alone: when enabled every launch of the forward is bracketed by a cudaEvent pair on the
+ * launching stream, and `h` launches without "pdl" so that each pair times one kernel.  avsep_profile_report
+ * synchronises and writes one "label launches total_ms" line per kernel class. */
 AVSEP_API int avsep_set_profile(avsep_handle* h, int32_t enable);
 AVSEP_API int avsep_profile_report(avsep_handle* h, char* buf, size_t capacity, int32_t reset);
 
