@@ -26,6 +26,11 @@ class EngineConfig:
     precision: str = "bf16"
 
 
+def _ptr(t):
+    """Device pointer of a tensor for the C ABI, NULL for None."""
+    return None if t is None else t.data_ptr()
+
+
 def _prec_code(p: str) -> int:
     if p in ("bf16", "bfloat16"):
         return _lib.PREC_BF16
@@ -128,9 +133,7 @@ class Engine:
             shp = (C.c_int64 * len(shape))(*shape)
             self._check(self.lib.avsep_set_weight(self.h, key.encode(), arr.ctypes.data_as(C.c_void_p),
                                                   _lib.DTYPE_F32, shp, len(shape)), "avsep_set_weight")
-        with torch.cuda.device(self.device):
-            stream = torch.cuda.current_stream().cuda_stream
-            self._check(self.lib.avsep_finalize_weights(self.h, C.c_void_p(stream)), "avsep_finalize_weights")
+        self._check(self.lib.avsep_finalize_weights(self.h, self._stream()), "avsep_finalize_weights")
 
     # ---- helpers ---------------------------------------------------------------------------------
     def _dev_f32(self, t: torch.Tensor, name: str) -> torch.Tensor:
@@ -235,9 +238,8 @@ class Engine:
         mixed = self._dev_f32(mixed, "mixed_spec")
         frames = self._dev_f32(frames, "lip_frames")
         B, T, N, Hh, Ww = self._check_inputs("forward", mixed=mixed, frames=frames, out=out)
-        with torch.cuda.device(self.device):
-            lens = self._lengths(lengths, "lengths", B, T)
-            flens = self._lengths(frame_lengths, "frame_lengths", B, N)
+        lens = self._lengths(lengths, "lengths", B, T)
+        flens = self._lengths(frame_lengths, "frame_lengths", B, N)
         F, S = self.cfg.freq_bins, self.cfg.num_speakers
         if out is None:
             # one allocation for both outputs: the caching allocator then recycles a handful of blocks, so the
@@ -249,21 +251,9 @@ class Engine:
             for t in out:
                 if not t.is_cuda or t.device.index != self.device:
                     raise ValueError(f"forward: output buffers must live on cuda:{self.device}")
-        if lens is None and flens is None:
-            fn, what = self.lib.avsep_forward, "avsep_forward"
-            args = (self.h, mixed.data_ptr(), frames.data_ptr(), B, T, N, Hh, Ww, sep.data_ptr(), masks.data_ptr(),
-                    None, 0, self._stream())
-        else:
-            fn, what = self.lib.avsep_forward_varlen, "avsep_forward_varlen"
-            args = (self.h, mixed.data_ptr(), frames.data_ptr(), None if lens is None else lens.data_ptr(),
-                    None if flens is None else flens.data_ptr(), B, T, N, Hh, Ww, sep.data_ptr(), masks.data_ptr(),
-                    None, 0, self._stream())
-        if torch.cuda.current_device() == self.device:      # the library selects its device itself; only restore the
-            rc = fn(*args)                                   # caller's when it differs
-        else:
-            with torch.cuda.device(self.device):
-                rc = fn(*args)
-        self._check(rc, what)
+        rc = self.lib.avsep_forward_varlen(self.h, mixed.data_ptr(), frames.data_ptr(), _ptr(lens), _ptr(flens), B, T, N,
+                                           Hh, Ww, sep.data_ptr(), masks.data_ptr(), None, 0, self._stream())
+        self._check(rc, "avsep_forward_varlen")
         return sep, masks
 
     @staticmethod
@@ -286,9 +276,8 @@ class Engine:
         self._check_inputs("forward_host", mixed=mixed, out=(sep, masks))
         if sep.is_cuda or masks.is_cuda:
             raise ValueError("forward_host: output buffers must be CPU tensors")
-        with torch.cuda.device(self.device):
-            rc = self.lib.avsep_forward_host(self.h, mixed.data_ptr(), frames.data_ptr(), B, T, N, Hh, Ww,
-                                             sep.data_ptr(), masks.data_ptr(), self._stream())
+        rc = self.lib.avsep_forward_host(self.h, mixed.data_ptr(), frames.data_ptr(), B, T, N, Hh, Ww, sep.data_ptr(),
+                                         masks.data_ptr(), self._stream())
         self._check(rc, "avsep_forward_host")
         return sep, masks
 
@@ -300,9 +289,8 @@ class Engine:
             if t.is_cuda or t.dtype != torch.float32 or not t.is_contiguous():
                 raise ValueError("forward_host_async: contiguous float32 CPU tensors required")
         B, T, N, Hh, Ww = self._check_inputs("forward_host_async", mixed=mixed, frames=frames, out=(sep, masks))
-        with torch.cuda.device(self.device):
-            rc = self.lib.avsep_forward_host_async(self.h, mixed.data_ptr(), frames.data_ptr(), B, T, N, Hh, Ww,
-                                                   sep.data_ptr(), masks.data_ptr(), int(slot), self._stream())
+        rc = self.lib.avsep_forward_host_async(self.h, mixed.data_ptr(), frames.data_ptr(), B, T, N, Hh, Ww,
+                                               sep.data_ptr(), masks.data_ptr(), int(slot), self._stream())
         self._check(rc, "avsep_forward_host_async")
 
     # ---- packed variable-length batches (include/avsep.h: utterances back to back, no padding) ------------------
@@ -369,12 +357,11 @@ class Engine:
         frames_p = self._dev_f32(frames_p, "frames_packed")
         B, T, N, Hh, Ww, lens, flens, (sep, masks) = self._packed_plan(what, mixed_p, frames_p, lengths, frame_lengths,
                                                                        max_len, max_frames, out, True)
-        with torch.cuda.device(self.device):
-            lens = self._lengths(lens, "lengths", B, T, what)
-            flens = self._lengths(flens, "frame_lengths", B, N, what)
-            rc = self.lib.avsep_forward_packed(self.h, mixed_p.data_ptr(), frames_p.data_ptr(), lens.data_ptr(),
-                                               flens.data_ptr(), B, T, N, Hh, Ww, sep.data_ptr(), masks.data_ptr(),
-                                               None, 0, self._stream())
+        lens = self._lengths(lens, "lengths", B, T, what)
+        flens = self._lengths(flens, "frame_lengths", B, N, what)
+        rc = self.lib.avsep_forward_packed(self.h, mixed_p.data_ptr(), frames_p.data_ptr(), lens.data_ptr(),
+                                           flens.data_ptr(), B, T, N, Hh, Ww, sep.data_ptr(), masks.data_ptr(), None, 0,
+                                           self._stream())
         self._check(rc, "avsep_forward_packed")
         return sep, masks
 
@@ -386,10 +373,9 @@ class Engine:
         frames_p = self._host_f32(frames_p, "frames_packed")
         B, T, N, Hh, Ww, lens, flens, (sep, masks) = self._packed_plan(what, mixed_p, frames_p, lengths, frame_lengths,
                                                                        max_len, max_frames, out, False)
-        with torch.cuda.device(self.device):
-            rc = self.lib.avsep_forward_host_packed(self.h, mixed_p.data_ptr(), frames_p.data_ptr(), lens.ctypes.data,
-                                                    flens.ctypes.data, B, T, N, Hh, Ww, sep.data_ptr(), masks.data_ptr(),
-                                                    self._stream())
+        rc = self.lib.avsep_forward_host_packed(self.h, mixed_p.data_ptr(), frames_p.data_ptr(), lens.ctypes.data,
+                                                flens.ctypes.data, B, T, N, Hh, Ww, sep.data_ptr(), masks.data_ptr(),
+                                                self._stream())
         self._check(rc, "avsep_forward_host_packed")
         return sep, masks
 
@@ -405,10 +391,9 @@ class Engine:
                 raise ValueError(f"{what}: contiguous float32 CPU tensors required")
         B, T, N, Hh, Ww, lens, flens, (sep, masks) = self._packed_plan(what, mixed_p, frames_p, lengths, frame_lengths,
                                                                        max_len, max_frames, out, False)
-        with torch.cuda.device(self.device):
-            rc = self.lib.avsep_forward_host_packed_async(self.h, mixed_p.data_ptr(), frames_p.data_ptr(),
-                                                          lens.ctypes.data, flens.ctypes.data, B, T, N, Hh, Ww,
-                                                          sep.data_ptr(), masks.data_ptr(), int(slot), self._stream())
+        rc = self.lib.avsep_forward_host_packed_async(self.h, mixed_p.data_ptr(), frames_p.data_ptr(), lens.ctypes.data,
+                                                      flens.ctypes.data, B, T, N, Hh, Ww, sep.data_ptr(),
+                                                      masks.data_ptr(), int(slot), self._stream())
         self._check(rc, "avsep_forward_host_packed_async")
 
     def host_wait(self, slot: int):
@@ -422,8 +407,7 @@ class Engine:
         mixed = self._dev_f32(mixed, "mixed_spec")
         B, T, _, _, _ = self._check_inputs("audio_encoder", mixed=mixed)
         out = torch.empty((B, T, self.cfg.d_model), device=mixed.device, dtype=torch.float32)
-        with torch.cuda.device(self.device):
-            rc = self.lib.avsep_audio_encoder(self.h, mixed.data_ptr(), B, T, out.data_ptr(), self._stream())
+        rc = self.lib.avsep_audio_encoder(self.h, mixed.data_ptr(), B, T, out.data_ptr(), self._stream())
         self._check(rc, "avsep_audio_encoder")
         return out
 
@@ -433,9 +417,8 @@ class Engine:
         if int(target_len) < 1:
             raise ValueError("visual_encoder: target_len must be >= 1")
         out = torch.empty((B, int(target_len), self.cfg.d_model), device=frames.device, dtype=torch.float32)
-        with torch.cuda.device(self.device):
-            rc = self.lib.avsep_visual_encoder(self.h, frames.data_ptr(), B, N, Hh, Ww, int(target_len),
-                                               out.data_ptr(), self._stream())
+        rc = self.lib.avsep_visual_encoder(self.h, frames.data_ptr(), B, N, Hh, Ww, int(target_len), out.data_ptr(),
+                                           self._stream())
         self._check(rc, "avsep_visual_encoder")
         return out
 
@@ -446,9 +429,7 @@ class Engine:
         B, T, d = audio.shape
         L = visual.shape[1]
         out = torch.empty_like(audio)
-        with torch.cuda.device(self.device):
-            rc = self.lib.avsep_fusion(self.h, audio.data_ptr(), visual.data_ptr(), B, T, L, out.data_ptr(),
-                                       self._stream())
+        rc = self.lib.avsep_fusion(self.h, audio.data_ptr(), visual.data_ptr(), B, T, L, out.data_ptr(), self._stream())
         self._check(rc, "avsep_fusion")
         return out
 
@@ -462,9 +443,8 @@ class Engine:
         F, S = self.cfg.freq_bins, self.cfg.num_speakers
         sep = torch.empty((B, S, F, T), device=fused.device, dtype=torch.float32)
         masks = torch.empty_like(sep)
-        with torch.cuda.device(self.device):
-            rc = self.lib.avsep_decoder(self.h, fused.data_ptr(), mixed.data_ptr(), B, T, sep.data_ptr(),
-                                        masks.data_ptr(), self._stream())
+        rc = self.lib.avsep_decoder(self.h, fused.data_ptr(), mixed.data_ptr(), B, T, sep.data_ptr(), masks.data_ptr(),
+                                    self._stream())
         self._check(rc, "avsep_decoder")
         return sep, masks
 
@@ -478,15 +458,9 @@ class Engine:
         mixed = self._dev_f32(mixed, "mixed_spec")
         B, T, _, _, _ = self._check_inputs("separate", mixed=mixed, out=(masks,) if out is None else (masks, out))
         sep = torch.empty_like(masks) if out is None else out
-        with torch.cuda.device(self.device):
-            if lengths is None:
-                rc = self.lib.avsep_separate(self.h, masks.data_ptr(), mixed.data_ptr(), B, T, sep.data_ptr(),
-                                             self._stream())
-                self._check(rc, "avsep_separate")
-                return sep
-            lens = self._lengths(lengths, "lengths", B, T, "separate")
-            rc = self.lib.avsep_separate_varlen(self.h, masks.data_ptr(), mixed.data_ptr(), lens.data_ptr(), B, T,
-                                                sep.data_ptr(), self._stream())
+        lens = self._lengths(lengths, "lengths", B, T, "separate")
+        rc = self.lib.avsep_separate_varlen(self.h, masks.data_ptr(), mixed.data_ptr(), _ptr(lens), B, T, sep.data_ptr(),
+                                            self._stream())
         self._check(rc, "avsep_separate_varlen")
         return sep
 
@@ -514,11 +488,8 @@ class Engine:
         mixed = torch.empty(B, F, T, device=dev)
         frames = torch.empty(B, S * nf, Hh, Ww, device=dev)
         clean = torch.empty(B, S, F, T, device=dev) if want_clean else None
-        with torch.cuda.device(self.device):
-            rc = self.lib.avsep_synth_batch(self.h, C.byref(cfg), B, amps.data_ptr(), freqs.data_ptr(), phases.data_ptr(),
-                                            noise.data_ptr() if noise is not None else None, mixed.data_ptr(),
-                                            frames.data_ptr(), clean.data_ptr() if clean is not None else None,
-                                            self._stream())
+        rc = self.lib.avsep_synth_batch(self.h, C.byref(cfg), B, amps.data_ptr(), freqs.data_ptr(), phases.data_ptr(),
+                                        _ptr(noise), mixed.data_ptr(), frames.data_ptr(), _ptr(clean), self._stream())
         self._check(rc, "avsep_synth_batch")
         return mixed, frames, clean
 
@@ -536,11 +507,8 @@ class Engine:
         out_snr = torch.empty(B, device=dev, dtype=torch.float64)
         perm = torch.empty(B, device=dev, dtype=torch.int32)
         si = torch.empty(B, device=dev, dtype=torch.float64)
-        with torch.cuda.device(self.device):
-            rc = self.lib.avsep_eval_snr(self.h, separated.data_ptr(), targets.data_ptr(),
-                                         mixed.data_ptr() if mixed is not None else None, B, S, F, T,
-                                         in_snr.data_ptr() if in_snr is not None else None, out_snr.data_ptr(),
-                                         perm.data_ptr(), si.data_ptr(), self._stream())
+        rc = self.lib.avsep_eval_snr(self.h, separated.data_ptr(), targets.data_ptr(), _ptr(mixed), B, S, F, T,
+                                     _ptr(in_snr), out_snr.data_ptr(), perm.data_ptr(), si.data_ptr(), self._stream())
         self._check(rc, "avsep_eval_snr")
         return in_snr, out_snr, perm, si
 
@@ -561,19 +529,12 @@ class Engine:
         F, T = n_fft // 2 + 1, 1 + L // hop_length
         spec = torch.empty(B, F, T, device=dev, dtype=torch.complex64)
         mag = torch.empty(B, F, T, device=dev, dtype=torch.float32) if want_mag else None
-        with torch.cuda.device(self.device):
-            if lengths is None:
-                rc = self.lib.avsep_stft(self.h, waves.data_ptr(), B, L, n_fft, hop_length, spec.data_ptr(),
-                                         mag.data_ptr() if want_mag else None, self._stream())
-                self._check(rc, "avsep_stft")
-                return spec, mag
-            lens = self._lengths(lengths, "lengths", B, L, "stft")
-            flens = self._stream_buf(("stft", "frame_lengths"), B)[:B]
-            rc = self.lib.avsep_stft_varlen(self.h, waves.data_ptr(), lens.data_ptr(), B, L, n_fft, hop_length,
-                                            spec.data_ptr(), mag.data_ptr() if want_mag else None, flens.data_ptr(),
-                                            self._stream())
+        lens = self._lengths(lengths, "lengths", B, L, "stft")
+        flens = None if lens is None else self._stream_buf(("stft", "frame_lengths"), B)[:B]
+        rc = self.lib.avsep_stft_varlen(self.h, waves.data_ptr(), _ptr(lens), B, L, n_fft, hop_length, spec.data_ptr(),
+                                        _ptr(mag), _ptr(flens), self._stream())
         self._check(rc, "avsep_stft_varlen")
-        return spec, mag, flens
+        return (spec, mag) if lens is None else (spec, mag, flens)
 
     def istft(self, spec, masks=None, length: int = None, n_fft: int = 512, hop_length: int = 128, lengths=None):
         """avsep_istft: complex64 (B, F, T) mixture spectrum (+ (B, S, F, T) float32 masks) -> (B, S, L) float32
@@ -597,16 +558,9 @@ class Engine:
                 raise ValueError("istft: masks / spec shape mismatch")
         L = (T - 1) * hop_length if length is None else int(length)
         waves = torch.empty(B, S, L, device=dev, dtype=torch.float32)
-        with torch.cuda.device(self.device):
-            if lengths is None:
-                rc = self.lib.avsep_istft(self.h, spec.data_ptr(), masks.data_ptr() if masks is not None else None, B,
-                                          S, T, n_fft, hop_length, L, waves.data_ptr(), self._stream())
-                self._check(rc, "avsep_istft")
-                return waves
-            lens = self._lengths(lengths, "lengths", B, L, "istft")
-            rc = self.lib.avsep_istft_varlen(self.h, spec.data_ptr(), masks.data_ptr() if masks is not None else None,
-                                             lens.data_ptr(), B, S, T, n_fft, hop_length, L, waves.data_ptr(),
-                                             self._stream())
+        lens = self._lengths(lengths, "lengths", B, L, "istft")
+        rc = self.lib.avsep_istft_varlen(self.h, spec.data_ptr(), _ptr(masks), _ptr(lens), B, S, T, n_fft, hop_length, L,
+                                         waves.data_ptr(), self._stream())
         self._check(rc, "avsep_istft_varlen")
         return waves
 

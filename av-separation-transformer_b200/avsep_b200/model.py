@@ -378,9 +378,8 @@ class AVSeparationTransformer(_InferenceOnly):
             raise ValueError(f"separate_waveforms: mixed_wave must be (B, L), got {tuple(mixed_wave.shape)}")
         B, L = mixed_wave.shape
         _, _, N, _, _ = eng._check_inputs("separate_waveforms", frames=lip_frames)
-        with torch.cuda.device(eng.device):
-            lens = eng._lengths(lengths, "lengths", B, L, "separate_waveforms")
-            flens = eng._lengths(frame_lengths, "frame_lengths", B, N, "separate_waveforms")
+        lens = eng._lengths(lengths, "lengths", B, L, "separate_waveforms")
+        flens = eng._lengths(frame_lengths, "frame_lengths", B, N, "separate_waveforms")
         if lens is None:
             spec, mag = eng.stft(mixed_wave, n_fft, hop_length)
             t_lens = None

@@ -36,6 +36,10 @@ __global__ void interp_rows_kernel(const float* __restrict__ x, float* __restric
   float* o = out + (static_cast<size_t>(b) * T + t) * d;
   for (int c = threadIdx.x; c < d; c += blockDim.x) o[c] = k.w0 * r0[c] + k.w1 * r1[c];
 }
+const char* launch_interp_rows(cudaStream_t s, const float* x, float* out, int B, int N, int T, int d) {
+  interp_rows_kernel<<<dim3(T, B), 128, 0, s>>>(x, out, N, T, d);
+  return cudaGetLastError() == cudaSuccess ? nullptr : "interp_rows: launch failed";
+}
 
 // Profiling aid: keeps the GPU busy while the host enqueues a whole forward, so that the per-kernel event pairs
 // measure device time and not host launch latency.
@@ -220,6 +224,28 @@ int fail(avsep_handle* h, const std::string& msg) {
   return 1;
 }
 
+// Selects `device` unless it is current, and selects the caller's device again when it goes out of scope.
+struct DeviceScope {
+  int caller = 0;
+  bool switched = false;
+  cudaError_t err;
+  explicit DeviceScope(int device) : err(cudaGetDevice(&caller)) {
+    if (err == cudaSuccess && caller != device) {
+      err = cudaSetDevice(device);
+      switched = err == cudaSuccess;
+    }
+  }
+  ~DeviceScope() {
+    if (switched) cudaSetDevice(caller);
+  }
+};
+// The rest of the calling C-ABI function runs on `device`, and no call changes which device the calling thread has
+// current, on any return path.
+#define ON_DEVICE(h, device)              \
+  const DeviceScope device_scope(device); \
+  if (device_scope.err != cudaSuccess)    \
+    return fail(h, std::string("cannot select the device: ") + cudaGetErrorString(device_scope.err))
+
 int prof_begin(avsep_handle* h, const char* label, cudaStream_t s) {
   if (h->ev_used + 2 > h->ev_pool.size()) {
     for (int i = 0; i < 64; ++i) {
@@ -240,8 +266,8 @@ void prof_end(avsep_handle* h, cudaStream_t s) {
 cudaStream_t stream_of(LaunchCtx lc) { return lc.stream; }
 cudaStream_t stream_of(cudaStream_t s) { return s; }
 
-// Launcher call fn(on, ...), where `on` is the LaunchCtx of a launch_pdl launcher or the stream of a <<<>>> one.  With
-// profiling on, the call is bracketed by an event pair on that same stream.
+// Launcher call fn(on, ...), where `on` is the LaunchCtx of a launch_pdl launcher or the stream of a <<<>>> one, counted
+// as one launch of the call.  With profiling on, the call is bracketed by an event pair on that same stream.
 #define CKL(label, on, fn, ...)                                         \
   do {                                                                  \
     const cudaStream_t _s = stream_of(on);                              \
@@ -266,6 +292,14 @@ void drop_graphs(avsep_handle* h) { h->graphs.clear(); }   // cached graphs hold
 // The launch settings of h's forward-path kernels on stream s: per-launch event pairs (profiling) must time the kernels
 // one at a time, so profiling turns PDL off.
 LaunchCtx launch_ctx(const avsep_handle* h, cudaStream_t s) { return {s, h->pdl && !h->profile}; }
+
+// The entry of every C-ABI call that enqueues device work on the caller's stream: the call runs on h's device, the
+// launch count starts again from 0, and `lc` holds h's launch settings on that stream.
+#define ENTER(h, stream)                                                 \
+  if (!h) return 1;                                                      \
+  ON_DEVICE(h, h->cfg.device);                                           \
+  h->launches = 0;                                                       \
+  const LaunchCtx lc = launch_ctx(h, static_cast<cudaStream_t>(stream))
 
 size_t op_size(const avsep_handle* h) { return h->cfg.precision == AVSEP_PREC_TF32 ? 4 : 2; }
 
@@ -756,7 +790,8 @@ int forward_cached(avsep_handle* h, LaunchCtx lc, Workspace& w, const void* ws_b
     return forward_device(h, lc, w, mixed, frames, separated, masks);   // warm-up, also sets kernel attributes
   }
   ent->last_use = ++h->graph_clock;
-  if (ent->exec == nullptr) {
+  if (ent->exec == nullptr) {   // the capture counts the launches it records; a replay adds them
+    const int64_t before = h->launches;
     CUDA_OK(make_stream(h->cap_stream));
     CUDA_OK(cudaStreamBeginCapture(h->cap_stream.get(), cudaStreamCaptureModeRelaxed));
     const int rc = forward_device(h, {h->cap_stream.get(), lc.pdl}, w, mixed, frames, separated, masks);
@@ -772,9 +807,10 @@ int forward_cached(avsep_handle* h, LaunchCtx lc, Workspace& w, const void* ws_b
     cudaGraphDestroy(graph);
     if (ci != cudaSuccess) return fail(h, std::string("cudaGraphInstantiate: ") + cudaGetErrorString(ci));
     ent->exec.reset(exec);
-    ent->launches = h->launches;
+    ent->launches = h->launches - before;
+  } else {
+    h->launches += ent->launches;
   }
-  h->launches = ent->launches;
   CUDA_OK(cudaGraphLaunch(ent->exec.get(), lc.stream));
   return 0;
 }
@@ -790,10 +826,8 @@ int forward_packed_run(avsep_handle* h, LaunchCtx lc, Workspace& w, const Stagin
       st.frames);
   w.lens = lens ? lens + b0 : nullptr;
   w.frame_lens = flens ? flens + b0 : nullptr;
-  h->launches = 0;   // a graph replay sets the forward's own count
   if (forward_cached(h, lc, w, ws_base, st.mixed, st.frames, st.sep, st.masks)) return 1;
   CKL("pack", lc, launch_pack, st.sep, st.masks, lens, b0, w.B, S, F, w.T, sep_p, masks_p);
-  ++h->launches;     // the unpack
   return 0;
 }
 
@@ -918,7 +952,7 @@ int avsep_create(const avsep_config* cfg, avsep_handle** out) {
   cudaDeviceProp prop;
   if (cudaGetDeviceProperties(&prop, cfg->device) != cudaSuccess) return fail(nullptr, "avsep_create: device query failed");
   if (prop.major != 10) return fail(nullptr, "avsep_create: kernels are built for sm_100a (B200) only");
-  if (cudaSetDevice(cfg->device) != cudaSuccess) return fail(nullptr, "avsep_create: cudaSetDevice failed");
+  ON_DEVICE(nullptr, cfg->device);
   if (const char* e = tma_init()) return fail(nullptr, e);
   if (const char* e = fft512_init_tables()) return fail(nullptr, e);
   avsep_handle* h = new avsep_handle();
@@ -945,7 +979,7 @@ int avsep_create(const avsep_config* cfg, avsep_handle** out) {
 
 void avsep_destroy(avsep_handle* h) {
   if (!h) return;
-  cudaSetDevice(h->cfg.device);   // the handle's resources belong to its device
+  const DeviceScope device_scope(h->cfg.device);   // the handle's resources belong to its device
   delete h;
 }
 
@@ -970,9 +1004,7 @@ int avsep_set_weight(avsep_handle* h, const char* key, const void* host_data, in
 }
 
 int avsep_finalize_weights(avsep_handle* h, void* cuda_stream) {
-  if (!h) return 1;
-  cudaStream_t s = static_cast<cudaStream_t>(cuda_stream);
-  CUDA_OK(cudaSetDevice(h->cfg.device));
+  ENTER(h, cuda_stream);
   const int64_t d = h->cfg.d_model, F = h->cfg.freq_bins, S = h->cfg.num_speakers, Fp = h->Fp;
   const int Le = h->cfg.num_encoder_layers, Lf = h->cfg.num_fusion_layers;
   const bool tf32 = h->cfg.precision == AVSEP_PREC_TF32;
@@ -1118,8 +1150,8 @@ int avsep_finalize_weights(avsep_handle* h, void* cuda_stream) {
   // upload
   drop_graphs(h);
   CUDA_OK(h->weights.alloc(ar.bytes.size()));
-  CUDA_OK(cudaMemcpyAsync(h->weights.get(), ar.bytes.data(), ar.bytes.size(), cudaMemcpyHostToDevice, s));
-  CUDA_OK(cudaStreamSynchronize(s));
+  CUDA_OK(cudaMemcpyAsync(h->weights.get(), ar.bytes.data(), ar.bytes.size(), cudaMemcpyHostToDevice, lc.stream));
+  CUDA_OK(cudaStreamSynchronize(lc.stream));
   ar.patch(h->weights.get());
   if (h->xs_a != nullptr) {
     h->xs_a_np = h->xs_a + xformer_pro_bytes(3, h->cfg.d_model);
@@ -1145,16 +1177,13 @@ int avsep_forward(avsep_handle* h, const float* mixed_spec, const float* lip_fra
 int avsep_forward_varlen(avsep_handle* h, const float* mixed_spec, const float* lip_frames, const int32_t* lengths,
                          const int32_t* frame_lengths, int32_t B, int32_t T, int32_t N, int32_t Hh, int32_t Ww,
                          float* separated, float* masks, void* workspace, size_t workspace_bytes, void* cuda_stream) {
-  if (!h) return 1;
+  ENTER(h, cuda_stream);
   if (!mixed_spec || !lip_frames || !separated || !masks) return fail(h, "avsep_forward: null buffer");
   if (check_shape(h, B, T, N, Hh, Ww)) return 1;
-  CUDA_OK(cudaSetDevice(h->cfg.device));
   Workspace w;
   if (get_workspace(h, w, workspace, workspace_bytes, B, T, N, Hh, Ww)) return 1;
   w.lens = lengths; w.frame_lens = frame_lengths;
-  h->launches = 0;
-  return forward_cached(h, launch_ctx(h, static_cast<cudaStream_t>(cuda_stream)), w,
-                        workspace ? workspace : h->own_ws.get(), mixed_spec, lip_frames, separated, masks);
+  return forward_cached(h, lc, w, workspace ? workspace : h->own_ws.get(), mixed_spec, lip_frames, separated, masks);
 }
 
 size_t avsep_packed_workspace_bytes(avsep_handle* h, int32_t B, int32_t T, int32_t N, int32_t Hh, int32_t Ww) {
@@ -1168,14 +1197,13 @@ int avsep_forward_packed(avsep_handle* h, const float* mixed_packed, const float
                          const int32_t* frame_lengths, int32_t B, int32_t T, int32_t N, int32_t Hh, int32_t Ww,
                          float* separated_packed, float* masks_packed, void* workspace, size_t workspace_bytes,
                          void* cuda_stream) {
-  if (!h) return 1;
+  ENTER(h, cuda_stream);
   if (!mixed_packed || !frames_packed || !separated_packed || !masks_packed)
     return fail(h, "avsep_forward_packed: null buffer");
   if ((reinterpret_cast<uintptr_t>(mixed_packed) | reinterpret_cast<uintptr_t>(frames_packed) |
        reinterpret_cast<uintptr_t>(separated_packed) | reinterpret_cast<uintptr_t>(masks_packed)) & 3)
     return fail(h, "avsep_forward_packed: buffers must be 4-byte aligned");
   if (check_shape(h, B, T, N, Hh, Ww)) return 1;
-  CUDA_OK(cudaSetDevice(h->cfg.device));
   Workspace w;
   Staging st;
   uint8_t* base = nullptr;
@@ -1183,9 +1211,8 @@ int avsep_forward_packed(avsep_handle* h, const float* mixed_packed, const float
                      "avsep_packed_workspace_bytes", base))
     return 1;
   carve_packed(h, w, st, base, B, T, N, Hh, Ww);
-  h->launches = 0;
-  return forward_packed_run(h, launch_ctx(h, static_cast<cudaStream_t>(cuda_stream)), w, st, base, mixed_packed,
-                            frames_packed, lengths, frame_lengths, 0, separated_packed, masks_packed);
+  return forward_packed_run(h, lc, w, st, base, mixed_packed, frames_packed, lengths, frame_lengths, 0,
+                            separated_packed, masks_packed);
 }
 
 namespace {
@@ -1218,7 +1245,6 @@ int host_submit(avsep_handle* h, const float* mixed_spec, const float* lip_frame
   }
   auto t_at = [&](size_t b) { return packed ? pt[b] : b * T; };
   auto n_at = [&](size_t b) { return packed ? pn[b] : b * N; };
-  CUDA_OK(cudaSetDevice(h->cfg.device));
   avsep_handle::HostSlot& sl = h->slot[slot_id];
   const size_t F = h->cfg.freq_bins, S = h->cfg.num_speakers;
   const size_t mixed_per = F * T, frames_per = static_cast<size_t>(N) * Hh * Ww, out_per = S * F * T;
@@ -1309,7 +1335,6 @@ int host_submit(avsep_handle* h, const float* mixed_spec, const float* lip_frame
     CUDA_OK(cudaEventRecord(sl.ev_lens.get(), s_in));
   }
   const size_t HW = static_cast<size_t>(Hh) * Ww, SF = S * F;
-  int64_t launches = 0;
   for (int c = 0; c < nchunks; ++c) {
     const size_t b0 = starts[c];
     const int bc = sizes[c];
@@ -1330,13 +1355,11 @@ int host_submit(avsep_handle* h, const float* mixed_spec, const float* lip_frame
                                     static_cast<int>(b0), io_sep, io_masks)
                : forward_cached(h, comp, wc, ws_lane, io_mixed + m0, io_frames + f0, io_sep + o0, io_masks + o0))
       return 1;
-    launches += h->launches;
     CUDA_OK(cudaEventRecord(sl.ev[2 * c + 1].get(), comp.stream));
     CUDA_OK(cudaStreamWaitEvent(s_out, sl.ev[2 * c + 1].get(), 0));
     CUDA_OK(cudaMemcpyAsync(separated + o0, io_sep + o0, on * 4, cudaMemcpyDeviceToHost, s_out));
     CUDA_OK(cudaMemcpyAsync(masks + o0, io_masks + o0, on * 4, cudaMemcpyDeviceToHost, s_out));
   }
-  h->launches = launches;
   for (int l = 0; l < lanes; ++l) CUDA_OK(cudaEventRecord(sl.ev_lane[l].get(), h->host_comp[l].get()));
   // The caller's stream is deliberately NOT made to wait for the results: that would chain call i+1 (which is ordered
   // after the caller's stream) behind call i's copy-out.  Results are consumed on the host after avsep_host_wait.
@@ -1347,9 +1370,8 @@ int host_submit(avsep_handle* h, const float* mixed_spec, const float* lip_frame
 
 int avsep_forward_host(avsep_handle* h, const float* mixed_spec, const float* lip_frames, int32_t B, int32_t T,
                        int32_t N, int32_t Hh, int32_t Ww, float* separated, float* masks, void* cuda_stream) {
-  if (!h) return 1;
-  if (host_submit(h, mixed_spec, lip_frames, B, T, N, Hh, Ww, separated, masks, 0, static_cast<cudaStream_t>(cuda_stream), false))
-    return 1;
+  ENTER(h, cuda_stream);
+  if (host_submit(h, mixed_spec, lip_frames, B, T, N, Hh, Ww, separated, masks, 0, lc.stream, false)) return 1;
   CUDA_OK(cudaEventSynchronize(h->slot[0].ev_end.get()));
   return 0;
 }
@@ -1357,17 +1379,16 @@ int avsep_forward_host(avsep_handle* h, const float* mixed_spec, const float* li
 int avsep_forward_host_async(avsep_handle* h, const float* mixed_spec, const float* lip_frames, int32_t B, int32_t T,
                              int32_t N, int32_t Hh, int32_t Ww, float* separated, float* masks, int32_t slot,
                              void* cuda_stream) {
-  if (!h) return 1;
-  return host_submit(h, mixed_spec, lip_frames, B, T, N, Hh, Ww, separated, masks, slot,
-                     static_cast<cudaStream_t>(cuda_stream), true);
+  ENTER(h, cuda_stream);
+  return host_submit(h, mixed_spec, lip_frames, B, T, N, Hh, Ww, separated, masks, slot, lc.stream, true);
 }
 
 int avsep_forward_host_packed(avsep_handle* h, const float* mixed_packed, const float* frames_packed,
                               const int32_t* lengths, const int32_t* frame_lengths, int32_t B, int32_t T, int32_t N,
                               int32_t Hh, int32_t Ww, float* separated_packed, float* masks_packed, void* cuda_stream) {
-  if (!h) return 1;
-  if (host_submit(h, mixed_packed, frames_packed, B, T, N, Hh, Ww, separated_packed, masks_packed, 0,
-                  static_cast<cudaStream_t>(cuda_stream), false, true, lengths, frame_lengths))
+  ENTER(h, cuda_stream);
+  if (host_submit(h, mixed_packed, frames_packed, B, T, N, Hh, Ww, separated_packed, masks_packed, 0, lc.stream, false,
+                  true, lengths, frame_lengths))
     return 1;
   CUDA_OK(cudaEventSynchronize(h->slot[0].ev_end.get()));
   return 0;
@@ -1377,16 +1398,16 @@ int avsep_forward_host_packed_async(avsep_handle* h, const float* mixed_packed, 
                                     const int32_t* lengths, const int32_t* frame_lengths, int32_t B, int32_t T,
                                     int32_t N, int32_t Hh, int32_t Ww, float* separated_packed, float* masks_packed,
                                     int32_t slot, void* cuda_stream) {
-  if (!h) return 1;
-  return host_submit(h, mixed_packed, frames_packed, B, T, N, Hh, Ww, separated_packed, masks_packed, slot,
-                     static_cast<cudaStream_t>(cuda_stream), true, true, lengths, frame_lengths);
+  ENTER(h, cuda_stream);
+  return host_submit(h, mixed_packed, frames_packed, B, T, N, Hh, Ww, separated_packed, masks_packed, slot, lc.stream,
+                     true, true, lengths, frame_lengths);
 }
 
 int avsep_host_wait(avsep_handle* h, int32_t slot) {
   if (!h) return 1;
   if (slot < 0 || slot >= AVSEP_HOST_SLOTS) return fail(h, "avsep_host_wait: slot must be 0 .. AVSEP_HOST_SLOTS - 1");
   if (!h->slot[slot].ev_end) return 0;       // nothing was ever submitted on this slot
-  CUDA_OK(cudaSetDevice(h->cfg.device));
+  ON_DEVICE(h, h->cfg.device);
   CUDA_OK(cudaEventSynchronize(h->slot[slot].ev_end.get()));
   return 0;
 }
@@ -1394,10 +1415,9 @@ int avsep_host_wait(avsep_handle* h, int32_t slot) {
 int avsep_synth_batch(avsep_handle* h, const avsep_synth_config* cfg, int32_t B, const double* amps, const double* freqs,
                       const double* phases, const float* noise, float* mixed_spec, float* lip_frames,
                       float* clean_specs, void* cuda_stream) {
-  if (!h) return 1;
+  ENTER(h, cuda_stream);
   if (!cfg || !amps || !freqs || !phases || !mixed_spec || !lip_frames) return fail(h, "avsep_synth_batch: null argument");
   if (B < 1) return fail(h, "avsep_synth_batch: empty batch");
-  CUDA_OK(cudaSetDevice(h->cfg.device));
   SynthProblem p{};
   p.B = B; p.S = cfg->num_speakers; p.n = cfg->num_samples_audio; p.nfft = cfg->n_fft; p.hop = cfg->hop_length;
   p.nf = cfg->num_frames; p.Hh = cfg->frame_h; p.Ww = cfg->frame_w; p.duration = cfg->duration;
@@ -1407,23 +1427,20 @@ int avsep_synth_batch(avsep_handle* h, const avsep_synth_config* cfg, int32_t B,
   const size_t need = static_cast<size_t>(B) * (p.S + 1) * p.n;
   if (h->synth_waves.cap < need) CUDA_OK(h->synth_waves.alloc(need));
   p.waves = h->synth_waves.get();
-  h->launches = 0;
-  const cudaStream_t s = static_cast<cudaStream_t>(cuda_stream);
-  CK(s, launch_synth, p);
-  h->launches = 3;
+  CK(lc.stream, launch_synth_waves, p);
+  CK(lc.stream, launch_stft, p.waves, nullptr, B, p.S + 1, p.n, p.nfft, p.hop, nullptr, mixed_spec, clean_specs,
+     nullptr);
+  CK(lc.stream, launch_synth_lips, p);
   return 0;
 }
 
 int avsep_eval_snr(avsep_handle* h, const float* separated, const float* targets, const float* mixed, int32_t B,
                    int32_t S, int32_t F, int32_t T, double* input_snr, double* output_snr, int32_t* best_perm,
                    double* si_snr, void* cuda_stream) {
-  if (!h) return 1;
+  ENTER(h, cuda_stream);
   if (!separated || !targets) return fail(h, "avsep_eval_snr: null argument");
   if (B < 1 || F < 1 || T < 1) return fail(h, "avsep_eval_snr: empty problem");
-  CUDA_OK(cudaSetDevice(h->cfg.device));
-  const cudaStream_t s = static_cast<cudaStream_t>(cuda_stream);
-  CK(s, launch_eval_snr, separated, targets, mixed, B, S, F * T, input_snr, output_snr, best_perm, si_snr);
-  h->launches = 1;
+  CK(lc.stream, launch_eval_snr, separated, targets, mixed, B, S, F * T, input_snr, output_snr, best_perm, si_snr);
   return 0;
 }
 
@@ -1434,15 +1451,12 @@ int avsep_stft(avsep_handle* h, const float* waves, int32_t B, int32_t L, int32_
 
 int avsep_stft_varlen(avsep_handle* h, const float* waves, const int32_t* lengths, int32_t B, int32_t L, int32_t n_fft,
                       int32_t hop_length, float* spec, float* mag, int32_t* frame_lengths_out, void* cuda_stream) {
-  if (!h) return 1;
+  ENTER(h, cuda_stream);
   if (!waves || !spec) return fail(h, "avsep_stft: null argument");
   if (B <= 0 || L <= 0) return fail(h, "stft: empty problem");
   if (!fft_geometry_ok(n_fft, hop_length))
     return fail(h, "stft: n_fft must be a power of two in [8, 2048], 1 <= hop <= n_fft");
-  CUDA_OK(cudaSetDevice(h->cfg.device));
-  const cudaStream_t s = static_cast<cudaStream_t>(cuda_stream);
-  CK(s, launch_stft, waves, lengths, B, 0, L, n_fft, hop_length, spec, mag, nullptr, frame_lengths_out);
-  h->launches = 1;
+  CK(lc.stream, launch_stft, waves, lengths, B, 0, L, n_fft, hop_length, spec, mag, nullptr, frame_lengths_out);
   return 0;
 }
 
@@ -1454,12 +1468,9 @@ int avsep_istft(avsep_handle* h, const float* spec, const float* masks, int32_t 
 int avsep_istft_varlen(avsep_handle* h, const float* spec, const float* masks, const int32_t* lengths, int32_t B,
                        int32_t S, int32_t T, int32_t n_fft, int32_t hop_length, int32_t L, float* waves,
                        void* cuda_stream) {
-  if (!h) return 1;
+  ENTER(h, cuda_stream);
   if (!spec || !waves) return fail(h, "avsep_istft: null argument");
-  CUDA_OK(cudaSetDevice(h->cfg.device));
-  const cudaStream_t s = static_cast<cudaStream_t>(cuda_stream);
-  CK(s, launch_istft_masked, spec, masks, lengths, B, S, T, n_fft, hop_length, L, waves);
-  h->launches = 1;
+  CK(lc.stream, launch_istft_masked, spec, masks, lengths, B, S, T, n_fft, hop_length, L, waves);
   return 0;
 }
 
@@ -1470,7 +1481,7 @@ int avsep_shared_alloc(avsep_handle* h, size_t bytes, void** dev_ptr, unsigned c
   if (!h) return 1;
   if (!dev_ptr || !handle_out || bytes == 0) return fail(h, "avsep_shared_alloc: bad argument");
   static_assert(sizeof(cudaIpcMemHandle_t) == AVSEP_IPC_HANDLE_BYTES, "IPC handle size");
-  CUDA_OK(cudaSetDevice(h->cfg.device));
+  ON_DEVICE(h, h->cfg.device);
   void* ptr = nullptr;
   CUDA_OK(cudaMalloc(&ptr, bytes));       // a dedicated allocation: an IPC handle always names a whole cudaMalloc block
   cudaIpcMemHandle_t ih;
@@ -1487,9 +1498,9 @@ int avsep_shared_alloc(avsep_handle* h, size_t bytes, void** dev_ptr, unsigned c
 
 int avsep_shared_free(avsep_handle* h, void* dev_ptr) {
   if (!h) return 1;
+  ON_DEVICE(h, h->cfg.device);
   for (size_t i = 0; i < h->shared_owned.size(); ++i)
     if (h->shared_owned[i] == dev_ptr) {
-      CUDA_OK(cudaSetDevice(h->cfg.device));
       h->shared_owned.erase(h->shared_owned.begin() + i);
       CUDA_OK(cudaFree(dev_ptr));
       return 0;
@@ -1500,7 +1511,7 @@ int avsep_shared_free(avsep_handle* h, void* dev_ptr) {
 int avsep_shared_open(avsep_handle* h, const unsigned char handle[AVSEP_IPC_HANDLE_BYTES], void** dev_ptr) {
   if (!h) return 1;
   if (!handle || !dev_ptr) return fail(h, "avsep_shared_open: bad argument");
-  CUDA_OK(cudaSetDevice(h->cfg.device));
+  ON_DEVICE(h, h->cfg.device);
   cudaIpcMemHandle_t ih;
   memcpy(&ih, handle, sizeof ih);
   void* ptr = nullptr;
@@ -1512,9 +1523,9 @@ int avsep_shared_open(avsep_handle* h, const unsigned char handle[AVSEP_IPC_HAND
 
 int avsep_shared_close(avsep_handle* h, void* dev_ptr) {
   if (!h) return 1;
+  ON_DEVICE(h, h->cfg.device);
   for (size_t i = 0; i < h->shared_mapped.size(); ++i)
     if (h->shared_mapped[i] == dev_ptr) {
-      CUDA_OK(cudaSetDevice(h->cfg.device));
       h->shared_mapped.erase(h->shared_mapped.begin() + i);
       CUDA_OK(cudaIpcCloseMemHandle(dev_ptr));
       return 0;
@@ -1523,11 +1534,10 @@ int avsep_shared_close(avsep_handle* h, void* dev_ptr) {
 }
 
 int avsep_copy_async(avsep_handle* h, void* dst, const void* src, size_t bytes, void* cuda_stream) {
-  if (!h) return 1;
+  ENTER(h, cuda_stream);
   if (!dst || !src) return fail(h, "avsep_copy_async: null buffer");
   if (bytes == 0) return 0;
-  CUDA_OK(cudaSetDevice(h->cfg.device));
-  CUDA_OK(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDefault, static_cast<cudaStream_t>(cuda_stream)));
+  CUDA_OK(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDefault, lc.stream));
   return 0;
 }
 
@@ -1538,13 +1548,11 @@ int avsep_separate(avsep_handle* h, const float* masks, const float* mixed_spec,
 
 int avsep_separate_varlen(avsep_handle* h, const float* masks, const float* mixed_spec, const int32_t* lengths,
                           int32_t B, int32_t T, float* separated, void* cuda_stream) {
-  if (!h) return 1;
+  ENTER(h, cuda_stream);
   if (!masks || !mixed_spec || !separated) return fail(h, "avsep_separate: null buffer");
   if (B < 1 || T < 1) return fail(h, "avsep_separate: B and T must be >= 1");
-  CUDA_OK(cudaSetDevice(h->cfg.device));
-  const char* e = launch_separate(static_cast<cudaStream_t>(cuda_stream), masks, mixed_spec, separated, B,
-                                  h->cfg.num_speakers, h->cfg.freq_bins, T, lengths);
-  return e ? fail(h, e) : 0;
+  CK(lc.stream, launch_separate, masks, mixed_spec, separated, B, h->cfg.num_speakers, h->cfg.freq_bins, T, lengths);
+  return 0;
 }
 
 namespace {
@@ -1560,37 +1568,32 @@ int make_flag_set(avsep_handle* h, uint32_t* const* flags, int32_t n, FlagSet& f
 }  // namespace
 
 int avsep_flag_signal(avsep_handle* h, uint32_t* const* flags, int32_t n, uint32_t value, void* cuda_stream) {
-  if (!h) return 1;
+  ENTER(h, cuda_stream);
   FlagSet f;
   if (make_flag_set(h, flags, n, f, "avsep_flag_signal")) return 1;
-  CUDA_OK(cudaSetDevice(h->cfg.device));
-  const char* e = launch_flag_signal(static_cast<cudaStream_t>(cuda_stream), f, value);
-  return e ? fail(h, e) : 0;
+  CK(lc.stream, launch_flag_signal, f, value);
+  return 0;
 }
 
 int avsep_flag_wait(avsep_handle* h, uint32_t* const* flags, int32_t n, uint32_t value, double timeout_s,
                     void* cuda_stream) {
-  if (!h) return 1;
+  ENTER(h, cuda_stream);
   FlagSet f;
   if (make_flag_set(h, flags, n, f, "avsep_flag_wait")) return 1;
   if (!(timeout_s > 0.0) || timeout_s > 3600.0) return fail(h, "avsep_flag_wait: timeout_s must be in (0, 3600]");
-  CUDA_OK(cudaSetDevice(h->cfg.device));
-  const char* e = launch_flag_wait(static_cast<cudaStream_t>(cuda_stream), f, value, timeout_s);
-  return e ? fail(h, e) : 0;
+  CK(lc.stream, launch_flag_wait, f, value, timeout_s);
+  return 0;
 }
 
 // ---- sub-module forwards ------------------------------------------------------------------------
 int avsep_audio_encoder(avsep_handle* h, const float* mixed_spec, int32_t B, int32_t T, float* out_BTd,
                         void* cuda_stream) {
-  if (!h) return 1;
+  ENTER(h, cuda_stream);
   if (!mixed_spec || !out_BTd) return fail(h, "avsep_audio_encoder: null buffer");
   if (check_shape(h, B, T, 1, 1, 1)) return 1;
-  CUDA_OK(cudaSetDevice(h->cfg.device));
-  const LaunchCtx lc = launch_ctx(h, static_cast<cudaStream_t>(cuda_stream));
   Workspace w;
   if (get_workspace(h, w, nullptr, 0, B, T, 1, 1, 1)) return 1;
   const int d = h->cfg.d_model, Ma = B * T;
-  h->launches = 0;
   if (audio_frontend(h, lc, w, mixed_spec, Plan{})) return 1;
   if (encoder_stack(h, lc, h->enc_a, B, T, w.x_a, w.y_a, w.a_op, w.qkv_a, w.attn_a, w.ffn_a, nullptr, nullptr)) return 1;
   CUDA_OK(cudaMemcpyAsync(out_BTd, w.x_a, static_cast<size_t>(Ma) * d * 4, cudaMemcpyDeviceToDevice, lc.stream));
@@ -1599,36 +1602,28 @@ int avsep_audio_encoder(avsep_handle* h, const float* mixed_spec, int32_t B, int
 
 int avsep_visual_encoder(avsep_handle* h, const float* lip_frames, int32_t B, int32_t N, int32_t Hh, int32_t Ww,
                          int32_t target_len, float* out_BTd, void* cuda_stream) {
-  if (!h) return 1;
+  ENTER(h, cuda_stream);
   if (!lip_frames || !out_BTd) return fail(h, "avsep_visual_encoder: null buffer");
   if (check_shape(h, B, 1, N, Hh, Ww)) return 1;
   if (target_len < 1) return fail(h, "avsep_visual_encoder: target_len must be >= 1");
-  CUDA_OK(cudaSetDevice(h->cfg.device));
-  const LaunchCtx lc = launch_ctx(h, static_cast<cudaStream_t>(cuda_stream));
   Workspace w;
   if (get_workspace(h, w, nullptr, 0, B, 1, N, Hh, Ww)) return 1;
   const int d = h->cfg.d_model;
-  h->launches = 0;
   if (visual_frontend(h, lc, w, lip_frames, Plan{})) return 1;
   if (encoder_stack(h, lc, h->enc_v, B, N, w.x_v, w.y_v, w.v_op, w.qkv_v, w.attn_v, w.ffn_v, nullptr, nullptr)) return 1;
-  interp_rows_kernel<<<dim3(target_len, B), 128, 0, lc.stream>>>(w.x_v, out_BTd, N, target_len, d);
-  CUDA_OK(cudaGetLastError());
-  ++h->launches;
+  CKL("interp_rows", lc.stream, launch_interp_rows, w.x_v, out_BTd, B, N, target_len, d);
   return 0;
 }
 
 int avsep_fusion(avsep_handle* h, const float* audio_BTd, const float* visual_BLd, int32_t B, int32_t T, int32_t L,
                  float* out_BTd, void* cuda_stream) {
-  if (!h) return 1;
+  ENTER(h, cuda_stream);
   if (!audio_BTd || !visual_BLd || !out_BTd) return fail(h, "avsep_fusion: null buffer");
   if (check_shape(h, B, T, L, 1, 1)) return 1;
   if (L != T) return fail(h, "avsep_fusion: audio and visual must have the same length (model.py:131-133)");
-  CUDA_OK(cudaSetDevice(h->cfg.device));
-  const LaunchCtx lc = launch_ctx(h, static_cast<cudaStream_t>(cuda_stream));
   Workspace w;
   if (get_workspace(h, w, nullptr, 0, B, T, L, 1, 1)) return 1;
   const int d = h->cfg.d_model, Ma = B * T, Mv = B * L, prec = h->cfg.precision;
-  h->launches = 0;
   CUDA_OK(cudaMemcpyAsync(w.x_a, audio_BTd, static_cast<size_t>(Ma) * d * 4, cudaMemcpyDeviceToDevice, lc.stream));
   CKL("add_layernorm", lc, launch_add_layernorm, prec, w.x_a, nullptr, h->fus[0].n1g, h->fus[0].n1b, nullptr, w.a_op,
       Ma, d);
@@ -1646,15 +1641,12 @@ int avsep_fusion(avsep_handle* h, const float* audio_BTd, const float* visual_BL
 
 int avsep_decoder(avsep_handle* h, const float* fused_BTd, const float* mixed_spec, int32_t B, int32_t T,
                   float* separated, float* masks, void* cuda_stream) {
-  if (!h) return 1;
+  ENTER(h, cuda_stream);
   if (!fused_BTd || !mixed_spec || !separated || !masks) return fail(h, "avsep_decoder: null buffer");
   if (check_shape(h, B, T, 1, 1, 1)) return 1;
-  CUDA_OK(cudaSetDevice(h->cfg.device));
-  const LaunchCtx lc = launch_ctx(h, static_cast<cudaStream_t>(cuda_stream));
   Workspace w;
   if (get_workspace(h, w, nullptr, 0, B, T, 1, 1, 1)) return 1;
   const int d = h->cfg.d_model, Ma = B * T;
-  h->launches = 0;
   CKL("add_layernorm", lc, launch_add_layernorm, h->cfg.precision, fused_BTd, nullptr, nullptr, nullptr, nullptr,
       w.a_op, Ma, d);
   return decoder_stage(h, lc, w, mixed_spec, separated, masks);
@@ -1675,6 +1667,7 @@ int avsep_debug_get_stage(avsep_handle* h, const char* name, float* host_out, si
   *count = snap.count;
   if (host_out == nullptr) return 0;
   if (capacity < snap.count) return fail(h, "avsep_debug_get_stage: buffer too small");
+  ON_DEVICE(h, h->cfg.device);
   CUDA_OK(cudaDeviceSynchronize());
   CUDA_OK(cudaMemcpy(host_out, snap.buf.get(), snap.count * sizeof(float), cudaMemcpyDeviceToHost));
   return 0;
@@ -1690,6 +1683,7 @@ int avsep_set_profile(avsep_handle* h, int32_t enable) {
 // "label count total_ms\n" lines into buf.  reset != 0 clears the totals afterwards.
 int avsep_profile_report(avsep_handle* h, char* buf, size_t capacity, int32_t reset) {
   if (!h || !buf || capacity == 0) return fail(h, "avsep_profile_report: bad argument");
+  ON_DEVICE(h, h->cfg.device);
   CUDA_OK(cudaDeviceSynchronize());
   for (auto& mk : h->ev_marks) {
     float ms = 0.f;
@@ -1716,11 +1710,10 @@ int avsep_profile_report(avsep_handle* h, char* buf, size_t capacity, int32_t re
 // ---- kernel-level test hooks -----------------------------------------------------------------------
 int avsep_test_gemm(avsep_handle* h, const void* A, const void* W, const float* bias, float* out, int32_t M, int32_t N,
                     int32_t K, int32_t act, int32_t force_bn, void* cuda_stream) {
-  if (!h) return 1;
+  ENTER(h, cuda_stream);
   const GemmProblem p = dense(A, M, K, W, N);
   GemmEpilogue e;
   e.bias = bias; e.act = act; e.out_f32 = out; e.ld_f32 = N;
-  const LaunchCtx lc = launch_ctx(h, static_cast<cudaStream_t>(cuda_stream));
   CK(lc, launch_gemm, h->cfg.precision, p, e, h->num_sms, force_bn);
   return 0;
 }
@@ -1729,13 +1722,12 @@ int avsep_test_gemm(avsep_handle* h, const void* A, const void* W, const float* 
 // out_op = LN_{gamma,beta}(x) in operand precision.
 int avsep_test_gemm_ln(avsep_handle* h, const void* A, const void* W, const float* bias, float* x, const float* gamma,
                        const float* beta, void* out_op, int32_t M, int32_t N, int32_t K, void* cuda_stream) {
-  if (!h) return 1;
+  ENTER(h, cuda_stream);
   const GemmProblem p = dense(A, M, K, W, N);
   GemmEpilogue e;
   e.kind = EPI_LN;
   e.bias = bias; e.resid = x; e.out_f32 = x; e.ld_f32 = N; e.ln_gamma = gamma; e.ln_beta = beta;
   e.out_op = out_op; e.ld_op = N;
-  const LaunchCtx lc = launch_ctx(h, static_cast<cudaStream_t>(cuda_stream));
   CK(lc, launch_gemm, h->cfg.precision, p, e, h->num_sms);
   return 0;
 }
@@ -1746,7 +1738,7 @@ int avsep_test_gemm_ln(avsep_handle* h, const void* A, const void* W, const floa
 int avsep_test_gemm_trace(avsep_handle* h, const void* A, const void* W, const float* bias, float* x_or_out,
                           const float* gamma, const float* beta, void* out_op, int32_t M, int32_t N, int32_t K,
                           int32_t ln, int32_t act, unsigned long long* trace_dev, void* cuda_stream) {
-  if (!h) return 1;
+  ENTER(h, cuda_stream);
   const GemmProblem p = dense(A, M, K, W, N);
   GemmEpilogue e;
   e.bias = bias; e.act = act;
@@ -1769,7 +1761,6 @@ int avsep_test_gemm_trace(avsep_handle* h, const void* A, const void* W, const f
     e.out_op = out_op; e.ld_op = N;
     e.out_f32 = out_op ? nullptr : x_or_out; e.ld_f32 = N;
   }
-  const LaunchCtx lc = launch_ctx(h, static_cast<cudaStream_t>(cuda_stream));
   CK(lc, launch_gemm, h->cfg.precision, p, e, h->num_sms, 0, trace_dev);
   return 0;
 }
@@ -1778,8 +1769,7 @@ int avsep_test_gemm_trace(avsep_handle* h, const void* A, const void* W, const f
 int avsep_test_ffn_fused(avsep_handle* h, const void* a, const void* w1, const float* b1, const void* w2,
                          const float* b2, int32_t act, float* x_inout, const float* gamma, const float* beta,
                          void* out_op, int32_t M, void* cuda_stream) {
-  if (!h) return 1;
-  const LaunchCtx lc = launch_ctx(h, static_cast<cudaStream_t>(cuda_stream));
+  ENTER(h, cuda_stream);
   CK(lc, launch_ffn_fused, a, w1, b1, w2, b2, act, x_inout, x_inout, gamma, beta, out_op, M, h->num_sms, nullptr);
   return 0;
 }
@@ -1789,8 +1779,7 @@ int avsep_test_ffn_fused(avsep_handle* h, const void* a, const void* w1, const f
 int avsep_test_ffn_fused_trace(avsep_handle* h, const void* a, const void* w1, const float* b1, const void* w2,
                                const float* b2, int32_t act, float* x_inout, const float* gamma, const float* beta,
                                void* out_op, int32_t M, unsigned long long* trace_dev, void* cuda_stream) {
-  if (!h) return 1;
-  const LaunchCtx lc = launch_ctx(h, static_cast<cudaStream_t>(cuda_stream));
+  ENTER(h, cuda_stream);
   CK(lc, launch_ffn_fused, a, w1, b1, w2, b2, act, x_inout, x_inout, gamma, beta, out_op, M, h->num_sms, trace_dev);
   return 0;
 }
@@ -1801,7 +1790,7 @@ int avsep_test_ffn_fused_trace(avsep_handle* h, const void* a, const void* w1, c
 // audio encoder, fusion.norm after the fusion stack; the visual encoder has none -- else a plain cast).
 int avsep_test_xformer_stack(avsep_handle* h, int32_t which, const float* x_in, const void* kv, int32_t B, int32_t L,
                              float* out_x, void* out_op, int32_t final_ln, long long* trace_dev, void* cuda_stream) {
-  if (!h) return 1;
+  ENTER(h, cuda_stream);
   if (!h->finalized) return fail(h, "weights not finalized");
   if (which < 0 || which > 2) return fail(h, "test_xformer_stack: which must be 0, 1 or 2");
   if (h->xs_a == nullptr || !xformer_stack_usable(h->cfg.precision, h->cfg.d_model, h->cfg.nhead, L))
@@ -1810,12 +1799,12 @@ int avsep_test_xformer_stack(avsep_handle* h, int32_t which, const float* x_in, 
   sp.x_in = x_in; sp.out_x = out_x; sp.out_op = out_op; sp.kv = kv; sp.B = B; sp.L = L; sp.trace = trace_dev;
   if (final_ln && which == 0) { sp.fin_gamma = h->fus[0].n1g; sp.fin_beta = h->fus[0].n1b; }
   if (final_ln && which == 2) { sp.fin_gamma = h->fng; sp.fin_beta = h->fnb; }
-  return run_stack(h, launch_ctx(h, static_cast<cudaStream_t>(cuda_stream)), which, sp);
+  return run_stack(h, lc, which, sp);
 }
 
 int avsep_test_fusion_decoder(avsep_handle* h, const float* x_in, const void* kv, int32_t B, int32_t L, const float* mixed,
                               float* separated, float* masks, long long* trace_dev, void* cuda_stream) {
-  if (!h) return 1;
+  ENTER(h, cuda_stream);
   if (!h->finalized) return fail(h, "weights not finalized");
   if (h->xs_f == nullptr || !h->xs_f_decoder || !xformer_stack_usable(h->cfg.precision, h->cfg.d_model, h->cfg.nhead, L))
     return fail(h, "test_fusion_decoder: the fused stack kernel does not support this configuration");
@@ -1823,11 +1812,12 @@ int avsep_test_fusion_decoder(avsep_handle* h, const float* x_in, const void* kv
   StackProblem sp{};
   sp.x_in = x_in; sp.fin_gamma = h->fng; sp.fin_beta = h->fnb; sp.kv = kv; sp.B = B; sp.L = L; sp.trace = trace_dev;
   sp.mixed = mixed; sp.separated = separated; sp.masks = masks;
-  return run_stack(h, launch_ctx(h, static_cast<cudaStream_t>(cuda_stream)), 2, sp);
+  return run_stack(h, lc, 2, sp);
 }
 
 int avsep_set_option(avsep_handle* h, const char* name, int32_t value) {
   if (!h || !name) return 1;
+  ON_DEVICE(h, h->cfg.device);   // drop_graphs destroys graph execs of h's device
   if (strcmp(name, "host_chunk") == 0) { h->host_chunk = value; return 0; }
   if (strcmp(name, "host_lanes") == 0) { h->host_lanes = value; return 0; }
   if (strcmp(name, "pdl") == 0) { h->pdl = value != 0; drop_graphs(h); return 0; }
@@ -1840,58 +1830,56 @@ int avsep_set_option(avsep_handle* h, const char* name, int32_t value) {
 
 int avsep_test_conv1d(avsep_handle* h, const void* A_padded, const void* W3, const float* bias, float* out, int32_t B,
                       int32_t L, int32_t N, int32_t K, void* cuda_stream) {
-  if (!h) return 1;
+  ENTER(h, cuda_stream);
   GemmProblem p{};
   const int Mp = B * (L + 2);
   p.A = A_padded; p.lda = K; p.rowsA = Mp; p.M = Mp; p.W = W3; p.ldw = 3 * K; p.N = N; p.K = K;
   p.taps = 3; p.tap_stride = K; p.row_shift = -1;
   GemmEpilogue e;
   e.bias = bias; e.rowmap = ROW_PAD2COMPACT; e.Lp = L + 2; e.out_f32 = out; e.ld_f32 = N;
-  const LaunchCtx lc = launch_ctx(h, static_cast<cudaStream_t>(cuda_stream));
   CK(lc, launch_gemm, h->cfg.precision, p, e, h->num_sms);
   return 0;
 }
 
 int avsep_test_attention(avsep_handle* h, const void* q, const void* k, const void* v, void* out, int32_t B, int32_t H,
                          int32_t hd, int32_t Lq, int32_t Lk, int32_t lerp_src, void* cuda_stream) {
-  if (!h) return 1;
+  ENTER(h, cuda_stream);
   AttnProblem ap{};
   ap.q = q; ap.ldq = H * hd; ap.k = k; ap.v = v; ap.ldkv = H * hd; ap.out = out; ap.ldo = H * hd;
   ap.B = B; ap.H = H; ap.hd = hd; ap.Lq = Lq; ap.Lk = Lk; ap.lerp_src = lerp_src; ap.tc_mode = h->attn_tc;
-  const LaunchCtx lc = launch_ctx(h, static_cast<cudaStream_t>(cuda_stream));
   Buf<__nv_bfloat16> scratch;
-  if (lerp_src > 0) {   // same routing as fusion_stack: K then V columns side by side in one interpolated buffer
-    AttnProblem tp = ap;
-    tp.lerp_src = 0; tp.ldkv = 2 * H * hd;
-    if (attention_tc_wanted(h->cfg.precision, tp)) {
-      const int dm = H * hd;
-      if (scratch.alloc(static_cast<size_t>(B) * Lk * 2 * dm) != cudaSuccess)
-        return fail(h, "test_attention: cudaMalloc failed");
-      tp.k = scratch.get(); tp.v = scratch.get() + dm;
-      CK(lc, launch_lerp_rows, static_cast<const float*>(k), dm, B, lerp_src, Lk, dm, scratch.get(), 2 * dm);
-      CK(lc, launch_lerp_rows, static_cast<const float*>(v), dm, B, lerp_src, Lk, dm, scratch.get() + dm, 2 * dm);
-      ap = tp;
+  const int rc = [&] {
+    if (lerp_src > 0) {   // same routing as fusion_stack: K then V columns side by side in one interpolated buffer
+      AttnProblem tp = ap;
+      tp.lerp_src = 0; tp.ldkv = 2 * H * hd;
+      if (attention_tc_wanted(h->cfg.precision, tp)) {
+        const int dm = H * hd;
+        if (scratch.alloc(static_cast<size_t>(B) * Lk * 2 * dm) != cudaSuccess)
+          return fail(h, "test_attention: cudaMalloc failed");
+        tp.k = scratch.get(); tp.v = scratch.get() + dm;
+        CK(lc, launch_lerp_rows, static_cast<const float*>(k), dm, B, lerp_src, Lk, dm, scratch.get(), 2 * dm);
+        CK(lc, launch_lerp_rows, static_cast<const float*>(v), dm, B, lerp_src, Lk, dm, scratch.get() + dm, 2 * dm);
+        ap = tp;
+      }
     }
-  }
-  const char* err = launch_attention(lc, h->cfg.precision, ap);
-  if (scratch.get()) cudaStreamSynchronize(lc.stream);   // before scratch is freed
-  if (err) return fail(h, err);
-  return 0;
+    CK(lc, launch_attention, h->cfg.precision, ap);
+    return 0;
+  }();
+  if (scratch.get()) cudaStreamSynchronize(lc.stream);   // before scratch is freed, on every return path
+  return rc;
 }
 
 int avsep_test_add_layernorm(avsep_handle* h, const float* x, const float* y, const float* gamma, const float* beta,
                              float* x_out, void* out_op, int32_t M, int32_t d, void* cuda_stream) {
-  if (!h) return 1;
-  const LaunchCtx lc = launch_ctx(h, static_cast<cudaStream_t>(cuda_stream));
+  ENTER(h, cuda_stream);
   CKL("add_layernorm", lc, launch_add_layernorm, h->cfg.precision, x, y, gamma, beta, x_out, out_op, M, d);
   return 0;
 }
 
 int avsep_test_visual_cnn(avsep_handle* h, const float* frames, int32_t M, int32_t Hh, int32_t Ww, void* pooled,
                           void* cuda_stream) {
-  if (!h) return 1;
+  ENTER(h, cuda_stream);
   if (!h->finalized) return fail(h, "weights not finalized");
-  const LaunchCtx lc = launch_ctx(h, static_cast<cudaStream_t>(cuda_stream));
   CK(lc, run_visual_cnn, h, frames, M, Hh, Ww, pooled);
   return 0;
 }
@@ -1899,9 +1887,8 @@ int avsep_test_visual_cnn(avsep_handle* h, const float* frames, int32_t M, int32
 // Debug: tcgen05 CNN with a phase trace ([grid][64] globaltimer stamps of each CTA's second frame group).
 int avsep_test_visual_cnn_trace(avsep_handle* h, const float* frames, int32_t M, void* pooled,
                                 unsigned long long* trace_dev, void* cuda_stream) {
-  if (!h) return 1;
+  ENTER(h, cuda_stream);
   if (!h->finalized) return fail(h, "weights not finalized");
-  const LaunchCtx lc = launch_ctx(h, static_cast<cudaStream_t>(cuda_stream));
   CK(lc, run_visual_cnn, h, frames, M, 32, 32, pooled, trace_dev);
   return 0;
 }

@@ -298,7 +298,11 @@ struct SynthProblem {
   float* waves;                          // scratch (B, S+1, n)
   float *mixed_spec, *lip_frames, *clean_specs;
 };
-const char* launch_synth(cudaStream_t s, const SynthProblem& p);
+// A batch is three launches: launch_synth_waves checks the whole problem and writes the (B, S+1, n) signals, the
+// mixture first; launch_stft in the synthesis layout turns them into mixed_spec and clean_specs; launch_synth_lips draws
+// the lip frames from them.
+const char* launch_synth_waves(cudaStream_t s, const SynthProblem& p);
+const char* launch_synth_lips(cudaStream_t s, const SynthProblem& p);
 const char* launch_eval_snr(cudaStream_t s, const float* separated, const float* targets, const float* mixed, int B,
                             int S, int FT, double* input_snr, double* output_snr, int* best_perm, double* si_snr);
 

@@ -202,7 +202,7 @@ __global__ void eval_snr_kernel(const float* __restrict__ separated, const float
 
 }  // namespace
 
-const char* launch_synth(cudaStream_t s, const SynthProblem& p) {
+const char* launch_synth_waves(cudaStream_t s, const SynthProblem& p) {
   if (p.B <= 0) return "synth: empty batch";
   if (p.S < 1 || p.S > 8) return "synth: num_speakers must be 1..8";
   if (!fft_size_ok(p.nfft)) return "synth: n_fft must be a power of two in [8, 2048]";
@@ -211,9 +211,10 @@ const char* launch_synth(cudaStream_t s, const SynthProblem& p) {
   if (static_cast<long long>(p.B) * (p.S + 1) > 65535) return "synth: batch * (speakers + 1) above 65535";
   synth_wave_kernel<<<dim3((p.n + 255) / 256, p.B), 256, 0, s>>>(p.amps, p.freqs, p.phases, p.S, p.n,
                                                                  p.duration / static_cast<double>(p.n), p.waves);
-  if (const char* e = launch_stft(s, p.waves, nullptr, p.B, p.S + 1, p.n, p.nfft, p.hop, nullptr, p.mixed_spec,
-                                  p.clean_specs, nullptr))
-    return e;
+  return cudaGetLastError() == cudaSuccess ? nullptr : "synth: launch failed";
+}
+
+const char* launch_synth_lips(cudaStream_t s, const SynthProblem& p) {
   const long long lip_warps = static_cast<long long>(p.B) * p.S * p.nf;
   lip_frames_kernel<<<static_cast<unsigned>((lip_warps + 7) / 8), 256, 0, s>>>(p.waves, p.noise, p.B, p.S, p.n, p.nf,
                                                                               p.Hh, p.Ww, p.lip_frames);

@@ -15,6 +15,8 @@
  *     No C++ exception crosses this boundary.
  *   - a handle is bound to one CUDA device; calls are stream-ordered on the caller's stream and never
  *     synchronise internally (except avsep_forward_host and the *_debug / *_test helpers).
+ *   - every call runs on its handle's device, whichever device the calling thread has current, and selects the
+ *     caller's current device again before it returns.
  *   - device buffers are owned by the caller; the library owns only the prepacked weights and, when the
  *     caller passes workspace == NULL, a cached workspace per shape.
  *   - eval-mode semantics only (dropout = identity, BatchNorm running statistics): model.py:159,164,197,288.
@@ -148,7 +150,10 @@ AVSEP_API int avsep_forward_host_packed_async(avsep_handle* h, const float* mixe
                                               int32_t T, int32_t N, int32_t Hh, int32_t Ww, float* separated_packed,
                                               float* masks_packed, int32_t slot, void* cuda_stream);
 
-/* Number of kernels the last avsep_forward on this handle launched. */
+/* Number of kernels the last call on `h` that enqueues device work - every call with a cuda_stream argument - enqueued:
+ * a replayed CUDA graph counts the kernels it holds, and avsep_copy_async and avsep_finalize_weights, which only copy,
+ * count 0.  Every other call (options, profiling and debug switches and reports, avsep_host_wait, sizes, the shared
+ * buffers) leaves the count as it is. */
 AVSEP_API int64_t avsep_last_launch_count(const avsep_handle* h);
 
 /* Sub-module forwards (reference: AudioEncoder.forward model.py:54-60, VisualEncoder.forward model.py:103-117,
