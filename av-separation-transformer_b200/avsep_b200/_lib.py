@@ -76,6 +76,10 @@ SIGNATURES = {
     "avsep_istft": (C.c_int, [_P, _P, _P, _I, _I, _I, _I, _I, _I, _P, _P]),
     "avsep_stft_varlen": (C.c_int, [_P, _P, _P, _I, _I, _I, _I, _P, _P, _P, _P]),
     "avsep_istft_varlen": (C.c_int, [_P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _P, _P]),
+    "avsep_waveform_workspace_bytes": (C.c_size_t, [_P, _I, _I, _I, _I, _I, _I, _I]),
+    "avsep_separate_waveforms": (C.c_int, [_P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _P, _P, _P, C.c_size_t, _P]),
+    "avsep_separate_waveforms_host": (C.c_int, [_P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _P, _P, _P]),
+    "avsep_separate_waveforms_host_async": (C.c_int, [_P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _P, _P, _I, _P]),
     "avsep_test_xformer_stack": (C.c_int, [_P, _I, _P, _P, _I, _I, _P, _P, _I, _P, _P]),
     "avsep_test_fusion_decoder": (C.c_int, [_P, _P, _P, _I, _I, _P, _P, _P, _P, _P]),
     "avsep_shared_alloc": (C.c_int, [_P, C.c_size_t, C.POINTER(_P), C.c_char_p]),

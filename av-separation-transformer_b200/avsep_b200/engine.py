@@ -564,6 +564,91 @@ class Engine:
         self._check(rc, "avsep_istft_varlen")
         return waves
 
+    # ---- waveforms in, waveforms out in one call -------------------------------------------------------------
+    def _wave_shapes(self, what, waves, frames, n_fft, hop_length):
+        """(B, L, N, Hh, Ww, T) of a waveform call; raises ValueError.  n_fft and the FFT geometry are checked by the
+        library (RuntimeError naming the call)."""
+        if waves.dim() != 2:
+            raise ValueError(f"{what}: mixed_wave must be (B, L), got {tuple(waves.shape)}")
+        B, L = waves.shape
+        _, _, N, Hh, Ww = self._check_inputs(what, frames=frames)
+        if frames.shape[0] != B:
+            raise ValueError(f"{what}: batch size of mixed_wave ({B}) and lip_frames ({frames.shape[0]}) differ")
+        if int(hop_length) < 1:
+            raise ValueError(f"{what}: hop_length must be >= 1")
+        return B, L, N, Hh, Ww, 1 + L // int(hop_length)
+
+    def separate_waveforms(self, waves, frames, n_fft: int = 512, hop_length: int = 128, lengths=None,
+                           frame_lengths=None, want_masks: bool = True):
+        """avsep_separate_waveforms: (B, L) float32 waveforms and (B, N, H, W) lip frames on the device -> (waves (B, S,
+        L), masks (B, S, F, T) or None).  Bit-identical to ``stft`` -> ``forward`` on the magnitude -> ``istft`` with the
+        masks, in one call whose forward is a cached CUDA graph.  ``lengths`` (B,) samples and ``frame_lengths`` (B,)
+        lip frames per utterance as for ``stft`` / ``forward``."""
+        what = "separate_waveforms"
+        dev = torch.device("cuda", self.device)
+        if waves.device != dev or waves.dtype != torch.float32 or not waves.is_contiguous():
+            raise ValueError(f"{what}: mixed_wave must be a contiguous float32 tensor on cuda:{self.device}")
+        frames = self._dev_f32(frames, "lip_frames")
+        B, L, N, Hh, Ww, T = self._wave_shapes(what, waves, frames, n_fft, hop_length)
+        lens = self._lengths(lengths, "lengths", B, L, what)
+        flens = self._lengths(frame_lengths, "frame_lengths", B, N, what)
+        F, S = self.cfg.freq_bins, self.cfg.num_speakers
+        out = torch.empty(B, S, L, device=dev, dtype=torch.float32)
+        masks = torch.empty(B, S, F, T, device=dev, dtype=torch.float32) if want_masks else None
+        rc = self.lib.avsep_separate_waveforms(self.h, waves.data_ptr(), frames.data_ptr(), _ptr(lens), _ptr(flens), B, L,
+                                               N, Hh, Ww, int(n_fft), int(hop_length), out.data_ptr(), _ptr(masks),
+                                               None, 0, self._stream())
+        self._check(rc, "avsep_separate_waveforms")
+        return out, masks
+
+    def separate_waveforms_host(self, waves, frames, n_fft: int = 512, hop_length: int = 128, want_masks: bool = True,
+                                out=None):
+        """avsep_separate_waveforms_host: CPU tensors in, CPU tensors out (full batches; pinned memory for overlap).
+        Returns (waves (B, S, L), masks (B, S, F, T) or None); without masks only the samples cross back.  ``out``:
+        optional (waves, masks-or-None) CPU buffers."""
+        what = "separate_waveforms_host"
+        waves = self._host_f32(waves, "mixed_wave")
+        frames = self._host_f32(frames, "lip_frames")
+        B, L, N, Hh, Ww, T = self._wave_shapes(what, waves, frames, n_fft, hop_length)
+        F, S = self.cfg.freq_bins, self.cfg.num_speakers
+        if out is None:
+            out = (torch.empty(B, S, L, dtype=torch.float32).pin_memory(),
+                   torch.empty(B, S, F, T, dtype=torch.float32).pin_memory() if want_masks else None)
+        w_out, masks = out
+        self._check_wave_out(what, w_out, masks, B, S, L, F, T)
+        rc = self.lib.avsep_separate_waveforms_host(self.h, waves.data_ptr(), frames.data_ptr(), B, L, N, Hh, Ww,
+                                                    int(n_fft), int(hop_length), w_out.data_ptr(), _ptr(masks),
+                                                    self._stream())
+        self._check(rc, "avsep_separate_waveforms_host")
+        return w_out, masks
+
+    def separate_waveforms_host_async(self, waves, frames, waves_out, masks, slot: int, n_fft: int = 512,
+                                      hop_length: int = 128):
+        """Streaming form of ``separate_waveforms_host`` on I/O slot 0 .. 3 (shared with ``forward_host_async``);
+        ``host_wait(slot)`` completes it.  All tensors must be contiguous float32 CPU tensors (pinned for overlap) that
+        outlive the wait; masks may be None."""
+        what = "separate_waveforms_host_async"
+        for t in (waves, frames, waves_out) + (() if masks is None else (masks,)):
+            if t.is_cuda or t.dtype != torch.float32 or not t.is_contiguous():
+                raise ValueError(f"{what}: contiguous float32 CPU tensors required")
+        B, L, N, Hh, Ww, T = self._wave_shapes(what, waves, frames, n_fft, hop_length)
+        self._check_wave_out(what, waves_out, masks, B, self.cfg.num_speakers, L, self.cfg.freq_bins, T)
+        rc = self.lib.avsep_separate_waveforms_host_async(self.h, waves.data_ptr(), frames.data_ptr(), B, L, N, Hh, Ww,
+                                                          int(n_fft), int(hop_length), waves_out.data_ptr(),
+                                                          _ptr(masks), int(slot), self._stream())
+        self._check(rc, "avsep_separate_waveforms_host_async")
+
+    @staticmethod
+    def _check_wave_out(what, waves_out, masks, B, S, L, F, T):
+        for t, want in ((waves_out, (B, S, L)), (masks, (B, S, F, T))):
+            if t is None:
+                continue
+            if tuple(t.shape) != want or t.dtype != torch.float32 or not t.is_contiguous() or t.is_cuda:
+                raise ValueError(f"{what}: output buffers must be contiguous float32 CPU tensors {want}, "
+                                 f"got {tuple(t.shape)}")
+        if waves_out is None:
+            raise ValueError(f"{what}: a waves output buffer is required")
+
     def set_option(self, name: str, value: int):
         """Execution options of avsep_set_option (include/avsep.h): 'use_graph', 'two_stream', 'pdl' (0/1), 'attn_tc'
         (0 never, 1 long sequences, 2 whenever usable), 'host_chunk', 'host_lanes' (0 = auto), 'profile_spin_us'.

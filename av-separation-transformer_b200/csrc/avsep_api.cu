@@ -102,9 +102,11 @@ struct GraphKey {
   int B, T, N, Hh, Ww;
   const void *mixed, *frames, *sep, *masks, *ws;
   const int *lens, *frame_lens;   // the kernels read the lengths at run time: their contents are not part of the key
+  bool xp_ready;                  // the forward of avsep_separate_waveforms (forward_device): never shares a graph
   bool operator==(const GraphKey& o) const {
     return B == o.B && T == o.T && N == o.N && Hh == o.Hh && Ww == o.Ww && mixed == o.mixed && frames == o.frames &&
-           sep == o.sep && masks == o.masks && ws == o.ws && lens == o.lens && frame_lens == o.frame_lens;
+           sep == o.sep && masks == o.masks && ws == o.ws && lens == o.lens && frame_lens == o.frame_lens &&
+           xp_ready == o.xp_ready;
   }
 };
 struct GraphEntry {
@@ -368,6 +370,31 @@ int get_workspace(avsep_handle* h, Workspace& w, void* user_ws, size_t user_byte
   return 0;
 }
 
+// avsep_separate_waveforms: behind the forward's own workspace the complex spectrum (B, F, T), the masks (B, S, F, T)
+// of a call without a masks buffer, the per-utterance frame counts T_b of a variable-length batch (int32 [B]), and the
+// magnitude (B, F, T) and `separated` (B, S, F, T) that the fused fusion + decoder kernel reads and writes.
+struct WaveStaging {
+  float *spec, *masks;
+  int32_t* tlens;
+  float *mag, *sep;
+};
+size_t carve_waves(const avsep_handle* h, Workspace& w, WaveStaging& st, uint8_t* base, int B, int T, int N, int Hh,
+                   int Ww) {
+  size_t off = carve_workspace(h, w, base, B, T, N, Hh, Ww);
+  auto take = [&](size_t bytes) {
+    void* p = base ? base + off : nullptr;
+    off += align_up(bytes, 1024);
+    return p;
+  };
+  const size_t FT = static_cast<size_t>(h->cfg.freq_bins) * T;
+  st.spec = static_cast<float*>(take(B * FT * 8));
+  st.masks = static_cast<float*>(take(B * h->cfg.num_speakers * FT * 4));
+  st.tlens = static_cast<int32_t*>(take(static_cast<size_t>(B) * 4));
+  st.mag = static_cast<float*>(take(B * FT * 4));
+  st.sep = static_cast<float*>(take(B * h->cfg.num_speakers * FT * 4));
+  return off;
+}
+
 // Padded staging of a packed batch: the varlen forward's inputs and outputs, (B, F, T), (B, N, Hh, Ww) and 2 x
 // (B, S, F, T), carved behind the forward's own workspace.  Returns the bytes of both.
 struct Staging {
@@ -568,11 +595,12 @@ int encoder_stack(avsep_handle* h, LaunchCtx lc, const std::vector<LayerW>& laye
 // AudioEncoder up to (not including) the transformer: Conv1d+ReLU x2, +PE (model.py:56-58), then the first
 // layer's LayerNorm: x_a (fp32) and a_op = LN_{layer0.norm1}(x_a).
 // pl.stack_a: the stack kernel computes the first LayerNorm itself, so only the fp32 residual rows are written, and with
-// pl.pro it runs Conv1d #2 + ReLU + PE too, on h1.
-int audio_frontend(avsep_handle* h, LaunchCtx lc, Workspace& w, const float* mixed, const Plan& pl) {
+// pl.pro it runs Conv1d #2 + ReLU + PE too, on h1.  xp_ready: the STFT has already written w.xp.
+int audio_frontend(avsep_handle* h, LaunchCtx lc, Workspace& w, const float* mixed, const Plan& pl,
+                   bool xp_ready = false) {
   const int d = h->cfg.d_model, F = h->cfg.freq_bins, B = w.B, T = w.T, prec = h->cfg.precision;
   const int Map = B * (T + 2);
-  CKL("prep_audio", lc, launch_prep_audio, prec, mixed, w.xp, B, F, T, h->Fp, w.lens);
+  if (!xp_ready) CKL("prep_audio", lc, launch_prep_audio, prec, mixed, w.xp, B, F, T, h->Fp, w.lens);
   {
     GemmProblem p{};
     p.A = w.xp; p.lda = h->Fp; p.rowsA = Map; p.M = Map; p.W = h->wc1; p.ldw = 3 * h->Fp; p.N = d; p.K = h->Fp;
@@ -705,8 +733,11 @@ int decoder_stage(avsep_handle* h, LaunchCtx lc, Workspace& w, const float* mixe
   return 0;
 }
 
+// xp_ready (avsep_separate_waveforms): w.xp already holds the Conv1d operand, so prep_audio is not launched, and the
+// per-layer decoder (EPI_TAIL) writes masks only.  The fused fusion + decoder kernel keeps reading `mixed` and writing
+// `separated` (staging): its masks-only variant measured 3x slower on a B200.  The Plan is the same either way.
 int forward_device(avsep_handle* h, LaunchCtx lc, Workspace& w, const float* mixed, const float* frames,
-                   float* separated, float* masks) {
+                   float* separated, float* masks, bool xp_ready = false) {
   const int d = h->cfg.d_model;
   const int Ma = w.B * w.T, Mv = w.B * w.N;
   const Plan pl = forward_plan(h, w.T, w.N);
@@ -742,7 +773,7 @@ int forward_device(avsep_handle* h, LaunchCtx lc, Workspace& w, const float* mix
   }
   if (snapshot(h, sv.stream, "visual_enc", w.x_v, static_cast<size_t>(Mv) * d, false)) return 1;
   // --- audio branch ---
-  if (audio_frontend(h, lc, w, mixed, pl)) return 1;
+  if (audio_frontend(h, lc, w, mixed, pl, xp_ready)) return 1;
   if (pl.stack_a) {
     StackProblem sp{};
     sp.x_in = w.x_a; sp.out_x = w.x_a; sp.out_op = pl.stack_f ? nullptr : w.a_op;
@@ -764,15 +795,17 @@ int forward_device(avsep_handle* h, LaunchCtx lc, Workspace& w, const float* mix
   }
   // --- fusion + decoder ---
   if (pl.stack_f ? fusion_stack_fused(h, lc, w, pl, mixed, separated, masks) : fusion_stack(h, lc, w, w.N)) return 1;
-  return pl.dec ? 0 : decoder_stage(h, lc, w, mixed, separated, masks);
+  return pl.dec ? 0 : decoder_stage(h, lc, w, xp_ready ? nullptr : mixed, xp_ready ? nullptr : separated, masks);
 }
 
 // Eager on the first use of a (shape, buffer set); captured into a CUDA graph on the second; replayed afterwards.
 // The graph bakes in the kernel parameters (tensor maps included), so a replay costs one host call.
 int forward_cached(avsep_handle* h, LaunchCtx lc, Workspace& w, const void* ws_base, const float* mixed,
-                   const float* frames, float* separated, float* masks) {
-  if (!h->use_graph || h->profile || h->debug) return forward_device(h, lc, w, mixed, frames, separated, masks);
-  const GraphKey key{w.B, w.T, w.N, w.Hh, w.Ww, mixed, frames, separated, masks, ws_base, w.lens, w.frame_lens};
+                   const float* frames, float* separated, float* masks, bool xp_ready = false) {
+  if (!h->use_graph || h->profile || h->debug)
+    return forward_device(h, lc, w, mixed, frames, separated, masks, xp_ready);
+  const GraphKey key{w.B, w.T, w.N, w.Hh, w.Ww, mixed, frames, separated, masks, ws_base, w.lens, w.frame_lens,
+                     xp_ready};
   GraphEntry* ent = nullptr;
   for (auto& g : h->graphs)
     if (g.key == key) { ent = &g; break; }
@@ -787,14 +820,14 @@ int forward_cached(avsep_handle* h, LaunchCtx lc, Workspace& w, const void* ws_b
     g.key = key;
     g.last_use = ++h->graph_clock;
     h->graphs.push_back(std::move(g));
-    return forward_device(h, lc, w, mixed, frames, separated, masks);   // warm-up, also sets kernel attributes
+    return forward_device(h, lc, w, mixed, frames, separated, masks, xp_ready);   // warm-up, also sets kernel attributes
   }
   ent->last_use = ++h->graph_clock;
   if (ent->exec == nullptr) {   // the capture counts the launches it records; a replay adds them
     const int64_t before = h->launches;
     CUDA_OK(make_stream(h->cap_stream));
     CUDA_OK(cudaStreamBeginCapture(h->cap_stream.get(), cudaStreamCaptureModeRelaxed));
-    const int rc = forward_device(h, {h->cap_stream.get(), lc.pdl}, w, mixed, frames, separated, masks);
+    const int rc = forward_device(h, {h->cap_stream.get(), lc.pdl}, w, mixed, frames, separated, masks, xp_ready);
     cudaGraph_t graph = nullptr;
     const cudaError_t ce = cudaStreamEndCapture(h->cap_stream.get(), &graph);
     if (rc != 0) {
@@ -829,6 +862,36 @@ int forward_packed_run(avsep_handle* h, LaunchCtx lc, Workspace& w, const Stagin
   if (forward_cached(h, lc, w, ws_base, st.mixed, st.frames, st.sep, st.masks)) return 1;
   CKL("pack", lc, launch_pack, st.sep, st.masks, lens, b0, w.B, S, F, w.T, sep_p, masks_p);
   return 0;
+}
+
+// Waveforms in, waveforms out on the device (avsep_separate_waveforms): the STFT writes the complex spectrum and the
+// magnitude to the staging and the Conv1d operand to w.xp (and T_b to st.tlens when lens is given), the forward (cached
+// graph) runs without prep_audio (forward_device's xp_ready), the masked inverse writes waves_out.  masks == null: the
+// masks go to the staging.  lens: DEVICE sample lengths, flens: DEVICE lip-frame lengths, or null.  Sets w.lens /
+// w.frame_lens.
+int waves_run(avsep_handle* h, LaunchCtx lc, Workspace& w, const WaveStaging& st, const void* ws_base,
+              const float* waves, const float* frames, const int* lens, const int* flens, int L, int n_fft, int hop,
+              float* waves_out, float* masks) {
+  float* const mk = masks ? masks : st.masks;
+  CKL("stft", lc.stream, launch_stft, waves, lens, w.B, 0, L, n_fft, hop, st.spec, st.mag, nullptr,
+      lens ? st.tlens : nullptr, w.xp, h->Fp, h->cfg.precision);
+  w.lens = lens ? st.tlens : nullptr;
+  w.frame_lens = flens;
+  if (forward_cached(h, lc, w, ws_base, st.mag, frames, st.sep, mk, true)) return 1;
+  CKL("istft", lc.stream, launch_istft_masked, st.spec, mk, lens, w.B, h->cfg.num_speakers, w.T, n_fft, hop, L,
+      waves_out);
+  return 0;
+}
+
+// Geometry of a waveform call: sets T = 1 + L / hop and checks it as check_shape does.
+int check_waves(avsep_handle* h, const char* who, int B, int L, int N, int Hh, int Ww, int n_fft, int hop, int& T) {
+  if (B < 1 || L < 1) return fail(h, std::string(who) + ": empty input: B and L must be >= 1");
+  if (n_fft != 2 * (h->cfg.freq_bins - 1))
+    return fail(h, std::string(who) + ": n_fft must be 2 * (freq_bins - 1) = " + std::to_string(2 * (h->cfg.freq_bins - 1)));
+  if (!fft_geometry_ok(n_fft, hop))
+    return fail(h, std::string(who) + ": n_fft must be a power of two in [8, 2048], 1 <= hop <= n_fft");
+  T = 1 + L / hop;
+  return check_shape(h, B, T, N, Hh, Ww);
 }
 
 // ---- weight access helpers ---------------------------------------------------------------------
@@ -1216,52 +1279,61 @@ int avsep_forward_packed(avsep_handle* h, const float* mixed_packed, const float
 }
 
 namespace {
-// packed: the buffers hold packed batches (include/avsep.h) with HOST lengths lens / flens (null: all T / all N); each
-// chunk's copies then cover its packed span and its kernels are forward_packed_run's.
-int host_submit(avsep_handle* h, const float* mixed_spec, const float* lip_frames, int B, int T, int N, int Hh, int Ww,
-                float* separated, float* masks, int slot_id, cudaStream_t s, bool streaming, bool packed = false,
-                const int32_t* lens = nullptr, const int32_t* flens = nullptr) {
+// A host tensor of a host-buffer call and the element offsets of its utterances: utterances [b0, b1) are the span
+// [at[b0], at[b1]) (packed or padded).
+struct HostIn {
+  const float* host;
+  std::vector<size_t> at;
+};
+struct HostOut {
+  float* host;
+  std::vector<size_t> at;
+};
+std::vector<size_t> padded_at(int B, size_t per) {
+  std::vector<size_t> at(B + 1);
+  for (int b = 0; b <= B; ++b) at[b] = b * per;
+  return at;
+}
+
+// What distinguishes the host-buffer forms (padded, packed and waveform forward): the spans each chunk copies in and
+// out - input i is mirrored by the slot's device buffer io[i], output j by io[in.size() + j] - and the chunk's device
+// step.  Slots, events, lanes and the chunk / lane choice are host_submit's.
+struct HostCall {
+  std::string who;
+  int B = 0;
+  std::vector<HostIn> in;
+  std::vector<HostOut> out;
+  std::vector<int32_t> lens;   // uploaded once per call to the slot's lens_dev (empty: nothing to upload)
+  // workspace bytes of one compute lane that runs chunks of up to Bc utterances
+  std::function<size_t(int Bc)> lane_bytes;
+  // enqueues utterances [b0, b0 + bc) on lc with the lane's workspace ws (carved for Bc), the slot's device buffers io
+  // and the uploaded lengths (or null)
+  std::function<int(LaunchCtx lc, uint8_t* ws, int Bc, int b0, int bc, float* const* io, const int32_t* lens)> step;
+};
+
+int host_submit(avsep_handle* h, const HostCall& c, int slot_id, cudaStream_t s, bool streaming) {
   // Software pipeline over chunks of the batch: H2D of chunk i+1, kernels of chunk i and D2H of chunk i-1 run
   // concurrently on separate streams (PCIe is full duplex), so a call costs ~max(copy-in, compute, copy-out); the
-  // two slots extend the same pipeline across consecutive calls.
-  const std::string who = packed ? "avsep_forward_host_packed" : "avsep_forward_host";
-  if (!mixed_spec || !lip_frames || !separated || !masks) return fail(h, who + ": null buffer");
-  if (slot_id < 0 || slot_id >= AVSEP_HOST_SLOTS) return fail(h, who + "_async: slot must be 0 .. AVSEP_HOST_SLOTS - 1");
-  if (check_shape(h, B, T, N, Hh, Ww)) return 1;
-  // packed spans: utterances [0, b) hold t_at(b) audio and n_at(b) lip frames; host lengths size the copies, so a
-  // value out of range is an error here, not clamped
-  std::vector<size_t> pt, pn;
-  if (packed) {
-    pt.assign(B + 1, 0);
-    pn.assign(B + 1, 0);
-    for (int b = 0; b < B; ++b) {
-      const int tb = lens ? lens[b] : T, nb = flens ? flens[b] : N;
-      if (tb < 1 || tb > T || nb < 1 || nb > N)
-        return fail(h, who + ": lengths[" + std::to_string(b) + "] = " + std::to_string(tb) + ", frame_lengths[" +
-                           std::to_string(b) + "] = " + std::to_string(nb) + " outside [1, T] / [1, N]");
-      pt[b + 1] = pt[b] + tb;
-      pn[b + 1] = pn[b] + nb;
-    }
-  }
-  auto t_at = [&](size_t b) { return packed ? pt[b] : b * T; };
-  auto n_at = [&](size_t b) { return packed ? pn[b] : b * N; };
+  // slots extend the same pipeline across consecutive calls.
+  if (slot_id < 0 || slot_id >= AVSEP_HOST_SLOTS) return fail(h, c.who + "_async: slot must be 0 .. AVSEP_HOST_SLOTS - 1");
+  const int B = c.B;
   avsep_handle::HostSlot& sl = h->slot[slot_id];
-  const size_t F = h->cfg.freq_bins, S = h->cfg.num_speakers;
-  const size_t mixed_per = F * T, frames_per = static_cast<size_t>(N) * Hh * Ww, out_per = S * F * T;
-  const size_t need[4] = {B * mixed_per, B * frames_per, B * out_per, B * out_per};
-  for (int i = 0; i < 4; ++i) {
-    if (sl.io[i].cap < need[i]) {
+  const size_t nin = c.in.size(), nio = nin + c.out.size();
+  for (size_t i = 0; i < nio; ++i) {
+    const size_t need = i < nin ? c.in[i].at[B] : c.out[i - nin].at[B];
+    if (sl.io[i].cap < need) {
       if (sl.ev_end) CUDA_OK(cudaEventSynchronize(sl.ev_end.get()));   // the slot's previous call still owns the buffer
-      CUDA_OK(sl.io[i].alloc(need[i]));
+      CUDA_OK(sl.io[i].alloc(need));
     }
   }
-  float *io_mixed = sl.io[0].get(), *io_frames = sl.io[1].get(), *io_sep = sl.io[2].get(), *io_masks = sl.io[3].get();
+  float* io[4];
+  for (int i = 0; i < 4; ++i) io[i] = sl.io[i].get();
   for (Stream& st : h->hs) CUDA_OK(make_stream(st));
   CUDA_OK(make_event(sl.ev_start));
   CUDA_OK(make_event(sl.ev_end));
-  const bool upload = packed && (lens || flens);
+  const bool upload = !c.lens.empty();
   if (upload) {
-    const size_t n = 2 * static_cast<size_t>(B);   // the call's lengths, then its frame lengths
+    const size_t n = c.lens.size();
     if (sl.lens_dev.cap < n || sl.lens_host.cap < n) {
       CUDA_OK(cudaEventSynchronize(sl.ev_end.get()));     // the slot's previous call still reads them
       CUDA_OK(sl.lens_dev.alloc(n));
@@ -1269,13 +1341,8 @@ int host_submit(avsep_handle* h, const float* mixed_spec, const float* lip_frame
     }
     CUDA_OK(make_event(sl.ev_lens));
     CUDA_OK(cudaEventSynchronize(sl.ev_lens.get()));      // the previous upload from lens_host has been read
-    for (int b = 0; b < B; ++b) {
-      sl.lens_host.get()[b] = lens ? lens[b] : T;
-      sl.lens_host.get()[B + b] = flens ? flens[b] : N;
-    }
+    memcpy(sl.lens_host.get(), c.lens.data(), n * sizeof(int32_t));
   }
-  const int32_t* d_lens = upload && lens ? sl.lens_dev.get() : nullptr;
-  const int32_t* d_flens = upload && flens ? sl.lens_dev.get() + B : nullptr;
   // Chunk size: a stack kernel takes as long for 64 utterances as for 256 (one tile per CTA either way), so chunks are
   // a trade between pipelining inside one call and kernel time.  Measured at B = 256 (tools/e2e_probe.py): the one-call
   // form is fastest with ~56-utterance chunks on two compute lanes (copy-in of chunk i+1 under the kernels of chunk i),
@@ -1284,12 +1351,7 @@ int host_submit(avsep_handle* h, const float* mixed_spec, const float* lip_frame
   const int auto_chunk = streaming ? 128 : 56;
   const int want_chunk = h->host_chunk > 0 ? h->host_chunk : auto_chunk;
   const int Bc = want_chunk < B ? want_chunk : B;
-  std::vector<int> starts, sizes;
-  for (int b0 = 0; b0 < B; b0 += Bc) {
-    starts.push_back(b0);
-    sizes.push_back((B - b0) < Bc ? (B - b0) : Bc);
-  }
-  const int nchunks = static_cast<int>(starts.size());
+  const int nchunks = (B + Bc - 1) / Bc;
   while (static_cast<int>(sl.ev.size()) < 2 * nchunks) {
     Event e;
     CUDA_OK(make_event(e));
@@ -1299,21 +1361,13 @@ int host_submit(avsep_handle* h, const float* mixed_spec, const float* lip_frame
   // of consecutive chunks are allowed to overlap
   const int want_lanes = h->host_lanes > 0 ? h->host_lanes : (streaming ? 1 : 2);
   const int lanes = want_lanes > 3 ? 3 : want_lanes;
-  Workspace wl[3];
-  Staging stl[3];
-  const size_t per_lane = packed ? carve_packed(h, wl[0], stl[0], nullptr, Bc, T, N, Hh, Ww)
-                                 : carve_workspace(h, wl[0], nullptr, Bc, T, N, Hh, Ww);
+  const size_t per_lane = c.lane_bytes(Bc);
   if (h->host_ws.cap < per_lane * lanes) {
     CUDA_OK(cudaDeviceSynchronize());          // the other slot may still be using the old workspace
     drop_graphs(h);                            // the cached graphs hold pointers into it
     CUDA_OK(h->host_ws.alloc(per_lane * lanes));
   }
   for (int l = 0; l < lanes; ++l) {
-    uint8_t* lane_base = h->host_ws.get() + l * per_lane;
-    if (packed)
-      carve_packed(h, wl[l], stl[l], lane_base, Bc, T, N, Hh, Ww);
-    else
-      carve_workspace(h, wl[l], lane_base, Bc, T, N, Hh, Ww);
     CUDA_OK(make_stream(h->host_comp[l]));
     CUDA_OK(make_event(sl.ev_lane[l]));
   }
@@ -1330,35 +1384,30 @@ int host_submit(avsep_handle* h, const float* mixed_spec, const float* lip_frame
   }
   CUDA_OK(cudaStreamWaitEvent(s_out, sl.ev_start.get(), 0));
   if (upload) {
-    CUDA_OK(cudaMemcpyAsync(sl.lens_dev.get(), sl.lens_host.get(), 2 * sizeof(int32_t) * B, cudaMemcpyHostToDevice,
-                            s_in));
+    CUDA_OK(cudaMemcpyAsync(sl.lens_dev.get(), sl.lens_host.get(), sizeof(int32_t) * c.lens.size(),
+                            cudaMemcpyHostToDevice, s_in));
     CUDA_OK(cudaEventRecord(sl.ev_lens.get(), s_in));
   }
-  const size_t HW = static_cast<size_t>(Hh) * Ww, SF = S * F;
-  for (int c = 0; c < nchunks; ++c) {
-    const size_t b0 = starts[c];
-    const int bc = sizes[c];
-    const int lane = c % lanes;
+  for (int ci = 0; ci < nchunks; ++ci) {
+    const int b0 = ci * Bc, bc = B - b0 < Bc ? B - b0 : Bc;
+    const int lane = ci % lanes;
     const LaunchCtx comp = launch_ctx(h, h->host_comp[lane].get());
-    // element offsets and counts of the chunk's span in each tensor (packed or padded)
-    const size_t m0 = F * t_at(b0), mn = F * (t_at(b0 + bc) - t_at(b0));
-    const size_t f0 = HW * n_at(b0), fn = HW * (n_at(b0 + bc) - n_at(b0));
-    const size_t o0 = SF * t_at(b0), on = SF * (t_at(b0 + bc) - t_at(b0));
-    CUDA_OK(cudaMemcpyAsync(io_mixed + m0, mixed_spec + m0, mn * 4, cudaMemcpyHostToDevice, s_in));
-    CUDA_OK(cudaMemcpyAsync(io_frames + f0, lip_frames + f0, fn * 4, cudaMemcpyHostToDevice, s_in));
-    CUDA_OK(cudaEventRecord(sl.ev[2 * c].get(), s_in));
-    CUDA_OK(cudaStreamWaitEvent(comp.stream, sl.ev[2 * c].get(), 0));
-    Workspace wc = wl[lane];
-    wc.B = bc;
-    const uint8_t* ws_lane = h->host_ws.get() + lane * per_lane;
-    if (packed ? forward_packed_run(h, comp, wc, stl[lane], ws_lane, io_mixed, io_frames, d_lens, d_flens,
-                                    static_cast<int>(b0), io_sep, io_masks)
-               : forward_cached(h, comp, wc, ws_lane, io_mixed + m0, io_frames + f0, io_sep + o0, io_masks + o0))
+    for (size_t i = 0; i < nin; ++i) {
+      const std::vector<size_t>& at = c.in[i].at;
+      CUDA_OK(cudaMemcpyAsync(io[i] + at[b0], c.in[i].host + at[b0], (at[b0 + bc] - at[b0]) * 4,
+                              cudaMemcpyHostToDevice, s_in));
+    }
+    CUDA_OK(cudaEventRecord(sl.ev[2 * ci].get(), s_in));
+    CUDA_OK(cudaStreamWaitEvent(comp.stream, sl.ev[2 * ci].get(), 0));
+    if (c.step(comp, h->host_ws.get() + lane * per_lane, Bc, b0, bc, io, upload ? sl.lens_dev.get() : nullptr))
       return 1;
-    CUDA_OK(cudaEventRecord(sl.ev[2 * c + 1].get(), comp.stream));
-    CUDA_OK(cudaStreamWaitEvent(s_out, sl.ev[2 * c + 1].get(), 0));
-    CUDA_OK(cudaMemcpyAsync(separated + o0, io_sep + o0, on * 4, cudaMemcpyDeviceToHost, s_out));
-    CUDA_OK(cudaMemcpyAsync(masks + o0, io_masks + o0, on * 4, cudaMemcpyDeviceToHost, s_out));
+    CUDA_OK(cudaEventRecord(sl.ev[2 * ci + 1].get(), comp.stream));
+    CUDA_OK(cudaStreamWaitEvent(s_out, sl.ev[2 * ci + 1].get(), 0));
+    for (size_t j = 0; j < c.out.size(); ++j) {
+      const std::vector<size_t>& at = c.out[j].at;
+      CUDA_OK(cudaMemcpyAsync(c.out[j].host + at[b0], io[nin + j] + at[b0], (at[b0 + bc] - at[b0]) * 4,
+                              cudaMemcpyDeviceToHost, s_out));
+    }
   }
   for (int l = 0; l < lanes; ++l) CUDA_OK(cudaEventRecord(sl.ev_lane[l].get(), h->host_comp[l].get()));
   // The caller's stream is deliberately NOT made to wait for the results: that would chain call i+1 (which is ordered
@@ -1366,12 +1415,111 @@ int host_submit(avsep_handle* h, const float* mixed_spec, const float* lip_frame
   CUDA_OK(cudaEventRecord(sl.ev_end.get(), s_out));
   return 0;
 }
+
+// The spectrogram forms.  packed: the buffers hold packed batches (include/avsep.h) with HOST lengths lens / flens
+// (null: all T / all N); each chunk's copies then cover its packed span and its kernels are forward_packed_run's.
+int host_spec_call(avsep_handle* h, HostCall& c, const float* mixed_spec, const float* lip_frames, int B, int T, int N,
+                   int Hh, int Ww, float* separated, float* masks, bool packed = false, const int32_t* lens = nullptr,
+                   const int32_t* flens = nullptr) {
+  c.who = packed ? "avsep_forward_host_packed" : "avsep_forward_host";
+  if (!mixed_spec || !lip_frames || !separated || !masks) return fail(h, c.who + ": null buffer");
+  if (check_shape(h, B, T, N, Hh, Ww)) return 1;
+  // packed spans: utterances [0, b) hold pt[b] audio and pn[b] lip frames; host lengths size the copies, so a value
+  // out of range is an error here, not clamped
+  std::vector<size_t> pt = padded_at(B, T), pn = padded_at(B, N);
+  if (packed) {
+    for (int b = 0; b < B; ++b) {
+      const int tb = lens ? lens[b] : T, nb = flens ? flens[b] : N;
+      if (tb < 1 || tb > T || nb < 1 || nb > N)
+        return fail(h, c.who + ": lengths[" + std::to_string(b) + "] = " + std::to_string(tb) + ", frame_lengths[" +
+                           std::to_string(b) + "] = " + std::to_string(nb) + " outside [1, T] / [1, N]");
+      pt[b + 1] = pt[b] + tb;
+      pn[b + 1] = pn[b] + nb;
+    }
+    if (lens || flens) {   // the call's lengths, then its frame lengths
+      c.lens.resize(2 * static_cast<size_t>(B));
+      for (int b = 0; b < B; ++b) {
+        c.lens[b] = lens ? lens[b] : T;
+        c.lens[B + b] = flens ? flens[b] : N;
+      }
+    }
+  }
+  auto scaled = [](std::vector<size_t> at, size_t k) {
+    for (size_t& v : at) v *= k;
+    return at;
+  };
+  const size_t F = h->cfg.freq_bins, SF = h->cfg.num_speakers * F, HW = static_cast<size_t>(Hh) * Ww;
+  c.B = B;
+  c.in = {{mixed_spec, scaled(pt, F)}, {lip_frames, scaled(pn, HW)}};
+  c.out = {{separated, scaled(pt, SF)}, {masks, scaled(pt, SF)}};
+  const bool has_lens = lens != nullptr, has_flens = flens != nullptr;
+  if (packed) {
+    c.lane_bytes = [=](int Bc) {
+      Workspace w;
+      Staging st;
+      return carve_packed(h, w, st, nullptr, Bc, T, N, Hh, Ww);
+    };
+    c.step = [=](LaunchCtx lc, uint8_t* ws, int Bc, int b0, int bc, float* const* io, const int32_t* d_lens) {
+      Workspace w;
+      Staging st;
+      carve_packed(h, w, st, ws, Bc, T, N, Hh, Ww);
+      w.B = bc;
+      return forward_packed_run(h, lc, w, st, ws, io[0], io[1], has_lens ? d_lens : nullptr,
+                                has_flens ? d_lens + B : nullptr, b0, io[2], io[3]);
+    };
+  } else {
+    c.lane_bytes = [=](int Bc) {
+      Workspace w;
+      return carve_workspace(h, w, nullptr, Bc, T, N, Hh, Ww);
+    };
+    c.step = [=](LaunchCtx lc, uint8_t* ws, int Bc, int b0, int bc, float* const* io, const int32_t*) {
+      Workspace w;
+      carve_workspace(h, w, ws, Bc, T, N, Hh, Ww);
+      w.B = bc;
+      const size_t o = SF * T * b0;
+      return forward_cached(h, lc, w, ws, io[0] + F * T * b0, io[1] + HW * N * b0, io[2] + o, io[3] + o);
+    };
+  }
+  return 0;
+}
+
+// The waveform form (full batches): samples and lip frames in, separated samples (and the masks when masks != null) out.
+int host_wave_call(avsep_handle* h, HostCall& c, const float* waves, const float* lip_frames, int B, int L, int N,
+                   int Hh, int Ww, int n_fft, int hop, float* waves_out, float* masks) {
+  c.who = "avsep_separate_waveforms_host";
+  if (!waves || !lip_frames || !waves_out) return fail(h, c.who + ": null buffer");
+  int T = 0;
+  if (check_waves(h, c.who.c_str(), B, L, N, Hh, Ww, n_fft, hop, T)) return 1;
+  const size_t S = h->cfg.num_speakers, SFT = S * h->cfg.freq_bins * T, HW = static_cast<size_t>(Hh) * Ww;
+  c.B = B;
+  c.in = {{waves, padded_at(B, L)}, {lip_frames, padded_at(B, N * HW)}};
+  c.out = {{waves_out, padded_at(B, S * L)}};
+  if (masks) c.out.push_back({masks, padded_at(B, SFT)});
+  c.lane_bytes = [=](int Bc) {
+    Workspace w;
+    WaveStaging st;
+    return carve_waves(h, w, st, nullptr, Bc, T, N, Hh, Ww);
+  };
+  const bool want_masks = masks != nullptr;
+  c.step = [=](LaunchCtx lc, uint8_t* ws, int Bc, int b0, int bc, float* const* io, const int32_t*) {
+    Workspace w;
+    WaveStaging st;
+    carve_waves(h, w, st, ws, Bc, T, N, Hh, Ww);
+    w.B = bc;
+    return waves_run(h, lc, w, st, ws, io[0] + static_cast<size_t>(L) * b0, io[1] + N * HW * b0, nullptr, nullptr, L,
+                     n_fft, hop, io[2] + S * L * b0, want_masks ? io[3] + SFT * b0 : nullptr);
+  };
+  return 0;
+}
 }  // namespace
 
 int avsep_forward_host(avsep_handle* h, const float* mixed_spec, const float* lip_frames, int32_t B, int32_t T,
                        int32_t N, int32_t Hh, int32_t Ww, float* separated, float* masks, void* cuda_stream) {
   ENTER(h, cuda_stream);
-  if (host_submit(h, mixed_spec, lip_frames, B, T, N, Hh, Ww, separated, masks, 0, lc.stream, false)) return 1;
+  HostCall c;
+  if (host_spec_call(h, c, mixed_spec, lip_frames, B, T, N, Hh, Ww, separated, masks) ||
+      host_submit(h, c, 0, lc.stream, false))
+    return 1;
   CUDA_OK(cudaEventSynchronize(h->slot[0].ev_end.get()));
   return 0;
 }
@@ -1380,15 +1528,19 @@ int avsep_forward_host_async(avsep_handle* h, const float* mixed_spec, const flo
                              int32_t N, int32_t Hh, int32_t Ww, float* separated, float* masks, int32_t slot,
                              void* cuda_stream) {
   ENTER(h, cuda_stream);
-  return host_submit(h, mixed_spec, lip_frames, B, T, N, Hh, Ww, separated, masks, slot, lc.stream, true);
+  HostCall c;
+  if (host_spec_call(h, c, mixed_spec, lip_frames, B, T, N, Hh, Ww, separated, masks)) return 1;
+  return host_submit(h, c, slot, lc.stream, true);
 }
 
 int avsep_forward_host_packed(avsep_handle* h, const float* mixed_packed, const float* frames_packed,
                               const int32_t* lengths, const int32_t* frame_lengths, int32_t B, int32_t T, int32_t N,
                               int32_t Hh, int32_t Ww, float* separated_packed, float* masks_packed, void* cuda_stream) {
   ENTER(h, cuda_stream);
-  if (host_submit(h, mixed_packed, frames_packed, B, T, N, Hh, Ww, separated_packed, masks_packed, 0, lc.stream, false,
-                  true, lengths, frame_lengths))
+  HostCall c;
+  if (host_spec_call(h, c, mixed_packed, frames_packed, B, T, N, Hh, Ww, separated_packed, masks_packed, true, lengths,
+                     frame_lengths) ||
+      host_submit(h, c, 0, lc.stream, false))
     return 1;
   CUDA_OK(cudaEventSynchronize(h->slot[0].ev_end.get()));
   return 0;
@@ -1399,8 +1551,62 @@ int avsep_forward_host_packed_async(avsep_handle* h, const float* mixed_packed, 
                                     int32_t N, int32_t Hh, int32_t Ww, float* separated_packed, float* masks_packed,
                                     int32_t slot, void* cuda_stream) {
   ENTER(h, cuda_stream);
-  return host_submit(h, mixed_packed, frames_packed, B, T, N, Hh, Ww, separated_packed, masks_packed, slot, lc.stream,
-                     true, true, lengths, frame_lengths);
+  HostCall c;
+  if (host_spec_call(h, c, mixed_packed, frames_packed, B, T, N, Hh, Ww, separated_packed, masks_packed, true, lengths,
+                     frame_lengths))
+    return 1;
+  return host_submit(h, c, slot, lc.stream, true);
+}
+
+size_t avsep_waveform_workspace_bytes(avsep_handle* h, int32_t B, int32_t L, int32_t N, int32_t Hh, int32_t Ww,
+                                      int32_t n_fft, int32_t hop_length) {
+  if (!h || B < 1 || L < 1 || N < 1 || Hh < 1 || Ww < 1 || !fft_geometry_ok(n_fft, hop_length) ||
+      n_fft != 2 * (h->cfg.freq_bins - 1))
+    return 0;
+  Workspace w;
+  WaveStaging st;
+  return carve_waves(h, w, st, nullptr, B, 1 + L / hop_length, N, Hh, Ww);
+}
+
+int avsep_separate_waveforms(avsep_handle* h, const float* waves, const float* lip_frames, const int32_t* lengths,
+                             const int32_t* frame_lengths, int32_t B, int32_t L, int32_t N, int32_t Hh, int32_t Ww,
+                             int32_t n_fft, int32_t hop_length, float* waves_out, float* masks, void* workspace,
+                             size_t workspace_bytes, void* cuda_stream) {
+  ENTER(h, cuda_stream);
+  if (!waves || !lip_frames || !waves_out) return fail(h, "avsep_separate_waveforms: null buffer");
+  int T = 0;
+  if (check_waves(h, "avsep_separate_waveforms", B, L, N, Hh, Ww, n_fft, hop_length, T)) return 1;
+  Workspace w;
+  WaveStaging st;
+  uint8_t* base = nullptr;
+  if (workspace_base(h, workspace, workspace_bytes, carve_waves(h, w, st, nullptr, B, T, N, Hh, Ww),
+                     "avsep_waveform_workspace_bytes", base))
+    return 1;
+  carve_waves(h, w, st, base, B, T, N, Hh, Ww);
+  return waves_run(h, lc, w, st, base, waves, lip_frames, lengths, frame_lengths, L, n_fft, hop_length, waves_out,
+                   masks);
+}
+
+int avsep_separate_waveforms_host(avsep_handle* h, const float* waves, const float* lip_frames, int32_t B, int32_t L,
+                                  int32_t N, int32_t Hh, int32_t Ww, int32_t n_fft, int32_t hop_length,
+                                  float* waves_out, float* masks, void* cuda_stream) {
+  ENTER(h, cuda_stream);
+  HostCall c;
+  if (host_wave_call(h, c, waves, lip_frames, B, L, N, Hh, Ww, n_fft, hop_length, waves_out, masks) ||
+      host_submit(h, c, 0, lc.stream, false))
+    return 1;
+  CUDA_OK(cudaEventSynchronize(h->slot[0].ev_end.get()));
+  return 0;
+}
+
+int avsep_separate_waveforms_host_async(avsep_handle* h, const float* waves, const float* lip_frames, int32_t B,
+                                        int32_t L, int32_t N, int32_t Hh, int32_t Ww, int32_t n_fft,
+                                        int32_t hop_length, float* waves_out, float* masks, int32_t slot,
+                                        void* cuda_stream) {
+  ENTER(h, cuda_stream);
+  HostCall c;
+  if (host_wave_call(h, c, waves, lip_frames, B, L, N, Hh, Ww, n_fft, hop_length, waves_out, masks)) return 1;
+  return host_submit(h, c, slot, lc.stream, true);
 }
 
 int avsep_host_wait(avsep_handle* h, int32_t slot) {

@@ -17,6 +17,7 @@
 // Epilogues (template EPI):
 //   EPI_STD  bias / ReLU / exact GELU / positional-encoding add / Conv1d halo handling, fp32 and/or bf16 stores
 //   EPI_TAIL SeparationDecoder head: sigmoid, x mixed_spec, (B,S,F,T) stores coalesced along T (model.py:204-220)
+//   EPI_TAIL_MASKS  the same head without the mixed_spec loads and the `separated` stores (masks only)
 //   EPI_LN   EPI_STD value + residual add, write the fp32 residual stream, then LayerNorm of the full row
 //            (n_tile == N == d_model <= 256, row held in registers, exact two-pass statistics merged across the
 //            two column halves) and write the normalised bf16 operand of the next GEMM -- the fused
@@ -250,6 +251,7 @@ __device__ __forceinline__ void value_chunk(const GemmEpilogue& e, const RowInfo
 // Whole chunks that do not cross a speaker boundary take branch-free bodies - the per-element guards and the frequency
 // wrap cost more instructions than the sigmoid.  All tests except `valid` are warp-uniform.
 // live == false: the row lies past its utterance's length; mixed_spec is not read there and both outputs are 0.
+// SEP == false (EPI_TAIL_MASKS): masks only; tail_load16 is not called and tail_store16 ignores mx.
 __device__ __forceinline__ void tail_load16(const GemmEpilogue& e, int N, int col0, const float* mixed_row, bool valid,
                                             bool live, float (&mx)[16]) {
   const int ncols = min(16, N - col0);
@@ -273,18 +275,19 @@ __device__ __forceinline__ void tail_load16(const GemmEpilogue& e, int N, int co
   }
 }
 
+template <bool SEP>
 __device__ __forceinline__ void tail_store16(const GemmEpilogue& e, int N, int col0, size_t out_base, bool valid,
                                              bool live, const uint32_t (&v)[16], const float* sb, const float (&mx)[16]) {
   const int ncols = min(16, N - col0);
   if (!valid || ncols <= 0) return;
   float* mo = e.masks + out_base + static_cast<size_t>(col0) * e.T;
-  float* so = e.separated + out_base + static_cast<size_t>(col0) * e.T;
+  float* so = SEP ? e.separated + out_base + static_cast<size_t>(col0) * e.T : nullptr;
   if (ncols == 16) {
 #pragma unroll
     for (int j = 0; j < 16; ++j) {
       const float mk = live ? sigmoid_fast(__uint_as_float(v[j]) + sb[j]) : 0.f;
       __stcs(mo + static_cast<size_t>(j) * e.T, mk);
-      __stcs(so + static_cast<size_t>(j) * e.T, mk * mx[j]);
+      if constexpr (SEP) __stcs(so + static_cast<size_t>(j) * e.T, mk * mx[j]);
     }
   } else {
 #pragma unroll
@@ -292,7 +295,7 @@ __device__ __forceinline__ void tail_store16(const GemmEpilogue& e, int N, int c
       if (j < ncols) {
         const float mk = live ? sigmoid_fast(__uint_as_float(v[j]) + sb[j]) : 0.f;
         __stcs(mo + static_cast<size_t>(j) * e.T, mk);
-        __stcs(so + static_cast<size_t>(j) * e.T, mk * mx[j]);
+        if constexpr (SEP) __stcs(so + static_cast<size_t>(j) * e.T, mk * mx[j]);
       }
     }
   }
@@ -328,6 +331,8 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
   const int m_tiles = (p.M + BM - 1) / BM;
   const int n_tiles = (p.N + p.n_tile - 1) / p.n_tile;
   const int total_tiles = m_tiles * n_tiles;
+  constexpr bool TAIL = EPI == EPI_TAIL || EPI == EPI_TAIL_MASKS;
+  constexpr bool SEP = EPI == EPI_TAIL;          // the tail also reads mixed_spec and writes `separated`
 
   if (threadIdx.x == 0) {
     TRACE(0);                                  // kernel entry
@@ -440,7 +445,7 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
       const int m = m0 + r;
       // stage this tile's bias slice in shared memory while the main loop is still running
       float* sb = sbias + (lt & 1) * BN_MAX;
-      if constexpr (EPI != EPI_TAIL) {
+      if constexpr (!TAIL) {
         const int i = threadIdx.x - 64;                       // 0..511 over the 16 epilogue warps
         if (i < BN_MAX) sb[i] = (e.bias != nullptr && i < p.n_tile && n0 + i < p.N) ? __ldg(e.bias + n0 + i) : 0.f;
       }
@@ -459,7 +464,7 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
       size_t t_out_base = 0;
       int t_cbeg = 0, t_cend = 0;
       float mxa[16], mxb[16];
-      if constexpr (EPI == EPI_TAIL) {
+      if constexpr (TAIL) {
         // SeparationDecoder head (model.py:204-207,220): column c = s*F + f, so masks[b,s,f,t] sits at
         // ((b*S*F + c)*T + t); lanes are consecutive t, so the (B,S,F,T) stores and the mixed_spec (B,F,T) loads are
         // both contiguous across the warp.
@@ -467,7 +472,7 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
         const int tb = m / e.T;
         const int tt = m - tb * e.T;
         t_live = e.lens == nullptr || (t_valid && tt < utt_len(e.lens, tb, e.T));
-        t_mixed_row = e.mixed + static_cast<size_t>(tb) * e.F * e.T + tt;
+        if constexpr (SEP) t_mixed_row = e.mixed + static_cast<size_t>(tb) * e.F * e.T + tt;
         t_out_base = static_cast<size_t>(tb) * e.S * e.F * e.T + tt;
         // Each column part takes a contiguous, balanced share of the tile in units of 16 columns (176 columns ->
         // 48/48/48/32); handing out whole 32-column chunks round-robin left two parts with twice the work of the
@@ -475,14 +480,14 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
         const int units = p.n_tile >> 4, ubase = units >> 2, urem = units & 3;
         t_cbeg = (part * ubase + min(part, urem)) << 4;
         t_cend = t_cbeg + ((ubase + (part < urem ? 1 : 0)) << 4);
-        if (t_cbeg < t_cend) tail_load16(e, p.N, n0 + t_cbeg, t_mixed_row, t_valid, t_live, mxa);
+        if (SEP && t_cbeg < t_cend) tail_load16(e, p.N, n0 + t_cbeg, t_mixed_row, t_valid, t_live, mxa);
         // each column part stages its own bias slice and synchronises only its 4 warps (same columns, same amount
         // of work): with one 512-thread barrier per tile every part waited ~1.2 us for the slowest of the 16 warps
         const int c = t_cbeg + r;
         if (c < t_cend) sb[c] = (e.bias != nullptr && n0 + c < p.N) ? __ldg(e.bias + n0 + c) : 0.f;
       }
       if (lt == 1 && threadIdx.x == 64) TRACE(2);               // [2] tile-1 epilogue entered (bias load issued)
-      if constexpr (EPI == EPI_TAIL) named_bar_sync(part_bar, 128);
+      if constexpr (TAIL) named_bar_sync(part_bar, 128);
       else asm volatile("bar.sync 5, 512;" ::: "memory");       // bias slice visible to all epilogue warps
       if (lt == 1 && threadIdx.x == 64) TRACE(3);               // [3] bias barrier passed
       mbar_wait(&tfull_bar[acc], aph);
@@ -490,7 +495,7 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
       if (threadIdx.x == 64) TRACE_TILE(lt, 2);     // accumulator ready
       const uint32_t taddr_row = tmem_base + (static_cast<uint32_t>(q * 32) << 16) + static_cast<uint32_t>(acc * BN_MAX);
 
-      if constexpr (EPI == EPI_TAIL) {
+      if constexpr (TAIL) {
         // 16 columns at a time (16 accumulator values + two 16-value mixed_spec buffers stay within the 96 registers
         // this 640-thread CTA allows), two chunks per iteration so that the buffers alternate statically.
         for (int c0 = t_cbeg; c0 < t_cend; c0 += 32) {
@@ -498,14 +503,14 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
           uint32_t v[16];
           tmem_ld_32x32b_x16(taddr_row + static_cast<uint32_t>(c0), v);
           const bool second = c0 + 16 < t_cend;
-          if (second) tail_load16(e, p.N, n0 + c0 + 16, t_mixed_row, t_valid, t_live, mxb);
+          if (SEP && second) tail_load16(e, p.N, n0 + c0 + 16, t_mixed_row, t_valid, t_live, mxb);
           tmem_ld_wait();
-          tail_store16(e, p.N, n0 + c0, t_out_base, t_valid, t_live, v, sb + c0, mxa);
+          tail_store16<SEP>(e, p.N, n0 + c0, t_out_base, t_valid, t_live, v, sb + c0, mxa);
           if (second && n0 + c0 + 16 < p.N) {
             tmem_ld_32x32b_x16(taddr_row + static_cast<uint32_t>(c0 + 16), v);
-            if (c0 + 32 < t_cend) tail_load16(e, p.N, n0 + c0 + 32, t_mixed_row, t_valid, t_live, mxa);
+            if (SEP && c0 + 32 < t_cend) tail_load16(e, p.N, n0 + c0 + 32, t_mixed_row, t_valid, t_live, mxa);
             tmem_ld_wait();
-            tail_store16(e, p.N, n0 + c0 + 16, t_out_base, t_valid, t_live, v, sb + c0 + 16, mxb);
+            tail_store16<SEP>(e, p.N, n0 + c0 + 16, t_out_base, t_valid, t_live, v, sb + c0 + 16, mxb);
           }
         }
       } else if constexpr (EPI == EPI_LN_TMA) {
@@ -986,7 +991,10 @@ const char* launch_gemm(LaunchCtx lc, int prec, const GemmProblem& p, const Gemm
   d.use_tma = use_tma ? 1 : 0;
   switch (e.kind) {
     case EPI_STD: return tf32 ? launch_cfg<EPI_STD, true>(lc, ta, tw, top, tf32m, d, num_sms) : launch_cfg<EPI_STD, false>(lc, ta, tw, top, tf32m, d, num_sms);
-    case EPI_TAIL: return tf32 ? launch_cfg<EPI_TAIL, true>(lc, ta, tw, top, tf32m, d, num_sms) : launch_cfg<EPI_TAIL, false>(lc, ta, tw, top, tf32m, d, num_sms);
+    case EPI_TAIL:
+      if (e.separated == nullptr)
+        return tf32 ? launch_cfg<EPI_TAIL_MASKS, true>(lc, ta, tw, top, tf32m, d, num_sms) : launch_cfg<EPI_TAIL_MASKS, false>(lc, ta, tw, top, tf32m, d, num_sms);
+      return tf32 ? launch_cfg<EPI_TAIL, true>(lc, ta, tw, top, tf32m, d, num_sms) : launch_cfg<EPI_TAIL, false>(lc, ta, tw, top, tf32m, d, num_sms);
     case EPI_LN:
       if (use_tma) return tf32 ? launch_cfg<EPI_LN_TMA, true>(lc, ta, tw, top, tf32m, d, num_sms) : launch_cfg<EPI_LN_TMA, false>(lc, ta, tw, top, tf32m, d, num_sms);
       return tf32 ? launch_cfg<EPI_LN, true>(lc, ta, tw, top, tf32m, d, num_sms) : launch_cfg<EPI_LN, false>(lc, ta, tw, top, tf32m, d, num_sms);

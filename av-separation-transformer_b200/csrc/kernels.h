@@ -69,7 +69,8 @@ enum Act { ACT_NONE = 0, ACT_RELU = 1, ACT_GELU = 2, ACT_GELU_BF16 = 3 };   // 3
 //                   the Conv1d zero padding); out row = m, halo rows are written as zeros
 //   ROW_PAD2COMPACT padded space in, compact (B*L) rows out; halo rows are dropped
 enum RowMap { ROW_IDENT = 0, ROW_PAD2PAD = 1, ROW_PAD2COMPACT = 2 };
-enum EpiKind { EPI_STD = 0, EPI_TAIL = 1, EPI_LN = 2, EPI_LN_TMA = 3 };   // EPI_LN_TMA is selected internally by launch_gemm
+// EPI_LN_TMA and EPI_TAIL_MASKS (EPI_TAIL with separated == null) are selected internally by launch_gemm
+enum EpiKind { EPI_STD = 0, EPI_TAIL = 1, EPI_LN = 2, EPI_LN_TMA = 3, EPI_TAIL_MASKS = 4 };
 
 struct GemmProblem {
   const void* A;   // [rowsA, K] K-major activations (bf16 or fp32/tf32), leading dimension lda (elements)
@@ -102,7 +103,8 @@ struct GemmEpilogue {
   const float* resid = nullptr;  // [rows, N] fp32, indexed by the OUTPUT row
   const float* ln_gamma = nullptr;
   const float* ln_beta = nullptr;
-  // EPI_TAIL (SeparationDecoder head): masks = sigmoid(acc + bias) -> masks[b,s,f,t]; separated = masks * mixed[b,f,t]
+  // EPI_TAIL (SeparationDecoder head): masks = sigmoid(acc + bias) -> masks[b,s,f,t]; separated = masks * mixed[b,f,t].
+  // separated == null: masks only, and mixed is never read (may be null).
   const float* mixed = nullptr;
   float* masks = nullptr;
   float* separated = nullptr;
@@ -317,9 +319,12 @@ const char* fft512_init_tables();   // window + twiddle tables of the n_fft = 51
 //           frame_lengths (device int32 [B], receives 1 + length / hop) is given.
 //   S1 > 0: the synthesis layout, waves (B, S1, L) with the mixture as signal 0 -> magnitudes only: mag (B, F, T) of
 //           the mixture, mag2 (B, S1 - 1, F, T) of the other signals or null.  spec, lengths, frame_lengths null.
+//   xp (S1 = 0 only, or null): also the forward's Conv1d operand, launch_prep_audio's xp [B * (T + 2), Fp] in operand
+//           precision xp_prec, bit-identical to launch_prep_audio of mag with the frame_lengths as its lens.
 // B * max(S1, 1) above 65535 is "stft: launch failed".
 const char* launch_stft(cudaStream_t s, const float* waves, const int* lengths, int B, int S1, int L, int nfft, int hop,
-                        float* spec, float* mag, float* mag2, int* frame_lengths);
+                        float* spec, float* mag, float* mag2, int* frame_lengths, void* xp = nullptr, int Fp = 0,
+                        int xp_prec = PREC_BF16);
 // lengths as for launch_stft: the istft runs its variable-length kernel when it is given.
 const char* launch_istft_masked(cudaStream_t s, const float* spec, const float* masks, const int* lengths, int B, int S,
                                 int T, int nfft, int hop, int L, float* waves);

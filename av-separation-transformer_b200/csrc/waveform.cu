@@ -68,6 +68,26 @@ __device__ __forceinline__ size_t stft_out_plane(int sig, int S1, int F, int T, 
 // the unscaled sums, the one magnitude expression of every analysis kernel and every layout.
 __device__ __forceinline__ float stft_mag(float2 z) { return 0.5f * hypotf(2.0f * z.x, 2.0f * z.y); }
 
+// The forward's Conv1d operand straight from the analysis (launch_prep_audio's layout): xp [B * (T + 2), Fp], bf16, or
+// tf32-rounded fp32 when tf32 != 0.  Of the CTA's nt frames t0 .. t0 + nt - 1 of signal sig, staged at stage[f * pitch
+// + g], the first nv are real: row sig * (T + 2) + t + 1 holds stft_mag of frame t converted exactly as prep_audio
+// converts the fp32 magnitude, so xp is bit-identical to prep_audio of this kernel's mag.  Frames at or past nv and the
+// columns [F, Fp) are 0; the CTA of frame 0 also zeroes the halo rows 0 and T + 1.  A frame's bins are one contiguous row.
+__device__ __forceinline__ void stft_store_xp(void* xp, int tf32, const float2* stage, int pitch, int sig, int t0,
+                                              int nt, int nv, int T, int F, int Fp, int tid, int nthr) {
+  const size_t row0 = static_cast<size_t>(sig) * (T + 2);
+  auto put = [&](size_t o, float v) {
+    if (tf32) static_cast<float*>(xp)[o] = round_tf32(v);
+    else static_cast<__nv_bfloat16*>(xp)[o] = __float2bfloat16_rn(v);
+  };
+  for (int e = tid; e < nt * Fp; e += nthr) {
+    const int g = e / Fp, f = e - g * Fp;
+    put((row0 + t0 + g + 1) * Fp + f, (g < nv && f < F) ? stft_mag(stage[f * pitch + g]) : 0.f);
+  }
+  if (t0 == 0)
+    for (int e = tid; e < 2 * Fp; e += nthr) put((row0 + (e < Fp ? 0 : T + 1)) * Fp + e % Fp, 0.f);
+}
+
 // Variable-length batch (VARLEN): utterance b owns the first nb = clamp(lengths[b], 1, n) samples of its row (all n
 // when lengths is null) and the first Tb = 1 + nb / hop frames.  Samples at or past nb are never read, frames at or
 // past Tb are neither staged nor transformed, and their outputs are stored as 0.  Frames are paired by absolute index
@@ -76,11 +96,12 @@ __device__ __forceinline__ float stft_mag(float2 z) { return 0.5f * hypotf(2.0f 
 // The uniform instantiation ignores the two trailing parameters.
 //
 // grid (ceil(T/TGA), number of signals), nfft/2 threads.  Outputs as stft_out_plane: spec (float2) and mag (float)
-// may each be null.  VARLEN is for the plain layout (S1 == 0) only.
+// may each be null; xp (plain layout only) as stft_store_xp, or null.  VARLEN is for the plain layout (S1 == 0) only.
 template <bool VARLEN>
 __global__ void stft_complex_kernel(const float* __restrict__ waves, int n, int nfft, int log2n, int hop, int T, int F,
                                     float2* __restrict__ spec, float* __restrict__ mag, float* __restrict__ mag2,
-                                    int S1, const int* __restrict__ lengths, int* __restrict__ frame_lengths) {
+                                    int S1, const int* __restrict__ lengths, int* __restrict__ frame_lengths,
+                                    void* __restrict__ xp, int Fp, int xp_tf32) {
   extern __shared__ __align__(16) uint8_t sm_raw[];
   double* win = reinterpret_cast<double*>(sm_raw);          // [nfft]
   float* re = reinterpret_cast<float*>(win + nfft);         // [nfft]
@@ -137,6 +158,7 @@ __global__ void stft_complex_kernel(const float* __restrict__ waves, int n, int 
     if (spec) spec[o] = v;
     if (m_out) m_out[o] = stft_mag(v);
   }
+  if (xp) stft_store_xp(xp, xp_tf32, stage, TGA + 1, sig, t0, min(TGA, T - t0), ng, T, F, Fp, tid, blockDim.x);
 }
 
 // grid (ceil(L/CH), S, B), nfft/2 threads.  spec (B, F, T) float2, masks (B, S, F, T) float or null (S = 1),
@@ -273,13 +295,14 @@ __device__ __forceinline__ void fft512_load_twiddles(float2* tw, int tid) {
   for (int m = tid; m < FFT512_TW; m += 256) tw[m] = g_tw512[m];
 }
 
-// grid (ceil(T/8), number of signals).  Outputs as stft_out_plane.  VARLEN (S1 == 0 only): the variable-length rule
+// grid (ceil(T/8), number of signals).  Outputs as stft_out_plane, xp as stft_store_xp.  VARLEN (S1 == 0 only): the variable-length rule
 // of stft_complex_kernel; pairs are (t0 + 2g, t0 + 2g + 1), again fixed by absolute frame index.
 template <bool VARLEN>
 __global__ void __launch_bounds__(256) stft512_kernel(const float* __restrict__ waves, int n, int hop, int T,
                                                       float2* __restrict__ spec, float* __restrict__ mag,
                                                       float* __restrict__ mag2, int S1,
-                                                      const int* __restrict__ lengths, int* __restrict__ frame_lengths) {
+                                                      const int* __restrict__ lengths, int* __restrict__ frame_lengths,
+                                                      void* __restrict__ xp, int Fp, int xp_tf32) {
   constexpr int NF = 512, F = 257;
   extern __shared__ __align__(16) uint8_t sm_raw[];
   float2* tw = reinterpret_cast<float2*>(sm_raw);                  // [FFT512_TW]
@@ -338,6 +361,7 @@ __global__ void __launch_bounds__(256) stft512_kernel(const float* __restrict__ 
     if (spec) spec[o] = z;
     if (m_out) m_out[o] = stft_mag(z);
   }
+  if (xp) stft_store_xp(xp, xp_tf32, stage, 9, sig, t0, min(8, T - t0), ng, T, F, Fp, tid, 256);
 }
 
 // grid (ceil(L/CH), S, B), CH = (9 - R) * hop with R = ceil(512 / hop) <= 8: exactly the (at most) 8 frames
@@ -456,21 +480,23 @@ const char* fft512_init_tables() {
 }
 
 const char* launch_stft(cudaStream_t s, const float* waves, const int* lengths, int B, int S1, int L, int nfft, int hop,
-                        float* spec, float* mag, float* mag2, int* frame_lengths) {
+                        float* spec, float* mag, float* mag2, int* frame_lengths, void* xp, int Fp, int xp_prec) {
   const int T = 1 + L / hop, F = nfft / 2 + 1;
   const dim3 grid((T + TGA - 1) / TGA, B * (S1 > 0 ? S1 : 1));
   const bool varlen = lengths || frame_lengths;
+  const int tf32 = xp_prec == PREC_TF32 ? 1 : 0;
+  if (xp && (S1 > 0 || Fp < F)) return "stft: the Conv1d operand needs the plain layout and Fp >= F";
   float2* spec2 = reinterpret_cast<float2*>(spec);
   if (nfft == 512) {
     auto kern = varlen ? stft512_kernel<true> : stft512_kernel<false>;
-    kern<<<grid, 256, kStft512Smem, s>>>(waves, L, hop, T, spec2, mag, mag2, S1, lengths, frame_lengths);
+    kern<<<grid, 256, kStft512Smem, s>>>(waves, L, hop, T, spec2, mag, mag2, S1, lengths, frame_lengths, xp, Fp, tf32);
   } else {
     const size_t smem = static_cast<size_t>(nfft) * sizeof(double) + 3 * static_cast<size_t>(nfft) * sizeof(float) +
                         static_cast<size_t>(F) * (TGA + 1) * sizeof(float2);
     auto kern = varlen ? stft_complex_kernel<true> : stft_complex_kernel<false>;
     if (!smem_opt_in(kern, static_cast<int>(smem))) return "stft: cannot raise the shared-memory limit";
     kern<<<grid, nfft / 2, smem, s>>>(waves, L, nfft, __builtin_ctz(nfft), hop, T, F, spec2, mag, mag2, S1, lengths,
-                                      frame_lengths);
+                                      frame_lengths, xp, Fp, tf32);
   }
   return cudaGetLastError() == cudaSuccess ? nullptr : "stft: launch failed";
 }

@@ -14,7 +14,8 @@
  *   - every function returns 0 on success, non-zero on error; avsep_last_error(h) gives the message.
  *     No C++ exception crosses this boundary.
  *   - a handle is bound to one CUDA device; calls are stream-ordered on the caller's stream and never
- *     synchronise internally (except avsep_forward_host and the *_debug / *_test helpers).
+ *     synchronise internally (except avsep_forward_host, avsep_forward_host_packed, avsep_separate_waveforms_host
+ *     and the *_debug / *_test helpers).
  *   - every call runs on its handle's device, whichever device the calling thread has current, and selects the
  *     caller's current device again before it returns.
  *   - device buffers are owned by the caller; the library owns only the prepacked weights and, when the
@@ -301,6 +302,50 @@ AVSEP_API int avsep_stft_varlen(avsep_handle* h, const float* waves, const int32
 AVSEP_API int avsep_istft_varlen(avsep_handle* h, const float* spec, const float* masks, const int32_t* lengths,
                                  int32_t B, int32_t S, int32_t T, int32_t n_fft, int32_t hop_length, int32_t L,
                                  float* waves, void* cuda_stream);
+
+/* Waveforms in, waveforms out in one call: the analysis above, AVSeparationTransformer.forward on its magnitude and the
+ * masked inverse, with n_fft = 2 * (freq_bins - 1), T = 1 + L / hop_length <= 5000 and F = freq_bins.
+ *   waves (B, L) float32, lip_frames (B, N, Hh, Ww) float32 -> waves_out (B, S, L) float32 and masks (B, S, F, T) float32,
+ *   or masks == NULL when only the waveforms are wanted.
+ * The results are bit-identical to avsep_stft_varlen -> avsep_forward_varlen (on the magnitude, with the frame_lengths
+ * the analysis returns) -> avsep_istft_varlen (on the spectrum and the masks, with the same sample lengths), with one
+ * launch fewer: the analysis writes the forward's Conv1d operand itself, so prep_audio does not run.  Where the forward
+ * runs its decoder as a separate GEMM (d_model != 256, TF32, T > 128, debug mode) that decoder writes the masks only:
+ * it neither reads the magnitude nor writes `separated`, which the inverse does not need.  Errors: a
+ * NULL input or waves_out, n_fft != 2 * (freq_bins - 1), an FFT geometry avsep_stft refuses, T > 5000 and the shape
+ * errors of avsep_forward; nothing is enqueued then. */
+
+/* Workspace of avsep_separate_waveforms: the forward's (avsep_workspace_bytes at T = 1 + L / hop_length) plus the
+ * complex spectrum, the masks and the per-utterance frame counts (0 on error). */
+AVSEP_API size_t avsep_waveform_workspace_bytes(avsep_handle* h, int32_t B, int32_t L, int32_t N, int32_t Hh, int32_t Ww,
+                                                int32_t n_fft, int32_t hop_length);
+
+/* DEVICE buffers.  lengths: DEVICE int32 [B] samples per utterance, frame_lengths: DEVICE int32 [B] lip frames per
+ * utterance, each left-aligned in its padded row; NULL = all L / all N, and values outside [1, L] / [1, N] behave as
+ * the nearest bound, as in avsep_stft_varlen / avsep_forward_varlen.  Utterance b's T_b = 1 + L_b / hop_length go from
+ * the analysis to the forward on the device.  Enqueues the analysis (spectrum into the workspace, Conv1d operand), the
+ * forward (a cached CUDA graph from the second call on the same buffers) and the masked inverse into waves_out.
+ * masks == NULL: the masks stay in the workspace.  workspace may be NULL (library-owned, cached per shape), else
+ * avsep_waveform_workspace_bytes(B, L, N, Hh, Ww, n_fft, hop_length) bytes, 1024-byte aligned. */
+AVSEP_API int avsep_separate_waveforms(avsep_handle* h, const float* waves, const float* lip_frames,
+                                       const int32_t* lengths, const int32_t* frame_lengths, int32_t B, int32_t L,
+                                       int32_t N, int32_t Hh, int32_t Ww, int32_t n_fft, int32_t hop_length,
+                                       float* waves_out, float* masks, void* workspace, size_t workspace_bytes,
+                                       void* cuda_stream);
+
+/* avsep_separate_waveforms with HOST buffers and full batches (pinned memory for overlap; pageable ones give the same
+ * results): the pipeline of avsep_forward_host ("host_chunk" utterances per chunk on "host_lanes" compute lanes), where
+ * a chunk copies in its samples and lip frames and copies out its waveforms, and its masks only when masks != NULL.
+ * Each chunk's kernels write straight into the slot's device buffers at the chunk's offset.  The results equal
+ * avsep_separate_waveforms bit for bit.  The async form uses the I/O slots and avsep_host_wait of
+ * avsep_forward_host_async, with the same rules; slots are shared with the spectrogram forms. */
+AVSEP_API int avsep_separate_waveforms_host(avsep_handle* h, const float* waves, const float* lip_frames, int32_t B,
+                                            int32_t L, int32_t N, int32_t Hh, int32_t Ww, int32_t n_fft,
+                                            int32_t hop_length, float* waves_out, float* masks, void* cuda_stream);
+AVSEP_API int avsep_separate_waveforms_host_async(avsep_handle* h, const float* waves, const float* lip_frames,
+                                                  int32_t B, int32_t L, int32_t N, int32_t Hh, int32_t Ww,
+                                                  int32_t n_fft, int32_t hop_length, float* waves_out, float* masks,
+                                                  int32_t slot, void* cuda_stream);
 
 /* Test hook: one whole transformer stack through the fused kernel (csrc/xformer_stack_sm100.cu) on the handle's
  * weights.  which: 0 = AudioEncoder.transformer (model.py:48-52,59), 1 = VisualEncoder.transformer (model.py:97-101,111),
